@@ -42,6 +42,7 @@ REFINE_MARGIN = float(os.environ.get("PKB_BENCH_REFINE_MARGIN", "0.02"))  # log-
 LL_TOL, ARGMAX_MIN, FEAT_TOL = 2e-2, 0.999, 1e-4
 SAMPLES_10S = 160000
 FRAMES_10S = 998
+DUMP_LIMIT = 64 << 20  # bytes of all the files --dump-outputs writes
 
 CONFIGS = {
     # name: (utts per GPU, hidden layers, width, pdfs, nnet?)
@@ -275,10 +276,31 @@ class Env:
             self.dist.destroy_process_group()
 
 
-def measure_batch(env, cfg, precision, n_utts, steps, warmup, sample_clocks):
+def dump_batch_outputs(batch, cfg, out_dir):
+    """Writes what one pass hands its caller: the log-likelihoods (the CMVN features for a config
+    without a net), every row when they fit in DUMP_LIMIT, otherwise a fixed seeded sample of
+    rows, in ascending row order, next to the row indices."""
+    import pocketkaldi_b200 as pk
+    which, name, cols = (pk.BUF_LOGLIK, "loglik", cfg["pdfs"]) if cfg["nnet"] else (pk.BUF_FEATS, "feats", 40)
+    n = batch.total_frames
+    k = min(n, (DUMP_LIMIT - 4096) // (4 * cols + 8))  # 4096: room for the two .npy headers
+    rows = np.sort(np.random.default_rng(0).choice(n, k, replace=False)) if k < n else np.arange(n)
+    out = np.empty((k, cols), np.float32)
+    # one copy per run of consecutive rows
+    for run in np.split(np.arange(k), np.flatnonzero(np.diff(rows) != 1) + 1):
+        if run.size:
+            batch.get_rows_async(which, int(rows[run[0]]), run.size, out[run[0]:])
+    batch.ctx.sync()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), out)
+    np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+
+
+def measure_batch(env, cfg, precision, n_utts, steps, warmup, sample_clocks, dump_dir=None):
     """Device-resident throughput of one config: W warm-up passes, K timed passes bracketed by a
     barrier + synchronize, CUDA events on the library's stream, max over ranks. Returns the
-    result dict plus the live (am, batch) for the legs that follow (parity, e2e)."""
+    result dict plus the live (am, batch) for the legs that follow (parity, e2e). With dump_dir,
+    rank 0 writes the output of the last timed pass there (dump_batch_outputs)."""
     import pocketkaldi_b200 as pk
     from pocketkaldi_b200 import sharding
     args, ctx, rank, local, dist, peaks = env.args, env.ctx, env.rank, env.local, env.dist, env.peaks
@@ -311,6 +333,8 @@ def measure_batch(env, cfg, precision, n_utts, steps, warmup, sample_clocks):
     ctx.profile_enable(False)
     ms_max, total_frames = reduce_timing(dist, local, ms, frames)
     value = total_frames * steps / (ms_max * 1e-3)
+    if dump_dir is not None and rank == 0:
+        dump_batch_outputs(batch, cfg, dump_dir)
     checksum = batch.checksum(pk.BUF_LOGLIK if cfg["nnet"] else pk.BUF_FEATS)
 
     gemm_launches = prof["gemm"][0] + prof["gemm_final"][0]
@@ -406,7 +430,8 @@ def run_gpu_arm(args, cfg):
     env = Env(args)
     rank, world = env.rank, env.world
     n_utts = args.utts or cfg["utts"]
-    main, am, batch = measure_batch(env, cfg, args.precision, n_utts, args.steps, args.warmup, True)
+    main, am, batch = measure_batch(env, cfg, args.precision, n_utts, args.steps, args.warmup, True,
+                                    dump_dir=args.dump_outputs)
 
     # ---- end to end through the host-buffer API: pinned PCM in, log-likelihoods out, per chunk
     e2e = None if args.no_e2e else run_e2e(env, cfg, am, n_utts, batch)
@@ -774,9 +799,10 @@ def measure_other_modes(env, cfg, ref_pack, skip):
     return out
 
 
-def measure_stream(env, cfg, precision, steps, warmup):
+def measure_stream(env, cfg, precision, steps, warmup, dump_dir=None):
     """BASELINE config 5: chunk latency from "chunk in pinned host memory" to "log-likelihoods in
-    pinned host memory" (host wall clock around the synchronous pkb_stream_push_i16)."""
+    pinned host memory" (host wall clock around the synchronous pkb_stream_push_i16). With
+    dump_dir, rank 0 writes the log-likelihoods of the last timed push there."""
     import pocketkaldi_b200 as pk
     from pocketkaldi_b200.binding import PinnedArray
     from pocketkaldi_b200.synth import synth_pcm
@@ -807,6 +833,9 @@ def measure_stream(env, cfg, precision, steps, warmup):
     barrier(dist, local)
     prof = ctx.profile_get()
     ms_max, frames_all = reduce_timing(dist, local, total_ms, frames)
+    if dump_dir is not None and rank == 0:
+        os.makedirs(dump_dir, exist_ok=True)
+        np.save(os.path.join(dump_dir, "loglik.npy"), np.ascontiguousarray(o))
     lat = np.array(lat)
     # the same with the compact output form (half the D2H bytes, finished per look-up by the consumer)
     st.flush(out=pin_out.array)
@@ -851,7 +880,7 @@ def measure_stream(env, cfg, precision, steps, warmup):
 def run_stream_arm(args, cfg):
     env = Env(args)
     sampler = ClockSampler(env.local) if env.rank == 0 else None
-    res = measure_stream(env, cfg, args.precision, args.steps, args.warmup)
+    res = measure_stream(env, cfg, args.precision, args.steps, args.warmup, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if sampler else None
     if env.rank == 0:
         line = {"metric": METRIC, "n_gpus": env.world, "higher_is_better": True, "scaling": "weak",
@@ -879,7 +908,15 @@ def main():
     ap.add_argument("--no-sub", action="store_true", help="skip the config 2/4/5 sub-objects")
     ap.add_argument("--no-modes", action="store_true", help="skip the other precision modes")
     ap.add_argument("--sub-utts4", type=int, default=512, help="utterances per GPU of the config-4 sub-run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step as DIR/<name>.npy (float32, row "
+                         "indices in float64; at most 64 MB in all, a fixed seeded row sample of "
+                         "larger outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference_arm(args, cfg)

@@ -1,11 +1,14 @@
-"""Parity gate at BASELINE.json's net sizes, against the compiled reference run live on the GPU
-box's host cores (oracle/_ref/libpkref.so ships with the snapshot; checker only).
+"""Parity gate at BASELINE.json's net sizes, against the compiled reference run live on the host
+cores where oracle/_ref/libpkref.so is built, otherwise against the C restatement pinned to it
+(oracle/pk_oracle.c); checker only.
 
 The precision under test is the one bench.py reports as `dtype` (bench.DEFAULT_PRECISION), so
 the headline number is always a parity-green number. Bars (BASELINE.json north_star):
 |dLL| <= 2e-2 on the unscaled AcousticModel::Compute output (src/am.cc:90-115), per-frame argmax
 pdf agreement >= 99.9 %, fbank / CMVN features within 1e-4 relative.
 """
+
+from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import pytest
@@ -32,9 +35,17 @@ def ctx():
     c.close()
 
 
-def reference_loglik(reference, cfg, pcms, g, tmp_path):
-    """fbank -> CMVN -> AcousticModel::Compute of the unmodified reference (unscaled)."""
+def reference_loglik(reference, oracle, cfg, pcms, g, tmp_path):
+    """fbank -> CMVN -> AcousticModel::Compute (unscaled) of the unmodified reference where it is
+    built (oracle/_ref), otherwise of the C restatement, which tests/test_oracle.py pins to the
+    reference's stored outputs (every step after the FFT in the reference's rounding order)."""
     conf, layers, prior = bench.write_reference_model(cfg, str(tmp_path))
+    if reference is None:
+        feats = [oracle.cmvn(oracle.fbank(pcm.astype(np.float32)), g) for pcm in pcms]
+        # the library calls release the GIL: one thread per utterance
+        with ThreadPoolExecutor(len(pcms)) as pool:
+            lls = list(pool.map(lambda ft: oracle.am_compute(ft, layers, prior, 5, 5), feats))
+        return layers, prior, feats, lls
     am = reference.am_load(conf)
     feats, lls = [], []
     for pcm in pcms:
@@ -46,13 +57,11 @@ def reference_loglik(reference, cfg, pcms, g, tmp_path):
 
 
 @pytest.mark.parametrize("config,n_utts", [("3", 3), ("4", 3)])
-def test_headline_precision_meets_the_parity_bar(ctx, reference, tmp_path, config, n_utts):
-    if reference is None:
-        pytest.skip("oracle/_ref/libpkref.so not built")
+def test_headline_precision_meets_the_parity_bar(ctx, reference, oracle, tmp_path, config, n_utts):
     cfg = bench.CONFIGS[config]
     g = synth_global_cmvn()
     pcms = [synth_pcm(1234, [u], bench.SAMPLES_10S)[0] for u in range(n_utts)]
-    layers, prior, ref_feats, ref_lls = reference_loglik(reference, cfg, pcms, g, tmp_path)
+    layers, prior, ref_feats, ref_lls = reference_loglik(reference, oracle, cfg, pcms, g, tmp_path)
     am = pk.AcousticModel(ctx, PRECISIONS[bench.DEFAULT_PRECISION]).from_layers(layers, prior, 5, 5)
     lls, feats = am.pcm_to_loglik(pcms, g, 1.0, want_feats=True)
     am.close()
@@ -66,15 +75,13 @@ def test_headline_precision_meets_the_parity_bar(ctx, reference, tmp_path, confi
     assert 1.0 - flips / frames >= ARGMAX_MIN, "%d of %d frames flipped" % (flips, frames)
 
 
-def test_single_pass_modes_are_reported_not_gated(ctx, reference, tmp_path):
+def test_single_pass_modes_are_reported_not_gated(ctx, reference, oracle, tmp_path):
     """The one-MMA modes on the config-3 net: measured error recorded next to the bar they miss
     (random-init nets have 1 % of frames with a top-2 margin below 3e-3, tools/precision_sim.py)."""
-    if reference is None:
-        pytest.skip("oracle/_ref/libpkref.so not built")
     cfg = bench.CONFIGS["3"]
     g = synth_global_cmvn()
     pcms = [synth_pcm(1234, [0], bench.SAMPLES_10S)[0]]
-    layers, prior, _, ref_lls = reference_loglik(reference, cfg, pcms, g, tmp_path)
+    layers, prior, _, ref_lls = reference_loglik(reference, oracle, cfg, pcms, g, tmp_path)
     for name, loose_ll, loose_arg in (("fp16", 2e-2, 0.99), ("bf16", 0.2, 0.95)):
         am = pk.AcousticModel(ctx, PRECISIONS[name]).from_layers(layers, prior, 5, 5)
         ll = am.pcm_to_loglik(pcms, g, 1.0)[0]

@@ -1,6 +1,7 @@
 """GPU Viterbi (SURVEY 8(f)-4, pkb_batch_decode) against the reference's own decoder: the
-unmodified reference CLI (oracle/_ref/pocketkaldi_ref: CPU nnet + src/decoder.cc) must print the
-same words, and the same per-frame weight, for every utterance."""
+unmodified reference CLI (oracle/_ref/pocketkaldi_ref: CPU nnet + src/decoder.cc), or where it is
+not built the host restatement of that path (oracle/decoder.py), must print the same words, and
+the same per-frame weight, for every utterance."""
 
 import os
 import subprocess
@@ -9,6 +10,7 @@ import numpy as np
 import pytest
 
 import pocketkaldi_b200 as pk
+from oracle.decoder import host_decode
 from pocketkaldi_b200 import formats
 from pocketkaldi_b200.synth import synth_global_cmvn, synth_pcm
 
@@ -120,11 +122,10 @@ def eps_graph(n_words, n_hmm, num_pdfs):
 
 
 @pytest.mark.parametrize("kind", ["loop", "eps", "loop_big"])
-def test_random_graphs_against_the_reference_cli(ctx, tmp_path, kind):
+def test_random_graphs_against_the_reference_cli(ctx, oracle, tmp_path, kind):
     # "loop" / "eps": small graphs, token tables in shared memory; "loop_big": 541 states, the
-    # tables live in the global workspace
-    if not os.path.exists(REF_CLI):
-        pytest.skip("oracle/_ref/pocketkaldi_ref not built")
+    # tables live in the global workspace. The reference CLI where oracle/_ref is built, otherwise
+    # the host restatement of its path (oracle/decoder.py, pinned by tests/test_oracle.py)
     rng = np.random.default_rng({"loop": 1, "eps": 2, "loop_big": 3}[kind])
     P = 600 if kind == "loop_big" else 96
     layers = formats.make_dnn(rng, 440, 96, 2, P)
@@ -153,7 +154,11 @@ def test_random_graphs_against_the_reference_cli(ctx, tmp_path, kind):
         formats.write_wav16(paths[-1], p)
     scp = str(tmp_path / "all.scp")
     open(scp, "w").write("\n".join(paths) + "\n")
-    ref = ref_cli(conf, scp)
+    if os.path.exists(REF_CLI):
+        ref = ref_cli(conf, scp)
+    else:
+        ref = [(words_of(ids, words), llpf)
+               for ids, llpf in host_decode(oracle, fst, tid2pdf, layers, prior, g, pcms)]
     hyps, wts, frames = gpu_decode(ctx, conf, pcms, g)
     assert len(ref) == len(hyps)
     for u, ((rh, rl), h, w, T) in enumerate(zip(ref, hyps, wts, frames)):

@@ -127,6 +127,28 @@ def test_decodable_vs_compiled_reference(oracle, golden, toy_conf):
     assert last.sum() == 1 and last[-1] == 1
 
 
+def test_host_decoder_reproduces_the_reference_toy_decodes(oracle, golden, toy_conf):
+    # the reference CLI's words and per-frame weight on its two test wavs (tests/golden/make_golden.py)
+    import importlib.util
+    import os
+    from oracle.decoder import host_decode
+    here = os.path.dirname(toy_conf)
+    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(here, "..", "make_golden.py"))
+    mg = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mg)
+    graph, _, _ = mg.toy_graph()
+    conf = formats.read_conf(toy_conf)
+    layers = formats.read_nnet(formats.conf_path(toy_conf, conf["nnet"]))
+    prior = formats.read_vector(formats.conf_path(toy_conf, conf["prior"]))
+    tid2pdf = formats.read_vector(formats.conf_path(toy_conf, conf["tid2pdf"]), dtype="<i4")
+    gold = [l.rstrip("\n").split("\t") for l in open(os.path.join(here, "..", "toy_decode_ref.txt"))]
+    got = host_decode(oracle, graph, tid2pdf, layers, prior, golden["cmvn_stats"],
+                      [golden[name + "_pcm"] for name, _, _ in gold])
+    for (name, hyp, llpf), (ids, w) in zip(gold, got):
+        assert " ".join(mg.TOY_WORDS[i] for i in ids) == hyp.strip(), name
+        assert abs(w - float(llpf)) < 1e-5, name
+
+
 # ---------------------------------------------------------------- live compiled reference
 def test_live_reference_random(oracle, reference, golden, tmp_path):
     if reference is None:
