@@ -345,22 +345,6 @@ int pkb_am_load(pkb_ctx_t *c, const char *conf_file, int precision, pkb_am_t **a
 void pkb_am_destroy(pkb_am_t *am) {
   if (!am) return;
   if (am->c) cudaSetDevice(am->c->device);
-  for (auto &st : am->stages) {
-    st.w_hi.release();
-    st.w_lo.release();
-    st.w8_hi.release();
-    st.w8_lo.release();
-    st.bias.release();
-  }
-  am->splice_stage.w_hi.release();
-  am->splice_stage.w_lo.release();
-  am->splice_stage.bias.release();
-  am->log_prior.release();
-  am->ws.release();
-  am->rf.release();
-  am->meta.dev.release();
-  am->in_f32.release();
-  am->out_f32.release();
   delete am;
 }
 
@@ -563,64 +547,51 @@ int pkb_batch_create(pkb_ctx_t *c, pkb_am_t *am, int n_utts, const int32_t *num_
   PKB_REQUIRE(!am || (am->has_splice_stage && am->feat_dim == pkb::kMel),
               "pkb_batch_create: the model's feature dim must be %d", pkb::kMel);
   PKB_CUDA(cudaSetDevice(c->device));
-  std::unique_ptr<pkb_batch> b(new pkb_batch());
+  std::unique_ptr<pkb_batch, decltype(&pkb_batch_destroy)> b(new pkb_batch(), pkb_batch_destroy);
   b->c = c;
   b->am = am;
   b->prob_scale = prob_scale;
   memcpy(b->global_stats, global_stats, sizeof(b->global_stats));
-  int rc = PKB_OK;
-  do {
-    if ((rc = b->meta.build_from_samples(num_samples, n_utts)) != PKB_OK) break;
-    if ((rc = b->meta.upload(c->stream)) != PKB_OK) break;
-    const BatchMeta &m = b->meta;
-    const size_t feat_bytes = static_cast<size_t>(m.total_frames) * pkb::kMel * sizeof(float);
-    if ((rc = b->pcm.ensure(std::max<size_t>(2, static_cast<size_t>(m.total_samples) * 2))) != PKB_OK) break;
-    if ((rc = b->raw.ensure(std::max<size_t>(4, feat_bytes))) != PKB_OK) break;
-    if ((rc = b->feats.ensure(std::max<size_t>(4, feat_bytes))) != PKB_OK) break;
-    if ((rc = b->sum.ensure(sizeof(double))) != PKB_OK) break;
-    if (am) {
-      std::vector<int64_t> &pad_off = b->pad_off;
-      pkb::padded_rows(m, am->left, am->right, &pad_off, &b->padded, &b->gemm_rows);
-      Workspace &ws = b->ws;
-      ws.fast_only = am->refine != 0;  // the FP8 operand planes only exist for the refined rows
-      if ((rc = pkb::workspace_ensure(am, &ws, b->gemm_rows)) != PKB_OK) break;
-      const int dp = am->feat_dim_pad;
-      const size_t plane_bytes = std::max<size_t>(16, static_cast<size_t>(b->padded) * dp * 2);
-      if ((rc = ws.feat_hi.ensure(plane_bytes)) != PKB_OK) break;
-      if (am->planes == 2 && (rc = ws.feat_lo.ensure(plane_bytes)) != PKB_OK) break;
-      if ((rc = ws.pad_off.ensure(std::max<size_t>(8, pad_off.size() * sizeof(int64_t)))) != PKB_OK) break;
-      if ((rc = ws.row_map.ensure(std::max<size_t>(4, static_cast<size_t>(b->gemm_rows) * 4))) != PKB_OK) break;
-      // padded-row layout: one output row per GEMM row
-      if ((rc = b->loglik.ensure(std::max<size_t>(4, static_cast<size_t>(b->gemm_rows) *
-                                                         am->num_pdfs * sizeof(float)))) != PKB_OK)
-        break;
-      if (!pad_off.empty() &&
-          (rc = pkb::upload(c, ws.pad_off.p, pad_off.data(), pad_off.size() * sizeof(int64_t))) != PKB_OK)
-        break;
-      // zero the planes once: rows of empty utterances are never written
-      cudaMemsetAsync(ws.feat_hi.p, 0, plane_bytes, c->stream);
-      if (am->planes == 2) cudaMemsetAsync(ws.feat_lo.p, 0, plane_bytes, c->stream);
-      if ((rc = pkb::launch_row_map(c, m, am->left, am->right, ws.pad_off.as<int64_t>(),
-                                    ws.row_map.as<int32_t>(), b->gemm_rows)) != PKB_OK)
-        break;
-      b->planes.hi = ws.feat_hi.as<__nv_bfloat16>();
-      b->planes.lo = am->planes == 2 ? ws.feat_lo.as<__nv_bfloat16>() : nullptr;
-      b->planes.d_pad_off = ws.pad_off.as<int64_t>();
-      b->planes.left = am->left;
-      b->planes.right = am->right;
-      b->planes.dim_pad = dp;
-      b->planes.fp16 = am->fp16;
-    }
-    if ((rc = pkb::prepare_cmvn_tables(c, global_stats)) != PKB_OK) break;
-    if (cudaStreamSynchronize(c->stream) != cudaSuccess) {
-      pkb::set_error("pkb_batch_create: %s", cudaGetErrorString(cudaGetLastError()));
-      rc = PKB_ERR_CUDA;
-    }
-  } while (0);
-  if (rc != PKB_OK) {
-    pkb_batch_destroy(b.release());
-    return rc;
+  PKB_TRY(b->meta.build_from_samples(num_samples, n_utts));
+  PKB_TRY(b->meta.upload(c->stream));
+  const BatchMeta &m = b->meta;
+  const size_t feat_bytes = static_cast<size_t>(m.total_frames) * pkb::kMel * sizeof(float);
+  PKB_TRY(b->pcm.ensure(std::max<size_t>(2, static_cast<size_t>(m.total_samples) * 2)));
+  PKB_TRY(b->raw.ensure(std::max<size_t>(4, feat_bytes)));
+  PKB_TRY(b->feats.ensure(std::max<size_t>(4, feat_bytes)));
+  PKB_TRY(b->sum.ensure(sizeof(double)));
+  if (am) {
+    std::vector<int64_t> &pad_off = b->pad_off;
+    pkb::padded_rows(m, am->left, am->right, &pad_off, &b->padded, &b->gemm_rows);
+    Workspace &ws = b->ws;
+    ws.fast_only = am->refine != 0;  // the FP8 operand planes only exist for the refined rows
+    PKB_TRY(pkb::workspace_ensure(am, &ws, b->gemm_rows));
+    const int dp = am->feat_dim_pad;
+    const size_t plane_bytes = std::max<size_t>(16, static_cast<size_t>(b->padded) * dp * 2);
+    PKB_TRY(ws.feat_hi.ensure(plane_bytes));
+    if (am->planes == 2) PKB_TRY(ws.feat_lo.ensure(plane_bytes));
+    PKB_TRY(ws.pad_off.ensure(std::max<size_t>(8, pad_off.size() * sizeof(int64_t))));
+    PKB_TRY(ws.row_map.ensure(std::max<size_t>(4, static_cast<size_t>(b->gemm_rows) * 4)));
+    // padded-row layout: one output row per GEMM row
+    PKB_TRY(b->loglik.ensure(
+        std::max<size_t>(4, static_cast<size_t>(b->gemm_rows) * am->num_pdfs * sizeof(float))));
+    if (!pad_off.empty())
+      PKB_TRY(pkb::upload(c, ws.pad_off.p, pad_off.data(), pad_off.size() * sizeof(int64_t)));
+    // zero the planes once: rows of empty utterances are never written
+    cudaMemsetAsync(ws.feat_hi.p, 0, plane_bytes, c->stream);
+    if (am->planes == 2) cudaMemsetAsync(ws.feat_lo.p, 0, plane_bytes, c->stream);
+    PKB_TRY(pkb::launch_row_map(c, m, am->left, am->right, ws.pad_off.as<int64_t>(),
+                                ws.row_map.as<int32_t>(), b->gemm_rows));
+    b->planes.hi = ws.feat_hi.as<__nv_bfloat16>();
+    b->planes.lo = am->planes == 2 ? ws.feat_lo.as<__nv_bfloat16>() : nullptr;
+    b->planes.d_pad_off = ws.pad_off.as<int64_t>();
+    b->planes.left = am->left;
+    b->planes.right = am->right;
+    b->planes.dim_pad = dp;
+    b->planes.fp16 = am->fp16;
   }
+  PKB_TRY(pkb::prepare_cmvn_tables(c, global_stats));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
   *out = b.release();
   return PKB_OK;
 }
@@ -631,19 +602,6 @@ void pkb_batch_destroy(pkb_batch_t *b) {
     cudaSetDevice(b->c->device);
     cudaStreamSynchronize(b->c->stream);
   }
-  b->pcm.release();
-  b->raw.release();
-  b->feats.release();
-  b->loglik.release();
-  b->loglik16.release();
-  b->loglik_off.release();
-  b->vit_work.release();
-  b->vit_out.release();
-  b->vit_tid2pdf.release();
-  b->sum.release();
-  b->ws.release();
-  b->rf.release();
-  b->meta.dev.release();
   delete b;
 }
 
@@ -887,7 +845,6 @@ int pkb_fst_load(pkb_ctx_t *c, const char *path, pkb_fst_t **fst) {
 void pkb_fst_destroy(pkb_fst_t *fst) {
   if (!fst) return;
   if (fst->c) cudaSetDevice(fst->c->device);
-  fst->buf.release();
   delete fst;
 }
 
@@ -942,26 +899,18 @@ int pkb_pcm_to_loglik_i16(pkb_ctx_t *c, pkb_am_t *am, const int16_t *pcm,
                           float prob_scale, float *loglik_out, float *feats_out,
                           int32_t *num_frames_out) {
   PKB_REQUIRE(c && am, "pkb_pcm_to_loglik_i16: NULL argument");
-  pkb_batch_t *b = nullptr;
-  PKB_TRY(pkb_batch_create(c, am, n_utts, num_samples, global_stats, prob_scale, &b));
-  int rc = PKB_OK;
-  do {
-    if (num_frames_out)
-      for (int u = 0; u < n_utts; ++u) num_frames_out[u] = b->meta.num_frames[u];
-    if (b->meta.total_frames == 0) break;
-    if ((rc = pkb_batch_set_pcm_i16(b, pcm)) != PKB_OK) break;
-    if ((rc = pkb_batch_run(b, PKB_STAGE_ALL)) != PKB_OK) break;
-    if (loglik_out && (rc = pkb_batch_get(b, PKB_BUF_LOGLIK, loglik_out)) != PKB_OK) break;
-    if (feats_out && (rc = pkb_batch_get(b, PKB_BUF_FEATS, feats_out)) != PKB_OK) break;
-    if (cudaStreamSynchronize(c->stream) != cudaSuccess) {
-      pkb::set_error("pkb_pcm_to_loglik_i16: %s", cudaGetErrorString(cudaGetLastError()));
-      rc = PKB_ERR_CUDA;
-    } else {
-      rc = pkb::check_device_error(c, "pkb_pcm_to_loglik_i16");
-    }
-  } while (0);
-  pkb_batch_destroy(b);
-  return rc;
+  pkb_batch_t *created = nullptr;
+  PKB_TRY(pkb_batch_create(c, am, n_utts, num_samples, global_stats, prob_scale, &created));
+  std::unique_ptr<pkb_batch, decltype(&pkb_batch_destroy)> b(created, pkb_batch_destroy);
+  if (num_frames_out)
+    for (int u = 0; u < n_utts; ++u) num_frames_out[u] = b->meta.num_frames[u];
+  if (b->meta.total_frames == 0) return PKB_OK;
+  PKB_TRY(pkb_batch_set_pcm_i16(b.get(), pcm));
+  PKB_TRY(pkb_batch_run(b.get(), PKB_STAGE_ALL));
+  if (loglik_out) PKB_TRY(pkb_batch_get(b.get(), PKB_BUF_LOGLIK, loglik_out));
+  if (feats_out) PKB_TRY(pkb_batch_get(b.get(), PKB_BUF_FEATS, feats_out));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  return pkb::check_device_error(c, "pkb_pcm_to_loglik_i16");
 }
 
 }  // extern "C"

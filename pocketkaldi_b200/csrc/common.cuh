@@ -9,6 +9,7 @@
 #include <string.h>
 
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "pkb200.h"
@@ -49,10 +50,15 @@ void set_error(const char *fmt, ...);
     }                                  \
   } while (0)
 
-// Grow-only device allocation.
+// Grow-only device allocation, freed when the buffer is destroyed.
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  DevBuf(DevBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+  ~DevBuf() { release(); }
   int ensure(size_t bytes);
   void release();
   template <typename T> T *as() const { return static_cast<T *>(p); }
@@ -74,6 +80,25 @@ struct ProfSpan {
   cudaEvent_t e0, e1;
 };
 
+// ---- metadata of a packed utterance batch (host side + device copy) -------
+struct BatchMeta {
+  int n_utts = 0;
+  int64_t total_samples = 0;
+  int64_t total_frames = 0;
+  int n_tiles = 0;                      // fbank tiles of kFramesPerTile frames
+  std::vector<int32_t> num_samples, num_frames, tile_prefix;
+  std::vector<int32_t> tile_utt;        // utterance of every fbank tile
+  std::vector<int64_t> sample_off, frame_off;
+  // device copies (one allocation)
+  DevBuf dev;
+  const int32_t *d_num_samples = nullptr, *d_num_frames = nullptr, *d_tile_prefix = nullptr;
+  const int32_t *d_tile_utt = nullptr;
+  const int64_t *d_sample_off = nullptr, *d_frame_off = nullptr;
+  int build_from_samples(const int32_t *ns, int n);
+  int build_from_frames(const int32_t *nf, int n);
+  int upload(cudaStream_t stream);
+};
+
 struct Ctx {
   int device = 0;
   int sm_count = 0;
@@ -91,7 +116,8 @@ struct Ctx {
   float cmvn_global[PKB_CMVN_STATS_DIM] = {0};
   bool cmvn_valid = false;
   // scratch for the host-buffer entry points
-  DevBuf s_in, s_meta, s_raw, s_out, s_flush;
+  DevBuf s_in, s_raw, s_out, s_flush;
+  BatchMeta meta;
   // device -> host error word (mapped pinned memory): a kernel that gives up on a bounded wait
   // stores a code here instead of trapping, which would poison the whole CUDA context
   int *err_host = nullptr;
@@ -103,6 +129,7 @@ struct Ctx {
   double total_ms[PKB_KERNEL_CLASSES] = {0};
   std::vector<ProfSpan> spans;
   std::vector<cudaEvent_t> free_events;
+  ~Ctx();  // the caller has made the device current and drained the stream
 };
 
 // Host -> device upload ordered on the context stream and complete on return. Plain cudaMemcpy
@@ -122,25 +149,6 @@ struct LaunchScope {
   bool timed;
   LaunchScope(Ctx *ctx, int cls);
   ~LaunchScope();
-};
-
-// ---- metadata of a packed utterance batch (host side + device copy) -------
-struct BatchMeta {
-  int n_utts = 0;
-  int64_t total_samples = 0;
-  int64_t total_frames = 0;
-  int n_tiles = 0;                      // fbank tiles of kFramesPerTile frames
-  std::vector<int32_t> num_samples, num_frames, tile_prefix;
-  std::vector<int32_t> tile_utt;        // utterance of every fbank tile
-  std::vector<int64_t> sample_off, frame_off;
-  // device copies (one allocation)
-  DevBuf dev;
-  const int32_t *d_num_samples = nullptr, *d_num_frames = nullptr, *d_tile_prefix = nullptr;
-  const int32_t *d_tile_utt = nullptr;
-  const int64_t *d_sample_off = nullptr, *d_frame_off = nullptr;
-  int build_from_samples(const int32_t *ns, int n);
-  int build_from_frames(const int32_t *nf, int n);
-  int upload(cudaStream_t stream);
 };
 
 constexpr int kFramesPerTile = 8;

@@ -5,6 +5,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <memory>
 
 #include "common.cuh"
 
@@ -47,6 +48,18 @@ void DevBuf::release() {
   if (p) cudaFree(p);
   p = nullptr;
   cap = 0;
+}
+
+Ctx::~Ctx() {
+  for (auto &s : spans) {
+    cudaEventDestroy(s.e0);
+    cudaEventDestroy(s.e1);
+  }
+  for (auto &e : free_events) cudaEventDestroy(e);
+  if (err_host) cudaFreeHost(err_host);
+  if (t0) cudaEventDestroy(t0);
+  if (t1) cudaEventDestroy(t1);
+  if (stream) cudaStreamDestroy(stream);
 }
 
 int upload(Ctx *c, void *dst, const void *src, size_t bytes) {
@@ -206,33 +219,18 @@ int pkb_create(int device, pkb_ctx_t **out) {
                    prop.major, prop.minor);
     return PKB_ERR_CUDA;
   }
-  pkb_ctx *c = new pkb_ctx();
+  std::unique_ptr<pkb_ctx, decltype(&pkb_destroy)> c(new pkb_ctx(), pkb_destroy);
   c->device = device;
   c->sm_count = prop.multiProcessorCount;
   snprintf(c->name, sizeof(c->name), "%s", prop.name);
-  int rc = PKB_OK;
-  do {
-    if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreate(&c->t0) != cudaSuccess || cudaEventCreate(&c->t1) != cudaSuccess) {
-      pkb::set_error("pkb_create: stream/event creation failed: %s",
-                     cudaGetErrorString(cudaGetLastError()));
-      rc = PKB_ERR_CUDA;
-      break;
-    }
-    if (cudaHostAlloc(reinterpret_cast<void **>(&c->err_host), sizeof(int), cudaHostAllocMapped) != cudaSuccess ||
-        cudaHostGetDevicePointer(reinterpret_cast<void **>(&c->err_dev), c->err_host, 0) != cudaSuccess) {
-      pkb::set_error("pkb_create: mapped error word: %s", cudaGetErrorString(cudaGetLastError()));
-      rc = PKB_ERR_CUDA;
-      break;
-    }
-    *c->err_host = 0;
-    rc = pkb::build_fbank_tables(c);
-  } while (0);
-  if (rc != PKB_OK) {
-    pkb_destroy(c);
-    return rc;
-  }
-  *out = c;
+  PKB_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
+  PKB_CUDA(cudaEventCreate(&c->t0));
+  PKB_CUDA(cudaEventCreate(&c->t1));
+  PKB_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&c->err_host), sizeof(int), cudaHostAllocMapped));
+  PKB_CUDA(cudaHostGetDevicePointer(reinterpret_cast<void **>(&c->err_dev), c->err_host, 0));
+  *c->err_host = 0;
+  PKB_TRY(pkb::build_fbank_tables(c.get()));
+  *out = c.release();
   return PKB_OK;
 }
 
@@ -240,22 +238,6 @@ void pkb_destroy(pkb_ctx_t *c) {
   if (!c) return;
   cudaSetDevice(c->device);
   if (c->stream) cudaStreamSynchronize(c->stream);
-  for (auto &s : c->spans) {
-    cudaEventDestroy(s.e0);
-    cudaEventDestroy(s.e1);
-  }
-  for (auto &e : c->free_events) cudaEventDestroy(e);
-  c->tables.release();
-  c->cmvn_tab.release();
-  c->s_in.release();
-  c->s_meta.release();
-  c->s_raw.release();
-  c->s_out.release();
-  c->s_flush.release();
-  if (c->err_host) cudaFreeHost(c->err_host);
-  if (c->t0) cudaEventDestroy(c->t0);
-  if (c->t1) cudaEventDestroy(c->t1);
-  if (c->stream) cudaStreamDestroy(c->stream);
   delete c;
 }
 

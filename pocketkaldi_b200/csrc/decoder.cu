@@ -23,6 +23,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <memory>
 
 #include "decoder.cuh"
 
@@ -773,7 +774,7 @@ int fst_build(Ctx *c, int num_states, int start, const float *final_w, const int
     has_eps = has_eps || il[a] == 0;
     max_il = std::max(max_il, il[a]);
   }
-  pkb_fst *f = new pkb_fst();
+  std::unique_ptr<pkb_fst, decltype(&pkb_fst_destroy)> f(new pkb_fst(), pkb_fst_destroy);
   f->c = c;
   f->num_states = num_states;
   f->num_arcs = num_arcs;
@@ -795,13 +796,8 @@ int fst_build(Ctx *c, int num_states, int start, const float *final_w, const int
     memcpy(h + o_ol, ol.data(), 4 * static_cast<size_t>(num_arcs));
     memcpy(h + o_w, wt.data(), 4 * static_cast<size_t>(num_arcs));
   }
-  int rc = f->buf.ensure(bytes);
-  if (rc == PKB_OK) rc = upload(c, f->buf.p, h, bytes);
-  if (rc != PKB_OK) {
-    f->buf.release();
-    delete f;
-    return rc;
-  }
+  PKB_TRY(f->buf.ensure(bytes));
+  PKB_TRY(upload(c, f->buf.p, h, bytes));
   const char *d = f->buf.as<char>();
   f->d_final = reinterpret_cast<const float *>(d + o_fin);
   f->d_arc_begin = reinterpret_cast<const int32_t *>(d + o_beg);
@@ -810,7 +806,7 @@ int fst_build(Ctx *c, int num_states, int start, const float *final_w, const int
   f->d_arc_il = reinterpret_cast<const int32_t *>(d + o_il);
   f->d_arc_ol = reinterpret_cast<const int32_t *>(d + o_ol);
   f->d_arc_w = reinterpret_cast<const float *>(d + o_w);
-  *out = f;
+  *out = f.release();
   return PKB_OK;
 }
 

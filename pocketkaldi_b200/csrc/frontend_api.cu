@@ -14,7 +14,7 @@ int fbank_host(pkb_ctx_t *c, const SampleT *wave, const int32_t *num_samples, in
   PKB_REQUIRE(c, "pkb_fbank: ctx is NULL");
   PKB_REQUIRE(n_utts == 0 || num_samples, "pkb_fbank: num_samples is NULL");
   PKB_CUDA(cudaSetDevice(c->device));
-  BatchMeta m;
+  BatchMeta &m = c->meta;
   PKB_TRY(m.build_from_samples(num_samples, n_utts));
   if (num_frames_out)
     for (int u = 0; u < n_utts; ++u) num_frames_out[u] = m.num_frames[u];
@@ -55,7 +55,7 @@ int pkb_cmvn(pkb_ctx_t *c, const float *raw, const int32_t *num_frames, int n_ut
   PKB_REQUIRE(global_stats, "pkb_cmvn: global_stats is NULL");
   PKB_REQUIRE(n_utts == 0 || num_frames, "pkb_cmvn: num_frames is NULL");
   PKB_CUDA(cudaSetDevice(c->device));
-  BatchMeta m;
+  BatchMeta &m = c->meta;
   PKB_TRY(m.build_from_frames(num_frames, n_utts));
   if (m.total_frames == 0) return PKB_OK;
   PKB_REQUIRE(raw && out, "pkb_cmvn: raw / out is NULL");

@@ -53,7 +53,6 @@ struct Workspace {
   bool fast_only = false;         // only single-plane passes run on this workspace (FP16R first pass)
   // padded feature planes of the batch pipeline
   DevBuf feat_hi, feat_lo, pad_off;
-  void release();
 };
 
 // Scratch of the selective second pass of PKB_PREC_FP16R (nnet_forward_refined).
@@ -64,7 +63,9 @@ struct Refine {
   Workspace ws;
   int32_t *h_n_sel = nullptr;     // pinned host copy of n_sel
   int64_t last_rows = 0, last_selected = 0;  // of the latest forward pass (pkb_batch_refine_stats)
-  void release();
+  ~Refine() {
+    if (h_n_sel) cudaFreeHost(h_n_sel);
+  }
 };
 
 }  // namespace pkb

@@ -13,6 +13,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <memory>
 
 #include "nnet.cuh"
 
@@ -134,6 +135,10 @@ struct pkb_stream {
   void *g_out[4] = {nullptr, nullptr, nullptr, nullptr}, *g_out2[4] = {nullptr, nullptr, nullptr, nullptr};
   int64_t g_launches[4][PKB_KERNEL_CLASSES] = {};
   bool graphs_off = false;
+  ~pkb_stream() {
+    for (cudaGraphExec_t g : gexec)
+      if (g) cudaGraphExecDestroy(g);
+  }
 };
 
 namespace {
@@ -191,7 +196,7 @@ int pkb_stream_create(pkb_ctx_t *c, pkb_am_t *am, int n_streams, int chunk_sampl
   PKB_REQUIRE(am->has_splice_stage && am->feat_dim == pkb::kMel,
               "pkb_stream_create: the model's feature dim must be %d", pkb::kMel);
   PKB_CUDA(cudaSetDevice(c->device));
-  pkb_stream *st = new pkb_stream();
+  std::unique_ptr<pkb_stream, decltype(&pkb_stream_destroy)> st(new pkb_stream(), pkb_stream_destroy);
   st->c = c;
   st->am = am;
   st->S = n_streams;
@@ -205,32 +210,24 @@ int pkb_stream_create(pkb_ctx_t *c, pkb_am_t *am, int n_streams, int chunk_sampl
   st->max_new = chunk_samples / pkb::kShift + 1;
   st->max_rows = st->L + st->R + std::max(st->max_new, st->R);  // flush appends R replicated rows
   st->pcm_stride = pkb::kFrame + chunk_samples;
-  int rc = PKB_OK;
-  do {
-    const size_t S = n_streams;
-    for (int i = 0; i < 2 && rc == PKB_OK; ++i) {
-      rc = st->pcm[i].ensure(S * st->pcm_stride * sizeof(int16_t));
-      if (rc == PKB_OK) rc = st->win_hi[i].ensure(S * st->max_rows * st->Dp * 2);
-      if (rc == PKB_OK && am->planes == 2) rc = st->win_lo[i].ensure(S * st->max_rows * st->Dp * 2);
-    }
-    if (rc != PKB_OK) break;
-    if ((rc = st->raw.ensure(S * st->max_new * pkb::kMel * sizeof(float))) != PKB_OK) break;
-    if ((rc = st->stat.ensure(S * pkb::kMel * sizeof(float))) != PKB_OK) break;
-    if ((rc = st->ring.ensure(S * pkb::kCmvnWindow * pkb::kMel * sizeof(float))) != PKB_OK) break;
-    if ((rc = st->tcount.ensure(2 * sizeof(int64_t))) != PKB_OK) break;
-    cudaMemsetAsync(st->tcount.p, 0, 2 * sizeof(int64_t), c->stream);
-    cudaMemsetAsync(st->stat.p, 0, S * pkb::kMel * sizeof(float), c->stream);
-    for (int i = 0; i < 2; ++i) {
-      cudaMemsetAsync(st->win_hi[i].p, 0, S * st->max_rows * st->Dp * 2, c->stream);
-      if (am->planes == 2) cudaMemsetAsync(st->win_lo[i].p, 0, S * st->max_rows * st->Dp * 2, c->stream);
-    }
-    if ((rc = pkb::prepare_cmvn_tables(c, global_stats)) != PKB_OK) break;
-  } while (0);
-  if (rc != PKB_OK) {
-    pkb_stream_destroy(st);
-    return rc;
+  const size_t S = n_streams;
+  for (int i = 0; i < 2; ++i) {
+    PKB_TRY(st->pcm[i].ensure(S * st->pcm_stride * sizeof(int16_t)));
+    PKB_TRY(st->win_hi[i].ensure(S * st->max_rows * st->Dp * 2));
+    if (am->planes == 2) PKB_TRY(st->win_lo[i].ensure(S * st->max_rows * st->Dp * 2));
   }
-  *out = st;
+  PKB_TRY(st->raw.ensure(S * st->max_new * pkb::kMel * sizeof(float)));
+  PKB_TRY(st->stat.ensure(S * pkb::kMel * sizeof(float)));
+  PKB_TRY(st->ring.ensure(S * pkb::kCmvnWindow * pkb::kMel * sizeof(float)));
+  PKB_TRY(st->tcount.ensure(2 * sizeof(int64_t)));
+  cudaMemsetAsync(st->tcount.p, 0, 2 * sizeof(int64_t), c->stream);
+  cudaMemsetAsync(st->stat.p, 0, S * pkb::kMel * sizeof(float), c->stream);
+  for (int i = 0; i < 2; ++i) {
+    cudaMemsetAsync(st->win_hi[i].p, 0, S * st->max_rows * st->Dp * 2, c->stream);
+    if (am->planes == 2) cudaMemsetAsync(st->win_lo[i].p, 0, S * st->max_rows * st->Dp * 2, c->stream);
+  }
+  PKB_TRY(pkb::prepare_cmvn_tables(c, global_stats));
+  *out = st.release();
   return PKB_OK;
 }
 
@@ -240,22 +237,6 @@ void pkb_stream_destroy(pkb_stream_t *st) {
     cudaSetDevice(st->c->device);
     cudaStreamSynchronize(st->c->stream);
   }
-  for (int i = 0; i < 2; ++i) {
-    st->pcm[i].release();
-    st->win_hi[i].release();
-    st->win_lo[i].release();
-  }
-  st->raw.release();
-  st->stat.release();
-  st->ring.release();
-  st->out.release();
-  st->out16.release();
-  st->out_off.release();
-  st->tcount.release();
-  for (int i = 0; i < 4; ++i)
-    if (st->gexec[i]) cudaGraphExecDestroy(st->gexec[i]);
-  st->ws.release();
-  st->meta.dev.release();
   delete st;
 }
 
