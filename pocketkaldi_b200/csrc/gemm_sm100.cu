@@ -770,8 +770,11 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
 #pragma unroll
               for (int i = 0; i < 32; ++i) z[i] = fmaxf(z[i], 0.0f);
             } else if (p.relu == 2) {  // sigmoid (not a reference layer type; parity unpinned)
+              // padding columns (z = 0) would become 0.5 and add 0.25 each to the NormalizeLayer
+              // sum of squares of the row: keep them 0 like ReLU and "no activation" do
 #pragma unroll
-              for (int i = 0; i < 32; ++i) z[i] = 1.0f / (1.0f + expf(-z[i]));
+              for (int i = 0; i < 32; ++i)
+                z[i] = col0 + h * 32 + i < p.N_valid ? 1.0f / (1.0f + expf(-z[i])) : 0.0f;
             }
             if (p.out_sumsq != nullptr) {
 #pragma unroll
