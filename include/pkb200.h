@@ -281,6 +281,36 @@ void pkb_fst_destroy(pkb_fst_t *fst);
 int pkb_batch_decode(pkb_batch_t *batch, const pkb_fst_t *fst, float beam, int max_tokens,
                      int max_words, int32_t *words_out, int32_t *n_words_out, float *weight_out);
 
+/* ---- online decoding: the GPU Viterbi search, chunk by chunk ----------------------------------
+ * n_streams searches whose tokens and word records stay on the device between calls, so that
+ * log-likelihood rows can arrive in any split: decoding a stream's rows 1, 7, 16 or all frames at a
+ * time gives bit-identical words and weight to pkb_batch_decode over the same rows. Streams advance
+ * together and finish together. */
+typedef struct pkb_decoder pkb_decoder_t;
+/* n_streams searches over `fst` with `am`'s tid2pdf map (the checks of pkb_batch_decode apply).
+ * The decoder keeps pointers to both: the model and the FST must outlive it.
+ * beam <= 0: 16; max_tokens <= 0: 4096 tokens per frame (graphs of more than 2048 states or 4096
+ * arcs); max_words: words returned per stream; max_records <= 0: 2^18 word records per stream.
+ * When an advance leaves the record store more than half full it is compacted to the word histories
+ * of the live tokens, so its use grows with the words spoken, not with frames x tokens. A stream
+ * whose live history does not fit, or whose tokens overflow, reports a negative word count. */
+int pkb_decoder_create(pkb_ctx_t *ctx, const pkb_am_t *am, const pkb_fst_t *fst, int n_streams, float beam,
+                       int max_tokens, int max_words, int max_records, pkb_decoder_t **dec);
+/* Detaches the decoder from its stream, if any. */
+void pkb_decoder_destroy(pkb_decoder_t *dec);
+/* Host rows: loglik [n_streams][frame_stride][num_pdfs]; stream s contributes its first n_frames[s]
+ * rows (n_frames[s] <= frame_stride). Synchronous. */
+int pkb_decoder_advance(pkb_decoder_t *dec, const float *loglik, int frame_stride, const int32_t *n_frames);
+/* Best-so-far per stream as of the last advance (or push / flush of the attached stream): the words
+ * ([n_streams][max_words], spoken order) of the lowest-cost token of the last frame, ties to the
+ * lowest state, without final weights; n_words_out < 0 when the search failed; its cost; frames
+ * decoded in this utterance. Any output may be NULL. Reads a host copy: no device work. */
+int pkb_decoder_partial(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words_out, float *cost_out,
+                        int64_t *frames_out);
+/* BestPath of every stream as pkb_batch_decode returns it, then a fresh utterance (InitDecoding).
+ * Synchronous. */
+int pkb_decoder_finish(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words_out, float *weight_out);
+
 /* Sum over all elements of a per-frame float buffer, computed on the device
  * in double (a cheap whole-output fingerprint for full-size runs). */
 int pkb_batch_checksum(pkb_batch_t *batch, int which, double *sum_out);
@@ -308,9 +338,18 @@ int pkb_stream_flush(pkb_stream_t *st, float *loglik_out, int32_t *frames_out);
  * Compact output of a stream (see pkb_batch_set_compact): h16_out [n_streams][max_frames][num_pdfs]
  * half bits and off_out [n_streams][max_frames] offsets instead of the FP32 rows. */
 int pkb_stream_set_compact(pkb_stream_t *st, int on);
+/* Number of pushes so far that replayed a captured CUDA graph (0 with PKB_STREAM_GRAPH=0). */
+int pkb_stream_graph_replays(const pkb_stream_t *st, int64_t *replays);
 int pkb_stream_push_compact_i16(pkb_stream_t *st, const int16_t *pcm, uint16_t *h16_out, float *off_out,
                                 int32_t *frames_out);
 int pkb_stream_flush_compact(pkb_stream_t *st, uint16_t *h16_out, float *off_out, int32_t *frames_out);
+/* Attaches a decoder of the same context, model and n_streams (NULL detaches). Every push and flush
+ * then advances it over the rows it emitted, on the device and inside the captured CUDA graph of
+ * the steady state; loglik_out may then be NULL (decode-only: no row crosses PCIe) and
+ * pkb_decoder_partial reads the result. Decoding reads the FP32 rows: a compact stream cannot have a
+ * decoder. After pkb_stream_flush, pkb_decoder_finish must be called before the next push.
+ * Destroying the stream leaves the decoder usable. */
+int pkb_stream_set_decoder(pkb_stream_t *st, pkb_decoder_t *dec);
 
 /* ---- batched ingestion (SURVEY 8(f)-2) --------------------------------------
  * Host-side readers that feed the batch pipeline without the reference's detour through

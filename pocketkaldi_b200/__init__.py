@@ -20,6 +20,7 @@ from .binding import (  # noqa: F401
     Decodable,
     Event,
     Batch,
+    Decoder,
     Fst,
     Stream,
     WavList,

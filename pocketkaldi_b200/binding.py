@@ -101,6 +101,12 @@ _SIGNATURES = [
     ("pkb_fst_create", C.c_int, [_VP, C.c_int, C.c_int, _VP, _VP, C.c_int, _VP, C.POINTER(_VP)]),
     ("pkb_fst_destroy", None, [_VP]),
     ("pkb_batch_decode", C.c_int, [_VP, _VP, C.c_float, C.c_int, C.c_int, _VP, _VP, _VP]),
+    ("pkb_decoder_create", C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
+                                     C.POINTER(_VP)]),
+    ("pkb_decoder_destroy", None, [_VP]),
+    ("pkb_decoder_advance", C.c_int, [_VP, _VP, C.c_int, _VP]),
+    ("pkb_decoder_partial", C.c_int, [_VP, _VP, _VP, _VP, _VP]),
+    ("pkb_decoder_finish", C.c_int, [_VP, _VP, _VP, _VP]),
     ("pkb_loglik16_expand", C.c_int, [_VP, _VP, C.c_int64, C.c_int, C.c_float, _VP]),
     ("pkb_stream_create", C.c_int, [_VP, _VP, C.c_int, C.c_int, _f32p, C.c_float, C.POINTER(_VP)]),
     ("pkb_stream_destroy", None, [_VP]),
@@ -108,8 +114,10 @@ _SIGNATURES = [
     ("pkb_stream_push_i16", C.c_int, [_VP, _VP, _VP, _VP]),
     ("pkb_stream_flush", C.c_int, [_VP, _VP, _VP]),
     ("pkb_stream_set_compact", C.c_int, [_VP, C.c_int]),
+    ("pkb_stream_graph_replays", C.c_int, [_VP, C.POINTER(C.c_int64)]),
     ("pkb_stream_push_compact_i16", C.c_int, [_VP, _VP, _VP, _VP, _VP]),
     ("pkb_stream_flush_compact", C.c_int, [_VP, _VP, _VP, _VP]),
+    ("pkb_stream_set_decoder", C.c_int, [_VP, _VP]),
     ("pkb_wav_probe", C.c_int, [C.c_char_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     ("pkb_wav_read_i16", C.c_int, [C.c_char_p, _VP, C.c_int32, C.POINTER(C.c_int32)]),
     ("pkb_wav_read_f32", C.c_int, [C.c_char_p, _VP, C.c_int32, C.POINTER(C.c_int32)]),
@@ -738,6 +746,62 @@ class Fst:
             pass
 
 
+def _hyps(words, nw, max_words):
+    return [None if n < 0 else [int(x) for x in words[s, :min(int(n), max_words)]] for s, n in enumerate(nw)]
+
+
+class Decoder:
+    """pkb_decoder_t: n_streams GPU Viterbi searches that advance chunk by chunk. Rows may arrive in
+    any split; the result equals Batch.decode over the same rows, bit for bit."""
+
+    def __init__(self, ctx, am, fst, n_streams, beam=0.0, max_tokens=0, max_words=256, max_records=0):
+        self.ctx, self.n_streams, self.max_words = ctx, n_streams, max_words
+        self.P = am.num_pdfs()
+        self.h = _VP()
+        _check(ctx.lib.pkb_decoder_create(ctx.h, am.h, fst.h, n_streams, beam, max_tokens, max_words,
+                                          max_records, C.byref(self.h)))
+        ctx._adopt(self)
+
+    def close(self):
+        if self.h:
+            self.ctx.lib.pkb_decoder_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def advance(self, loglik, n_frames=None):
+        """loglik: float32 [n_streams][frame_stride][num_pdfs]; stream s decodes its first
+        n_frames[s] rows (all of them when n_frames is None)."""
+        loglik = _f32(loglik)
+        assert loglik.ndim == 3 and loglik.shape[0] == self.n_streams and loglik.shape[2] == self.P
+        nf = _lens(np.full(self.n_streams, loglik.shape[1]) if n_frames is None else n_frames)
+        _check(self.ctx.lib.pkb_decoder_advance(self.h, loglik.ctypes.data if loglik.size else None,
+                                                loglik.shape[1], nf.ctypes.data))
+
+    def partial(self):
+        """Best-so-far per stream: (word lists or None where the search failed, costs, frames)."""
+        words = np.zeros((self.n_streams, self.max_words), np.int32)
+        nw = np.zeros(self.n_streams, np.int32)
+        cost = np.zeros(self.n_streams, np.float32)
+        frames = np.zeros(self.n_streams, np.int64)
+        _check(self.ctx.lib.pkb_decoder_partial(self.h, words.ctypes.data, nw.ctypes.data, cost.ctypes.data,
+                                                frames.ctypes.data))
+        return _hyps(words, nw, self.max_words), cost, frames
+
+    def finish(self):
+        """BestPath per stream (as Batch.decode: word lists, None where the search failed, and
+        weights), then fresh utterances."""
+        words = np.zeros((self.n_streams, self.max_words), np.int32)
+        nw = np.zeros(self.n_streams, np.int32)
+        wt = np.zeros(self.n_streams, np.float32)
+        _check(self.ctx.lib.pkb_decoder_finish(self.h, words.ctypes.data, nw.ctypes.data, wt.ctypes.data))
+        return _hyps(words, nw, self.max_words), wt
+
+
 class Stream:
     """pkb_stream_t: n_streams audio streams advancing in lock step with carried state
     (PCM tail, CMVN running sums + ring, splice context). No reference equivalent exists; the
@@ -765,20 +829,33 @@ class Stream:
         except Exception:
             pass
 
-    def push(self, pcm, out=None):
-        """pcm: int16 [n_streams][chunk]. Returns a view [n_streams][frames][P] (frames may be 0)."""
+    def push(self, pcm, out=None, rows=True):
+        """pcm: int16 [n_streams][chunk]. Returns a view [n_streams][frames][P] (frames may be 0).
+        rows=False (needs an attached decoder): no row is copied back; returns the frame count."""
         pcm = np.ascontiguousarray(pcm, dtype=np.int16)
         assert pcm.shape == (self.n_streams, self.chunk)
         out = self.out if out is None else out
         n = C.c_int32(0)
-        _check(self.ctx.lib.pkb_stream_push_i16(self.h, pcm.ctypes.data, out.ctypes.data, C.byref(n)))
-        return out[:, :n.value]
+        _check(self.ctx.lib.pkb_stream_push_i16(self.h, pcm.ctypes.data, out.ctypes.data if rows else None,
+                                                C.byref(n)))
+        return out[:, :n.value] if rows else n.value
 
-    def flush(self, out=None):
+    def flush(self, out=None, rows=True):
         out = self.out if out is None else out
         n = C.c_int32(0)
-        _check(self.ctx.lib.pkb_stream_flush(self.h, out.ctypes.data, C.byref(n)))
-        return out[:, :n.value]
+        _check(self.ctx.lib.pkb_stream_flush(self.h, out.ctypes.data if rows else None, C.byref(n)))
+        return out[:, :n.value] if rows else n.value
+
+    def graph_replays(self):
+        """Pushes so far that replayed a captured CUDA graph (pkb_stream_graph_replays)."""
+        n = C.c_int64(0)
+        _check(self.ctx.lib.pkb_stream_graph_replays(self.h, C.byref(n)))
+        return n.value
+
+    def set_decoder(self, dec):
+        """Attach a Decoder (None detaches): every push / flush advances it on the device."""
+        _check(self.ctx.lib.pkb_stream_set_decoder(self.h, dec.h if dec is not None else None))
+        self.decoder = dec
 
     def set_compact(self, on=True):
         """Half-size output rows (see pkb_stream_set_compact): push_compact / flush_compact."""

@@ -852,16 +852,9 @@ int pkb_batch_decode(pkb_batch_t *b, const pkb_fst_t *fst, float beam, int max_t
                      int32_t *words_out, int32_t *n_words_out, float *weight_out) {
   PKB_REQUIRE(b && fst, "pkb_batch_decode: NULL argument");
   PKB_REQUIRE(b->am, "pkb_batch_decode: the batch has no model");
-  PKB_REQUIRE(fst->c == b->c, "pkb_batch_decode: the FST belongs to another context");
   PKB_REQUIRE(!b->compact, "pkb_batch_decode: reads the FP32 log-likelihoods (switch the compact output off)");
-  PKB_REQUIRE(!b->am->tid2pdf.empty(), "pkb_batch_decode: the model has no tid2pdf map");
-  PKB_REQUIRE(fst->max_ilabel < static_cast<int>(b->am->tid2pdf.size()),
-              "pkb_batch_decode: the graph uses input label %d but the model's tid2pdf map has %zu entries",
-              fst->max_ilabel, b->am->tid2pdf.size());
-  for (int32_t v : b->am->tid2pdf)
-    PKB_REQUIRE(v >= 0 && v < b->am->num_pdfs, "pkb_batch_decode: tid2pdf entry %d outside [0, %d)", v,
-                b->am->num_pdfs);
-  PKB_REQUIRE(max_words > 0 && words_out && n_words_out && weight_out, "pkb_batch_decode: bad output arguments");
+  PKB_TRY(pkb::check_decode_graph(b->c, b->am, fst, "pkb_batch_decode"));
+  PKB_TRY(pkb::check_decode_outputs(max_words, words_out, n_words_out, weight_out, "pkb_batch_decode"));
   Ctx *c = b->c;
   PKB_CUDA(cudaSetDevice(c->device));
   const int n = b->meta.n_utts;

@@ -38,6 +38,37 @@ struct ViterbiConfig {
   int max_words = 256;       // words returned per utterance
 };
 
+// Kernel choice and workspace of one search (launch_viterbi picks the same for both entry points).
+struct VitPlan {
+  bool dense = false;   // dense shared-memory kernel (small graphs) instead of the hash-table kernel
+  bool small = false;   // table kernel with its tables in shared memory
+  int variant = 0;      // arcs per thread (dense) or lanes per token (table)
+  int max_tok = 0;      // token capacity per frame
+  uint32_t H = 0;       // hash-table slots
+  int grid = 0;
+  size_t stride = 0;    // global workspace bytes per block
+  size_t smem = 0;      // dynamic shared memory
+};
+
+// Carried state of the resumable search (pkb_decoder): what one stream keeps in global memory
+// between launches. A launch restores the tokens into its tables, runs the new frames with the
+// per-frame code of the batch search and saves them back.
+struct Carry {
+  int *hdr;              // [n][4]: live tokens (-1: fresh utterance), word records used, error, alive
+  long long *frames;     // [n] frames decoded in this utterance
+  int *tok_state;        // [n][cap] live tokens: state, cost, newest word record
+  float *tok_cost;
+  int *tok_bp;
+  int cap;
+  int frame_stride;      // the rows of stream s start at row s * frame_stride
+  int uniform_frames;    // new frames of every stream when num_frames is NULL
+  int finish;            // BestPath of the current tokens, then a fresh utterance
+  long long *p_frames;   // best-so-far per stream: frames, [n][max_words] words, word count, cost
+  int32_t *p_words;
+  int32_t *p_nw;
+  float *p_cost;
+};
+
 // Decodes n_utts utterances. loglik: [rows][num_pdfs] scaled log-likelihoods where utterance u owns
 // rows [row_off[u], row_off[u] + num_frames[u]). tid2pdf: device map of input labels.
 // words_out [n_utts][max_words] in spoken order, n_words_out[u] (-1: the search failed: token or
@@ -47,4 +78,56 @@ int launch_viterbi(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const f
                    const int32_t *d_tid2pdf, int n_tids, DevBuf *work, int32_t *d_words,
                    int32_t *d_n_words, float *d_weight);
 
+// The resumable search behind pkb_decoder: n streams, one thread block each, whose tokens and word
+// records stay in global memory between launches. advance() decodes the next rows of every stream
+// (stream s: rows [s * frame_stride, s * frame_stride + n_frames[s]) of d_loglik, or uniform_frames
+// rows each when d_n_frames is NULL) and leaves the best-so-far block in `out`; its arguments stay
+// fixed for fixed inputs, so it can be captured into a CUDA graph. finish() applies BestPath to the
+// current tokens (f_words / f_nw / f_weight, as launch_viterbi) and starts a fresh utterance.
+struct ResumableSearch {
+  Ctx *c = nullptr;
+  const pkb_fst *fst = nullptr;
+  ViterbiConfig cfg;
+  int num_pdfs = 0, n = 0;
+  VitPlan plan;
+  DevBuf work, carry, out, d_tid2pdf;
+  Carry cr{};
+  size_t partial_bytes = 0;  // the best-so-far block at the start of `out`
+  int32_t *f_words = nullptr, *f_nw = nullptr;
+  float *f_weight = nullptr;
+  int setup(Ctx *ctx, const pkb_fst *graph, const ViterbiConfig &config, const int32_t *tid2pdf, int n_tids,
+            int pdfs, int streams);
+  int advance(const float *d_loglik, int frame_stride, const int32_t *d_n_frames, int uniform_frames);
+  int finish();
+};
+
+// Checks shared by pkb_batch_decode and pkb_decoder_create / _finish: the FST is from context c, the
+// model has a tid2pdf map that covers the graph's input labels and points into its pdfs; the
+// output arguments exist.
+int check_decode_graph(const Ctx *c, const pkb_am *am, const pkb_fst *fst, const char *who);
+int check_decode_outputs(int max_words, const void *words_out, const void *n_words_out, const void *weight_out,
+                         const char *who);
+
+}  // namespace pkb
+
+// n_streams searches of pkb_decoder_create (include/pkb200.h).
+struct pkb_decoder {
+  pkb::Ctx *c = nullptr;
+  const pkb_am *am = nullptr;
+  int n = 0;
+  pkb::ResumableSearch search;
+  pkb::DevBuf rows, nfr;        // staging of the host-fed advance: rows, frames per stream
+  struct { void *p = nullptr; } partial;  // pinned host copy of the best-so-far block
+  pkb_stream *st = nullptr;     // attached stream (pkb_stream_set_decoder)
+  bool flushed = false;         // the attached stream was flushed: finish before its next push
+  pkb_decoder() = default;
+  pkb_decoder(const pkb_decoder &) = delete;
+  pkb_decoder &operator=(const pkb_decoder &) = delete;
+  ~pkb_decoder();
+};
+
+namespace pkb {
+// Queues an advance over device rows and the copy of its best-so-far block to the host.
+int decoder_enqueue_advance(pkb_decoder *dec, const float *d_rows, int frame_stride, const int32_t *d_n_frames,
+                            int uniform_frames);
 }  // namespace pkb

@@ -15,6 +15,7 @@
 #include <algorithm>
 #include <memory>
 
+#include "decoder.cuh"
 #include "nnet.cuh"
 
 namespace pkb {
@@ -135,16 +136,25 @@ struct pkb_stream {
   void *g_out[4] = {nullptr, nullptr, nullptr, nullptr}, *g_out2[4] = {nullptr, nullptr, nullptr, nullptr};
   int64_t g_launches[4][PKB_KERNEL_CLASSES] = {};
   bool graphs_off = false;
-  ~pkb_stream() {
-    for (cudaGraphExec_t g : gexec)
+  int64_t replays = 0;         // pushes run by replaying a captured graph
+  pkb_decoder *dec = nullptr;  // advanced over the emitted rows of every push (pkb_stream_set_decoder)
+  void drop_graphs() {
+    for (cudaGraphExec_t &g : gexec) {
       if (g) cudaGraphExecDestroy(g);
+      g = nullptr;
+    }
+  }
+  ~pkb_stream() {
+    if (dec) dec->st = nullptr;
+    drop_graphs();
   }
 };
 
 namespace {
 
-// Runs the nnet over the current feature window (rows per stream = `rows`) and copies the first
-// `emit` rows of every stream to the host.
+// Runs the nnet over the current feature window (rows per stream = `rows`), advances the attached
+// decoder over the first `emit` rows of every stream and copies those rows to the host unless
+// loglik_out is NULL.
 int stream_emit(pkb_stream *st, int rows, int emit, void *loglik_out, float *off_out) {
   pkb::Ctx *c = st->c;
   pkb_am *am = st->am;
@@ -176,6 +186,8 @@ int stream_emit(pkb_stream *st, int rows, int emit, void *loglik_out, float *off
   }
   PKB_TRY(pkb::nnet_forward(am, &st->ws, in, &am->splice_stage, pkb::kFinalLoglik, st->scale,
                             st->out.as<float>()));
+  if (st->dec) PKB_TRY(pkb::decoder_enqueue_advance(st->dec, st->out.as<float>(), rows, nullptr, emit));
+  if (!loglik_out) return PKB_OK;
   const size_t row_bytes = static_cast<size_t>(st->P) * sizeof(float);
   PKB_CUDA(cudaMemcpy2DAsync(loglik_out, max_frames * row_bytes, st->out.p, rows * row_bytes,
                              emit * row_bytes, st->S, cudaMemcpyDeviceToHost, c->stream));
@@ -241,6 +253,12 @@ void pkb_stream_destroy(pkb_stream_t *st) {
 }
 
 int pkb_stream_max_frames(const pkb_stream_t *st) { return st ? st->max_new + st->R : 0; }
+
+int pkb_stream_graph_replays(const pkb_stream_t *st, int64_t *replays) {
+  PKB_REQUIRE(st && replays, "pkb_stream_graph_replays: NULL argument");
+  *replays = st->replays;
+  return PKB_OK;
+}
 
 namespace {
 
@@ -316,7 +334,8 @@ int stream_push(pkb_stream *st, const int16_t *pcm, void *out, float *off_out, i
   sh.rows = sh.n_new > 0 ? sh.carry + sh.n_new : 0;
   sh.emit = sh.n_new > 0 ? std::max(0, sh.rows - (st->L + st->R)) : 0;
   PKB_REQUIRE(sh.rows <= st->max_rows, "%s: window overflow (%d rows)", who, sh.rows);
-  PKB_REQUIRE(sh.emit == 0 || out, "%s: the output buffer is NULL", who);
+  PKB_REQUIRE(!st->dec || !st->dec->flushed, "%s: the stream was flushed: finish its decoder first", who);
+  PKB_REQUIRE(sh.emit == 0 || out || st->dec, "%s: the output buffer is NULL", who);
   PKB_REQUIRE(sh.emit == 0 || !st->compact || off_out, "%s: the offset buffer is NULL", who);
   if (sh.n_new > 0) {
     if (st->meta_len != sh.win_len) {
@@ -368,6 +387,7 @@ int stream_push(pkb_stream *st, const int16_t *pcm, void *out, float *off_out, i
     }
     if (st->gexec[par] != nullptr) {
       PKB_CUDA(cudaGraphLaunch(st->gexec[par], c->stream));
+      ++st->replays;
       for (int k = 0; k < PKB_KERNEL_CLASSES; ++k) c->launches[k] += st->g_launches[par][k];
       done = true;
     }
@@ -407,14 +427,30 @@ int pkb_stream_push_compact_i16(pkb_stream_t *st, const int16_t *pcm, uint16_t *
 int pkb_stream_set_compact(pkb_stream_t *st, int on) {
   PKB_REQUIRE(st, "pkb_stream_set_compact: stream is NULL");
   PKB_REQUIRE(!on || st->am->softmax_last, "pkb_stream_set_compact: the model does not end in a softmax");
+  PKB_REQUIRE(!on || !st->dec, "pkb_stream_set_compact: the attached decoder reads the FP32 rows");
   if ((on != 0) == st->compact) return PKB_OK;
   PKB_CUDA(cudaSetDevice(st->c->device));
   PKB_CUDA(cudaStreamSynchronize(st->c->stream));
-  for (int i = 0; i < 4; ++i) {
-    if (st->gexec[i]) cudaGraphExecDestroy(st->gexec[i]);
-    st->gexec[i] = nullptr;
-  }
+  st->drop_graphs();
   st->compact = on != 0;
+  return PKB_OK;
+}
+
+int pkb_stream_set_decoder(pkb_stream_t *st, pkb_decoder_t *dec) {
+  PKB_REQUIRE(st, "pkb_stream_set_decoder: stream is NULL");
+  if (dec == st->dec) return PKB_OK;
+  if (dec) {
+    PKB_REQUIRE(dec->c == st->c && dec->am == st->am && dec->n == st->S,
+                "pkb_stream_set_decoder: the decoder has another context, model or stream count");
+    PKB_REQUIRE(!st->compact, "pkb_stream_set_decoder: the decoder reads the FP32 rows (switch the compact output off)");
+    PKB_REQUIRE(!dec->st, "pkb_stream_set_decoder: the decoder is attached to another stream");
+  }
+  PKB_CUDA(cudaSetDevice(st->c->device));
+  PKB_CUDA(cudaStreamSynchronize(st->c->stream));
+  st->drop_graphs();  // the captured pushes advance the old decoder, or none
+  if (st->dec) st->dec->st = nullptr;
+  st->dec = dec;
+  if (dec) dec->st = st;
   return PKB_OK;
 }
 
@@ -425,7 +461,7 @@ static int stream_flush(pkb_stream_t *st, void *loglik_out, float *off_out, int3
   int emit = 0;
   const int pending = static_cast<int>(st->n_feat - st->n_emit);
   if (pending > 0) {
-    PKB_REQUIRE(loglik_out && (!st->compact || off_out), "pkb_stream_flush: output buffer is NULL");
+    PKB_REQUIRE((loglik_out || st->dec) && (!st->compact || off_out), "pkb_stream_flush: output buffer is NULL");
     // rows = carry (pending + L); append R replicas of the last frame (src/am.cc:76)
     const int carry = pending + st->L;
     const int rows = carry + st->R;
@@ -460,6 +496,7 @@ static int stream_flush(pkb_stream_t *st, void *loglik_out, float *off_out, int3
   st->n_feat = st->n_emit = 0;
   st->prev_rows = 0;
   st->have_last = false;
+  if (st->dec) st->dec->flushed = true;
   PKB_CUDA(cudaMemsetAsync(st->stat.p, 0, static_cast<size_t>(st->S) * pkb::kMel * sizeof(float), c->stream));
   PKB_CUDA(cudaMemsetAsync(st->tcount.p, 0, 2 * sizeof(int64_t), c->stream));
   return pkb::check_device_error(c, "pkb_stream_flush");
