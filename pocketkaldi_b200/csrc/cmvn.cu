@@ -14,7 +14,6 @@
 // tabulated on the host with the reference's double/float arithmetic.
 
 #include <math.h>
-#include <stdlib.h>
 
 #include <algorithm>
 
@@ -130,14 +129,15 @@ __device__ __forceinline__ void cp_async_wait() {
 // One thread per pair of chains (utterance, dims 2k and 2k + 1): 20 threads per utterance. The
 // recurrence is a handful of dependent FP32 operations per frame, so what limits the kernel is
 // latency: every thread streams its x[t] and x[t - 600] pairs through a private shared-memory ring
-// with cp.async, kGroups - 1 groups of 8 frames ahead of the group it is consuming, and no thread
+// with cp.async, kCmvnGroups - 1 groups of 8 frames ahead of the group it is consuming, and no thread
 // ever reads another thread's slots (no block-level synchronisation in the loop).
 // Frames t < 600 fill the window (global stats blended in through the alpha / scale tables, which
 // hold alpha = 0 at t = 599); frames t >= 600 slide it. 600 is a multiple of the group size, so a
 // group lies in one phase.
 constexpr int kCmvnThreadsPerUtt = kMel / 2;
+constexpr int kCmvnGroups = 4;  // ring depth: 4 groups of kCmvnUnroll frames (32 frames)
 
-template <int kPlanes, bool kFp16, bool kOut, int kBlock, int kCmvnGroups>
+template <int kPlanes, bool kFp16, bool kOut, int kBlock>
 __global__ void __launch_bounds__(kBlock, kBlock == 160 ? 2 : 16)
 cmvn_kernel(const float *__restrict__ raw, const int64_t *__restrict__ frame_off,
             const int32_t *__restrict__ num_frames, int n_utts,
@@ -346,33 +346,22 @@ int launch_cmvn(Ctx *c, const float *d_raw, const BatchMeta &m, float *d_out,
   // single-warp blocks spread over all SM sub-partitions instead of a few 5-warp blocks
   const int block = threads >= static_cast<int64_t>(c->sm_count) * 2 * 160 ? 160 : 32;
   const int grid = static_cast<int>((threads + block - 1) / block);
-  // ring depth: 4 groups (32 frames); PKB_CMVN_GROUPS=8 doubles it (tuning knob)
-  static const int env_groups = getenv("PKB_CMVN_GROUPS") ? atoi(getenv("PKB_CMVN_GROUPS")) : 0;
-  const int groups = env_groups == 4 || env_groups == 8 ? env_groups : 4;
   // per-thread rings: x and x_old pairs
-  size_t dyn_smem = static_cast<size_t>(2) * groups * kCmvnUnroll * block * sizeof(float2);
-  // PKB_CMVN_BLOCKS_PER_SM=n (tuning knob): caps residency with unused dynamic shared memory
-  static const int max_blocks = getenv("PKB_CMVN_BLOCKS_PER_SM") ? atoi(getenv("PKB_CMVN_BLOCKS_PER_SM")) : 0;
-  if (max_blocks > 0) dyn_smem = std::max<size_t>(dyn_smem, (220 * 1024) / max_blocks - 6 * 1024);
+  const size_t dyn_smem = static_cast<size_t>(2) * kCmvnGroups * kCmvnUnroll * block * sizeof(float2);
   LaunchScope scope(c, PKB_KERNEL_CMVN);
   __nv_bfloat16 *hi = planes ? planes->hi : nullptr, *lo = planes ? planes->lo : nullptr;
   const int n_planes = hi ? (lo ? 2 : 1) : 0;
   const bool fp16 = planes && planes->fp16;
   PKB_REQUIRE(!planes || planes->dim_pad == kMel, "cmvn: operand planes must have a row pitch of %d elements", kMel);
-#define PKB_CMVN_LAUNCH4(PL, FP, OUT, BLK, GR)                                                           \
+#define PKB_CMVN_LAUNCH3(PL, FP, OUT, BLK)                                                               \
   do {                                                                                                  \
     if (dyn_smem > 40 * 1024)                                                                           \
-      cudaFuncSetAttribute(cmvn_kernel<PL, FP, OUT, BLK, GR>,                                           \
+      cudaFuncSetAttribute(cmvn_kernel<PL, FP, OUT, BLK>,                                               \
                            cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(dyn_smem));    \
-    cmvn_kernel<PL, FP, OUT, BLK, GR><<<grid, BLK, dyn_smem, c->stream>>>(                              \
+    cmvn_kernel<PL, FP, OUT, BLK><<<grid, BLK, dyn_smem, c->stream>>>(                                  \
         d_raw, m.d_frame_off, m.d_num_frames, m.n_utts, c->cmvn_tab.as<float>(), d_out, hi, lo,         \
         planes ? planes->d_pad_off : nullptr, planes ? planes->left : 0, planes ? planes->right : 0,    \
         planes ? planes->dim_pad : 0);                                                                  \
-  } while (0)
-#define PKB_CMVN_LAUNCH3(PL, FP, OUT, BLK)                \
-  do {                                                    \
-    if (groups == 8) PKB_CMVN_LAUNCH4(PL, FP, OUT, BLK, 8); \
-    else PKB_CMVN_LAUNCH4(PL, FP, OUT, BLK, 4);             \
   } while (0)
 #define PKB_CMVN_LAUNCH2(PL, FP, OUT)                    \
   do {                                                   \
@@ -391,7 +380,6 @@ int launch_cmvn(Ctx *c, const float *d_raw, const BatchMeta &m, float *d_out,
   else if (n_planes == 2 && !fp16) PKB_CMVN_LAUNCH(2, false);
   else PKB_CMVN_LAUNCH(2, true);
 #undef PKB_CMVN_LAUNCH3
-#undef PKB_CMVN_LAUNCH4
 #undef PKB_CMVN_LAUNCH2
 #undef PKB_CMVN_LAUNCH
   PKB_CUDA(cudaGetLastError());

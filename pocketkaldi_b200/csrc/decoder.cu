@@ -20,7 +20,6 @@
 // equal float costs are broken by arc index instead of by list order.
 
 #include <math.h>
-#include <stdlib.h>
 
 #include <algorithm>
 #include <memory>
@@ -999,8 +998,7 @@ VitPlan plan_viterbi(const Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg,
                      bool resume) {
   VitPlan p;
   const size_t log_bytes = (resume ? 3 : 2) * sizeof(int) * static_cast<size_t>(cfg.max_log);
-  static const char *env_dense = getenv("PKB_VIT_DENSE");  // tuning knob: 0 forces the table kernel
-  p.dense = fst->num_states <= 2048 && fst->num_arcs <= 16 * kVitThreads && !(env_dense && atoi(env_dense) == 0);
+  p.dense = fst->num_states <= 2048 && fst->num_arcs <= 16 * kVitThreads;
   if (p.dense) {
     // dense kernel: no token capacity to run out of; the global workspace holds the word records only
     p.max_tok = fst->num_states;
@@ -1027,9 +1025,7 @@ VitPlan plan_viterbi(const Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg,
   // persistent blocks: a few per SM, each walking its share of the utterances with one workspace
   p.grid = resume ? n_utts : std::min(n_utts, c->sm_count * 8);
   p.smem = p.small ? table_bytes : 0;
-  static const char *env_group = getenv("PKB_VIT_GROUP");  // tuning knob: 8 or 32
-  p.variant = (env_group ? atoi(env_group) == 32 : static_cast<double>(fst->num_arcs) >= 12.0 * fst->num_states)
-                  ? 32 : 8;
+  p.variant = static_cast<double>(fst->num_arcs) >= 12.0 * fst->num_states ? 32 : 8;
   return p;
 }
 

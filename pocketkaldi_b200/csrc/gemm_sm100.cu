@@ -51,15 +51,9 @@ constexpr int kMainThreads = 128;   // warps 0-3: TMA producer, MMA issuer, TMEM
 // registers, one pipeline stage less) is 5 % slower than one team, and dropping the back-off
 // sleeps of the producer / MMA waits changes nothing -- the hidden stages are bound by the
 // TMA -> MMA stream, not by the epilogue (PKB_GEMM_DEBUG=1 prints the per-tile cycle split).
-#ifndef PKB_HID_TEAMS
-#define PKB_HID_TEAMS 1
-#endif
-// PKB_FINAL_TEAMS=1 (one team of 16 warps, four column quarters per lane quadrant) is correct
-// but 6-14 % slower than two teams: pass 2 is bound by the turnaround of each warp's single TMA
-// staging tile and the exchange latency, which only another team's work can cover.
-#ifndef PKB_FINAL_TEAMS
-#define PKB_FINAL_TEAMS 2
-#endif
+// One output-stage team of 16 warps (four column quarters per lane quadrant) is correct but 6-14 %
+// slower than two teams: pass 2 is bound by the turnaround of each warp's single TMA staging tile
+// and the exchange latency, which only another team's work can cover.
 // `planes` is the operand mode of the main loop: 1 = one 16-bit plane, 2 = hi + lo planes (three
 // MMAs per product), 3 = FP16 + FP8 corrections (two MMA-equivalents per product).
 // Accumulator stages in TMEM. The output stage's drain (two passes over the accumulator with the
@@ -73,17 +67,11 @@ constexpr int kMainThreads = 128;   // warps 0-3: TMA producer, MMA issuer, TMEM
 // warp no longer waits for TMEM, but the extra write + read + write of every output tile competes
 // with the operand loads (wait for shared-memory stages 3.7k -> 7.3k cycles per tile) and the
 // in-place finish takes as long as the pass it replaces (41.3 -> 45.5 ms, 43.3 ms with CTA pairs).
-constexpr int acc_stages(bool final, int bn) { return (void(final), void(bn), 2); }
-constexpr int epi_teams(bool final, int planes, int bn = 256) {
-  return (void(bn), final ? PKB_FINAL_TEAMS : (planes == 1 ? PKB_HID_TEAMS : 1));
-}
-constexpr int team_warps(bool final, int planes, int bn = 256) {
-  return final ? 16 / epi_teams(final, planes, bn) : (planes == 2 ? 4 : PKB_HID_WARPS);
-}
-constexpr int epi_warps(bool final, int planes, int bn = 256) {
-  return epi_teams(final, planes, bn) * team_warps(final, planes, bn);
-}
-constexpr int num_threads(bool final, int planes, int bn = 256) { return kMainThreads + 32 * epi_warps(final, planes, bn); }
+constexpr int kAccStages = 2;
+constexpr int epi_teams(bool final) { return final ? 2 : 1; }
+constexpr int team_warps(bool final, int planes) { return final ? 8 : (planes == 2 ? 4 : kHidWarps); }
+constexpr int epi_warps(bool final, int planes) { return epi_teams(final) * team_warps(final, planes); }
+constexpr int num_threads(bool final, int planes) { return kMainThreads + 32 * epi_warps(final, planes); }
 // bytes of epilogue staging per warp of a hidden stage: one 32 x 128-byte tile per 16-bit output
 // plane, or the FP16 tile plus two 32 x 64-byte FP8 tiles
 constexpr uint32_t hid_stage_bytes(int planes, bool out8) { return (out8 || planes == 2) ? 8192u : 4096u; }
@@ -501,7 +489,7 @@ __device__ __forceinline__ bool get_tile(const GemmParams &p, int it, uint32_t r
 //   w_x = e4m3(W16 * 2^4); correction phase A = a_lo x w_x, phase B = a_x x w_lo, main = a_hi x w_hi.
 // OUT8 (hidden stages only): the epilogue writes the FP16C8 operand triple of the next stage.
 template <int BN, int PLANES, bool FINAL, int CG, bool OUT8>
-__global__ void __launch_bounds__(num_threads(FINAL, PLANES, BN), 1)
+__global__ void __launch_bounds__(num_threads(FINAL, PLANES), 1)
 gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
             const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo,
             const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ CUtensorMap tm_a_x,
@@ -515,9 +503,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
   uint64_t *bars = reinterpret_cast<uint64_t *>(smem + L.bar_off);
   uint64_t *full = bars;                       // [stages]
   uint64_t *empty = bars + kMaxStages;         // [stages]
-  constexpr int kAcc = acc_stages(FINAL, BN);  // accumulator stages of BN columns in TMEM
-  uint64_t *tfull = bars + 2 * kMaxStages;     // [kAcc <= 4]
-  uint64_t *tempty = bars + 2 * kMaxStages + 4;  // [kAcc <= 4]
+  uint64_t *tfull = bars + 2 * kMaxStages;     // [kAccStages <= 4]
+  uint64_t *tempty = bars + 2 * kMaxStages + 4;  // [kAccStages <= 4]
   uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 2 * kMaxStages + 8);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -543,14 +530,14 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], 1);
     }
-    for (int i = 0; i < kAcc; ++i) {
+    for (int i = 0; i < kAccStages; ++i) {
       mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], CG * team_warps(FINAL, PLANES, BN));  // both CTAs of a pair release the leader
+      mbar_init(&tempty[i], CG * team_warps(FINAL, PLANES));  // both CTAs of a pair release the leader
     }
     fence_barrier_init();
   }
   if (warp == 2) {
-    tmem_alloc<CG>(tmem_slot, kAcc * BN);
+    tmem_alloc<CG>(tmem_slot, kAccStages * BN);
     tmem_relinquish<CG>();
   }
   tc_fence_before();
@@ -620,7 +607,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
       uint32_t s = 0, ph = 0;
       int m_blk, n_blk;
       for (int it = 0; get_tile<CG>(p, it, cta_rank, m_blk, n_blk); ++it) {
-        const uint32_t as = it % kAcc, aph = (it / kAcc) & 1;
+        const uint32_t as = it % kAccStages, aph = (it / kAccStages) & 1;
         long long tw0 = 0, tw_full = 0;
         if (kProbes && p.dbg != nullptr) tw0 = clock64();
         mbar_wait<32>(&tempty[as], aph ^ 1);
@@ -688,8 +675,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
     const int q = warp & 3;  // TMEM lane quadrant
     // FINAL: team = accumulator stage; inside a team two warps per lane quadrant, each owning
     // half of the tile's columns
-    constexpr int kTeams = epi_teams(FINAL, PLANES, BN);
-    constexpr int kTeamWarps = team_warps(FINAL, PLANES, BN);
+    constexpr int kTeams = epi_teams(FINAL);
+    constexpr int kTeamWarps = team_warps(FINAL, PLANES);
     const int team = (warp - 4) / kTeamWarps;
     const int wt = (warp - 4) % kTeamWarps;
     constexpr int kHalves = kTeamWarps / 4;  // warps per lane quadrant
@@ -706,7 +693,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
     // grouped schedule: this CTA's column tile never changes, keep its bias / log-prior in smem
     float *s_bias = reinterpret_cast<float *>(smem + L.epi_off + (FINAL ? kFinalStageBytes : 16u * 4096u));
     float *s_lp = s_bias + BN;
-    constexpr int kEpiThreads = 32 * epi_warps(FINAL, PLANES, BN);
+    constexpr int kEpiThreads = 32 * epi_warps(FINAL, PLANES);
     if (FINAL && p.group_sched) {
       const int nb = (static_cast<int>(blockIdx.x) / CG) % p.n_tiles_n;
       for (int i = threadIdx.x - kMainThreads; i < BN; i += kEpiThreads) {
@@ -720,7 +707,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
     const int t_row = lane >> 3, t_chunk = lane & 7;            // transposed read role
     int m_blk, n_blk;
     for (int it = team; get_tile<CG>(p, it, cta_rank, m_blk, n_blk); it += kTeams) {
-      const uint32_t as = it % kAcc, aph = (it / kAcc) & 1;
+      const uint32_t as = it % kAccStages, aph = (it / kAccStages) & 1;
       const int m0 = m_blk * kBlockM;
       const int n0 = n_blk * BN;
       const int wrow0 = m0 + q * 32;  // first row of this warp
@@ -1208,7 +1195,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
   if (CG == 2) cluster_sync_all(); else __syncthreads();
   if (warp == 2) {
     tc_fence_after();
-    tmem_dealloc<CG>(tmem_base, kAcc * BN);
+    tmem_dealloc<CG>(tmem_base, kAccStages * BN);
   }
 }
 
@@ -1285,11 +1272,11 @@ int launch_one(Ctx *c, const GemmMaps &mp, const GemmParams &p) {
     void *args[] = {&m0, &m1, &m2, &m3, &out_map, &m5, &m6, &pp};
     if (CG == 1) {
       PKB_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<const void *>(kern), dim3(grid),
-                                           dim3(num_threads(FINAL, PLANES, BN)), args, L.total, c->stream));
+                                           dim3(num_threads(FINAL, PLANES)), args, L.total, c->stream));
     } else {
       cudaLaunchConfig_t cfg{};
       cfg.gridDim = dim3(grid);
-      cfg.blockDim = dim3(num_threads(FINAL, PLANES, BN));
+      cfg.blockDim = dim3(num_threads(FINAL, PLANES));
       cfg.dynamicSmemBytes = L.total;
       cfg.stream = c->stream;
       cudaLaunchAttribute attr[2];
@@ -1305,15 +1292,14 @@ int launch_one(Ctx *c, const GemmMaps &mp, const GemmParams &p) {
       // grid (<= one CTA per SM) holds without the attribute.
       static const bool tool_attached = getenv("CUDA_INJECTION64_PATH") != nullptr ||
                                         getenv("NV_COMPUTE_PROFILER_PERFWORKS_DIR") != nullptr ||
-                                        getenv("NV_NSIGHT_INJECTION_PORT_BASE") != nullptr ||
-                                        getenv("PKB_NO_COOP_CLUSTER") != nullptr;
+                                        getenv("NV_NSIGHT_INJECTION_PORT_BASE") != nullptr;
       cfg.numAttrs = tool_attached ? 1 : 2;
       PKB_CUDA(cudaLaunchKernelEx(&cfg, kern, m0, m1, m2, m3, out_map, m5, m6, pp));
     }
   } else if (CG == 2) {
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(num_threads(FINAL, PLANES, BN));
+    cfg.blockDim = dim3(num_threads(FINAL, PLANES));
     cfg.dynamicSmemBytes = L.total;
     cfg.stream = c->stream;
     cudaLaunchAttribute attr[1];
@@ -1325,8 +1311,8 @@ int launch_one(Ctx *c, const GemmMaps &mp, const GemmParams &p) {
     cfg.numAttrs = 1;
     PKB_CUDA(cudaLaunchKernelEx(&cfg, kern, *a_hi, *a_lo, *w_hi, *w_lo, out_map, *a_x, *w_x, pp));
   } else {
-    kern<<<grid, num_threads(FINAL, PLANES, BN), L.total, c->stream>>>(*a_hi, *a_lo, *w_hi, *w_lo, out_map, *a_x,
-                                                                   *w_x, pp);
+    kern<<<grid, num_threads(FINAL, PLANES), L.total, c->stream>>>(*a_hi, *a_lo, *w_hi, *w_lo, out_map, *a_x,
+                                                               *w_x, pp);
   }
   PKB_CUDA(cudaGetLastError());
   }
@@ -1458,7 +1444,6 @@ int launch_gemm(Ctx *c, int block_n, int planes, bool final, int cta_group, bool
   // CTA pairs (the W maps must have box rows block_n / 2)
   PKB_GEMM_CASE(256, 1, false, 2, false)
   PKB_GEMM_CASE(256, 2, false, 2, false)
-  PKB_GEMM_CASE(256, 1, true, 2, false)
   PKB_GEMM_CASE(256, 2, true, 2, false)
   PKB_GEMM_CASE(256, 2, false, 2, true)
   PKB_GEMM_CASE(256, 3, false, 2, true)

@@ -105,12 +105,10 @@ int make_output_map16(CUtensorMap *map, const uint16_t *base, uint64_t cols, uin
 
 int gemm_max_smem_bytes(int block_n, int planes);
 
-// Epilogue warps of a single-plane hidden stage: 8 (two per TMEM lane quadrant) or 4.
-#ifndef PKB_HID_WARPS
-#define PKB_HID_WARPS 8
-#endif
+// Epilogue warps of a single-plane hidden stage: two per TMEM lane quadrant.
+constexpr int kHidWarps = 8;
 // Sum-of-squares partials one hidden tile writes per row (= epilogue warps per lane quadrant)
 // for operand mode `planes`.
-inline int sumsq_parts(int planes) { return planes == 2 ? 1 : PKB_HID_WARPS / 4; }
+inline int sumsq_parts(int planes) { return planes == 2 ? 1 : kHidWarps / 4; }
 
 }  // namespace pkb

@@ -444,10 +444,8 @@ int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, const Stage *fi
     // of row blocks: always for hidden stages; for the output stage only in the multi-MMA modes,
     // where the halved W tile is what makes a second pipeline stage fit (its BF16/FP16 variant is
     // bound by the epilogue, not by operand traffic, and measured no gain from pairing)
-    static const bool no_pairs = getenv("PKB_GEMM_CG1") != nullptr;
-    static const bool final_pairs = getenv("PKB_GEMM_FINAL_CG2") != nullptr;
-    const bool want_pair = !final || mode >= 2 || final_pairs;
-    int cg = (want_pair && block_n == 256 && m_tiles >= 2 && !no_pairs) ? 2 : 1;
+    const bool want_pair = !final || mode >= 2;
+    int cg = (want_pair && block_n == 256 && m_tiles >= 2) ? 2 : 1;
     // the grouped schedule of the softmax stage needs one CTA (pair) per column tile on the device
     if (final && p.final_mode != 0 && cg == 2 && (c->sm_count / 2) / p.n_tiles_n < 1) cg = 1;
     GemmMaps maps;

@@ -316,8 +316,12 @@ def test_loader_errors_follow_the_reference_convention(ctx, tmp_path, toy_conf):
         pk.AcousticModel(ctx).Read(str(tmp_path / "nope.conf"))
     assert e.value.code == 2 and "IOError" in str(e.value)
     import shutil
+    # contents only: copied modes would leave the copies read-only where the test tree is
+    src = os.path.dirname(toy_conf)
     d = tmp_path / "m"
-    shutil.copytree(os.path.dirname(toy_conf), d)
+    d.mkdir()
+    for f in os.listdir(src):
+        shutil.copyfile(os.path.join(src, f), d / f)
     conf = str(d / "toy.conf")
     raw = bytearray(open(d / "toy.nnet", "rb").read())
     raw[0:4] = b"XXXX"
@@ -325,7 +329,7 @@ def test_loader_errors_follow_the_reference_convention(ctx, tmp_path, toy_conf):
     with pytest.raises(pk.PkbError) as e:
         pk.AcousticModel(ctx).Read(conf)
     assert e.value.code == 3 and "Corruption" in str(e.value)
-    shutil.copy(os.path.join(os.path.dirname(toy_conf), "toy.nnet"), d / "toy.nnet")
+    shutil.copyfile(os.path.join(src, "toy.nnet"), d / "toy.nnet")
     lines = [l for l in open(conf) if not l.startswith("prior")]
     open(conf, "w").writelines(lines)
     with pytest.raises(pk.PkbError) as e:

@@ -17,8 +17,6 @@ from oracle.decoder import host_viterbi
 from pocketkaldi_b200 import formats
 from pocketkaldi_b200.synth import synth_global_cmvn
 
-pytestmark = pytest.mark.gpu
-
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, HERE)
@@ -39,7 +37,7 @@ def make_model(ctx, kind):
     """(am, fst, graph, tid2pdf) for the graph kinds of test_gpu_viterbi.py, with acoustic scores
     made decisive the same way: "loop" 12 words (dense kernel), "eps" the epsilon hub, "loop_big"
     180 words / 541 states (table kernel, global tables), "loop_mid" 100 words / 301 states (table
-    kernel with shared-memory tables when the dense kernel is switched off)."""
+    kernel, shared-memory tables)."""
     rng = np.random.default_rng({"loop": 1, "eps": 2, "loop_big": 3, "loop_mid": 4}[kind])
     P = 600 if kind in ("loop_big", "loop_mid") else 96
     layers = formats.make_dnn(rng, 440, 96, 2, P)
@@ -87,8 +85,16 @@ def decode_in_splits(dec, rows, k, each=None):
     return dec.finish()
 
 
-def check_split_invariance(kind):
-    ctx = pk.Context(0)
+def test_loop_mid_takes_the_table_kernel_with_shared_memory_tables():
+    # plan_viterbi (decoder.cu): more than 4096 arcs rule out the dense kernel, at most 512 states
+    # put the token tables in shared memory (the graph of make_model(ctx, "loop_mid"))
+    num_states, _, _, arcs = demo.word_loop_graph(100, 3, 600)[0]
+    assert num_states <= 512 and len(arcs) > 4096
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("kind", ["loop", "eps", "loop_big", "loop_mid"])
+def test_split_invariance_bitwise_against_batch_decode(ctx, kind):
     am, fst, _, _ = make_model(ctx, kind)
     pcms = [coloured(100 + u, n) for u, n in enumerate(LENS)]
     hyps, wts, rows = batch_rows(ctx, am, fst, pcms)
@@ -99,12 +105,6 @@ def check_split_invariance(kind):
         assert got == hyps, (kind, k)
         assert np.array_equal(gw.view(np.int32), wts.view(np.int32)), (kind, k, gw, wts)
         dec.close()
-    ctx.close()
-
-
-@pytest.mark.parametrize("kind", ["loop", "eps", "loop_big"])
-def test_split_invariance_bitwise_against_batch_decode(kind):
-    check_split_invariance(kind)
 
 
 def run_child(code, **env):
@@ -114,11 +114,6 @@ def run_child(code, **env):
                        cwd=ROOT, env=e, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, timeout=900)
     assert r.returncode == 0, r.stdout.decode()[-4000:]
     assert b"CHILD OK" in r.stdout
-
-
-def test_split_invariance_table_kernel_shared_memory_tables():
-    run_child("import test_gpu_online_decode as t\nt.check_split_invariance('loop_mid')\nprint('CHILD OK')",
-              PKB_VIT_DENSE="0")
 
 
 # ---------------------------------------------------------------- host restatement with its tokens
@@ -168,6 +163,7 @@ def host_frames(graph, tid2pdf, loglik, beam=16.0):
         yield toks
 
 
+@pytest.mark.gpu
 @pytest.mark.parametrize("kind", ["loop", "eps"])
 def test_partials_follow_the_host_restatement(ctx, kind):
     am, fst, graph, tid2pdf = make_model(ctx, kind)
@@ -232,6 +228,7 @@ def stream_utterance(st, dec, ref, pcm, chunk, rows=True):
     return got, parts, emitting
 
 
+@pytest.mark.gpu
 @pytest.mark.parametrize("kind", ["loop", "eps"])
 @pytest.mark.parametrize("chunk", [160, 2560, 16000])
 def test_attached_stream_decodes_like_the_batch(ctx, kind, chunk):
@@ -298,10 +295,12 @@ def check_decode_only_pushes():
     ctx.close()
 
 
+@pytest.mark.gpu
 def test_decode_only_pushes_in_the_captured_graph():
     check_decode_only_pushes()
 
 
+@pytest.mark.gpu
 def test_decode_only_pushes_eager():
     run_child("import test_gpu_online_decode as t\nt.check_decode_only_pushes()\nprint('CHILD OK')",
               PKB_STREAM_GRAPH="0")
@@ -364,6 +363,7 @@ def host_record_counts(graph, tid2pdf, loglik, every, beam=16.0):
     return appended, live_max, adv_max
 
 
+@pytest.mark.gpu
 def test_record_compaction_on_a_long_stream(ctx):
     am, fst, graph, tid2pdf = make_model(ctx, "loop")
     pcm = coloured(500, 120 * 16000)
@@ -396,6 +396,7 @@ def test_record_compaction_on_a_long_stream(ctx):
 
 
 # ---------------------------------------------------------------- errors and lifetime
+@pytest.mark.gpu
 def test_invalid_uses_are_rejected(ctx):
     am, fst, graph, tid2pdf = make_model(ctx, "loop")
     g = synth_global_cmvn()
@@ -457,6 +458,7 @@ def test_invalid_uses_are_rejected(ctx):
     ctx2.close()
 
 
+@pytest.mark.gpu
 def test_token_overflow_is_reported_and_the_next_utterance_is_clean(ctx):
     rng = np.random.default_rng(3)
     P = 640
@@ -480,6 +482,7 @@ def test_token_overflow_is_reported_and_the_next_utterance_is_clean(ctx):
     am.close()
 
 
+@pytest.mark.gpu
 def test_create_attach_finish_destroy_cycles_do_not_leak(ctx):
     import torch
     am, fst, _, _ = make_model(ctx, "loop")
