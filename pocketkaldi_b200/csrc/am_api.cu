@@ -365,7 +365,7 @@ static int am_compute_device(pkb_ctx_t *c, pkb_am_t *am, const float *feats, con
                              std::vector<int64_t> *pad_off) {
   PKB_REQUIRE(c && am, "%s: NULL argument", who);
   PKB_REQUIRE(am->c == c, "%s: model belongs to another context", who);
-  PKB_REQUIRE(am->has_splice_stage && feat_dim == am->feat_dim,
+  PKB_REQUIRE(am->feat_dim > 0 && feat_dim == am->feat_dim,
               "%s: feat_dim %d does not match the model (nnet input %d, context %d+1+%d)", who,
               feat_dim, am->input_dim, am->left, am->right);
   PKB_CUDA(cudaSetDevice(c->device));
@@ -402,8 +402,8 @@ static int am_compute_device(pkb_ctx_t *c, pkb_am_t *am, const float *feats, con
   in.rows = rows;
   in.cols = (am->left + am->right + 1) * dp;
   in.pitch_elems = dp;
-  return pkb::nnet_forward_refined(am, &ws, &am->rf, in, &am->splice_stage, ws.row_map.as<int32_t>(),
-                                   pkb::kFinalLoglik, prob_scale, am->out_f32.as<float>());
+  return pkb::nnet_forward_refined(am, &ws, &am->rf, in, ws.row_map.as<int32_t>(), pkb::kFinalLoglik,
+                                   prob_scale, am->out_f32.as<float>());
 }
 
 int pkb_am_compute(pkb_ctx_t *c, pkb_am_t *am, const float *feats, const int32_t *num_frames,
@@ -512,7 +512,12 @@ int pkb_nnet_propagate(pkb_ctx_t *c, pkb_am_t *am, const float *in_host, int row
   PKB_CUDA(cudaSetDevice(c->device));
   Workspace &ws = am->ws;
   PKB_TRY(pkb::workspace_ensure(am, &ws, rows));
-  const int dp = (in_dim + 7) / 8 * 8;
+  // the column layout stage 0 was packed for: feat_dim_pad columns per context frame, or one
+  // group of in_dim columns padded to 16 bytes
+  const int group = am->feat_dim > 0 ? am->feat_dim : in_dim;
+  const int group_pad = am->feat_dim > 0 ? am->feat_dim_pad : (in_dim + 7) / 8 * 8;
+  const int groups = in_dim / group;
+  const int dp = groups * group_pad;
   const int out_dim = am->stages.back().out_dim;
   PKB_TRY(ws.feat_hi.ensure(static_cast<size_t>(rows) * dp * 2));
   if (am->planes == 2) PKB_TRY(ws.feat_lo.ensure(static_cast<size_t>(rows) * dp * 2));
@@ -523,7 +528,7 @@ int pkb_nnet_propagate(pkb_ctx_t *c, pkb_am_t *am, const float *in_host, int row
   PKB_CUDA(cudaMemcpyAsync(am->in_f32.p, in_host, in_bytes, cudaMemcpyHostToDevice, c->stream));
   __nv_bfloat16 *hi = ws.feat_hi.as<__nv_bfloat16>();
   __nv_bfloat16 *lo = am->planes == 2 ? ws.feat_lo.as<__nv_bfloat16>() : nullptr;
-  PKB_TRY(pkb::launch_pack_plain(c, am->in_f32.as<float>(), rows, in_dim, dp, hi, lo, am->fp16));
+  PKB_TRY(pkb::launch_pack_plain(c, am->in_f32.as<float>(), rows, groups, group, group_pad, hi, lo, am->fp16));
   InputView in;
   in.hi = hi;
   in.lo = lo;
@@ -531,7 +536,7 @@ int pkb_nnet_propagate(pkb_ctx_t *c, pkb_am_t *am, const float *in_host, int row
   in.cols = dp;
   in.pitch_elems = dp;
   const pkb::FinalMode mode = am->softmax_last ? pkb::kFinalProb : pkb::kFinalRaw;
-  PKB_TRY(pkb::nnet_forward(am, &ws, in, &am->stages[0], mode, 1.0f, am->out_f32.as<float>()));
+  PKB_TRY(pkb::nnet_forward(am, &ws, in, mode, 1.0f, am->out_f32.as<float>()));
   PKB_CUDA(cudaMemcpyAsync(out, am->out_f32.p, out_bytes, cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaStreamSynchronize(c->stream));
   return pkb::check_device_error(c, "pkb_nnet_propagate");
@@ -544,7 +549,7 @@ int pkb_batch_create(pkb_ctx_t *c, pkb_am_t *am, int n_utts, const int32_t *num_
   PKB_REQUIRE(global_stats, "pkb_batch_create: global_stats is NULL");
   PKB_REQUIRE(n_utts == 0 || num_samples, "pkb_batch_create: num_samples is NULL");
   PKB_REQUIRE(!am || am->c == c, "pkb_batch_create: model belongs to another context");
-  PKB_REQUIRE(!am || (am->has_splice_stage && am->feat_dim == pkb::kMel),
+  PKB_REQUIRE(!am || am->feat_dim == pkb::kMel,
               "pkb_batch_create: the model's feature dim must be %d", pkb::kMel);
   PKB_CUDA(cudaSetDevice(c->device));
   std::unique_ptr<pkb_batch, decltype(&pkb_batch_destroy)> b(new pkb_batch(), pkb_batch_destroy);
@@ -647,12 +652,11 @@ int pkb_batch_run(pkb_batch_t *b, int stages) {
     in.pitch_elems = am->feat_dim_pad;
     const int32_t *row_map = b->ws.row_map.as<int32_t>();
     if (b->compact)
-      PKB_TRY(pkb::nnet_forward_refined(am, &b->ws, &b->rf, in, &am->splice_stage, row_map,
-                                        pkb::kFinalCompact, b->prob_scale, nullptr,
-                                        b->loglik16.as<uint16_t>(), b->loglik_off.as<float>()));
+      PKB_TRY(pkb::nnet_forward_refined(am, &b->ws, &b->rf, in, row_map, pkb::kFinalCompact, b->prob_scale,
+                                        nullptr, b->loglik16.as<uint16_t>(), b->loglik_off.as<float>()));
     else
-      PKB_TRY(pkb::nnet_forward_refined(am, &b->ws, &b->rf, in, &am->splice_stage, row_map,
-                                        pkb::kFinalLoglik, b->prob_scale, b->loglik.as<float>()));
+      PKB_TRY(pkb::nnet_forward_refined(am, &b->ws, &b->rf, in, row_map, pkb::kFinalLoglik, b->prob_scale,
+                                        b->loglik.as<float>()));
   }
   return PKB_OK;
 }

@@ -1199,33 +1199,22 @@ gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *,
-                                  const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
-                                  const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void *sym = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &q) != cudaSuccess ||
-      q != cudaDriverEntryPointSuccess || sym == nullptr)
-    return nullptr;
-  fn = reinterpret_cast<EncodeTiledFn>(sym);
-  return fn;
-}
-
 template <int BN, int PLANES, bool FINAL, int CG, bool OUT8>
 int launch_one(Ctx *c, const GemmMaps &mp, const GemmParams &p) {
   const CUtensorMap *a_hi = mp.a_hi, *a_lo = mp.a_lo, *w_hi = mp.w_hi, *w_lo = mp.w_lo;
   const CUtensorMap *a_x = PLANES == 3 ? mp.a_x : mp.a_hi, *w_x = PLANES == 3 ? mp.w_x : mp.w_hi;
-  // FP32 output map of the final stage (hidden stages pass a dummy copy of the A map)
+  // output map of the final stage's TMA stores, boxes of 32 rows x 128 bytes; it needs a 16-byte
+  // row pitch (hidden stages pass a dummy copy of the A map)
   CUtensorMap out_map = *a_hi;
   if (FINAL && p.final_mode == 3) {
-    if ((p.ld_f32 & 7) == 0) PKB_TRY(make_output_map16(&out_map, p.out_h16, p.N_valid, p.M));
+    if ((p.ld_f32 & 7) == 0)
+      PKB_TRY(encode_tensor_map(&out_map, CU_TENSOR_MAP_DATA_TYPE_UINT16, p.out_h16, p.N_valid, p.M,
+                                static_cast<uint64_t>(p.N_valid) * sizeof(uint16_t), 64, 32,
+                                CU_TENSOR_MAP_L2_PROMOTION_NONE));
   } else if (FINAL && (p.ld_f32 & 3) == 0) {
-    PKB_TRY(make_output_map(&out_map, p.out_f32, p.N_valid, p.M));
+    PKB_TRY(encode_tensor_map(&out_map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, p.out_f32, p.N_valid, p.M,
+                              static_cast<uint64_t>(p.N_valid) * sizeof(float), 32, 32,
+                              CU_TENSOR_MAP_L2_PROMOTION_NONE));
   }
   const SmemLayout L = smem_layout(BN, PLANES, FINAL, CG, OUT8);
   auto kern = gemm_kernel<BN, PLANES, FINAL, CG, OUT8>;
@@ -1339,87 +1328,34 @@ int launch_one(Ctx *c, const GemmMaps &mp, const GemmParams &p) {
 
 int gemm_max_smem_bytes(int block_n, int planes) { return smem_layout(block_n, planes, true, 1, false).total; }
 
-int make_tensor_map8(CUtensorMap *map, const void *base, uint64_t cols, uint64_t rows,
-                     uint64_t pitch_bytes, uint32_t box_rows) {
-  EncodeTiledFn fn = get_encode_fn();
+int encode_tensor_map(CUtensorMap *map, CUtensorMapDataType type, const void *base, uint64_t cols,
+                      uint64_t rows, uint64_t pitch_bytes, uint32_t box_cols, uint32_t box_rows,
+                      CUtensorMapL2promotion l2) {
+  typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *,
+                                    const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
+                                    const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  static const EncodeTiledFn fn = [] {
+    void *sym = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &q) == cudaSuccess &&
+                    q == cudaDriverEntryPointSuccess && sym != nullptr;
+    return ok ? reinterpret_cast<EncodeTiledFn>(sym) : nullptr;
+  }();
   if (!fn) {
     set_error("cuTensorMapEncodeTiled entry point not available");
     return PKB_ERR_CUDA;
   }
   cuuint64_t dims[2] = {cols, rows};
   cuuint64_t strides[1] = {pitch_bytes};
-  cuuint32_t box[2] = {128, box_rows};
+  cuuint32_t box[2] = {box_cols, box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void *>(base), dims, strides, box,
-                  estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = fn(map, type, 2, const_cast<void *>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  CU_TENSOR_MAP_SWIZZLE_128B, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (FP8) failed (CUresult %d) cols=%llu rows=%llu pitch=%llu", (int)r,
-              (unsigned long long)cols, (unsigned long long)rows, (unsigned long long)pitch_bytes);
-    return PKB_ERR_CUDA;
-  }
-  return PKB_OK;
-}
-
-int make_tensor_map(CUtensorMap *map, const void *base, uint64_t cols, uint64_t rows,
-                    uint64_t pitch_bytes, uint32_t box_rows) {
-  EncodeTiledFn fn = get_encode_fn();
-  if (!fn) {
-    set_error("cuTensorMapEncodeTiled entry point not available");
-    return PKB_ERR_CUDA;
-  }
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {pitch_bytes};
-  cuuint32_t box[2] = {static_cast<cuuint32_t>(kBlockK), box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), dims, strides,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed (CUresult %d) cols=%llu rows=%llu pitch=%llu", (int)r,
-              (unsigned long long)cols, (unsigned long long)rows, (unsigned long long)pitch_bytes);
-    return PKB_ERR_CUDA;
-  }
-  return PKB_OK;
-}
-
-int make_output_map(CUtensorMap *map, const float *base, uint64_t cols, uint64_t rows) {
-  EncodeTiledFn fn = get_encode_fn();
-  if (!fn) {
-    set_error("cuTensorMapEncodeTiled entry point not available");
-    return PKB_ERR_CUDA;
-  }
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {cols * sizeof(float)};
-  cuuint32_t box[2] = {32, 32};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float *>(base), dims, strides,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (output) failed (CUresult %d) cols=%llu rows=%llu", (int)r,
-              (unsigned long long)cols, (unsigned long long)rows);
-    return PKB_ERR_CUDA;
-  }
-  return PKB_OK;
-}
-
-int make_output_map16(CUtensorMap *map, const uint16_t *base, uint64_t cols, uint64_t rows) {
-  EncodeTiledFn fn = get_encode_fn();
-  if (!fn) {
-    set_error("cuTensorMapEncodeTiled entry point not available");
-    return PKB_ERR_CUDA;
-  }
-  cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {cols * sizeof(uint16_t)};
-  cuuint32_t box[2] = {64, 32};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, const_cast<uint16_t *>(base), dims, strides,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled (16-bit output) failed (CUresult %d) cols=%llu rows=%llu", (int)r,
-              (unsigned long long)cols, (unsigned long long)rows);
+    set_error("cuTensorMapEncodeTiled failed (CUresult %d) type=%d cols=%llu rows=%llu pitch=%llu box=%ux%u", (int)r,
+              (int)type, (unsigned long long)cols, (unsigned long long)rows, (unsigned long long)pitch_bytes,
+              box_cols, box_rows);
     return PKB_ERR_CUDA;
   }
   return PKB_OK;

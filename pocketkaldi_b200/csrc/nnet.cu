@@ -76,14 +76,16 @@ __global__ void row_map_kernel(const int64_t *__restrict__ frame_off,
     row_map[base + t] = static_cast<int32_t>(f0 + t);
 }
 
+// one thread per (row, padded column); input column k goes to (k / group) * group_pad + k % group
 __global__ void pack_plain_kernel(const float *__restrict__ in, int64_t rows, int dim, int dim_pad,
-                                  __nv_bfloat16 *__restrict__ hi, __nv_bfloat16 *__restrict__ lo,
-                                  int fp16) {
+                                  int group, int group_pad, __nv_bfloat16 *__restrict__ hi,
+                                  __nv_bfloat16 *__restrict__ lo, int fp16) {
   const int64_t g = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const int64_t r = g / dim_pad;
   const int d = static_cast<int>(g % dim_pad);
   if (r >= rows) return;
-  const float v = d < dim ? in[r * dim + d] : 0.0f;
+  const int j = d % group_pad;
+  const float v = j < group ? in[r * dim + d / group_pad * group + j] : 0.0f;
   const __nv_bfloat16 h = operand_bits(v, fp16);
   hi[g] = h;
   if (lo) lo[g] = operand_bits(v - operand_value(h, fp16), fp16);
@@ -111,19 +113,48 @@ __global__ void pack_c8_kernel(const float *__restrict__ W, int out_dim, int in_
 }
 
 // ---------------------------------------------------------------- weight packing
-// W[out][in] float -> BF16 planes [n_pad][k_pad]; column c of the source goes to
-// column remap(c) (identity, or the padded splice layout).
-int pack_stage(Ctx *c, Stage *st, const float *W, const float *b, int out_dim, int in_dim,
-               int group, int group_pad, int planes, int fp16) {
+// What both packings share: the N tiling, the zero-padded bias, the device planes (`planes` 16-bit
+// ones, and the two E4M3 ones of FP16C8) and the weight maps. The caller sets the K layout first
+// (k_pad; c8 and k_pad8 for FP16C8) and fills the planes.
+int alloc_stage(Ctx *c, Stage *st, const float *b, int out_dim, int in_dim, int planes) {
   st->in_dim = in_dim;
   st->out_dim = out_dim;
-  const int groups = group > 0 ? in_dim / group : 1;
-  const int k_logical = group > 0 ? groups * group_pad : in_dim;
-  st->k_pad = round_up(k_logical, kBlockK);
   const int n128 = round_up(out_dim, 128), n256 = round_up(out_dim, 256);
   // wide tiles unless they cost more than 6% extra padding
   st->block_n = (n256 * 100 <= n128 * 106) ? 256 : 128;
   st->n_pad = st->block_n == 256 ? n256 : n128;
+  std::vector<float> bias(st->n_pad, 0.0f);
+  memcpy(bias.data(), b, sizeof(float) * out_dim);
+  PKB_TRY(st->bias.ensure(sizeof(float) * st->n_pad));
+  PKB_TRY(upload(c, st->bias.p, bias.data(), sizeof(float) * st->n_pad));
+  const size_t e16 = static_cast<size_t>(st->n_pad) * st->k_pad, e8 = static_cast<size_t>(st->n_pad) * st->k_pad8;
+  PKB_TRY(st->w_hi.ensure(e16 * 2));
+  if (planes == 2) PKB_TRY(st->w_lo.ensure(e16 * 2));
+  if (st->c8) {
+    PKB_TRY(st->w8_hi.ensure(e8));
+    PKB_TRY(st->w8_lo.ensure(e8));
+  }
+  const uint64_t p16 = static_cast<uint64_t>(st->k_pad) * 2, p8 = static_cast<uint64_t>(st->k_pad8);
+  for (int t = 0; t < 2; ++t) {
+    CUtensorMap *m = st->w_map[t];
+    const uint32_t box_rows = st->block_n >> t;
+    PKB_TRY(make_operand_map(&m[0], st->w_hi.p, false, st->k_pad, st->n_pad, p16, box_rows));
+    m[1] = m[2] = m[0];
+    if (planes == 2) PKB_TRY(make_operand_map(&m[1], st->w_lo.p, false, st->k_pad, st->n_pad, p16, box_rows));
+    if (st->c8) {
+      PKB_TRY(make_operand_map(&m[1], st->w8_lo.p, true, st->k_pad8, st->n_pad, p8, box_rows));
+      PKB_TRY(make_operand_map(&m[2], st->w8_hi.p, true, st->k_pad8, st->n_pad, p8, box_rows));
+    }
+  }
+  return PKB_OK;
+}
+
+// W[out][in] float -> BF16 planes [n_pad][k_pad]; column k of the source goes to column
+// (k / group) * group_pad + k % group (group = group_pad = in_dim: the identity).
+int pack_stage(Ctx *c, Stage *st, const float *W, const float *b, int out_dim, int in_dim,
+               int group, int group_pad, int planes, int fp16) {
+  st->k_pad = round_up(in_dim / group * group_pad, kBlockK);
+  PKB_TRY(alloc_stage(c, st, b, out_dim, in_dim, planes));
   const size_t elems = static_cast<size_t>(st->n_pad) * st->k_pad;
   std::vector<__nv_bfloat16> hi(elems, operand_bits(0.0f, fp16)), lo;
   if (planes == 2) lo.assign(elems, operand_bits(0.0f, fp16));
@@ -132,50 +163,23 @@ int pack_stage(Ctx *c, Stage *st, const float *W, const float *b, int out_dim, i
     __nv_bfloat16 *dh = hi.data() + static_cast<size_t>(o) * st->k_pad;
     __nv_bfloat16 *dl = planes == 2 ? lo.data() + static_cast<size_t>(o) * st->k_pad : nullptr;
     for (int k = 0; k < in_dim; ++k) {
-      const int kk = group > 0 ? (k / group) * group_pad + (k % group) : k;
+      const int kk = (k / group) * group_pad + (k % group);
       const __nv_bfloat16 h = operand_bits(src[k], fp16);
       dh[kk] = h;
       if (dl) dl[kk] = operand_bits(src[k] - operand_value(h, fp16), fp16);
     }
   }
-  std::vector<float> bias(st->n_pad, 0.0f);
-  memcpy(bias.data(), b, sizeof(float) * out_dim);
-  PKB_TRY(st->w_hi.ensure(elems * 2));
   PKB_TRY(upload(c, st->w_hi.p, hi.data(), elems * 2));
-  if (planes == 2) {
-    PKB_TRY(st->w_lo.ensure(elems * 2));
-    PKB_TRY(upload(c, st->w_lo.p, lo.data(), elems * 2));
-  }
-  PKB_TRY(st->bias.ensure(sizeof(float) * st->n_pad));
-  PKB_TRY(upload(c, st->bias.p, bias.data(), sizeof(float) * st->n_pad));
-  PKB_TRY(make_tensor_map(&st->tm_w_hi, st->w_hi.p, st->k_pad, st->n_pad,
-                          static_cast<uint64_t>(st->k_pad) * 2, st->block_n));
-  if (planes == 2)
-    PKB_TRY(make_tensor_map(&st->tm_w_lo, st->w_lo.p, st->k_pad, st->n_pad,
-                            static_cast<uint64_t>(st->k_pad) * 2, st->block_n));
-  else
-    st->tm_w_lo = st->tm_w_hi;
-  PKB_TRY(make_tensor_map(&st->tm_w_hi_half, st->w_hi.p, st->k_pad, st->n_pad,
-                          static_cast<uint64_t>(st->k_pad) * 2, st->block_n / 2));
-  if (planes == 2)
-    PKB_TRY(make_tensor_map(&st->tm_w_lo_half, st->w_lo.p, st->k_pad, st->n_pad,
-                            static_cast<uint64_t>(st->k_pad) * 2, st->block_n / 2));
-  else
-    st->tm_w_lo_half = st->tm_w_hi_half;
+  if (planes == 2) PKB_TRY(upload(c, st->w_lo.p, lo.data(), elems * 2));
   return PKB_OK;
 }
 
 // Operand mode 3 (FP16C8) planes of W[out][in]: W16 = fp16(W * 2^g) with max |W * 2^g| in [1, 2),
 // W_hi8 = e4m3(W16 * 2^4), W_lo8 = e4m3((W * 2^g - W16) * 2^13); see gemm_sm100.cu.
 int pack_stage_c8(Ctx *c, Stage *st, const float *W, const float *b, int out_dim, int in_dim) {
-  st->in_dim = in_dim;
-  st->out_dim = out_dim;
   st->c8 = true;
   st->k_pad = round_up(in_dim, kBlockK);
   st->k_pad8 = round_up(in_dim, 128);
-  const int n128 = round_up(out_dim, 128), n256 = round_up(out_dim, 256);
-  st->block_n = (n256 * 100 <= n128 * 106) ? 256 : 128;
-  st->n_pad = st->block_n == 256 ? n256 : n128;
   float wmax = 0.0f;
   for (size_t i = 0; i < static_cast<size_t>(out_dim) * in_dim; ++i) wmax = std::max(wmax, fabsf(W[i]));
   PKB_REQUIRE(std::isfinite(wmax), "linear layer: non-finite weight");
@@ -183,38 +187,19 @@ int pack_stage_c8(Ctx *c, Stage *st, const float *W, const float *b, int out_dim
   if (wmax > 0.0f) frexpf(wmax, &e);  // wmax = m * 2^e, m in [0.5, 1)
   st->w_exp = wmax > 0.0f ? 1 - e : 0; // W * 2^g has its maximum in [1, 2)
   const float sg = ldexpf(1.0f, st->w_exp);
-  const size_t e16 = static_cast<size_t>(st->n_pad) * st->k_pad, e8 = static_cast<size_t>(st->n_pad) * st->k_pad8;
-  std::vector<float> bias(st->n_pad, 0.0f);
-  memcpy(bias.data(), b, sizeof(float) * out_dim);
-  PKB_TRY(st->w_hi.ensure(e16 * 2));
-  PKB_TRY(st->w8_hi.ensure(e8));
-  PKB_TRY(st->w8_lo.ensure(e8));
-  PKB_TRY(st->bias.ensure(sizeof(float) * st->n_pad));
-  PKB_TRY(upload(c, st->bias.p, bias.data(), sizeof(float) * st->n_pad));
-  {
-    // the planes are rounded on the device: 2 x 8.8 M scalar FP8 conversions on the host would
-    // dominate the model load of the config-3 net
-    DevBuf tmp;
-    const size_t wbytes = static_cast<size_t>(out_dim) * in_dim * sizeof(float);
-    PKB_TRY(tmp.ensure(wbytes));
-    PKB_TRY(upload(c, tmp.p, W, wbytes));
-    const int64_t threads = static_cast<int64_t>(e8);
-    pack_c8_kernel<<<static_cast<unsigned>((threads + 255) / 256), 256, 0, c->stream>>>(
-        tmp.as<float>(), out_dim, in_dim, st->n_pad, st->k_pad, st->k_pad8, sg, st->w_hi.as<__nv_bfloat16>(),
-        st->w8_hi.as<uint8_t>(), st->w8_lo.as<uint8_t>());
-    PKB_CUDA(cudaGetLastError());
-    PKB_CUDA(cudaStreamSynchronize(c->stream));
-  }
-  const uint64_t p16 = static_cast<uint64_t>(st->k_pad) * 2, p8 = static_cast<uint64_t>(st->k_pad8);
-  PKB_TRY(make_tensor_map(&st->tm_w_hi, st->w_hi.p, st->k_pad, st->n_pad, p16, st->block_n));
-  PKB_TRY(make_tensor_map(&st->tm_w_hi_half, st->w_hi.p, st->k_pad, st->n_pad, p16, st->block_n / 2));
-  st->tm_w_lo = st->tm_w_hi;
-  st->tm_w_lo_half = st->tm_w_hi_half;
-  PKB_TRY(make_tensor_map8(&st->tm_w8_hi, st->w8_hi.p, st->k_pad8, st->n_pad, p8, st->block_n));
-  PKB_TRY(make_tensor_map8(&st->tm_w8_hi_half, st->w8_hi.p, st->k_pad8, st->n_pad, p8, st->block_n / 2));
-  PKB_TRY(make_tensor_map8(&st->tm_w8_lo, st->w8_lo.p, st->k_pad8, st->n_pad, p8, st->block_n));
-  PKB_TRY(make_tensor_map8(&st->tm_w8_lo_half, st->w8_lo.p, st->k_pad8, st->n_pad, p8, st->block_n / 2));
-  (void)c;
+  PKB_TRY(alloc_stage(c, st, b, out_dim, in_dim, 1));
+  // the planes are rounded on the device: 2 x 8.8 M scalar FP8 conversions on the host would
+  // dominate the model load of the config-3 net
+  DevBuf tmp;
+  const size_t wbytes = static_cast<size_t>(out_dim) * in_dim * sizeof(float);
+  PKB_TRY(tmp.ensure(wbytes));
+  PKB_TRY(upload(c, tmp.p, W, wbytes));
+  const int64_t threads = static_cast<int64_t>(st->n_pad) * st->k_pad8;
+  pack_c8_kernel<<<static_cast<unsigned>((threads + 255) / 256), 256, 0, c->stream>>>(
+      tmp.as<float>(), out_dim, in_dim, st->n_pad, st->k_pad, st->k_pad8, sg, st->w_hi.as<__nv_bfloat16>(),
+      st->w8_hi.as<uint8_t>(), st->w8_lo.as<uint8_t>());
+  PKB_CUDA(cudaGetLastError());
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
   return PKB_OK;
 }
 
@@ -266,16 +251,21 @@ int am_build(Ctx *c, int n_layers, const int32_t *types, const float *const *wei
     const int od = out_dims[lin], id = in_dims[lin];
     PKB_REQUIRE(od > 0 && id > 0 && (prev_out < 0 || id == prev_out),
                 "linear layer %d: shape [%d x %d] does not follow output dim %d", lin, od, id, prev_out);
+    int group = id, group_pad = id;
+    if (lin == 0) {
+      am->input_dim = id;
+      const int w = left + right + 1;
+      if (id % w == 0) {  // stage 0 reads the padded splice view: feat_dim_pad columns per frame
+        am->feat_dim = group = id / w;
+        am->feat_dim_pad = group_pad = round_up(am->feat_dim, 8);  // 16-byte row pitch for the TMA view
+      }
+    }
     am->stages.emplace_back();
     Stage &st = am->stages.back();
     // FP16C8: stage 0 reads the 16-bit feature planes (three MMAs), later stages the FP8 triple
     PKB_TRY((am->c8 && lin > 0) ? pack_stage_c8(c, &st, weights[lin], biases[lin], od, id)
-                                : pack_stage(c, &st, weights[lin], biases[lin], od, id, 0, 0, am->planes, am->fp16));
-    if (lin == 0) {
-      am->input_dim = id;
-      am->w0_host.assign(weights[0], weights[0] + static_cast<size_t>(od) * id);
-      am->b0_host.assign(biases[0], biases[0] + od);
-    }
+                                : pack_stage(c, &st, weights[lin], biases[lin], od, id, group, group_pad,
+                                             am->planes, am->fp16));
     prev_out = od;
     ++lin;
     ++i;
@@ -305,18 +295,6 @@ int am_build(Ctx *c, int n_layers, const int32_t *types, const float *const *wei
     for (int j = 0; j < am->num_pdfs; ++j) lp[j] = static_cast<float>(log(static_cast<double>(prior[j])));
   PKB_TRY(am->log_prior.ensure(sizeof(float) * lp_len));
   PKB_TRY(upload(c, am->log_prior.p, lp.data(), sizeof(float) * lp_len));
-  const int w = left + right + 1;
-  if (am->input_dim % w == 0) {
-    am->feat_dim = am->input_dim / w;
-    am->feat_dim_pad = round_up(am->feat_dim, 8);  // 16-byte row pitch for the TMA view
-    PKB_TRY(pack_stage(c, &am->splice_stage, am->w0_host.data(), am->b0_host.data(),
-                       am->stages[0].out_dim, am->input_dim, am->feat_dim, am->feat_dim_pad,
-                       am->planes, am->fp16));
-    am->splice_stage.relu = am->stages[0].relu;
-    am->splice_stage.sigmoid = am->stages[0].sigmoid;
-    am->splice_stage.normalize = am->stages[0].normalize;
-    am->has_splice_stage = true;
-  }
   if (tid2pdf && n_tid2pdf > 0) am->tid2pdf.assign(tid2pdf, tid2pdf + n_tid2pdf);
   *out = am.release();
   return PKB_OK;
@@ -352,9 +330,8 @@ int workspace_ensure(pkb_am *am, Workspace *ws, int64_t rows) {
   return PKB_OK;
 }
 
-int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, const Stage *first,
-                 FinalMode mode_out, float prob_scale, float *d_out, uint16_t *d_h16, float *d_off,
-                 bool fast, int *near_cnt, float near_margin) {
+int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, FinalMode mode_out, float prob_scale,
+                 float *d_out, uint16_t *d_h16, float *d_off, bool fast, int *near_cnt, float near_margin) {
   Ctx *c = am->c;
   const int64_t rows = ws->rows;
   if (rows == 0) return PKB_OK;
@@ -378,19 +355,19 @@ int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, const Stage *fi
   float in_dim = 0.0f;
   const int m_tiles = static_cast<int>((rows + kBlockM - 1) / kBlockM);
   for (size_t i = 0; i < ns; ++i) {
-    const Stage &st = i == 0 ? *first : am->stages[i];
+    const Stage &st = am->stages[i];
     const bool final = i + 1 == ns;
     // operand mode of this stage and the form its epilogue has to produce for the next one
     const int mode = fast ? 1 : (st.c8 ? 3 : am->planes);
     const bool out8 = !fast && !final && am->c8;
     CUtensorMap tm_a_hi, tm_a_lo, tm_a_x;
-    PKB_TRY(make_tensor_map(&tm_a_hi, a_hi, a_cols, rows, static_cast<uint64_t>(a_pitch) * 2, kBlockM));
+    PKB_TRY(make_operand_map(&tm_a_hi, a_hi, false, a_cols, rows, static_cast<uint64_t>(a_pitch) * 2, kBlockM));
     if (mode == 2) {
-      PKB_TRY(make_tensor_map(&tm_a_lo, a_lo, a_cols, rows, static_cast<uint64_t>(a_pitch) * 2, kBlockM));
+      PKB_TRY(make_operand_map(&tm_a_lo, a_lo, false, a_cols, rows, static_cast<uint64_t>(a_pitch) * 2, kBlockM));
       tm_a_x = tm_a_hi;
     } else if (mode == 3) {
-      PKB_TRY(make_tensor_map8(&tm_a_lo, a8_lo, a_cols, rows, static_cast<uint64_t>(a_pitch), kBlockM));
-      PKB_TRY(make_tensor_map8(&tm_a_x, a8_hi, a_cols, rows, static_cast<uint64_t>(a_pitch), kBlockM));
+      PKB_TRY(make_operand_map(&tm_a_lo, a8_lo, true, a_cols, rows, static_cast<uint64_t>(a_pitch), kBlockM));
+      PKB_TRY(make_operand_map(&tm_a_x, a8_hi, true, a_cols, rows, static_cast<uint64_t>(a_pitch), kBlockM));
     } else {
       tm_a_lo = tm_a_hi;
       tm_a_x = tm_a_hi;
@@ -448,18 +425,8 @@ int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, const Stage *fi
     int cg = (want_pair && block_n == 256 && m_tiles >= 2) ? 2 : 1;
     // the grouped schedule of the softmax stage needs one CTA (pair) per column tile on the device
     if (final && p.final_mode != 0 && cg == 2 && (c->sm_count / 2) / p.n_tiles_n < 1) cg = 1;
-    GemmMaps maps;
-    maps.a_hi = &tm_a_hi;
-    maps.a_lo = &tm_a_lo;
-    maps.a_x = &tm_a_x;
-    maps.w_hi = cg == 2 ? &st.tm_w_hi_half : &st.tm_w_hi;
-    if (mode == 3) {
-      maps.w_lo = cg == 2 ? &st.tm_w8_lo_half : &st.tm_w8_lo;
-      maps.w_x = cg == 2 ? &st.tm_w8_hi_half : &st.tm_w8_hi;
-    } else {
-      maps.w_lo = cg == 2 ? &st.tm_w_lo_half : &st.tm_w_lo;
-      maps.w_x = maps.w_hi;
-    }
+    const CUtensorMap *w = st.w_map[cg == 2 ? 1 : 0];
+    const GemmMaps maps{&tm_a_hi, &tm_a_lo, &tm_a_x, &w[0], &w[1], &w[2]};
     PKB_TRY(launch_gemm(c, block_n, mode, final, cg, out8, maps, p));
     if (!final) {
       a_hi = p.out_hi;
@@ -556,10 +523,10 @@ int launch_scatter(Ctx *c, const void *src, const int32_t *list, int n, size_t r
 }  // namespace
 
 int nnet_forward_refined(pkb_am *am, Workspace *ws, Refine *rf, const InputView &in,
-                         const Stage *first, const int32_t *row_map, FinalMode mode,
-                         float prob_scale, float *d_out, uint16_t *d_h16, float *d_off) {
+                         const int32_t *row_map, FinalMode mode, float prob_scale, float *d_out,
+                         uint16_t *d_h16, float *d_off) {
   if (!am->refine || (mode != kFinalLoglik && mode != kFinalCompact))
-    return nnet_forward(am, ws, in, first, mode, prob_scale, d_out, d_h16, d_off);
+    return nnet_forward(am, ws, in, mode, prob_scale, d_out, d_h16, d_off);
   Ctx *c = am->c;
   const int64_t rows = ws->rows;
   rf->last_rows = rows;
@@ -575,8 +542,8 @@ int nnet_forward_refined(pkb_am *am, Workspace *ws, Refine *rf, const InputView 
   PKB_CUDA(cudaMemsetAsync(rf->near_cnt.p, 0, static_cast<size_t>(rows) * sizeof(int), c->stream));
   PKB_CUDA(cudaMemsetAsync(rf->n_sel.p, 0, sizeof(int), c->stream));
   // pass 1: one FP16 MMA per product
-  PKB_TRY(nnet_forward(am, ws, in, first, mode, prob_scale, d_out, d_h16, d_off, true,
-                       rf->near_cnt.as<int>(), am->refine_margin));
+  PKB_TRY(nnet_forward(am, ws, in, mode, prob_scale, d_out, d_h16, d_off, true, rf->near_cnt.as<int>(),
+                       am->refine_margin));
   {
     LaunchScope scope(c, PKB_KERNEL_MISC);
     select_rows_kernel<<<static_cast<unsigned>((rows + 1023) / 1024), 1024, 0, c->stream>>>(
@@ -623,7 +590,7 @@ int nnet_forward_refined(pkb_am *am, Workspace *ws, Refine *rf, const InputView 
   in2.rows = n;
   in2.cols = in.cols;
   in2.pitch_elems = in.cols;
-  PKB_TRY(nnet_forward(am, &rf->ws, in2, first, mode, prob_scale, rf->out_f32.as<float>(),
+  PKB_TRY(nnet_forward(am, &rf->ws, in2, mode, prob_scale, rf->out_f32.as<float>(),
                        rf->out_h16.as<uint16_t>(), rf->out_off.as<float>()));
   if (mode == kFinalCompact) {
     PKB_TRY(launch_scatter(c, rf->out_h16.p, rf->list.as<int32_t>(), n, static_cast<size_t>(out_dim) * 2, d_h16));
@@ -722,13 +689,15 @@ int launch_pack_padded(Ctx *c, const float *d_feats, const BatchMeta &m, int dim
   return PKB_OK;
 }
 
-int launch_pack_plain(Ctx *c, const float *d_in, int64_t rows, int dim, int dim_pad,
+int launch_pack_plain(Ctx *c, const float *d_in, int64_t rows, int groups, int group, int group_pad,
                       __nv_bfloat16 *hi, __nv_bfloat16 *lo, int fp16) {
   if (rows == 0) return PKB_OK;
+  const int dim_pad = groups * group_pad;
   const int64_t threads = rows * dim_pad;
   const int grid = static_cast<int>((threads + 255) / 256);
   LaunchScope scope(c, PKB_KERNEL_MISC);
-  pack_plain_kernel<<<grid, 256, 0, c->stream>>>(d_in, rows, dim, dim_pad, hi, lo, fp16);
+  pack_plain_kernel<<<grid, 256, 0, c->stream>>>(d_in, rows, groups * group, dim_pad, group, group_pad, hi,
+                                                 lo, fp16);
   PKB_CUDA(cudaGetLastError());
   return PKB_OK;
 }

@@ -18,14 +18,15 @@ struct Stage {
   bool sigmoid = false;         // sigmoid follows (PKB_LAYER_SIGMOID; not a reference layer type)
   bool normalize = false;       // NormalizeLayer follows  (src/nnet.cc:62-75)
   DevBuf w_hi, w_lo, bias;      // [n_pad][k_pad] BF16 planes, [n_pad] FP32
-  CUtensorMap tm_w_hi, tm_w_lo;
-  CUtensorMap tm_w_hi_half, tm_w_lo_half;  // box rows block_n / 2: W halves of a CTA pair
   // operand mode 3 (FP16C8): w_hi holds fp16(W * 2^w_exp); E4M3 planes [n_pad][k_pad8]
   bool c8 = false;
   int w_exp = 0;                // g: stored weights are W * 2^g with max |W * 2^g| in [1, 2)
   int k_pad8 = 0;               // K padded to 128
   DevBuf w8_hi, w8_lo;          // e4m3(W16 * 2^4), e4m3((W * 2^g - W16) * 2^13)
-  CUtensorMap tm_w8_hi, tm_w8_lo, tm_w8_hi_half, tm_w8_lo_half;
+  // weight maps [tile][operand]: tile 0 has box rows block_n, tile 1 block_n / 2 (the W half of a
+  // CTA pair); operands 0, 1, 2 are GemmMaps::w_hi, w_lo, w_x and map w_hi; w_lo (FP16C8: w8_lo,
+  // one plane: w_hi); w8_hi (FP16C8) or w_hi
+  CUtensorMap w_map[2][3];
 };
 
 // How the final stage's logits are turned into the caller's output.
@@ -85,15 +86,11 @@ struct pkb_am {
   int feat_dim = 0;    // input_dim / (left + right + 1) when divisible, else 0
   int feat_dim_pad = 0;
   bool softmax_last = false;
+  // stages[0] reads feat_dim_pad columns per context frame (the padded splice view) when
+  // feat_dim > 0, the input_dim columns of a row otherwise
   std::vector<pkb::Stage> stages;
-  // stage 0 weights re-laid for the padded splice view (feat_dim_pad per context frame);
-  // identical to stages[0] when feat_dim % 8 == 0
-  pkb::Stage splice_stage;
-  bool has_splice_stage = false;
   pkb::DevBuf log_prior;  // [num_pdfs], log taken at load (src/am.cc:42-43)
   std::vector<int32_t> tid2pdf;
-  // host copies kept for building splice_stage
-  std::vector<float> w0_host, b0_host;
   // scratch of the synchronous host-buffer entry points (pkb_am_compute, pkb_nnet_propagate)
   pkb::Workspace ws;
   pkb::Refine rf;
@@ -111,18 +108,16 @@ int am_build(Ctx *c, int n_layers, const int32_t *types, const float *const *wei
 // Sizes `ws` for `rows` GEMM rows of model `am`.
 int workspace_ensure(pkb_am *am, Workspace *ws, int64_t rows);
 
-// Runs every stage. `first` selects the weights of stage 0 (am->stages[0] or
-// am->splice_stage). d_out is [ws->rows][out_dim]: GEMM row m -> output row m. For a padded
+// Runs every stage. d_out is [ws->rows][out_dim]: GEMM row m -> output row m. For a padded
 // batch the rows of utterance u start at pad_off[u] and the (left+right) rows between two
 // utterances hold garbage; copy_rows_compact() removes them on the way out.
 // kFinalCompact writes d_h16 [ws->rows][out_dim] (IEEE half bits) and d_off [ws->rows] instead of
 // d_out; prob_scale is then left to the consumer.
 // fast: every stage as one 16-bit plane (the hi planes of whatever the model holds).
 // near_cnt (kFinalLoglik / kFinalCompact): see GemmParams::near_cnt.
-int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, const Stage *first,
-                 FinalMode mode, float prob_scale, float *d_out, uint16_t *d_h16 = nullptr,
-                 float *d_off = nullptr, bool fast = false, int *near_cnt = nullptr,
-                 float near_margin = 0.0f);
+int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, FinalMode mode, float prob_scale,
+                 float *d_out, uint16_t *d_h16 = nullptr, float *d_off = nullptr, bool fast = false,
+                 int *near_cnt = nullptr, float near_margin = 0.0f);
 
 // nnet_forward for every precision; PKB_PREC_FP16R log-likelihoods take two passes:
 //   1. nnet_forward(fast) over all rows, counting per row the pdfs within am->refine_margin of
@@ -131,9 +126,8 @@ int nnet_forward(pkb_am *am, Workspace *ws, const InputView &in, const Stage *fi
 //      gathered, run through the FP16C8 stages and scattered over the first pass's output.
 // One host synchronisation in between (the number of selected rows sizes the second pass).
 int nnet_forward_refined(pkb_am *am, Workspace *ws, Refine *rf, const InputView &in,
-                         const Stage *first, const int32_t *row_map, FinalMode mode,
-                         float prob_scale, float *d_out, uint16_t *d_h16 = nullptr,
-                         float *d_off = nullptr);
+                         const int32_t *row_map, FinalMode mode, float prob_scale, float *d_out,
+                         uint16_t *d_h16 = nullptr, float *d_off = nullptr);
 
 // Device (padded rows) -> host (compact frames) copy of frames [frame0, frame0 + n): one
 // cudaMemcpyAsync per utterance touched.
@@ -149,8 +143,9 @@ int launch_checksum_rows(Ctx *c, const float *d, int cols, int64_t rows, const i
 int launch_pack_padded(Ctx *c, const float *d_feats, const BatchMeta &m, int dim, int dim_pad,
                        int left, int right, const int64_t *d_pad_off, __nv_bfloat16 *hi,
                        __nv_bfloat16 *lo, int32_t *row_map, int fp16);
-// float [rows][dim] -> BF16 planes [rows][dim_pad] (zero padded columns).
-int launch_pack_plain(Ctx *c, const float *d_in, int64_t rows, int dim, int dim_pad,
+// float [rows][groups * group] -> BF16 planes [rows][groups * group_pad]: column k goes to
+// (k / group) * group_pad + k % group, the padding columns are zero.
+int launch_pack_plain(Ctx *c, const float *d_in, int64_t rows, int groups, int group, int group_pad,
                       __nv_bfloat16 *hi, __nv_bfloat16 *lo, int fp16);
 // row_map for a padded batch without packing (the CMVN kernel wrote the planes).
 int launch_row_map(Ctx *c, const BatchMeta &m, int left, int right, const int64_t *d_pad_off,

@@ -175,8 +175,8 @@ int stream_emit(pkb_stream *st, int rows, int emit, void *loglik_out, float *off
   in.pitch_elems = st->Dp;
   const int max_frames = pkb_stream_max_frames(st);
   if (st->compact) {
-    PKB_TRY(pkb::nnet_forward(am, &st->ws, in, &am->splice_stage, pkb::kFinalCompact, st->scale, nullptr,
-                              st->out16.as<uint16_t>(), st->out_off.as<float>()));
+    PKB_TRY(pkb::nnet_forward(am, &st->ws, in, pkb::kFinalCompact, st->scale, nullptr, st->out16.as<uint16_t>(),
+                              st->out_off.as<float>()));
     const size_t row_bytes = static_cast<size_t>(st->P) * sizeof(uint16_t);
     PKB_CUDA(cudaMemcpy2DAsync(loglik_out, max_frames * row_bytes, st->out16.p, rows * row_bytes,
                                emit * row_bytes, st->S, cudaMemcpyDeviceToHost, c->stream));
@@ -184,8 +184,7 @@ int stream_emit(pkb_stream *st, int rows, int emit, void *loglik_out, float *off
                                emit * sizeof(float), st->S, cudaMemcpyDeviceToHost, c->stream));
     return PKB_OK;
   }
-  PKB_TRY(pkb::nnet_forward(am, &st->ws, in, &am->splice_stage, pkb::kFinalLoglik, st->scale,
-                            st->out.as<float>()));
+  PKB_TRY(pkb::nnet_forward(am, &st->ws, in, pkb::kFinalLoglik, st->scale, st->out.as<float>()));
   if (st->dec) PKB_TRY(pkb::decoder_enqueue_advance(st->dec, st->out.as<float>(), rows, nullptr, emit));
   if (!loglik_out) return PKB_OK;
   const size_t row_bytes = static_cast<size_t>(st->P) * sizeof(float);
@@ -205,7 +204,7 @@ int pkb_stream_create(pkb_ctx_t *c, pkb_am_t *am, int n_streams, int chunk_sampl
   PKB_REQUIRE(n_streams > 0, "pkb_stream_create: n_streams must be positive");
   PKB_REQUIRE(chunk_samples > 0 && chunk_samples % pkb::kShift == 0,
               "pkb_stream_create: chunk_samples must be a positive multiple of %d", pkb::kShift);
-  PKB_REQUIRE(am->has_splice_stage && am->feat_dim == pkb::kMel,
+  PKB_REQUIRE(am->feat_dim == pkb::kMel,
               "pkb_stream_create: the model's feature dim must be %d", pkb::kMel);
   PKB_CUDA(cudaSetDevice(c->device));
   std::unique_ptr<pkb_stream, decltype(&pkb_stream_destroy)> st(new pkb_stream(), pkb_stream_destroy);

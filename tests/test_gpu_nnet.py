@@ -2,6 +2,7 @@
 C ABI, against the compiled-reference golden vectors and the restatement oracle."""
 
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -9,6 +10,9 @@ import pytest
 import pocketkaldi_b200 as pk
 from pocketkaldi_b200 import formats
 from pocketkaldi_b200.synth import synth_pcm
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from test_gpu_gemm_matrix import C_MODE, PREC_ID, SCALE, make_net, make_prior, needed_c, splice  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -263,6 +267,29 @@ def test_nnet_propagate_without_softmax_and_odd_input_dim(ctx, oracle):
     ref = oracle.nnet(x, layers)
     assert y.shape == ref.shape == (77, 21)
     assert np.max(np.abs(y - ref)) < 1e-4
+
+
+@pytest.mark.parametrize("prec", ["bf16x3", "fp16c8"])
+def test_spliced_rows_with_unaligned_feat_dim_vs_float64(ctx, prec):
+    # feat_dim 13 is not a multiple of 8, so layer 0 is stored with 16 columns per context frame and
+    # pkb_nnet_propagate has to pack its 65-column rows in that layout. Nnet has no context, so the
+    # model is an AcousticModel passed to pkb_nnet_propagate directly.
+    rng = np.random.default_rng(13)
+    layers = make_net(rng, (65, 256, 300))
+    prior = make_prior(rng, 300)
+    feats = (rng.standard_normal((300, 13)) * 2.5).astype(np.float32)
+    x = splice(feats, 2, 2)
+    am = pk.AcousticModel(ctx, PREC_ID[prec]).from_layers(layers, prior, 2, 2)
+    try:
+        prob = np.empty((300, 300), np.float32)
+        rc = ctx.lib.pkb_nnet_propagate(ctx.h, am.h, x, 300, 65, prob)
+        assert rc == 0, ctx.lib.pkb_last_error().decode()
+        loglik = am.compute_batch([feats], SCALE)[0]
+    finally:
+        am.close()
+    for out, got in (("prob", prob), ("loglik", loglik)):
+        c, _ = needed_c(prec, out, got, x, layers, prior)
+        assert c <= C_MODE[prec], "%s %s: error needs c = %.3g > %.3g" % (prec, out, c, C_MODE[prec])
 
 
 def test_config3_size_properties(ctx, golden):
