@@ -281,6 +281,31 @@ void pkb_fst_destroy(pkb_fst_t *fst);
 int pkb_batch_decode(pkb_batch_t *batch, const pkb_fst_t *fst, float beam, int max_tokens,
                      int max_words, int32_t *words_out, int32_t *n_words_out, float *weight_out);
 
+/* ---- lattices of the batch search -------------------------------------------------------------
+ * Every arc the search of pkb_batch_decode relaxed under its beam, kept when the best complete path
+ * through it costs at most best + lattice_beam (backward costs in double over the search's arcs).
+ * Arcs come sorted by source time; within one time, epsilon arcs before emitting arcs, each group in
+ * ascending FST arc index. */
+typedef struct {           /* 28 bytes, no padding */
+  int32_t t;               /* time of the source node; an emitting arc reads row t and ends at t + 1 */
+  int32_t src, dst;        /* FST states of the source / destination nodes */
+  int32_t ilabel, olabel;
+  float graph_cost;        /* the arc's FST weight */
+  float acoustic_cost;     /* -loglik[t][tid2pdf[ilabel]] (scaled rows); 0 for an epsilon arc */
+} pkb_lattice_arc_t;
+/* Searches every utterance like pkb_batch_decode (same beam / max_tokens defaults) and keeps its
+ * lattice pruned to lattice_beam (> 0, may be +inf) on the device. max_arcs: unpruned arcs per
+ * utterance, 8 bytes of device log each (<= 0: (frames of the longest utterance + 1) x arcs of the
+ * graph, which no utterance can exceed; a word loop keeps nearly all its arcs inside the beam, so a
+ * caller short of memory passes less). n_arcs_out[u]: kept arcs, or a
+ * negative code (-1 tokens, -2 word records, -3 epsilon closure, -4 more than max_arcs arcs);
+ * best_cost_out[u]: min over final nodes of alpha + final (+inf: no final node or a failed search).
+ * Synchronous. */
+int pkb_batch_lattice(pkb_batch_t *batch, const pkb_fst_t *fst, float beam, float lattice_beam, int max_tokens,
+                      int max_arcs, int64_t *n_arcs_out, double *best_cost_out);
+/* The arcs of the latest pkb_batch_lattice, every utterance's back to back in utterance order. */
+int pkb_batch_lattice_get(pkb_batch_t *batch, pkb_lattice_arc_t *arcs_out);
+
 /* ---- online decoding: the GPU Viterbi search, chunk by chunk ----------------------------------
  * n_streams searches whose tokens and word records stay on the device between calls, so that
  * log-likelihood rows can arrive in any split: decoding a stream's rows 1, 7, 16 or all frames at a

@@ -22,6 +22,7 @@ from .binding import (  # noqa: F401
     Batch,
     Decoder,
     Fst,
+    LATTICE_ARC_DTYPE,
     Stream,
     WavList,
     read_wav,

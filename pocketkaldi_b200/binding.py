@@ -27,6 +27,11 @@ BUF_PCM, BUF_RAW, BUF_FEATS, BUF_LOGLIK = 0, 1, 2, 3
 BUF_LOGLIK16, BUF_LOGLIK_OFF = 4, 5  # compact output (Batch.set_compact)
 KERNEL_CLASSES = ("fbank", "cmvn", "gemm", "gemm_final", "misc")
 
+# pkb_lattice_arc_t (include/pkb200.h)
+LATTICE_ARC_DTYPE = np.dtype([("t", np.int32), ("src", np.int32), ("dst", np.int32), ("ilabel", np.int32),
+                              ("olabel", np.int32), ("graph_cost", np.float32), ("acoustic_cost", np.float32)])
+assert LATTICE_ARC_DTYPE.itemsize == 28
+
 _f32p = np.ctypeslib.ndpointer(dtype=np.float32, flags="C_CONTIGUOUS")
 _i32p = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
 _i16p = np.ctypeslib.ndpointer(dtype=np.int16, flags="C_CONTIGUOUS")
@@ -101,6 +106,8 @@ _SIGNATURES = [
     ("pkb_fst_create", C.c_int, [_VP, C.c_int, C.c_int, _VP, _VP, C.c_int, _VP, C.POINTER(_VP)]),
     ("pkb_fst_destroy", None, [_VP]),
     ("pkb_batch_decode", C.c_int, [_VP, _VP, C.c_float, C.c_int, C.c_int, _VP, _VP, _VP]),
+    ("pkb_batch_lattice", C.c_int, [_VP, _VP, C.c_float, C.c_float, C.c_int, C.c_int, _VP, _VP]),
+    ("pkb_batch_lattice_get", C.c_int, [_VP, _VP]),
     ("pkb_decoder_create", C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
                                      C.POINTER(_VP)]),
     ("pkb_decoder_destroy", None, [_VP]),
@@ -669,6 +676,22 @@ class Batch:
                                              nw.ctypes.data, wt.ctypes.data))
         hyps = [None if nw[u] < 0 else [int(x) for x in words[u, :min(int(nw[u]), max_words)]] for u in range(n)]
         return hyps, wt[:n].copy()
+
+    def lattice(self, fst, lattice_beam=8.0, beam=0.0, max_tokens=0, max_arcs=0):
+        """The search of decode() keeping its lattice pruned to lattice_beam (pkb_batch_lattice):
+        returns ([LATTICE_ARC_DTYPE array per utterance, None where the search failed],
+        best costs as float64)."""
+        n = len(self.num_samples)
+        na = np.zeros(max(n, 1), np.int64)
+        best = np.zeros(max(n, 1), np.float64)
+        _check(self.ctx.lib.pkb_batch_lattice(self.h, fst.h, beam, lattice_beam, max_tokens, max_arcs,
+                                              na.ctypes.data, best.ctypes.data))
+        kept = np.maximum(na[:n], 0)
+        arcs = np.empty(max(int(kept.sum()), 1), LATTICE_ARC_DTYPE)
+        _check(self.ctx.lib.pkb_batch_lattice_get(self.h, arcs.ctypes.data))
+        off = np.concatenate([[0], np.cumsum(kept)])
+        lats = [None if na[u] < 0 else arcs[off[u]:off[u + 1]].copy() for u in range(n)]
+        return lats, best[:n].copy()
 
     def refine_stats(self):
         """(GEMM rows, frames recomputed) of the latest run under PREC_FP16R."""

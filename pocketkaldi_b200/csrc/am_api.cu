@@ -281,6 +281,8 @@ struct pkb_batch {
   bool compact = false;             // nnet stage writes loglik16 + loglik_off instead of loglik
   pkb::DevBuf loglik16, loglik_off;
   pkb::DevBuf vit_work, vit_out, vit_tid2pdf;  // GPU Viterbi: workspace, results, device tid2pdf
+  pkb::DevBuf lat_log, lat_aux, lat_arcs;      // lattices: arc logs, offsets and results, kept arcs
+  int64_t lat_total = -1;                      // kept arcs of the latest pkb_batch_lattice
   Workspace ws;
   pkb::Refine rf;
   pkb::PaddedPlanes planes;
@@ -888,6 +890,84 @@ int pkb_batch_decode(pkb_batch_t *b, const pkb_fst_t *fst, float beam, int max_t
   PKB_CUDA(cudaMemcpyAsync(weight_out, d_wt, sizeof(float) * n, cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaStreamSynchronize(c->stream));
   return pkb::check_device_error(c, "pkb_batch_decode");
+}
+
+static_assert(sizeof(pkb_lattice_arc_t) == 28 && offsetof(pkb_lattice_arc_t, acoustic_cost) == 24,
+              "pkb_lattice_arc_t is 28 bytes without padding");
+
+int pkb_batch_lattice(pkb_batch_t *b, const pkb_fst_t *fst, float beam, float lattice_beam, int max_tokens,
+                      int max_arcs, int64_t *n_arcs_out, double *best_cost_out) {
+  PKB_REQUIRE(b && fst && n_arcs_out && best_cost_out, "pkb_batch_lattice: NULL argument");
+  PKB_REQUIRE(b->am, "pkb_batch_lattice: the batch has no model");
+  PKB_REQUIRE(!b->compact, "pkb_batch_lattice: reads the FP32 log-likelihoods (switch the compact output off)");
+  PKB_REQUIRE(lattice_beam > 0.0f, "pkb_batch_lattice: lattice_beam must be > 0 (got %g)", lattice_beam);
+  PKB_TRY(pkb::check_decode_graph(b->c, b->am, fst, "pkb_batch_lattice"));
+  Ctx *c = b->c;
+  PKB_CUDA(cudaSetDevice(c->device));
+  b->lat_total = 0;
+  const int n = b->meta.n_utts;
+  if (n == 0) return PKB_OK;
+  pkb::ViterbiConfig cfg;
+  if (beam > 0.0f) cfg.beam = beam;
+  if (max_tokens > 0) cfg.max_tokens = max_tokens;
+  pkb_am *am = b->am;
+  const size_t tid_bytes = am->tid2pdf.size() * sizeof(int32_t);
+  if (b->vit_tid2pdf.cap < tid_bytes) {
+    PKB_TRY(b->vit_tid2pdf.ensure(tid_bytes));
+    PKB_CUDA(cudaMemcpyAsync(b->vit_tid2pdf.p, am->tid2pdf.data(), tid_bytes, cudaMemcpyHostToDevice, c->stream));
+  }
+  int t_max = 0;
+  for (int u = 0; u < n; ++u) t_max = std::max(t_max, b->meta.num_frames[u]);
+  pkb::Lattice lat{};
+  // default: the most the search can log, every arc of the graph at every time of the longest
+  // utterance (1.84 M entries, 14.7 MB, for 10 s on the 40-word loop; 33 M, 267 MB, on the 180-word loop)
+  const int64_t bound = static_cast<int64_t>(t_max + 1) * std::max(fst->num_arcs, 1);
+  lat.max_arcs = max_arcs > 0 ? max_arcs : static_cast<int>(std::min<int64_t>(bound, INT32_MAX));
+  lat.grp_stride = 2 * (t_max + 1);
+  lat.beam = lattice_beam;
+  // per utterance: the log; group offsets; kept count, best cost and first output record
+  PKB_TRY(b->lat_log.ensure(static_cast<size_t>(n) * lat.max_arcs * sizeof(unsigned long long)));
+  const size_t grp_bytes = (static_cast<size_t>(n) * lat.grp_stride * sizeof(int) + 7) & ~static_cast<size_t>(7);
+  PKB_TRY(b->lat_aux.ensure(grp_bytes + 3 * sizeof(int64_t) * static_cast<size_t>(n)));
+  lat.log = b->lat_log.as<unsigned long long>();
+  lat.grp = b->lat_aux.as<int>();
+  lat.n_out = reinterpret_cast<long long *>(b->lat_aux.as<char>() + grp_bytes);
+  lat.best_out = reinterpret_cast<double *>(lat.n_out + n);
+  long long *d_first = lat.n_out + 2 * n;
+  PKB_TRY(pkb::launch_lattice(c, fst, cfg, b->loglik.as<float>(), am->num_pdfs, b->ws.pad_off.as<int64_t>(),
+                              b->meta.d_num_frames, n, b->vit_tid2pdf.as<int32_t>(), &b->vit_work, lat));
+  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
+  PKB_CUDA(cudaMemcpyAsync(n_arcs_out, lat.n_out, sizeof(int64_t) * n, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaMemcpyAsync(best_cost_out, lat.best_out, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  PKB_TRY(pkb::check_device_error(c, "pkb_batch_lattice"));
+  // the kept arcs as records, every utterance's back to back
+  std::vector<long long> first(n);
+  int64_t total = 0;
+  for (int u = 0; u < n; ++u) {
+    first[u] = total;
+    total += std::max<int64_t>(n_arcs_out[u], 0);
+  }
+  PKB_TRY(b->lat_arcs.ensure(std::max<int64_t>(total, 1) * sizeof(pkb_lattice_arc_t)));
+  PKB_CUDA(cudaMemcpyAsync(d_first, first.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, c->stream));
+  PKB_TRY(pkb::lattice_expand(c, fst, lat, b->loglik.as<float>(), am->num_pdfs, b->ws.pad_off.as<int64_t>(), n,
+                              b->vit_tid2pdf.as<int32_t>(), d_first, b->lat_arcs.as<pkb_lattice_arc_t>()));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  PKB_TRY(pkb::check_device_error(c, "pkb_batch_lattice"));
+  b->lat_total = total;
+  return PKB_OK;
+}
+
+int pkb_batch_lattice_get(pkb_batch_t *b, pkb_lattice_arc_t *arcs_out) {
+  PKB_REQUIRE(b, "pkb_batch_lattice_get: the batch is NULL");
+  PKB_REQUIRE(b->lat_total >= 0, "pkb_batch_lattice_get: no pkb_batch_lattice on this batch yet");
+  if (b->lat_total == 0) return PKB_OK;
+  PKB_REQUIRE(arcs_out, "pkb_batch_lattice_get: NULL argument");
+  PKB_CUDA(cudaSetDevice(b->c->device));
+  PKB_CUDA(cudaMemcpyAsync(arcs_out, b->lat_arcs.p, sizeof(pkb_lattice_arc_t) * b->lat_total,
+                           cudaMemcpyDeviceToHost, b->c->stream));
+  PKB_CUDA(cudaStreamSynchronize(b->c->stream));
+  return pkb::check_device_error(b->c, "pkb_batch_lattice_get");
 }
 
 // ---------------------------------------------------------------- fused host path

@@ -218,13 +218,205 @@ __device__ void carry_reset(const Carry &cr, int u) {
   }
 }
 
-template <int kVitGroup, bool kResume>
+// ---------------------------------------------------------------------------------------------
+// Lattice mode of the batch search (Lattice in decoder.cuh). Only the lattice instantiations
+// reference this block's shared state.
+constexpr int kLatScanMax = 16 * (kVitThreads / 32);  // flags per thread x warps of block_scan
+constexpr unsigned long long kKept = 1ull << 63;      // a log entry's mark (arc indices are < 2^31)
+
+struct LatShared {
+  int count;                    // log entries of the current utterance
+  int changed;
+  int cnt[kLatScanMax + 1];
+  unsigned long long best;      // ord64 of the best final cost
+};
+__device__ __forceinline__ LatShared &lat_shared() {
+  __shared__ LatShared s;
+  return s;
+}
+
+// Exclusive block-wide prefix count of K flags per thread, in the order (k, thread): pos[k] is the
+// number of set flags before flag k of this thread. Returns the total. Everyone must call it.
+template <int K>
+__device__ int block_scan(const bool (&flag)[K], int (&pos)[K]) {
+  int *cnt = lat_shared().cnt;
+  const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
+#pragma unroll
+  for (int k = 0; k < K; ++k) {
+    const unsigned m = __ballot_sync(0xffffffffu, flag[k]);
+    pos[k] = __popc(m & ((1u << lane) - 1u));
+    if (lane == 0) cnt[k * (kVitThreads / 32) + wp] = __popc(m);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int run = 0;
+    for (int i = 0; i < K * (kVitThreads / 32); ++i) { const int v = cnt[i]; cnt[i] = run; run += v; }
+    cnt[K * (kVitThreads / 32)] = run;
+  }
+  __syncthreads();
+#pragma unroll
+  for (int k = 0; k < K; ++k) pos[k] += cnt[k * (kVitThreads / 32) + wp];
+  const int total = cnt[K * (kVitThreads / 32)];
+  __syncthreads();
+  return total;
+}
+
+// Appends group g to the log in the order (k, thread), i.e. by arc index when arc k of a thread is
+// tid + 256 k: the arcs whose flag is set, with their source's cost. Everyone must call it.
+template <int K>
+__device__ void lat_append_ordered(const Lattice &lat, unsigned long long *lg, int *go, int g,
+                                   const bool (&flag)[K], const float (&src_cost)[K], int *err) {
+  LatShared &ls = lat_shared();
+  const int base = ls.count;
+  int pos[K];
+  const int total = block_scan<K>(flag, pos);
+#pragma unroll
+  for (int k = 0; k < K; ++k) {
+    const int r = base + pos[k];
+    if (flag[k] && r < lat.max_arcs)
+      lg[r] = (static_cast<unsigned long long>(threadIdx.x + k * kVitThreads) << 32) | __float_as_uint(src_cost[k]);
+  }
+  if (threadIdx.x == 0) {
+    go[g] = base;
+    ls.count = base + total;
+    if (base + total > lat.max_arcs && !*err) *err = 4;
+  }
+  __syncthreads();
+}
+
+// After a pass that appended with atomics: a log past max_arcs fails the utterance with 4, unless
+// the pass already failed it otherwise (the reported code does not depend on the order of atomics).
+__device__ __forceinline__ void lat_check_overflow(const Lattice &lat, int *err) {
+  if (threadIdx.x == 0 && !*err && lat_shared().count > lat.max_arcs) *err = 4;
+  __syncthreads();
+}
+
+// Sorts a[0, n) ascending: bitonic network whose comparators all put the minimum first, so that
+// the missing elements up to the next power of two act as +inf and are never touched.
+__device__ void block_sort(unsigned long long *a, int n) {
+  int P = 1;
+  while (P < n) P <<= 1;
+  for (int k = 2; k <= P; k <<= 1) {
+    for (int j = k >> 1; j >= 1; j >>= 1) {
+      for (int idx = threadIdx.x; idx < P / 2; idx += kVitThreads) {
+        const int i = (idx / j) * 2 * j + idx % j;
+        const int l = j == (k >> 1) ? (i ^ (k - 1)) : i + j;
+        if (l < n) {
+          const unsigned long long x = a[i], y = a[l];
+          if (x > y) { a[i] = y; a[l] = x; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// Backward pass over utterance u's log once its search is complete, with `best` finite:
+//   beta(T, s) = final(s); beta(t, s) = min over logged arcs leaving (t, s) of
+//   (w + ac) + beta(head), epsilon arcs of a time relaxed to a fixpoint (also at T);
+//   an arc is kept when beta(head) is finite and ((alpha(tail) + w) + ac) + beta(head) <= best + beam,
+// all in double, ac re-read from the row. `beta` keeps two times, b = t & 1: reset(b), get(b, s)
+// (+inf when absent) and relax(b, s, v) (min; true when it lowered the value). The kept arcs are
+// then moved to the front of the log as (group << 32 | arc) and, unless the log was written in
+// arc order, sorted. Returns the kept count.
+template <class Reset, class Get, class Relax>
+__device__ int lattice_prune(const FstDev &fst, const Lattice &lat, unsigned long long *lg, const int *go, int T,
+                             const float *ll0, int num_pdfs, const int32_t *tid2pdf, double best, bool sort,
+                             int *err, Reset reset, Get get, Relax relax) {
+  LatShared &ls = lat_shared();
+  const int tid = threadIdx.x;
+  const double bound = best + static_cast<double>(lat.beam);
+  auto beta = [&](int b, int s, bool at_end) {
+    const double v = get(b, s);
+    return at_end ? fmin(v, static_cast<double>(__ldg(&fst.final_w[s]))) : v;
+  };
+  for (int t = T; t >= 0; --t) {
+    const int b = t & 1;
+    const bool end = t == T;
+    reset(b);
+    if (!end) {
+      // emitting arcs from t to t + 1
+      const float *ll = ll0 + static_cast<int64_t>(t) * num_pdfs;
+      for (int i = go[2 * t + 1] + tid; i < go[2 * t + 2]; i += kVitThreads) {
+        const unsigned long long e = lg[i];
+        const int a = static_cast<int>(e >> 32);
+        const double bh = beta(b ^ 1, __ldg(&fst.arc_dst[a]), t + 1 == T);
+        if (bh == INFINITY) continue;
+        const double w = static_cast<double>(__ldg(&fst.arc_w[a]));
+        const double ac = static_cast<double>(-__ldg(&ll[__ldg(&tid2pdf[__ldg(&fst.arc_il[a])])]));
+        relax(b, __ldg(&fst.arc_src[a]), (w + ac) + bh);
+        if (((static_cast<double>(__uint_as_float(static_cast<uint32_t>(e))) + w) + ac) + bh <= bound)
+          lg[i] = e | kKept;
+      }
+      __syncthreads();
+    }
+    // epsilon arcs within t
+    const int p0 = go[2 * t], p1 = go[2 * t + 1];
+    if (p1 > p0) {
+      for (int round = 0;; ++round) {
+        if (tid == 0) ls.changed = 0;
+        __syncthreads();
+        for (int i = p0 + tid; i < p1; i += kVitThreads) {
+          const int a = static_cast<int>(lg[i] >> 32);
+          const double bh = beta(b, __ldg(&fst.arc_dst[a]), end);
+          if (bh != INFINITY && relax(b, __ldg(&fst.arc_src[a]), static_cast<double>(__ldg(&fst.arc_w[a])) + bh))
+            ls.changed = 1;
+        }
+        __syncthreads();
+        const int changed = ls.changed;
+        __syncthreads();
+        if (!changed) break;
+        if (round == 4096) {
+          if (tid == 0) *err = 3;
+          __syncthreads();
+          return 0;
+        }
+      }
+      for (int i = p0 + tid; i < p1; i += kVitThreads) {
+        const unsigned long long e = lg[i];
+        const int a = static_cast<int>(e >> 32);
+        const double bh = beta(b, __ldg(&fst.arc_dst[a]), end);
+        const double w = static_cast<double>(__ldg(&fst.arc_w[a]));
+        if (bh != INFINITY && ((static_cast<double>(__uint_as_float(static_cast<uint32_t>(e))) + w) + 0.0) + bh <= bound)
+          lg[i] = e | kKept;
+      }
+      __syncthreads();
+    }
+    if (*err) return 0;
+  }
+  // kept arcs to the front, in order (a write never passes a read of a later block of entries)
+  const int n_log = go[2 * T + 1];
+  int kept = 0;
+  for (int b0 = 0; b0 < n_log; b0 += kVitThreads) {
+    const int r = b0 + tid;
+    const unsigned long long e = r < n_log ? lg[r] : 0ull;
+    bool keep[1] = {(e & kKept) != 0};
+    int pos[1];
+    unsigned long long key = 0;
+    if (keep[0]) {
+      int lo = 0, hi = 2 * T + 1;  // the last group that starts at or before r
+      while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (go[mid] <= r) lo = mid; else hi = mid - 1;
+      }
+      key = (static_cast<unsigned long long>(lo) << 32) | ((e >> 32) & 0x7fffffffull);
+    }
+    const int total = block_scan<1>(keep, pos);
+    if (keep[0]) lg[kept + pos[0]] = key;
+    kept += total;
+    __syncthreads();
+  }
+  if (sort) block_sort(lg, kept);
+  return kept;
+}
+
+template <int kVitGroup, bool kResume, bool kLattice>
 __global__ void __launch_bounds__(kVitThreads)
 viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, int max_words,
                const float *__restrict__ loglik, int num_pdfs, const int64_t *__restrict__ row_off,
                const int32_t *__restrict__ num_frames, int n_utts, const int32_t *__restrict__ tid2pdf,
                char *work_base, size_t work_stride, int tables_in_smem, int32_t *__restrict__ words_out,
-               int32_t *__restrict__ n_words_out, float *__restrict__ weight_out, Carry cr) {
+               int32_t *__restrict__ n_words_out, float *__restrict__ weight_out, Carry cr, Lattice lat) {
   __shared__ int s_ntok[2], s_nfront[2], s_log, s_err, s_unres;
   __shared__ unsigned long long s_min;
 
@@ -371,11 +563,40 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
     __syncthreads();
   };
 
+  // lattice mode: group g of the log, the epsilon arcs of table c's final tokens under `cutoff`
+  // (the closure's bound), in token-list order; lattice_prune sorts the kept ones
+  auto lat_log_eps = [&](unsigned long long *lg, int *go, int c, int g, double cutoff) {
+    LatShared &ls = lat_shared();
+    if (tid == 0) go[g] = ls.count;
+    __syncthreads();
+    if (fst.has_eps) {
+      const Tab &tc = w.tab[c];
+      const int n = min(s_ntok[c], max_tok);
+      for (int i = grp; i < n; i += kVitGroups) {
+        const int slot = tc.list[i];
+        const float cost = cost_of(tc.vals[slot]);
+        const int state = tc.keys[slot] - 1;
+        const int a1 = __ldg(&fst.arc_begin[state + 1]);
+        for (int a = __ldg(&fst.arc_begin[state]) + gl; a < a1; a += kVitGroup) {
+          if (__ldg(&fst.arc_il[a]) != 0) continue;
+          if (static_cast<double>(cost) + static_cast<double>(__ldg(&fst.arc_w[a])) > cutoff) continue;
+          const int r = atomicAdd(&ls.count, 1);
+          if (r < lat.max_arcs) lg[r] = (static_cast<unsigned long long>(a) << 32) | __float_as_uint(cost);
+        }
+      }
+    }
+    __syncthreads();
+    lat_check_overflow(lat, &s_err);
+  };
+
   for (int u = blockIdx.x; u < n_utts; u += gridDim.x) {
     const int T = kResume ? (cr.finish ? 0 : num_frames ? num_frames[u] : cr.uniform_frames) : num_frames[u];
     const float *ll0 = loglik + (kResume ? static_cast<int64_t>(u) * cr.frame_stride : row_off[u]) * num_pdfs;
     const int *hdr = kResume ? cr.hdr + 4 * u : nullptr;
     const bool fresh = !kResume || hdr[0] < 0;
+    unsigned long long *lg = kLattice ? lat.log + static_cast<size_t>(u) * lat.max_arcs : nullptr;
+    int *go = kLattice ? lat.grp + static_cast<size_t>(u) * lat.grp_stride : nullptr;
+    if (kLattice && tid == 0) lat_shared().count = 0;
     if (tid == 0) { s_ntok[0] = s_ntok[1] = 0; s_log = fresh ? 0 : hdr[1]; s_err = fresh ? 0 : hdr[2]; }
     __syncthreads();
     int cur = 0;
@@ -387,6 +608,7 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
       }
       __syncthreads();
       close_and_resolve(0, 1, INFINITY);
+      if (kLattice && !s_err) lat_log_eps(lg, go, 0, 0, INFINITY);
     } else {
       // ---- the carried tokens of the previous advance
       const int n = hdr[2] ? 0 : hdr[0];
@@ -447,6 +669,10 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
       __syncthreads();
       if (s_min == ~0ull) { alive = false; break; }  // no arc left the beam: the reference has no tokens either
       const double next_cutoff = unord64(s_min) + static_cast<double>(beam);
+      if (kLattice) {
+        if (tid == 0) go[2 * f + 1] = lat_shared().count;
+        __syncthreads();
+      }
       // ---- pass 2: create / improve the tokens of this frame
       for (int i = grp; i < n_prev; i += kVitGroups) {
         const int slot = tp.list[i];
@@ -462,14 +688,20 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
           const double total = static_cast<double>(cost) + static_cast<double>(__ldg(&fst.arc_w[a])) +
                                static_cast<double>(ac);
           if (total > next_cutoff) continue;
+          if (kLattice) {
+            const int r = atomicAdd(&lat_shared().count, 1);
+            if (r < lat.max_arcs) lg[r] = (static_cast<unsigned long long>(a) << 32) | __float_as_uint(cost);
+          }
           const int s2 = tab_insert(tc, __ldg(&fst.arc_dst[a]), mask, &s_ntok[cur], max_tok);
           if (s2 < 0) { s_err = 1; continue; }
           atomicMin(&tc.vals[s2], pack(static_cast<float>(total), static_cast<uint32_t>(a)));
         }
       }
       __syncthreads();
+      if (kLattice) lat_check_overflow(lat, &s_err);
       // ProcessEmitting returns the bound as a float (src/decoder.cc:240)
       if (!s_err) close_and_resolve(cur, prev, static_cast<double>(static_cast<float>(next_cutoff)));
+      if (kLattice && !s_err) lat_log_eps(lg, go, cur, 2 * (f + 1), static_cast<double>(static_cast<float>(next_cutoff)));
       clear_tab(prev);
     }
 
@@ -485,6 +717,20 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
       }
       __syncthreads();
       carry_end_advance(cr, u, n, T, w.log_prev, w.log_ol, mark, max_log, max_words, s_log, s_err, alive);
+    } else if (kLattice) {
+      // best complete path: min over the final tokens of double(alpha) + double(final)
+      LatShared &ls = lat_shared();
+      if (tid == 0) { ls.best = ~0ull; go[2 * T + 1] = ls.count; }
+      __syncthreads();
+      const Tab &tb = w.tab[cur];
+      const int n = (alive && !s_err) ? min(s_ntok[cur], max_tok) : 0;
+      for (int i = tid; i < n; i += kVitThreads) {
+        const int slot = tb.list[i];
+        const double c = static_cast<double>(cost_of(tb.vals[slot])) +
+                         static_cast<double>(fst.final_w[tb.keys[slot] - 1]);
+        if (c != INFINITY) atomicMin(&ls.best, ord64(c));
+      }
+      __syncthreads();
     } else {
     // ---- BestPath (src/decoder.cc:300-339)
     if (tid == 0) s_min = ~0ull;
@@ -539,6 +785,44 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
       clear_tab(0);
       clear_tab(1);
     }
+    if (kLattice) {
+      // backward pass with beta keyed by state in the two (clean) token tables
+      const unsigned long long bst = lat_shared().best;
+      const double best = bst == ~0ull ? INFINITY : unord64(bst);
+      int kept = 0;
+      if (!s_err && best != INFINITY) {
+        auto reset = [&](int b) { clear_tab(b); };
+        auto get = [&](int b, int s) -> double {
+          const int sl = tab_find(w.tab[b], s, mask);
+          if (sl < 0) return INFINITY;
+          const unsigned long long v = *reinterpret_cast<volatile unsigned long long *>(&w.tab[b].vals[sl]);
+          return v == kEmptyVal ? INFINITY : unord64(v);
+        };
+        auto relax = [&](int b, int s, double v) -> bool {
+          const int sl = tab_insert(w.tab[b], s, mask, &s_ntok[b], max_tok);
+          if (sl < 0) { s_err = 1; return false; }
+          const unsigned long long o = ord64(v);
+          return atomicMin(&w.tab[b].vals[sl], o) > o;
+        };
+        kept = lattice_prune(fst, lat, lg, go, T, ll0, num_pdfs, tid2pdf, best, true, &s_err, reset, get, relax);
+        if (s_err) {
+          // an overflowing insert leaves a claimed slot in no list
+          for (uint32_t i = tid; i < H; i += kVitThreads)
+            for (int k = 0; k < 2; ++k) { w.tab[k].keys[i] = 0; w.tab[k].vals[i] = kEmptyVal; }
+          __syncthreads();
+          if (tid == 0) s_ntok[0] = s_ntok[1] = 0;
+          __syncthreads();
+        } else {
+          clear_tab(0);
+          clear_tab(1);
+        }
+      }
+      if (tid == 0) {
+        lat.n_out[u] = s_err ? -s_err : kept;
+        lat.best_out[u] = s_err ? INFINITY : best;
+      }
+      __syncthreads();
+    }
   }
 }
 
@@ -553,13 +837,13 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
 //   bp[s]    newest word record of the token
 constexpr uint32_t kInactive = 0xffffffffu;
 
-template <int kArcsPerThread, bool kResume>
+template <int kArcsPerThread, bool kResume, bool kLattice>
 __global__ void __launch_bounds__(kVitThreads, kArcsPerThread <= 8 ? 3 : 1)
 viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_words,
                      const float *__restrict__ loglik, int num_pdfs, const int64_t *__restrict__ row_off,
                      const int32_t *__restrict__ num_frames, int n_utts, const int32_t *__restrict__ tid2pdf,
                      char *work_base, size_t work_stride, int32_t *__restrict__ words_out,
-                     int32_t *__restrict__ n_words_out, float *__restrict__ weight_out, Carry cr) {
+                     int32_t *__restrict__ n_words_out, float *__restrict__ weight_out, Carry cr, Lattice lat) {
   extern __shared__ __align__(16) char s_dense[];
   __shared__ int s_log, s_err, s_unres, s_changed;
   __shared__ unsigned long long s_min;
@@ -739,16 +1023,36 @@ viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_
     __syncthreads();
   };
 
+  // lattice mode: group g of the log, the emitting arcs still live after pass 2 (source costs in
+  // table p) or the epsilon arcs of table c's final tokens under `cutoff`, in arc order
+  auto lat_log = [&](unsigned long long *lg, int *go, int g, int tab, bool emitting, double cutoff,
+                     const bool (&live)[kArcsPerThread]) {
+    bool flag[kArcsPerThread];
+    float alpha[kArcsPerThread];
+#pragma unroll
+    for (int k = 0; k < kArcsPerThread; ++k) {
+      const uint32_t cs = has_arc(k) ? cost[tab][src_of(k)] : kInactive;
+      alpha[k] = unord32(cs);
+      if (emitting) flag[k] = live[k];
+      else flag[k] = fst.has_eps && has_arc(k) && a_pdf[k] < 0 && cs != kInactive &&
+                     static_cast<double>(alpha[k]) + static_cast<double>(a_w[k]) <= cutoff;
+    }
+    lat_append_ordered<kArcsPerThread>(lat, lg, go, g, flag, alpha, &s_err);
+  };
+
   for (int u = blockIdx.x; u < n_utts; u += gridDim.x) {
     const int T = kResume ? (cr.finish ? 0 : num_frames ? num_frames[u] : cr.uniform_frames) : num_frames[u];
     const float *ll0 = loglik + (kResume ? static_cast<int64_t>(u) * cr.frame_stride : row_off[u]) * num_pdfs;
     const int *hdr = kResume ? cr.hdr + 4 * u : nullptr;
     const bool fresh = !kResume || hdr[0] < 0;
+    unsigned long long *lg = kLattice ? lat.log + static_cast<size_t>(u) * lat.max_arcs : nullptr;
+    int *go = kLattice ? lat.grp + static_cast<size_t>(u) * lat.grp_stride : nullptr;
     for (int s = tid; s < S; s += kVitThreads) {
       cost[0][s] = cost[1][s] = kInactive;
       warc[0][s] = warc[1][s] = kInactive;
       bp[0][s] = bp[1][s] = -1;
     }
+    if (kLattice && tid == 0) lat_shared().count = 0;
     if (tid == 0) { s_log = fresh ? 0 : hdr[1]; s_err = fresh ? 0 : hdr[2]; }
     __syncthreads();
     int cur = 0;
@@ -773,6 +1077,7 @@ viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_
 #pragma unroll
       for (int k = 0; k < kArcsPerThread; ++k) { td[k] = 0.0; live[k] = false; }
       finish_frame(0, 1, INFINITY, td, live);
+      if (kLattice) lat_log(lg, go, 0, 0, false, INFINITY, live);
     }
     end_frame(0, 1);
     bool alive = fresh || hdr[3] != 0;
@@ -825,7 +1130,9 @@ viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_
         if (live[k]) atomicMin(&cost[cur][dst_of(k)], ord32(static_cast<float>(td[k])));
       }
       __syncthreads();
+      if (kLattice) lat_log(lg, go, 2 * f + 1, prev, true, 0.0, live);
       finish_frame(cur, prev, static_cast<double>(static_cast<float>(next_cutoff)), td, live);
+      if (kLattice) lat_log(lg, go, 2 * (f + 1), cur, false, static_cast<double>(static_cast<float>(next_cutoff)), live);
       {
         float *ll_nx = s_ll + ((f + 1) & 1) * Dmax;  // last read two frames ago
 #pragma unroll
@@ -854,6 +1161,44 @@ viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_
       __syncthreads();
       carry_end_advance(cr, u, s_nsave, T, log_prev, log_ol, log_ol + max_log, max_log, max_words, s_log, s_err,
                         alive);
+      continue;
+    }
+    if (kLattice) {
+      // best complete path: min over the final tokens of double(alpha) + double(final)
+      LatShared &ls = lat_shared();
+      if (tid == 0) { ls.best = ~0ull; go[2 * T + 1] = ls.count; }
+      __syncthreads();
+      if (alive && !s_err)
+        for (int s = tid; s < S; s += kVitThreads) {
+          if (cost[cur][s] == kInactive) continue;
+          const double c = static_cast<double>(unord32(cost[cur][s])) + static_cast<double>(fst.final_w[s]);
+          if (c != INFINITY) atomicMin(&ls.best, ord64(c));
+        }
+      __syncthreads();
+      const double best = ls.best == ~0ull ? INFINITY : unord64(ls.best);
+      int kept = 0;
+      if (alive && !s_err && best != INFINITY) {
+        // backward pass with beta in the cost / warc arrays the search is done with: 2 S doubles
+        unsigned long long *bt = reinterpret_cast<unsigned long long *>(s_dense);
+        auto reset = [&](int b) {
+          for (int s = tid; s < S; s += kVitThreads) bt[b * S + s] = kEmptyVal;
+          __syncthreads();
+        };
+        auto get = [&](int b, int s) -> double {
+          const unsigned long long v = *reinterpret_cast<volatile unsigned long long *>(&bt[b * S + s]);
+          return v == kEmptyVal ? INFINITY : unord64(v);
+        };
+        auto relax = [&](int b, int s, double v) -> bool {
+          const unsigned long long o = ord64(v);
+          return atomicMin(&bt[b * S + s], o) > o;
+        };
+        kept = lattice_prune(fst, lat, lg, go, T, ll0, num_pdfs, tid2pdf, best, false, &s_err, reset, get, relax);
+      }
+      if (tid == 0) {
+        lat.n_out[u] = s_err ? -s_err : kept;
+        lat.best_out[u] = s_err ? INFINITY : best;
+      }
+      __syncthreads();
       continue;
     }
     // ---- BestPath (src/decoder.cc:300-339)
@@ -892,6 +1237,31 @@ viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_
     }
     if (kResume) carry_reset(cr, u);
     __syncthreads();
+  }
+}
+
+// The kept arcs of utterance u (lattice_prune's keys) as records from out + first[u] on.
+__global__ void __launch_bounds__(kVitThreads)
+lattice_expand_kernel(FstDev fst, Lattice lat, const float *__restrict__ loglik, int num_pdfs,
+                      const int64_t *__restrict__ row_off, const int32_t *__restrict__ tid2pdf,
+                      const long long *__restrict__ first, pkb_lattice_arc_t *__restrict__ out) {
+  const int u = blockIdx.x;
+  const long long n = lat.n_out[u];
+  const unsigned long long *lg = lat.log + static_cast<size_t>(u) * lat.max_arcs;
+  pkb_lattice_arc_t *o = out + first[u];
+  for (long long i = threadIdx.x; i < n; i += kVitThreads) {
+    const unsigned long long key = lg[i];
+    const int t = static_cast<int>(key >> 33), a = static_cast<int>(key & 0xffffffffull);
+    const int il = __ldg(&fst.arc_il[a]);
+    pkb_lattice_arc_t r;
+    r.t = t;
+    r.src = __ldg(&fst.arc_src[a]);
+    r.dst = __ldg(&fst.arc_dst[a]);
+    r.ilabel = il;
+    r.olabel = __ldg(&fst.arc_ol[a]);
+    r.graph_cost = __ldg(&fst.arc_w[a]);
+    r.acoustic_cost = il ? -__ldg(&loglik[(row_off[u] + t) * num_pdfs + __ldg(&tid2pdf[il])]) : 0.0f;
+    o[i] = r;
   }
 }
 
@@ -1042,21 +1412,21 @@ int init_workspace(Ctx *c, const VitPlan &p, DevBuf *work) {
   return PKB_OK;
 }
 
-template <bool kResume>
+template <bool kResume, bool kLattice>
 int launch_plan(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfig &cfg, const float *d_loglik,
                 int num_pdfs, const int64_t *d_row_off, const int32_t *d_num_frames, int n_utts,
                 const int32_t *d_tid2pdf, DevBuf *work, int32_t *d_words, int32_t *d_n_words, float *d_weight,
-                const Carry &cr) {
+                const Carry &cr, const Lattice &lat) {
   const FstDev fd = fst_dev(fst);
   LaunchScope scope(c, PKB_KERNEL_MISC);
 #define PKB_VIT_DENSE(APT)                                                                                   \
   do {                                                                                                       \
     if (p.smem > 48 * 1024)                                                                                  \
-      PKB_CUDA(cudaFuncSetAttribute(viterbi_dense_kernel<APT, kResume>,                                      \
+      PKB_CUDA(cudaFuncSetAttribute(viterbi_dense_kernel<APT, kResume, kLattice>,                            \
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(p.smem))); \
-    viterbi_dense_kernel<APT, kResume><<<p.grid, kVitThreads, p.smem, c->stream>>>(                          \
+    viterbi_dense_kernel<APT, kResume, kLattice><<<p.grid, kVitThreads, p.smem, c->stream>>>(                \
         fd, fst->num_arcs, cfg.beam, cfg.max_log, cfg.max_words, d_loglik, num_pdfs, d_row_off,              \
-        d_num_frames, n_utts, d_tid2pdf, work->as<char>(), p.stride, d_words, d_n_words, d_weight, cr);      \
+        d_num_frames, n_utts, d_tid2pdf, work->as<char>(), p.stride, d_words, d_n_words, d_weight, cr, lat); \
   } while (0)
   // (staging each frame's log-likelihood row in shared memory with cp.async was measured slower in
   // the table kernel, 44 vs 26 ms for 128 utterances: the larger carve-out takes the L1 space that
@@ -1064,12 +1434,12 @@ int launch_plan(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfi
 #define PKB_VIT_LAUNCH(G)                                                                                    \
   do {                                                                                                       \
     if (p.smem > 48 * 1024)                                                                                  \
-      PKB_CUDA(cudaFuncSetAttribute(viterbi_kernel<G, kResume>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                    static_cast<int>(p.smem)));                                              \
-    viterbi_kernel<G, kResume><<<p.grid, kVitThreads, p.smem, c->stream>>>(                                  \
+      PKB_CUDA(cudaFuncSetAttribute(viterbi_kernel<G, kResume, kLattice>,                                    \
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(p.smem))); \
+    viterbi_kernel<G, kResume, kLattice><<<p.grid, kVitThreads, p.smem, c->stream>>>(                        \
         fd, cfg.beam, p.max_tok, p.H - 1, cfg.max_log, cfg.max_words, d_loglik, num_pdfs, d_row_off,         \
         d_num_frames, n_utts, d_tid2pdf, work->as<char>(), p.stride, p.small ? 1 : 0, d_words, d_n_words,    \
-        d_weight, cr);                                                                                       \
+        d_weight, cr, lat);                                                                                  \
   } while (0)
   if (p.dense) {
     if (p.variant == 4) PKB_VIT_DENSE(4);
@@ -1098,8 +1468,32 @@ int launch_viterbi(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const f
   const VitPlan p = plan_viterbi(c, fst, cfg, num_pdfs, n_utts, false);
   PKB_TRY(work->ensure(p.stride * p.grid));
   if (!p.dense && !p.small) PKB_TRY(init_workspace(c, p, work));
-  return launch_plan<false>(c, fst, p, cfg, d_loglik, num_pdfs, d_row_off, d_num_frames, n_utts, d_tid2pdf, work,
-                            d_words, d_n_words, d_weight, Carry{});
+  return launch_plan<false, false>(c, fst, p, cfg, d_loglik, num_pdfs, d_row_off, d_num_frames, n_utts, d_tid2pdf,
+                                   work, d_words, d_n_words, d_weight, Carry{}, Lattice{});
+}
+
+int launch_lattice(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const float *d_loglik, int num_pdfs,
+                   const int64_t *d_row_off, const int32_t *d_num_frames, int n_utts, const int32_t *d_tid2pdf,
+                   DevBuf *work, const Lattice &lat) {
+  if (n_utts == 0) return PKB_OK;
+  PKB_REQUIRE(cfg.max_tokens >= 16 && cfg.max_log >= 16 && cfg.beam > 0.0f && lat.max_arcs > 0 && lat.beam > 0.0f,
+              "pkb_batch_lattice: bad configuration");
+  const VitPlan p = plan_viterbi(c, fst, cfg, num_pdfs, n_utts, false);
+  PKB_TRY(work->ensure(p.stride * p.grid));
+  if (!p.dense && !p.small) PKB_TRY(init_workspace(c, p, work));
+  return launch_plan<false, true>(c, fst, p, cfg, d_loglik, num_pdfs, d_row_off, d_num_frames, n_utts, d_tid2pdf,
+                                  work, nullptr, nullptr, nullptr, Carry{}, lat);
+}
+
+int lattice_expand(Ctx *c, const pkb_fst *fst, const Lattice &lat, const float *d_loglik, int num_pdfs,
+                   const int64_t *d_row_off, int n_utts, const int32_t *d_tid2pdf, const long long *d_first,
+                   pkb_lattice_arc_t *d_out) {
+  if (n_utts == 0) return PKB_OK;
+  LaunchScope scope(c, PKB_KERNEL_MISC);
+  lattice_expand_kernel<<<n_utts, kVitThreads, 0, c->stream>>>(fst_dev(fst), lat, d_loglik, num_pdfs, d_row_off,
+                                                               d_tid2pdf, d_first, d_out);
+  PKB_CUDA(cudaGetLastError());
+  return PKB_OK;
 }
 
 int ResumableSearch::setup(Ctx *ctx, const pkb_fst *graph, const ViterbiConfig &config, const int32_t *tid2pdf,
@@ -1150,15 +1544,15 @@ int ResumableSearch::advance(const float *d_loglik, int frame_stride, const int3
   Carry a = cr;
   a.frame_stride = frame_stride;
   a.uniform_frames = uniform_frames;
-  return launch_plan<true>(c, fst, plan, cfg, d_loglik, num_pdfs, nullptr, d_n_frames, n,
-                           d_tid2pdf.as<int32_t>(), &work, nullptr, nullptr, nullptr, a);
+  return launch_plan<true, false>(c, fst, plan, cfg, d_loglik, num_pdfs, nullptr, d_n_frames, n,
+                                  d_tid2pdf.as<int32_t>(), &work, nullptr, nullptr, nullptr, a, Lattice{});
 }
 
 int ResumableSearch::finish() {
   Carry a = cr;
   a.finish = 1;
-  return launch_plan<true>(c, fst, plan, cfg, nullptr, num_pdfs, nullptr, nullptr, n, d_tid2pdf.as<int32_t>(),
-                           &work, f_words, f_nw, f_weight, a);
+  return launch_plan<true, false>(c, fst, plan, cfg, nullptr, num_pdfs, nullptr, nullptr, n,
+                                  d_tid2pdf.as<int32_t>(), &work, f_words, f_nw, f_weight, a, Lattice{});
 }
 
 }  // namespace pkb

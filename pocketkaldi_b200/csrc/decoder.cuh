@@ -69,6 +69,20 @@ struct Carry {
   float *p_cost;
 };
 
+// Lattice output of the batch search (pkb_batch_lattice). Utterance u logs every arc the search
+// relaxed under its bounds as (arc << 32 | float bits of the tail's cost) at log + u * max_arcs, in
+// the groups eps(0), emit(0), eps(1), ..., whose start offsets go to grp + u * grp_stride
+// (2 (T + 1) ints; grp[2T + 1] is the log's length). After the last frame the block runs the
+// backward pass and leaves the kept arcs at the start of its log as (group << 32 | arc), in order.
+struct Lattice {
+  unsigned long long *log;
+  int *grp;
+  long long *n_out;    // [n] kept arcs, or -(error code)
+  double *best_out;    // [n] min over final nodes of double(alpha) + double(final)
+  int max_arcs, grp_stride;
+  float beam;          // lattice beam
+};
+
 // Decodes n_utts utterances. loglik: [rows][num_pdfs] scaled log-likelihoods where utterance u owns
 // rows [row_off[u], row_off[u] + num_frames[u]). tid2pdf: device map of input labels.
 // words_out [n_utts][max_words] in spoken order, n_words_out[u] (-1: the search failed: token or
@@ -77,6 +91,16 @@ int launch_viterbi(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const f
                    int num_pdfs, const int64_t *d_row_off, const int32_t *d_num_frames, int n_utts,
                    const int32_t *d_tid2pdf, int n_tids, DevBuf *work, int32_t *d_words,
                    int32_t *d_n_words, float *d_weight);
+
+// The search of launch_viterbi in lattice mode: per utterance lat.n_out / lat.best_out and the kept
+// arcs in lat.log (see Lattice). lattice_expand then writes utterance u's kept arcs as records from
+// out + first[u] on.
+int launch_lattice(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const float *d_loglik, int num_pdfs,
+                   const int64_t *d_row_off, const int32_t *d_num_frames, int n_utts, const int32_t *d_tid2pdf,
+                   DevBuf *work, const Lattice &lat);
+int lattice_expand(Ctx *c, const pkb_fst *fst, const Lattice &lat, const float *d_loglik, int num_pdfs,
+                   const int64_t *d_row_off, int n_utts, const int32_t *d_tid2pdf, const long long *d_first,
+                   pkb_lattice_arc_t *d_out);
 
 // The resumable search behind pkb_decoder: n streams, one thread block each, whose tokens and word
 // records stay in global memory between launches. advance() decodes the next rows of every stream
