@@ -335,6 +335,28 @@ int pkb_decoder_partial(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words
 /* BestPath of every stream as pkb_batch_decode returns it, then a fresh utterance (InitDecoding).
  * Synchronous. */
 int pkb_decoder_finish(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words_out, float *weight_out);
+/* Lattices of the online search: with lattice_beam > 0 (may be +inf) every pkb_decoder_finish also
+ * leaves each stream's lattice on the device, bit-identical to pkb_batch_lattice over the same rows
+ * with the same beam, lattice_beam and max_tokens, however the rows were split across advances or
+ * pushes; words, weights and partials stay exactly those of a decoder without lattices. Each
+ * advance copies its rows into a per-stream store for the backward pass of the finish.
+ * max_frames (<= 0: 6000, 60 s): frames per utterance and stream the store keeps; max_arcs: log
+ * entries per stream as in pkb_batch_lattice (<= 0: (max_frames + 1) x arcs of the graph; at most
+ * INT32_MAX - arcs of the graph, the default capped there). Device
+ * memory per stream: 8 max_arcs + 4 max_frames x num_pdfs bytes. lattice_beam = 0 switches lattices
+ * off and frees the buffers; negative or NaN is rejected. Only between utterances (after create or
+ * pkb_decoder_finish); an attached stream captures its CUDA graphs again. A failed allocation
+ * leaves the decoder working without lattices. */
+int pkb_decoder_set_lattice(pkb_decoder_t *dec, float lattice_beam, int max_frames, int max_arcs);
+/* Per stream, for the latest finish: kept arcs or a negative code (those of pkb_batch_lattice, and
+ * -5 more than max_frames frames; a lattice error fails only that stream's lattice) and the best
+ * cost. Valid until the next advance, push or flush; rejected after one, or when the latest finish
+ * ran without lattices. If the finish could not expand the lattices into records (their device
+ * buffer could not be allocated), the finish still succeeds with its words and this call is
+ * rejected with the reason. */
+int pkb_decoder_lattice(pkb_decoder_t *dec, int64_t *n_arcs_out, double *best_cost_out);
+/* The arcs of the latest finish, every stream's back to back in stream order (same validity). */
+int pkb_decoder_lattice_get(pkb_decoder_t *dec, pkb_lattice_arc_t *arcs_out);
 
 /* Sum over all elements of a per-frame float buffer, computed on the device
  * in double (a cheap whole-output fingerprint for full-size runs). */

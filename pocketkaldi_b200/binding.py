@@ -114,6 +114,9 @@ _SIGNATURES = [
     ("pkb_decoder_advance", C.c_int, [_VP, _VP, C.c_int, _VP]),
     ("pkb_decoder_partial", C.c_int, [_VP, _VP, _VP, _VP, _VP]),
     ("pkb_decoder_finish", C.c_int, [_VP, _VP, _VP, _VP]),
+    ("pkb_decoder_set_lattice", C.c_int, [_VP, C.c_float, C.c_int, C.c_int]),
+    ("pkb_decoder_lattice", C.c_int, [_VP, _VP, _VP]),
+    ("pkb_decoder_lattice_get", C.c_int, [_VP, _VP]),
     ("pkb_loglik16_expand", C.c_int, [_VP, _VP, C.c_int64, C.c_int, C.c_float, _VP]),
     ("pkb_stream_create", C.c_int, [_VP, _VP, C.c_int, C.c_int, _f32p, C.c_float, C.POINTER(_VP)]),
     ("pkb_stream_destroy", None, [_VP]),
@@ -823,6 +826,24 @@ class Decoder:
         wt = np.zeros(self.n_streams, np.float32)
         _check(self.ctx.lib.pkb_decoder_finish(self.h, words.ctypes.data, nw.ctypes.data, wt.ctypes.data))
         return _hyps(words, nw, self.max_words), wt
+
+    def set_lattice(self, lattice_beam=8.0, max_frames=0, max_arcs=0):
+        """Every finish() also keeps each stream's lattice pruned to lattice_beam, equal to
+        Batch.lattice over the same rows (pkb_decoder_set_lattice); 0 switches lattices off. Only
+        between utterances."""
+        _check(self.ctx.lib.pkb_decoder_set_lattice(self.h, lattice_beam, max_frames, max_arcs))
+
+    def lattice(self):
+        """The lattices of the latest finish(): ([LATTICE_ARC_DTYPE array per stream, None where it
+        failed], best costs as float64), as Batch.lattice returns them."""
+        na = np.zeros(self.n_streams, np.int64)
+        best = np.zeros(self.n_streams, np.float64)
+        _check(self.ctx.lib.pkb_decoder_lattice(self.h, na.ctypes.data, best.ctypes.data))
+        kept = np.maximum(na, 0)
+        arcs = np.empty(max(int(kept.sum()), 1), LATTICE_ARC_DTYPE)
+        _check(self.ctx.lib.pkb_decoder_lattice_get(self.h, arcs.ctypes.data))
+        off = np.concatenate([[0], np.cumsum(kept)])
+        return [None if na[s] < 0 else arcs[off[s]:off[s + 1]].copy() for s in range(self.n_streams)], best
 
 
 class Stream:

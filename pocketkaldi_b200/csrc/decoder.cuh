@@ -6,6 +6,7 @@
 // [frames x pdfs] matrix over PCIe and walks it on one host core per utterance.
 #pragma once
 
+#include <string>
 #include <vector>
 
 #include "common.cuh"
@@ -81,6 +82,13 @@ struct Lattice {
   double *best_out;    // [n] min over final nodes of double(alpha) + double(final)
   int max_arcs, grp_stride;
   float beam;          // lattice beam
+  // Resumable search only (pkb_decoder_set_lattice). Groups are indexed by utterance time, so an
+  // advance that starts at frame t0 logs emit(t) / eps(t + 1) at grp[2 (t0 + t) + 1 / + 2]. Each
+  // advance copies its rows to rows + (s * max_frames + t0) * num_pdfs for the backward pass of
+  // the finish, which reads them back as its loglik with frame_stride = max_frames.
+  int *state;          // [n][2]: log length, lattice error (4 arcs, 5 frames; apart from the search's)
+  float *rows;         // [n][max_frames][num_pdfs]
+  int max_frames;
 };
 
 // Decodes n_utts utterances. loglik: [rows][num_pdfs] scaled log-likelihoods where utterance u owns
@@ -119,10 +127,22 @@ struct ResumableSearch {
   size_t partial_bytes = 0;  // the best-so-far block at the start of `out`
   int32_t *f_words = nullptr, *f_nw = nullptr;
   float *f_weight = nullptr;
+  // lattice mode (set_lattice): lat.log == nullptr when off. lat_aux holds the group offsets, the
+  // per-stream state, the finish results and the row offsets / first records of lattice_expand.
+  Lattice lat{};
+  DevBuf lat_log, lat_aux, lat_rows, lat_arcs;
+  long long *lat_first = nullptr;
+  int64_t *lat_row_off = nullptr;
   int setup(Ctx *ctx, const pkb_fst *graph, const ViterbiConfig &config, const int32_t *tid2pdf, int n_tids,
             int pdfs, int streams);
+  // lattice_beam > 0 switches lattice mode on (buffers for max_frames frames and max_arcs log
+  // entries per stream), 0 off. Only between utterances.
+  int set_lattice(float lattice_beam, int max_frames, int max_arcs);
   int advance(const float *d_loglik, int frame_stride, const int32_t *d_n_frames, int uniform_frames);
   int finish();
+  // after a finish in lattice mode: the kept arcs of every stream as records in lat_arcs, back to
+  // back; n_out / best_out on the host. Returns the total in *total.
+  int expand_lattice(int64_t *n_out, double *best_out, int64_t *total);
 };
 
 // Checks shared by pkb_batch_decode and pkb_decoder_create / _finish: the FST is from context c, the
@@ -144,6 +164,12 @@ struct pkb_decoder {
   struct { void *p = nullptr; } partial;  // pinned host copy of the best-so-far block
   pkb_stream *st = nullptr;     // attached stream (pkb_stream_set_decoder)
   bool flushed = false;         // the attached stream was flushed: finish before its next push
+  bool in_utt = false;          // an advance, push or flush since create or the last finish
+  // results of the latest finish in lattice mode, valid until the next advance, push or flush
+  int64_t lat_total = -1;       // records in search.lat_arcs (-1: none valid, for the reason in lat_why)
+  std::string lat_why = "no pkb_decoder_finish yet";
+  std::vector<int64_t> lat_n;
+  std::vector<double> lat_best;
   pkb_decoder() = default;
   pkb_decoder(const pkb_decoder &) = delete;
   pkb_decoder &operator=(const pkb_decoder &) = delete;
@@ -154,4 +180,10 @@ namespace pkb {
 // Queues an advance over device rows and the copy of its best-so-far block to the host.
 int decoder_enqueue_advance(pkb_decoder *dec, const float *d_rows, int frame_stride, const int32_t *d_n_frames,
                             int uniform_frames);
+// Host state of a decoder whose utterance moves on (an advance, or a push / flush of the attached
+// stream, whose captured graph advances the decoder without host code): the lattice results of
+// the last finish stop being valid and lattice mode can no longer change.
+void decoder_begin_step(pkb_decoder *dec);
+// Destroys the captured CUDA graphs of a stream's pushes (stream_api.cu).
+void stream_drop_graphs(pkb_stream *st);
 }  // namespace pkb

@@ -35,6 +35,12 @@ int decoder_enqueue_advance(pkb_decoder *dec, const float *d_rows, int frame_str
   return PKB_OK;
 }
 
+void decoder_begin_step(pkb_decoder *dec) {
+  dec->in_utt = true;
+  dec->lat_total = -1;
+  dec->lat_why = "an advance, push or flush came after the latest pkb_decoder_finish";
+}
+
 }  // namespace pkb
 
 pkb_decoder::~pkb_decoder() {
@@ -89,6 +95,7 @@ int pkb_decoder_advance(pkb_decoder_t *dec, const float *loglik, int frame_strid
   PKB_REQUIRE(loglik || most == 0, "pkb_decoder_advance: loglik is NULL");
   pkb::Ctx *c = dec->c;
   PKB_CUDA(cudaSetDevice(c->device));
+  pkb::decoder_begin_step(dec);
   const size_t row_bytes = static_cast<size_t>(dec->am->num_pdfs) * sizeof(float);
   const size_t bytes = static_cast<size_t>(dec->n) * frame_stride * row_bytes;
   if (bytes) {
@@ -134,7 +141,65 @@ int pkb_decoder_finish(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words_
   PKB_CUDA(cudaMemcpyAsync(dec->partial.p, r.out.p, r.partial_bytes, cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaStreamSynchronize(c->stream));
   dec->flushed = false;
-  return pkb::check_device_error(c, "pkb_decoder_finish");
+  dec->in_utt = false;
+  dec->lat_total = -1;
+  dec->lat_why = "the latest pkb_decoder_finish ran without lattices";
+  PKB_TRY(pkb::check_device_error(c, "pkb_decoder_finish"));
+  if (r.lat.log) {
+    // the words above are complete and the utterance is over: a lattice that cannot be expanded
+    // (the records of a large graph can take gigabytes) is reported by pkb_decoder_lattice instead
+    dec->lat_n.resize(S);
+    dec->lat_best.resize(S);
+    int64_t total = 0;
+    if (r.expand_lattice(dec->lat_n.data(), dec->lat_best.data(), &total) == PKB_OK) {
+      dec->lat_total = total;
+    } else {
+      dec->lat_why = std::string("expanding the lattices of the latest pkb_decoder_finish failed: ") + pkb_last_error();
+      cudaGetLastError();
+    }
+  }
+  return PKB_OK;
+}
+
+int pkb_decoder_set_lattice(pkb_decoder_t *dec, float lattice_beam, int max_frames, int max_arcs) {
+  PKB_REQUIRE(dec, "pkb_decoder_set_lattice: decoder is NULL");
+  PKB_REQUIRE(lattice_beam >= 0.0f, "pkb_decoder_set_lattice: lattice_beam must be >= 0 (got %g)", lattice_beam);
+  PKB_REQUIRE(max_frames <= (1 << 24), "pkb_decoder_set_lattice: max_frames %d is more than %d", max_frames, 1 << 24);
+  // the log count is an int and passes max_arcs by at most one group (at most the graph's arcs)
+  const int arcs_cap = INT32_MAX - std::max(dec->search.fst->num_arcs, 1);
+  PKB_REQUIRE(max_arcs <= arcs_cap, "pkb_decoder_set_lattice: max_arcs %d is more than %d", max_arcs, arcs_cap);
+  PKB_REQUIRE(!dec->in_utt,
+              "pkb_decoder_set_lattice: only between utterances (after create or pkb_decoder_finish)");
+  pkb::Ctx *c = dec->c;
+  PKB_CUDA(cudaSetDevice(c->device));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  // the attached stream's captured pushes launch the advance with the old lattice arguments (or
+  // none): they are captured again
+  if (dec->st) pkb::stream_drop_graphs(dec->st);
+  dec->lat_total = -1;
+  dec->lat_why = "pkb_decoder_set_lattice came after the latest pkb_decoder_finish";
+  return dec->search.set_lattice(lattice_beam, max_frames, max_arcs);
+}
+
+int pkb_decoder_lattice(pkb_decoder_t *dec, int64_t *n_arcs_out, double *best_cost_out) {
+  PKB_REQUIRE(dec && n_arcs_out && best_cost_out, "pkb_decoder_lattice: NULL argument");
+  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_lattice: no lattice: %s", dec->lat_why.c_str());
+  memcpy(n_arcs_out, dec->lat_n.data(), sizeof(int64_t) * dec->n);
+  memcpy(best_cost_out, dec->lat_best.data(), sizeof(double) * dec->n);
+  return PKB_OK;
+}
+
+int pkb_decoder_lattice_get(pkb_decoder_t *dec, pkb_lattice_arc_t *arcs_out) {
+  PKB_REQUIRE(dec, "pkb_decoder_lattice_get: decoder is NULL");
+  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_lattice_get: no lattice: %s", dec->lat_why.c_str());
+  if (dec->lat_total == 0) return PKB_OK;
+  PKB_REQUIRE(arcs_out, "pkb_decoder_lattice_get: NULL argument");
+  pkb::Ctx *c = dec->c;
+  PKB_CUDA(cudaSetDevice(c->device));
+  PKB_CUDA(cudaMemcpyAsync(arcs_out, dec->search.lat_arcs.p, sizeof(pkb_lattice_arc_t) * dec->lat_total,
+                           cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  return pkb::check_device_error(c, "pkb_decoder_lattice_get");
 }
 
 }  // extern "C"

@@ -195,6 +195,10 @@ int stream_emit(pkb_stream *st, int rows, int emit, void *loglik_out, float *off
 
 }  // namespace
 
+namespace pkb {
+void stream_drop_graphs(pkb_stream *st) { st->drop_graphs(); }
+}  // namespace pkb
+
 extern "C" {
 
 int pkb_stream_create(pkb_ctx_t *c, pkb_am_t *am, int n_streams, int chunk_samples,
@@ -336,6 +340,7 @@ int stream_push(pkb_stream *st, const int16_t *pcm, void *out, float *off_out, i
   PKB_REQUIRE(!st->dec || !st->dec->flushed, "%s: the stream was flushed: finish its decoder first", who);
   PKB_REQUIRE(sh.emit == 0 || out || st->dec, "%s: the output buffer is NULL", who);
   PKB_REQUIRE(sh.emit == 0 || !st->compact || off_out, "%s: the offset buffer is NULL", who);
+  if (st->dec) pkb::decoder_begin_step(st->dec);
   if (sh.n_new > 0) {
     if (st->meta_len != sh.win_len) {
       std::vector<int32_t> ns(S, sh.win_len);
@@ -457,6 +462,7 @@ static int stream_flush(pkb_stream_t *st, void *loglik_out, float *off_out, int3
   PKB_REQUIRE(st, "pkb_stream_flush: stream is NULL");
   pkb::Ctx *c = st->c;
   PKB_CUDA(cudaSetDevice(c->device));
+  if (st->dec) pkb::decoder_begin_step(st->dec);
   int emit = 0;
   const int pending = static_cast<int>(st->n_feat - st->n_emit);
   if (pending > 0) {
