@@ -305,6 +305,35 @@ int pkb_batch_lattice(pkb_batch_t *batch, const pkb_fst_t *fst, float beam, floa
                       int max_arcs, int64_t *n_arcs_out, double *best_cost_out);
 /* The arcs of the latest pkb_batch_lattice, every utterance's back to back in utterance order. */
 int pkb_batch_lattice_get(pkb_batch_t *batch, pkb_lattice_arc_t *arcs_out);
+/* ---- N-best lists over a lattice ----------------------------------------------------------------
+ * A path of a lattice runs from (0, start) to (T, s) with final(s) finite, where T is the last
+ * emitting record's t + 1 (0 without one); an emitting record goes from (t, src) to (t + 1, dst), an
+ * epsilon record from (t, src) to (t, dst). Along a path, its words are the nonzero olabels in path
+ * order, its graph cost ((g1 + g2) + ...) + final(s) and its acoustic cost (a1 + a2) + ..., both
+ * summed in double in path order from the records' floats; cost = graph + acoustic. A word sequence
+ * is represented by its best path: least cost, then least graph cost. The N-best list holds the n
+ * first distinct word sequences ordered by cost, then graph cost, then the word sequences compared
+ * from the last word backwards (a suffix of the other comes first), then acoustic cost. The list is
+ * taken over the lattice's paths: a sequence whose cost is above best + lattice_beam may have had
+ * cheaper alignments pruned, so its cost is then only an upper bound on its best cost over the
+ * search's arcs. A zero-frame utterance whose start state is final gives one empty sequence of cost
+ * final(start).
+ * Device memory per call: the outputs, 2 x states x n x 24 bytes of lists per utterance in flight,
+ * and a word-history table of 8-byte slots for at least 1.5 x n x (min(labelled emitting records,
+ * T x states entered by a labelled emitting arc) + 4 x min(labelled epsilon records, (T + 1) x states
+ * entered by a labelled epsilon arc)) histories per utterance in flight; utterances run in waves of
+ * at most 8 GiB (or half the free memory) of these.
+ * n_hyps_out codes besides those of the lattice: -6 an epsilon closure that did not settle in
+ * (records of the group + 1) x (n + 1) passes (only cycles that never settle), -7 more word
+ * histories than the table holds (only an epsilon closure of more than 4 passes can need more). */
+/* N-best lists of the latest pkb_batch_lattice of this batch (fst: the graph of that call; another
+ * one is rejected). 1 <= n <= 1024, max_words > 0. words_out [n_utts][n][max_words] in spoken order,
+ * n_words_out / graph_cost_out / acoustic_cost_out [n_utts][n] (n_words may exceed max_words: the
+ * list is then truncated, as in pkb_batch_decode); n_hyps_out[u]: entries of utterance u (<= n;
+ * 0 when the lattice has no complete path), or that lattice's negative code. Synchronous; the
+ * lattice itself is left unchanged. */
+int pkb_batch_nbest(pkb_batch_t *batch, const pkb_fst_t *fst, int n, int max_words, int32_t *words_out,
+                    int32_t *n_words_out, double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out);
 
 /* ---- online decoding: the GPU Viterbi search, chunk by chunk ----------------------------------
  * n_streams searches whose tokens and word records stay on the device between calls, so that
@@ -357,6 +386,9 @@ int pkb_decoder_set_lattice(pkb_decoder_t *dec, float lattice_beam, int max_fram
 int pkb_decoder_lattice(pkb_decoder_t *dec, int64_t *n_arcs_out, double *best_cost_out);
 /* The arcs of the latest finish, every stream's back to back in stream order (same validity). */
 int pkb_decoder_lattice_get(pkb_decoder_t *dec, pkb_lattice_arc_t *arcs_out);
+/* pkb_batch_nbest for the lattices of the latest pkb_decoder_finish; valid when pkb_decoder_lattice is. */
+int pkb_decoder_nbest(pkb_decoder_t *dec, int n, int max_words, int32_t *words_out, int32_t *n_words_out,
+                      double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out);
 
 /* Sum over all elements of a per-frame float buffer, computed on the device
  * in double (a cheap whole-output fingerprint for full-size runs). */

@@ -108,6 +108,7 @@ _SIGNATURES = [
     ("pkb_batch_decode", C.c_int, [_VP, _VP, C.c_float, C.c_int, C.c_int, _VP, _VP, _VP]),
     ("pkb_batch_lattice", C.c_int, [_VP, _VP, C.c_float, C.c_float, C.c_int, C.c_int, _VP, _VP]),
     ("pkb_batch_lattice_get", C.c_int, [_VP, _VP]),
+    ("pkb_batch_nbest", C.c_int, [_VP, _VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
     ("pkb_decoder_create", C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
                                      C.POINTER(_VP)]),
     ("pkb_decoder_destroy", None, [_VP]),
@@ -117,6 +118,7 @@ _SIGNATURES = [
     ("pkb_decoder_set_lattice", C.c_int, [_VP, C.c_float, C.c_int, C.c_int]),
     ("pkb_decoder_lattice", C.c_int, [_VP, _VP, _VP]),
     ("pkb_decoder_lattice_get", C.c_int, [_VP, _VP]),
+    ("pkb_decoder_nbest", C.c_int, [_VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
     ("pkb_loglik16_expand", C.c_int, [_VP, _VP, C.c_int64, C.c_int, C.c_float, _VP]),
     ("pkb_stream_create", C.c_int, [_VP, _VP, C.c_int, C.c_int, _f32p, C.c_float, C.POINTER(_VP)]),
     ("pkb_stream_destroy", None, [_VP]),
@@ -696,6 +698,13 @@ class Batch:
         lats = [None if na[u] < 0 else arcs[off[u]:off[u + 1]].copy() for u in range(n)]
         return lats, best[:n].copy()
 
+    def nbest(self, fst, n=10, max_words=256):
+        """N-best lists of distinct word sequences over the latest lattice() (pkb_batch_nbest; fst
+        is the graph of that call): per utterance None where its lattice failed, otherwise a list
+        of (words, graph_cost, acoustic_cost), best first."""
+        return _nbest(len(self.num_samples), n, max_words,
+                      lambda *out: self.ctx.lib.pkb_batch_nbest(self.h, fst.h, n, max_words, *out))
+
     def refine_stats(self):
         """(GEMM rows, frames recomputed) of the latest run under PREC_FP16R."""
         rows, sel = C.c_int64(0), C.c_int64(0)
@@ -844,6 +853,31 @@ class Decoder:
         _check(self.ctx.lib.pkb_decoder_lattice_get(self.h, arcs.ctypes.data))
         off = np.concatenate([[0], np.cumsum(kept)])
         return [None if na[s] < 0 else arcs[off[s]:off[s + 1]].copy() for s in range(self.n_streams)], best
+
+    def nbest(self, n=10, max_words=256):
+        """Batch.nbest over the lattices of the latest finish() (pkb_decoder_nbest)."""
+        return _nbest(self.n_streams, n, max_words,
+                      lambda *out: self.ctx.lib.pkb_decoder_nbest(self.h, n, max_words, *out))
+
+
+def _nbest(n_utts, n, max_words, call):
+    """Runs call(words, n_words, graph, acoustic, n_hyps) over output arrays for n_utts utterances and
+    unpacks them as Batch.nbest returns them."""
+    u = max(n_utts, 1)
+    words = np.zeros((u, max(n, 1), max(max_words, 1)), np.int32)
+    nw = np.zeros((u, max(n, 1)), np.int32)
+    g = np.zeros((u, max(n, 1)), np.float64)
+    a = np.zeros((u, max(n, 1)), np.float64)
+    nh = np.zeros(u, np.int32)
+    _check(call(words.ctypes.data, nw.ctypes.data, g.ctypes.data, a.ctypes.data, nh.ctypes.data))
+    out = []
+    for i in range(n_utts):
+        if nh[i] < 0:
+            out.append(None)
+            continue
+        out.append([([int(x) for x in words[i, j, :min(int(nw[i, j]), max_words)]], float(g[i, j]), float(a[i, j]))
+                    for j in range(int(nh[i]))])
+    return out
 
 
 class Stream:

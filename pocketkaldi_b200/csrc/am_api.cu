@@ -283,6 +283,9 @@ struct pkb_batch {
   pkb::DevBuf vit_work, vit_out, vit_tid2pdf;  // GPU Viterbi: workspace, results, device tid2pdf
   pkb::DevBuf lat_log, lat_aux, lat_arcs;      // lattices: arc logs, offsets and results, kept arcs
   int64_t lat_total = -1;                      // kept arcs of the latest pkb_batch_lattice
+  const pkb_fst *lat_fst = nullptr;            // its graph, while its records are valid
+  pkb::LatticeRecords lat_rec;                 // its records on the device
+  pkb::DevBuf nbest_work;                      // outputs of pkb_batch_nbest
   Workspace ws;
   pkb::Refine rf;
   pkb::PaddedPlanes planes;
@@ -905,8 +908,13 @@ int pkb_batch_lattice(pkb_batch_t *b, const pkb_fst_t *fst, float beam, float la
   Ctx *c = b->c;
   PKB_CUDA(cudaSetDevice(c->device));
   b->lat_total = 0;
+  b->lat_fst = nullptr;
   const int n = b->meta.n_utts;
-  if (n == 0) return PKB_OK;
+  if (n == 0) {
+    b->lat_fst = fst;
+    b->lat_rec = pkb::LatticeRecords{};
+    return PKB_OK;
+  }
   pkb::ViterbiConfig cfg;
   if (beam > 0.0f) cfg.beam = beam;
   if (max_tokens > 0) cfg.max_tokens = max_tokens;
@@ -955,6 +963,12 @@ int pkb_batch_lattice(pkb_batch_t *b, const pkb_fst_t *fst, float beam, float la
   PKB_CUDA(cudaStreamSynchronize(c->stream));
   PKB_TRY(pkb::check_device_error(c, "pkb_batch_lattice"));
   b->lat_total = total;
+  b->lat_fst = fst;
+  b->lat_rec.arcs = b->lat_arcs.as<pkb_lattice_arc_t>();
+  b->lat_rec.first = d_first;
+  b->lat_rec.n_arcs = lat.n_out;
+  b->lat_rec.best = lat.best_out;
+  b->lat_rec.n_utts = n;
   return PKB_OK;
 }
 
@@ -968,6 +982,19 @@ int pkb_batch_lattice_get(pkb_batch_t *b, pkb_lattice_arc_t *arcs_out) {
                            cudaMemcpyDeviceToHost, b->c->stream));
   PKB_CUDA(cudaStreamSynchronize(b->c->stream));
   return pkb::check_device_error(b->c, "pkb_batch_lattice_get");
+}
+
+int pkb_batch_nbest(pkb_batch_t *b, const pkb_fst_t *fst, int n, int max_words, int32_t *words_out,
+                    int32_t *n_words_out, double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out) {
+  PKB_REQUIRE(b && fst, "pkb_batch_nbest: NULL argument");
+  PKB_REQUIRE(b->lat_fst, "pkb_batch_nbest: no valid pkb_batch_lattice on this batch");
+  PKB_REQUIRE(b->lat_fst == fst, "pkb_batch_nbest: the FST is not the one of the latest pkb_batch_lattice");
+  PKB_TRY(pkb::check_nbest_args(n, max_words, words_out, n_words_out, graph_cost_out, acoustic_cost_out,
+                                n_hyps_out, "pkb_batch_nbest"));
+  PKB_CUDA(cudaSetDevice(b->c->device));
+  PKB_TRY(pkb::launch_nbest(b->c, fst, b->lat_rec, n, max_words, &b->nbest_work, words_out, n_words_out,
+                            graph_cost_out, acoustic_cost_out, n_hyps_out));
+  return pkb::check_device_error(b->c, "pkb_batch_nbest");
 }
 
 // ---------------------------------------------------------------- fused host path

@@ -110,6 +110,26 @@ int lattice_expand(Ctx *c, const pkb_fst *fst, const Lattice &lat, const float *
                    const int64_t *d_row_off, int n_utts, const int32_t *d_tid2pdf, const long long *d_first,
                    pkb_lattice_arc_t *d_out);
 
+// The kept records of the latest lattice call, as the search left them on the device: utterance u's
+// n_arcs[u] records (or its negative code) from arcs + first[u] on, and its best cost.
+struct LatticeRecords {
+  const pkb_lattice_arc_t *arcs = nullptr;
+  const long long *first = nullptr, *n_arcs = nullptr;
+  const double *best = nullptr;
+  int n_utts = 0;
+};
+
+// N-best lists of distinct word sequences over the records of every utterance (nbest.cu), with the
+// arguments and host outputs of pkb_batch_nbest. work keeps the outputs and statistics; the
+// per-block lists (2 x states x n x 24 bytes) and word-history tables are allocated per call.
+int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, int max_words, DevBuf *work,
+                 int32_t *words_out, int32_t *n_words_out, double *graph_cost_out, double *acoustic_cost_out,
+                 int32_t *n_hyps_out);
+// The argument checks shared by pkb_batch_nbest and pkb_decoder_nbest.
+int check_nbest_args(int n, int max_words, const void *words_out, const void *n_words_out,
+                     const void *graph_cost_out, const void *acoustic_cost_out, const void *n_hyps_out,
+                     const char *who);
+
 // The resumable search behind pkb_decoder: n streams, one thread block each, whose tokens and word
 // records stay in global memory between launches. advance() decodes the next rows of every stream
 // (stream s: rows [s * frame_stride, s * frame_stride + n_frames[s]) of d_loglik, or uniform_frames
@@ -170,6 +190,7 @@ struct pkb_decoder {
   std::string lat_why = "no pkb_decoder_finish yet";
   std::vector<int64_t> lat_n;
   std::vector<double> lat_best;
+  pkb::DevBuf nbest_work;       // outputs of pkb_decoder_nbest
   pkb_decoder() = default;
   pkb_decoder(const pkb_decoder &) = delete;
   pkb_decoder &operator=(const pkb_decoder &) = delete;

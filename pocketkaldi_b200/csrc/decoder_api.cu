@@ -27,6 +27,16 @@ int check_decode_outputs(int max_words, const void *words_out, const void *n_wor
   return PKB_OK;
 }
 
+int check_nbest_args(int n, int max_words, const void *words_out, const void *n_words_out,
+                     const void *graph_cost_out, const void *acoustic_cost_out, const void *n_hyps_out,
+                     const char *who) {
+  PKB_REQUIRE(n >= 1 && n <= 1024, "%s: n must be in [1, 1024] (got %d)", who, n);
+  PKB_REQUIRE(max_words > 0, "%s: max_words must be > 0 (got %d)", who, max_words);
+  PKB_REQUIRE(words_out && n_words_out && graph_cost_out && acoustic_cost_out && n_hyps_out,
+              "%s: NULL output argument", who);
+  return PKB_OK;
+}
+
 int decoder_enqueue_advance(pkb_decoder *dec, const float *d_rows, int frame_stride, const int32_t *d_n_frames,
                             int uniform_frames) {
   PKB_TRY(dec->search.advance(d_rows, frame_stride, d_n_frames, uniform_frames));
@@ -200,6 +210,26 @@ int pkb_decoder_lattice_get(pkb_decoder_t *dec, pkb_lattice_arc_t *arcs_out) {
                            cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaStreamSynchronize(c->stream));
   return pkb::check_device_error(c, "pkb_decoder_lattice_get");
+}
+
+int pkb_decoder_nbest(pkb_decoder_t *dec, int n, int max_words, int32_t *words_out, int32_t *n_words_out,
+                      double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out) {
+  PKB_REQUIRE(dec, "pkb_decoder_nbest: decoder is NULL");
+  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_nbest: no lattice: %s", dec->lat_why.c_str());
+  PKB_TRY(pkb::check_nbest_args(n, max_words, words_out, n_words_out, graph_cost_out, acoustic_cost_out,
+                                n_hyps_out, "pkb_decoder_nbest"));
+  pkb::Ctx *c = dec->c;
+  PKB_CUDA(cudaSetDevice(c->device));
+  const pkb::ResumableSearch &r = dec->search;
+  pkb::LatticeRecords lr;
+  lr.arcs = r.lat_arcs.as<pkb_lattice_arc_t>();
+  lr.first = r.lat_first;
+  lr.n_arcs = r.lat.n_out;
+  lr.best = r.lat.best_out;
+  lr.n_utts = dec->n;
+  PKB_TRY(pkb::launch_nbest(c, r.fst, lr, n, max_words, &dec->nbest_work, words_out, n_words_out, graph_cost_out,
+                            acoustic_cost_out, n_hyps_out));
+  return pkb::check_device_error(c, "pkb_decoder_nbest");
 }
 
 }  // extern "C"
