@@ -334,6 +334,53 @@ int pkb_batch_lattice_get(pkb_batch_t *batch, pkb_lattice_arc_t *arcs_out);
  * lattice itself is left unchanged. */
 int pkb_batch_nbest(pkb_batch_t *batch, const pkb_fst_t *fst, int n, int max_words, int32_t *words_out,
                     int32_t *n_words_out, double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out);
+/* ---- arc and frame posteriors over a lattice ---------------------------------------------------
+ * Paths, T and final(s) as in the N-best comment above. Per utterance, in double from the
+ * records' floats: the scaled cost of a record c(r) = graph_scale x graph_cost + acoustic_scale x
+ * acoustic_cost, and of a final weight graph_scale x final(s) (the rows already carry prob_scale,
+ * so scales of 1 give the search's own costs). Forward and backward costs alpha(t, s), beta(t, s)
+ * are negative logs of path sums, with lse(a, b) = m - log1p(exp(m - M)), m = min(a, b),
+ * M = max(a, b), +inf the identity:
+ *   alpha(0, start) = 0; a node folds its incoming records alpha(t, src) + c(r) in ascending record
+ *   order (so emitting records before the epsilon records of its time).
+ *   beta(T, s) = graph_scale x final(s) (+inf when not final), folded with the outgoing epsilon
+ *   records of time T; an earlier node folds its outgoing records c(r) + beta(head) in ascending
+ *   record order.
+ *   Within one time, the epsilon records are processed in topological order: a node is folded once
+ *   all its sources (forward) or heads (backward) are complete, so nothing depends on scheduling.
+ * total = lse over the final states s, in ascending order, of alpha(T, s) + graph_scale x final(s)
+ * (+inf without a complete path). The posterior of a record from (t, src) to (t', dst) is
+ * exp(total - ((alpha(t, src) + c(r)) + beta(t', dst))) (0 without a complete path); the frame
+ * posterior of (t, pdf) is the double sum, in record order, of the posteriors of the emitting
+ * records of time t whose tid2pdf[ilabel] is pdf, returned as a float when that float is
+ * >= min_post. Every complete path crosses one emitting record per frame, so for each t < T the
+ * emitting posteriors of time t, and the frame posteriors at min_post = 0, sum to 1. The sums run
+ * over the lattice's paths: with a finite lattice_beam they are those of the pruned lattice, not
+ * of every path of the search.
+ * n_post_out codes besides those of the lattice: -8 the kept epsilon records of one time form a
+ * cycle (forward-backward needs an acyclic lattice); only that utterance fails, its total and arc
+ * posteriors are NaN and it has no frame entries. A failed lattice keeps its code and a NaN total.
+ * Device memory per call: the results, 4 bytes per record and 12 per frame entry, kept until the
+ * next call; 12 bytes per record of frame scratch; and per utterance in flight 8 bytes per record
+ * (alpha) plus 12 bytes per graph arc and, for graphs whose per-state arrays pass 48 KiB, those
+ * arrays (36 bytes per state and 16 per state or pdf, whichever are more); utterances run in waves of at most 8 GiB (or
+ * half the free memory) of the latter. */
+typedef struct {           /* 12 bytes, no padding */
+  int32_t t;               /* frame */
+  int32_t pdf;
+  float post;
+} pkb_frame_post_t;
+/* Posteriors of the latest pkb_batch_lattice of this batch (fst: the graph of that call; another
+ * one is rejected). acoustic_scale > 0 and graph_scale >= 0, both finite; 0 <= min_post <= 1.
+ * total_out[u]; n_post_out[u]: frame entries of utterance u, or its negative code. Synchronous;
+ * the lattice, N-best and decode results are left unchanged. */
+int pkb_batch_posteriors(pkb_batch_t *batch, const pkb_fst_t *fst, float acoustic_scale, float graph_scale,
+                         float min_post, double *total_out, int64_t *n_post_out);
+/* The results of the latest pkb_batch_posteriors, valid until the next lattice or posteriors call
+ * on the batch. arc_post_out: one float per record of pkb_batch_lattice_get, in the same order;
+ * frame_post_out: every utterance's entries back to back, each in (t, pdf) order. Either may be
+ * NULL. */
+int pkb_batch_posteriors_get(pkb_batch_t *batch, float *arc_post_out, pkb_frame_post_t *frame_post_out);
 
 /* ---- online decoding: the GPU Viterbi search, chunk by chunk ----------------------------------
  * n_streams searches whose tokens and word records stay on the device between calls, so that
@@ -389,6 +436,12 @@ int pkb_decoder_lattice_get(pkb_decoder_t *dec, pkb_lattice_arc_t *arcs_out);
 /* pkb_batch_nbest for the lattices of the latest pkb_decoder_finish; valid when pkb_decoder_lattice is. */
 int pkb_decoder_nbest(pkb_decoder_t *dec, int n, int max_words, int32_t *words_out, int32_t *n_words_out,
                       double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out);
+/* pkb_batch_posteriors for the lattices of the latest pkb_decoder_finish; valid when
+ * pkb_decoder_lattice is. */
+int pkb_decoder_posteriors(pkb_decoder_t *dec, float acoustic_scale, float graph_scale, float min_post,
+                           double *total_out, int64_t *n_post_out);
+/* The results of the latest pkb_decoder_posteriors, valid until the next advance, push or flush. */
+int pkb_decoder_posteriors_get(pkb_decoder_t *dec, float *arc_post_out, pkb_frame_post_t *frame_post_out);
 
 /* Sum over all elements of a per-frame float buffer, computed on the device
  * in double (a cheap whole-output fingerprint for full-size runs). */

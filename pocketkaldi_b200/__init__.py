@@ -23,6 +23,7 @@ from .binding import (  # noqa: F401
     Decoder,
     Fst,
     LATTICE_ARC_DTYPE,
+    FRAME_POST_DTYPE,
     Stream,
     WavList,
     read_wav,

@@ -31,6 +31,9 @@ KERNEL_CLASSES = ("fbank", "cmvn", "gemm", "gemm_final", "misc")
 LATTICE_ARC_DTYPE = np.dtype([("t", np.int32), ("src", np.int32), ("dst", np.int32), ("ilabel", np.int32),
                               ("olabel", np.int32), ("graph_cost", np.float32), ("acoustic_cost", np.float32)])
 assert LATTICE_ARC_DTYPE.itemsize == 28
+# pkb_frame_post_t (include/pkb200.h)
+FRAME_POST_DTYPE = np.dtype([("t", np.int32), ("pdf", np.int32), ("post", np.float32)])
+assert FRAME_POST_DTYPE.itemsize == 12
 
 _f32p = np.ctypeslib.ndpointer(dtype=np.float32, flags="C_CONTIGUOUS")
 _i32p = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
@@ -109,6 +112,8 @@ _SIGNATURES = [
     ("pkb_batch_lattice", C.c_int, [_VP, _VP, C.c_float, C.c_float, C.c_int, C.c_int, _VP, _VP]),
     ("pkb_batch_lattice_get", C.c_int, [_VP, _VP]),
     ("pkb_batch_nbest", C.c_int, [_VP, _VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
+    ("pkb_batch_posteriors", C.c_int, [_VP, _VP, C.c_float, C.c_float, C.c_float, _VP, _VP]),
+    ("pkb_batch_posteriors_get", C.c_int, [_VP, _VP, _VP]),
     ("pkb_decoder_create", C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
                                      C.POINTER(_VP)]),
     ("pkb_decoder_destroy", None, [_VP]),
@@ -119,6 +124,8 @@ _SIGNATURES = [
     ("pkb_decoder_lattice", C.c_int, [_VP, _VP, _VP]),
     ("pkb_decoder_lattice_get", C.c_int, [_VP, _VP]),
     ("pkb_decoder_nbest", C.c_int, [_VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
+    ("pkb_decoder_posteriors", C.c_int, [_VP, C.c_float, C.c_float, C.c_float, _VP, _VP]),
+    ("pkb_decoder_posteriors_get", C.c_int, [_VP, _VP, _VP]),
     ("pkb_loglik16_expand", C.c_int, [_VP, _VP, C.c_int64, C.c_int, C.c_float, _VP]),
     ("pkb_stream_create", C.c_int, [_VP, _VP, C.c_int, C.c_int, _f32p, C.c_float, C.POINTER(_VP)]),
     ("pkb_stream_destroy", None, [_VP]),
@@ -696,6 +703,7 @@ class Batch:
         _check(self.ctx.lib.pkb_batch_lattice_get(self.h, arcs.ctypes.data))
         off = np.concatenate([[0], np.cumsum(kept)])
         lats = [None if na[u] < 0 else arcs[off[u]:off[u + 1]].copy() for u in range(n)]
+        self._lat_n = na[:n].copy()
         return lats, best[:n].copy()
 
     def nbest(self, fst, n=10, max_words=256):
@@ -704,6 +712,17 @@ class Batch:
         of (words, graph_cost, acoustic_cost), best first."""
         return _nbest(len(self.num_samples), n, max_words,
                       lambda *out: self.ctx.lib.pkb_batch_nbest(self.h, fst.h, n, max_words, *out))
+
+    def posteriors(self, fst, acoustic_scale=1.0, graph_scale=1.0, min_post=0.0):
+        """Arc and frame posteriors over the latest lattice() (pkb_batch_posteriors; fst is the graph
+        of that call): (totals as float64, per utterance the float32 posteriors of its lattice()
+        records or None where its lattice failed, per utterance a FRAME_POST_DTYPE array of its
+        (t, pdf) entries or None where its lattice or its posteriors failed)."""
+        lib = self.ctx.lib
+        return _posteriors(getattr(self, "_lat_n", np.zeros(0, np.int64)), len(self.num_samples),
+                           lambda tot, npost: lib.pkb_batch_posteriors(self.h, fst.h, acoustic_scale, graph_scale,
+                                                                      min_post, tot, npost),
+                           lambda arc, fr: lib.pkb_batch_posteriors_get(self.h, arc, fr))
 
     def refine_stats(self):
         """(GEMM rows, frames recomputed) of the latest run under PREC_FP16R."""
@@ -859,6 +878,17 @@ class Decoder:
         return _nbest(self.n_streams, n, max_words,
                       lambda *out: self.ctx.lib.pkb_decoder_nbest(self.h, n, max_words, *out))
 
+    def posteriors(self, acoustic_scale=1.0, graph_scale=1.0, min_post=0.0):
+        """Batch.posteriors over the lattices of the latest finish() (pkb_decoder_posteriors)."""
+        lib = self.ctx.lib
+        na = np.zeros(self.n_streams, np.int64)
+        best = np.zeros(self.n_streams, np.float64)
+        _check(lib.pkb_decoder_lattice(self.h, na.ctypes.data, best.ctypes.data))
+        return _posteriors(na, self.n_streams,
+                           lambda tot, npost: lib.pkb_decoder_posteriors(self.h, acoustic_scale, graph_scale,
+                                                                        min_post, tot, npost),
+                           lambda arc, fr: lib.pkb_decoder_posteriors_get(self.h, arc, fr))
+
 
 def _nbest(n_utts, n, max_words, call):
     """Runs call(words, n_words, graph, acoustic, n_hyps) over output arrays for n_utts utterances and
@@ -878,6 +908,27 @@ def _nbest(n_utts, n, max_words, call):
         out.append([([int(x) for x in words[i, j, :min(int(nw[i, j]), max_words)]], float(g[i, j]), float(a[i, j]))
                     for j in range(int(nh[i]))])
     return out
+
+
+def _posteriors(n_arcs, n_utts, call, get):
+    """Runs call(totals, n_post) and get(arc_posts, frame_entries) for n_utts utterances whose
+    lattices have n_arcs records (or negative codes) and unpacks them as Batch.posteriors returns
+    them."""
+    tot = np.zeros(max(n_utts, 1), np.float64)
+    npost = np.zeros(max(n_utts, 1), np.int64)
+    _check(call(tot.ctypes.data, npost.ctypes.data))
+    if len(n_arcs) != n_utts:
+        raise PkbError(1, "posteriors: the record counts of the latest lattice() are unknown")
+    kept = np.maximum(n_arcs, 0)
+    nf = np.maximum(npost[:n_utts], 0)
+    arc = np.empty(max(int(kept.sum()), 1), np.float32)
+    fr = np.empty(max(int(nf.sum()), 1), FRAME_POST_DTYPE)
+    _check(get(arc.ctypes.data, fr.ctypes.data))
+    ao = np.concatenate([[0], np.cumsum(kept)])
+    fo = np.concatenate([[0], np.cumsum(nf)])
+    arcs = [None if n_arcs[u] < 0 else arc[ao[u]:ao[u + 1]].copy() for u in range(n_utts)]
+    frames = [None if npost[u] < 0 else fr[fo[u]:fo[u + 1]].copy() for u in range(n_utts)]
+    return tot[:n_utts].copy(), arcs, frames
 
 
 class Stream:

@@ -286,6 +286,7 @@ struct pkb_batch {
   const pkb_fst *lat_fst = nullptr;            // its graph, while its records are valid
   pkb::LatticeRecords lat_rec;                 // its records on the device
   pkb::DevBuf nbest_work;                      // outputs of pkb_batch_nbest
+  pkb::PosteriorResults post;                  // results of pkb_batch_posteriors
   Workspace ws;
   pkb::Refine rf;
   pkb::PaddedPlanes planes;
@@ -909,6 +910,7 @@ int pkb_batch_lattice(pkb_batch_t *b, const pkb_fst_t *fst, float beam, float la
   PKB_CUDA(cudaSetDevice(c->device));
   b->lat_total = 0;
   b->lat_fst = nullptr;
+  b->post.n_arcs = -1;
   const int n = b->meta.n_utts;
   if (n == 0) {
     b->lat_fst = fst;
@@ -995,6 +997,30 @@ int pkb_batch_nbest(pkb_batch_t *b, const pkb_fst_t *fst, int n, int max_words, 
   PKB_TRY(pkb::launch_nbest(b->c, fst, b->lat_rec, n, max_words, &b->nbest_work, words_out, n_words_out,
                             graph_cost_out, acoustic_cost_out, n_hyps_out));
   return pkb::check_device_error(b->c, "pkb_batch_nbest");
+}
+
+static_assert(sizeof(pkb_frame_post_t) == 12 && offsetof(pkb_frame_post_t, post) == 8,
+              "pkb_frame_post_t is 12 bytes without padding");
+
+int pkb_batch_posteriors(pkb_batch_t *b, const pkb_fst_t *fst, float acoustic_scale, float graph_scale,
+                         float min_post, double *total_out, int64_t *n_post_out) {
+  PKB_REQUIRE(b && fst, "pkb_batch_posteriors: NULL argument");
+  PKB_REQUIRE(b->lat_fst, "pkb_batch_posteriors: no valid pkb_batch_lattice on this batch");
+  PKB_REQUIRE(b->lat_fst == fst, "pkb_batch_posteriors: the FST is not the one of the latest pkb_batch_lattice");
+  PKB_TRY(pkb::check_posterior_args(acoustic_scale, graph_scale, min_post, total_out, n_post_out,
+                                    "pkb_batch_posteriors"));
+  PKB_CUDA(cudaSetDevice(b->c->device));
+  PKB_TRY(pkb::launch_posteriors(b->c, fst, b->lat_rec, b->vit_tid2pdf.as<int32_t>(), b->am->num_pdfs,
+                                 acoustic_scale, graph_scale, min_post, &b->post, total_out, n_post_out));
+  return pkb::check_device_error(b->c, "pkb_batch_posteriors");
+}
+
+int pkb_batch_posteriors_get(pkb_batch_t *b, float *arc_post_out, pkb_frame_post_t *frame_post_out) {
+  PKB_REQUIRE(b, "pkb_batch_posteriors_get: the batch is NULL");
+  PKB_REQUIRE(b->post.n_arcs >= 0, "pkb_batch_posteriors_get: no pkb_batch_posteriors since the latest pkb_batch_lattice");
+  PKB_CUDA(cudaSetDevice(b->c->device));
+  PKB_TRY(pkb::posteriors_get(b->c, b->post, arc_post_out, frame_post_out));
+  return pkb::check_device_error(b->c, "pkb_batch_posteriors_get");
 }
 
 // ---------------------------------------------------------------- fused host path

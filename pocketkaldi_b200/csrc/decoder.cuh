@@ -130,6 +130,25 @@ int check_nbest_args(int n, int max_words, const void *words_out, const void *n_
                      const void *graph_cost_out, const void *acoustic_cost_out, const void *n_hyps_out,
                      const char *who);
 
+// Results of the latest posteriors call, kept on the device for the _get call: one float per
+// record, and every utterance's frame entries back to back.
+struct PosteriorResults {
+  DevBuf arc, frames;
+  int64_t n_arcs = -1;   // records covered (-1: no valid results)
+  int64_t n_frames = 0;  // frame entries
+};
+// Arc and frame posteriors over the records of every utterance (posterior.cu), with the arguments
+// and host outputs of pkb_batch_posteriors; d_tid2pdf maps input labels to pdfs in [0, num_pdfs).
+// Alpha (8 bytes per record) and the per-block workspace are allocated per call, in waves.
+int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, const int32_t *d_tid2pdf, int num_pdfs,
+                      float acoustic_scale, float graph_scale, float min_post, PosteriorResults *res,
+                      double *total_out, int64_t *n_post_out);
+// The argument checks shared by pkb_batch_posteriors and pkb_decoder_posteriors.
+int check_posterior_args(float acoustic_scale, float graph_scale, float min_post, const void *total_out,
+                         const void *n_post_out, const char *who);
+// Copies the results out (either output may be NULL).
+int posteriors_get(Ctx *c, const PosteriorResults &res, float *arc_post_out, pkb_frame_post_t *frame_post_out);
+
 // The resumable search behind pkb_decoder: n streams, one thread block each, whose tokens and word
 // records stay in global memory between launches. advance() decodes the next rows of every stream
 // (stream s: rows [s * frame_stride, s * frame_stride + n_frames[s]) of d_loglik, or uniform_frames
@@ -191,6 +210,7 @@ struct pkb_decoder {
   std::vector<int64_t> lat_n;
   std::vector<double> lat_best;
   pkb::DevBuf nbest_work;       // outputs of pkb_decoder_nbest
+  pkb::PosteriorResults post;   // results of pkb_decoder_posteriors, valid as the lattice results are
   pkb_decoder() = default;
   pkb_decoder(const pkb_decoder &) = delete;
   pkb_decoder &operator=(const pkb_decoder &) = delete;

@@ -154,6 +154,7 @@ int pkb_decoder_finish(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words_
   dec->in_utt = false;
   dec->lat_total = -1;
   dec->lat_why = "the latest pkb_decoder_finish ran without lattices";
+  dec->post.n_arcs = -1;
   PKB_TRY(pkb::check_device_error(c, "pkb_decoder_finish"));
   if (r.lat.log) {
     // the words above are complete and the utterance is over: a lattice that cannot be expanded
@@ -230,6 +231,36 @@ int pkb_decoder_nbest(pkb_decoder_t *dec, int n, int max_words, int32_t *words_o
   PKB_TRY(pkb::launch_nbest(c, r.fst, lr, n, max_words, &dec->nbest_work, words_out, n_words_out, graph_cost_out,
                             acoustic_cost_out, n_hyps_out));
   return pkb::check_device_error(c, "pkb_decoder_nbest");
+}
+
+int pkb_decoder_posteriors(pkb_decoder_t *dec, float acoustic_scale, float graph_scale, float min_post,
+                           double *total_out, int64_t *n_post_out) {
+  PKB_REQUIRE(dec, "pkb_decoder_posteriors: decoder is NULL");
+  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_posteriors: no lattice: %s", dec->lat_why.c_str());
+  PKB_TRY(pkb::check_posterior_args(acoustic_scale, graph_scale, min_post, total_out, n_post_out,
+                                    "pkb_decoder_posteriors"));
+  pkb::Ctx *c = dec->c;
+  PKB_CUDA(cudaSetDevice(c->device));
+  const pkb::ResumableSearch &r = dec->search;
+  pkb::LatticeRecords lr;
+  lr.arcs = r.lat_arcs.as<pkb_lattice_arc_t>();
+  lr.first = r.lat_first;
+  lr.n_arcs = r.lat.n_out;
+  lr.best = r.lat.best_out;
+  lr.n_utts = dec->n;
+  PKB_TRY(pkb::launch_posteriors(c, r.fst, lr, r.d_tid2pdf.as<int32_t>(), r.num_pdfs, acoustic_scale, graph_scale,
+                                 min_post, &dec->post, total_out, n_post_out));
+  return pkb::check_device_error(c, "pkb_decoder_posteriors");
+}
+
+int pkb_decoder_posteriors_get(pkb_decoder_t *dec, float *arc_post_out, pkb_frame_post_t *frame_post_out) {
+  PKB_REQUIRE(dec, "pkb_decoder_posteriors_get: decoder is NULL");
+  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_posteriors_get: no lattice: %s", dec->lat_why.c_str());
+  PKB_REQUIRE(dec->post.n_arcs >= 0, "pkb_decoder_posteriors_get: no pkb_decoder_posteriors since the latest finish");
+  pkb::Ctx *c = dec->c;
+  PKB_CUDA(cudaSetDevice(c->device));
+  PKB_TRY(pkb::posteriors_get(c, dec->post, arc_post_out, frame_post_out));
+  return pkb::check_device_error(c, "pkb_decoder_posteriors_get");
 }
 
 }  // extern "C"

@@ -1,0 +1,535 @@
+// Arc and frame posteriors over the kept records of a lattice (pkb_batch_posteriors,
+// pkb_decoder_posteriors): a forward-backward pass in the log semiring, one thread block per
+// utterance, in the fold order of include/pkb200.h.
+//
+// The block walks the groups eps(0), emit(0), eps(1), ... forward and then backward, with the
+// costs of two times live as per-state double arrays (in shared memory when they fit):
+//   emit(t) forward   the group's records are grouped by destination with a stable counting sort
+//                     (below), then one thread per destination folds its incoming records in
+//                     record order into alpha(t + 1, dst).
+//   eps(t)            Kahn levels over the group: a node is folded once every source (forward) or
+//                     every head (backward) is complete, so the fold order is fixed and the result
+//                     does not depend on scheduling. Nodes left over when the levels stop lie on a
+//                     cycle of epsilon records: the utterance fails with -8.
+//   backward          the records of a group are already grouped by source (the FST's arcs are
+//                     sorted by source state), so a node folds its outgoing epsilon records, then
+//                     its outgoing emitting records, from two contiguous ranges.
+// The forward pass saves alpha(t, src) per record (8 bytes), so the backward pass finishes each
+// record's posterior as soon as beta at its head is known. The frame posteriors of time t are the
+// emitting posteriors of the group grouped by pdf with the same stable sort, summed in record
+// order, thresholded and written in pdf order. The backward pass produces times in descending
+// order, so an utterance's entries are written from the end of its record range downwards and
+// gathered into (t, pdf) order afterwards. No float atomics: repeated calls are bit-identical.
+
+#include <math.h>
+
+#include <algorithm>
+#include <cub/block/block_radix_sort.cuh>
+#include <cub/block/block_scan.cuh>
+
+#include "decoder.cuh"
+
+namespace pkb {
+namespace {
+
+constexpr int kPoThreads = 512;
+constexpr int kPoItems = 4;                        // records per thread of a sort tile
+constexpr int kPoTile = kPoThreads * kPoItems;     // records per sort tile
+constexpr int kPoTileBits = 11;                    // log2(kPoTile)
+static_assert((1 << kPoTileBits) == kPoTile, "tile bits");
+constexpr size_t kPoSmemState = 48 << 10;          // per-state arrays go to shared memory up to this
+
+struct PostArgs {
+  const pkb_lattice_arc_t *arcs;
+  const long long *first, *n_arcs;
+  const double *best;
+  const float *final_w;
+  const int32_t *tid2pdf;
+  int num_states, num_pdfs, num_arcs, start, u0;
+  double as, gs;
+  float min_post;
+  char *work;               // per block: sort order and group posteriors [, per-state arrays]
+  size_t work_stride;
+  bool smem_state;          // per-state arrays in dynamic shared memory
+  double *alpha;            // alpha(t, src) of record first[u] + i at alpha[first[u] - rec0 + i]
+  long long rec0;
+  float *arc_post;          // [records]
+  pkb_frame_post_t *tail;   // [records]: utterance u's entries end at first[u] + n_arcs[u]
+  double *total;            // [n_utts]
+  long long *n_post;        // [n_utts]
+};
+
+__device__ __forceinline__ int group_of(const pkb_lattice_arc_t &r) { return 2 * r.t + (r.ilabel != 0); }
+
+// -log(exp(-a) + exp(-b)); +inf is the identity
+__device__ __forceinline__ double lse(double a, double b) {
+  const double m = fmin(a, b), M = fmax(a, b);
+  return M == INFINITY ? m : m - log1p(exp(m - M));
+}
+
+__device__ __forceinline__ double scaled_cost(const PostArgs &A, const pkb_lattice_arc_t &r) {
+  return __dadd_rn(__dmul_rn(A.gs, static_cast<double>(r.graph_cost)),
+                   __dmul_rn(A.as, static_cast<double>(r.acoustic_cost)));
+}
+
+__device__ __forceinline__ double arc_posterior(double total, double alpha, double c, double beta) {
+  return total < INFINITY ? exp(total - ((alpha + c) + beta)) : 0.0;
+}
+
+__device__ __forceinline__ int bit_width(unsigned x) { return 32 - __clz(x); }
+
+__global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
+  using Scan = cub::BlockScan<int, kPoThreads>;
+  using Sort = cub::BlockRadixSort<unsigned long long, kPoThreads, kPoItems>;
+  __shared__ union {
+    typename Scan::TempStorage scan;
+    typename Sort::TempStorage sort;
+  } tmp;
+  __shared__ int tkey[kPoTile];
+  __shared__ double s_total;
+  extern __shared__ double smem_state[];
+  const int w = blockIdx.x, u = A.u0 + w, tid = threadIdx.x;
+  const long long na = A.n_arcs[u];
+  if (na < 0) {
+    if (tid == 0) {
+      A.total[u] = NAN;
+      A.n_post[u] = na;
+    }
+    return;
+  }
+  const long long f0 = A.first[u];
+  if (!(A.best[u] < INFINITY)) {  // no complete path, so no records
+    for (long long i = tid; i < na; i += kPoThreads) A.arc_post[f0 + i] = 0.0f;
+    if (tid == 0) {
+      A.total[u] = INFINITY;
+      A.n_post[u] = 0;
+    }
+    return;
+  }
+  const pkb_lattice_arc_t *recs = A.arcs + f0;
+  double *alpha = A.alpha + (f0 - A.rec0);
+  const int S = A.num_states, P = A.num_pdfs, K = max(S, P), NA = A.num_arcs;
+  char *g = A.work + A.work_stride * w;
+  int *perm = reinterpret_cast<int *>(g);                                           // [NA]
+  double *pd = reinterpret_cast<double *>(g + ((sizeof(int) * NA + 7) & ~size_t(7)));  // [NA]
+  char *st = A.smem_state ? reinterpret_cast<char *>(smem_state) : reinterpret_cast<char *>(pd + NA);
+  double *X = reinterpret_cast<double *>(st);  // [S] costs of the current time
+  double *Y = X + S;                           // [S] costs of the neighbouring time
+  double *acc = Y + S;                         // [K] frame posteriors by pdf
+  int *done = reinterpret_cast<int *>(acc + K);  // [S] Kahn state: 0 open, 1 folded this level, 2 complete
+  int *fill = done + S;                        // [K]
+  int *seg = fill + K;                         // [K + 1]
+  int *eb = seg + K + 1, *ee = eb + S, *mb = ee + S, *me = mb + S;  // [S] each: runs by source
+
+  // the first index in [lo, min(na, lo + NA)] whose group is > grp (a group holds at most NA
+  // records); every thread probes once per round, so two rounds cover 2^18 records
+  auto group_end = [&](long long lo, int grp) {
+    long long a = lo, b = min(na, lo + NA);
+    while (b > a) {
+      const long long step = (b - a + kPoThreads - 1) / kPoThreads, p = a + tid * step;
+      const int k = __syncthreads_count(p < b && group_of(recs[p]) <= grp);
+      if (k == 0) break;
+      const long long nb = min(b, a + k * step);
+      a += (k - 1) * step + 1;
+      b = nb;
+    }
+    return a;
+  };
+  // Groups records [0, m) by key(i) in [0, K) stably: key k's records are perm[seg[k] .. seg[k + 1])
+  // in ascending order. Counts and a scan give the segments; then tiles of kPoTile records in
+  // order are radix-sorted by (key, index) and appended to their segments.
+  auto group_by_key = [&](int m, auto key) {
+    __syncthreads();
+    for (int k = tid; k < K; k += kPoThreads) fill[k] = 0;
+    __syncthreads();
+    for (int i = tid; i < m; i += kPoThreads) atomicAdd(&fill[key(i)], 1);
+    __syncthreads();
+    const int per = (K + kPoThreads - 1) / kPoThreads, k0 = min(K, tid * per), k1 = min(K, k0 + per);
+    int sum = 0;
+    for (int k = k0; k < k1; ++k) sum += fill[k];
+    int base = 0;
+    Scan(tmp.scan).ExclusiveSum(sum, base);
+    __syncthreads();
+    for (int k = k0; k < k1; ++k) {
+      const int c = fill[k];
+      seg[k] = base;
+      fill[k] = base;
+      base += c;
+    }
+    if (tid == 0) seg[K] = m;
+    const int end_bit = kPoTileBits + bit_width(static_cast<unsigned>(K));
+    for (int b0 = 0; b0 < m; b0 += kPoTile) {
+      unsigned long long keys[kPoItems];
+      for (int j = 0; j < kPoItems; ++j) {
+        const int li = tid * kPoItems + j;
+        keys[j] = b0 + li < m ? (static_cast<unsigned long long>(key(b0 + li)) << kPoTileBits) | li : ~0ull;
+      }
+      __syncthreads();
+      Sort(tmp.sort).Sort(keys, 0, end_bit);
+      for (int j = 0; j < kPoItems; ++j) {
+        const int r = tid * kPoItems + j;
+        tkey[r] = r < m - b0 ? static_cast<int>(keys[j] >> kPoTileBits) : -1;
+      }
+      __syncthreads();
+      // the first rank of each key's run in this tile moves its fill pointer back by that rank,
+      // every rank then lands at fill + rank, and the run's last rank moves it past the run
+      for (int j = 0; j < kPoItems; ++j) {
+        const int r = tid * kPoItems + j, k = tkey[r];
+        if (k >= 0 && (r == 0 || tkey[r - 1] != k)) fill[k] -= r;
+      }
+      __syncthreads();
+      for (int j = 0; j < kPoItems; ++j) {
+        const int r = tid * kPoItems + j, k = tkey[r];
+        if (k >= 0) perm[fill[k] + r] = b0 + static_cast<int>(keys[j] & (kPoTile - 1));
+      }
+      __syncthreads();
+      for (int j = 0; j < kPoItems; ++j) {
+        const int r = tid * kPoItems + j, k = tkey[r];
+        if (k >= 0 && (r == kPoTile - 1 || tkey[r + 1] != k)) fill[k] += r + 1;
+      }
+    }
+    __syncthreads();
+  };
+
+  // T: the last emitting record's t + 1 (records end with eps(T))
+  int T = 0;
+  if (na > 0) {
+    const pkb_lattice_arc_t last = recs[na - 1];
+    if (last.ilabel) {
+      T = last.t + 1;
+    } else {
+      const long long b = group_end(max(0ll, na - NA), 2 * last.t - 1);
+      T = b > 0 ? recs[b - 1].t + 1 : 0;
+    }
+  }
+
+  // ---- forward: alpha(t, .) in X
+  for (int s = tid; s < S; s += kPoThreads) X[s] = s == A.start ? 0.0 : INFINITY;
+  int err = 0;
+  long long pos = 0;
+  for (int t = 0;; ++t) {
+    const long long e_end = group_end(pos, 2 * t);
+    const int ne = static_cast<int>(e_end - pos);
+    if (ne > 0) {
+      const pkb_lattice_arc_t *E = recs + pos;
+      group_by_key(ne, [&](int i) { return E[i].dst; });
+      for (int s = tid; s < S; s += kPoThreads) done[s] = seg[s + 1] > seg[s] ? 0 : 2;
+      __syncthreads();
+      for (;;) {
+        for (int d = tid; d < S; d += kPoThreads) {
+          if (done[d]) continue;
+          bool ready = true;
+          for (int j = seg[d]; j < seg[d + 1] && ready; ++j) ready = done[E[perm[j]].src] == 2;
+          if (!ready) continue;
+          double a = X[d];
+          for (int j = seg[d]; j < seg[d + 1]; ++j) {
+            const pkb_lattice_arc_t &r = E[perm[j]];
+            a = lse(a, X[r.src] + scaled_cost(A, r));
+          }
+          X[d] = a;
+          done[d] = 1;
+        }
+        __syncthreads();
+        int progress = 0;
+        for (int d = tid; d < S; d += kPoThreads)
+          if (done[d] == 1) {
+            done[d] = 2;
+            progress = 1;
+          }
+        if (!__syncthreads_or(progress)) break;
+      }
+      int open = 0;
+      for (int d = tid; d < S && !open; d += kPoThreads) open = done[d] == 0;
+      if (__syncthreads_or(open)) {
+        err = 8;
+        break;
+      }
+    }
+    const long long m_end = t < T ? group_end(e_end, 2 * t + 1) : e_end;
+    for (long long i = pos + tid; i < m_end; i += kPoThreads) alpha[i] = X[recs[i].src];
+    if (t == T) break;
+    const int nm = static_cast<int>(m_end - e_end);
+    const pkb_lattice_arc_t *M = recs + e_end;
+    for (int s = tid; s < S; s += kPoThreads) Y[s] = INFINITY;
+    if (nm > 0) {
+      group_by_key(nm, [&](int i) { return M[i].dst; });
+      for (int d = tid; d < S; d += kPoThreads) {
+        if (seg[d + 1] == seg[d]) continue;
+        double a = INFINITY;
+        for (int j = seg[d]; j < seg[d + 1]; ++j) {
+          const pkb_lattice_arc_t &r = M[perm[j]];
+          a = lse(a, X[r.src] + scaled_cost(A, r));
+        }
+        Y[d] = a;
+      }
+    }
+    __syncthreads();
+    double *tx = X;
+    X = Y;
+    Y = tx;
+    pos = m_end;
+  }
+  if (err) {
+    for (long long i = tid; i < na; i += kPoThreads) A.arc_post[f0 + i] = NAN;
+    if (tid == 0) {
+      A.total[u] = NAN;
+      A.n_post[u] = -err;
+    }
+    return;
+  }
+  if (tid == 0) {
+    double tot = INFINITY;
+    for (int s = 0; s < S; ++s) {
+      const float f = A.final_w[s];
+      if (f < INFINITY) tot = lse(tot, X[s] + __dmul_rn(A.gs, static_cast<double>(f)));
+    }
+    s_total = tot;
+  }
+  __syncthreads();
+  const double total = s_total;
+
+  // ---- backward: beta(t, .) in X, beta(t + 1, .) in Y
+  long long end = na;
+  int nout = 0;
+  for (int t = T; t >= 0; --t) {
+    const long long m_beg = t < T ? group_end(max(0ll, end - NA), 2 * t) : end;
+    const long long e_beg = t > 0 ? group_end(max(0ll, m_beg - NA), 2 * t - 1) : 0;
+    const pkb_lattice_arc_t *E = recs + e_beg, *M = recs + m_beg;
+    const int ne = static_cast<int>(m_beg - e_beg), nm = static_cast<int>(end - m_beg);
+    if (nm > 0) {
+      // posteriors of emit(t), then its frame posteriors
+      for (int i = tid; i < nm; i += kPoThreads) {
+        const pkb_lattice_arc_t &r = M[i];
+        const double p = arc_posterior(total, alpha[m_beg + i], scaled_cost(A, r), Y[r.dst]);
+        pd[i] = p;
+        A.arc_post[f0 + m_beg + i] = static_cast<float>(p);
+      }
+      group_by_key(nm, [&](int i) { return A.tid2pdf[M[i].ilabel]; });
+      const int per = (P + kPoThreads - 1) / kPoThreads, k0 = min(P, tid * per), k1 = min(P, k0 + per);
+      int cnt = 0;
+      for (int k = k0; k < k1; ++k) {
+        if (seg[k + 1] == seg[k]) continue;
+        double sum = 0.0;
+        for (int j = seg[k]; j < seg[k + 1]; ++j) sum += pd[perm[j]];
+        acc[k] = sum;
+        cnt += static_cast<float>(sum) >= A.min_post;
+      }
+      int base = 0, kept = 0;
+      Scan(tmp.scan).ExclusiveSum(cnt, base, kept);
+      pkb_frame_post_t *out = A.tail + f0 + na - nout - kept;
+      for (int k = k0; k < k1; ++k) {
+        if (seg[k + 1] == seg[k]) continue;
+        const float v = static_cast<float>(acc[k]);
+        if (v >= A.min_post) out[base++] = pkb_frame_post_t{t, k, v};
+      }
+      nout += kept;
+    }
+    // beta(t, s): the final weight at T, then the outgoing epsilon and emitting records of s in
+    // record order
+    for (int s = tid; s < S; s += kPoThreads) {
+      eb[s] = ee[s] = mb[s] = me[s] = 0;
+      done[s] = 0;
+    }
+    __syncthreads();
+    for (int i = tid; i < ne; i += kPoThreads) {
+      const int s = E[i].src;
+      if (i == 0 || E[i - 1].src != s) eb[s] = i;
+      if (i == ne - 1 || E[i + 1].src != s) ee[s] = i + 1;
+    }
+    for (int i = tid; i < nm; i += kPoThreads) {
+      const int s = M[i].src;
+      if (i == 0 || M[i - 1].src != s) mb[s] = i;
+      if (i == nm - 1 || M[i + 1].src != s) me[s] = i + 1;
+    }
+    __syncthreads();
+    for (;;) {
+      for (int s = tid; s < S; s += kPoThreads) {
+        if (done[s]) continue;
+        bool ready = true;
+        for (int i = eb[s]; i < ee[s] && ready; ++i) ready = done[E[i].dst] == 2;
+        if (!ready) continue;
+        double b = INFINITY;
+        if (t == T) {
+          const float f = A.final_w[s];
+          if (f < INFINITY) b = __dmul_rn(A.gs, static_cast<double>(f));
+        }
+        for (int i = eb[s]; i < ee[s]; ++i) b = lse(b, scaled_cost(A, E[i]) + X[E[i].dst]);
+        for (int i = mb[s]; i < me[s]; ++i) b = lse(b, scaled_cost(A, M[i]) + Y[M[i].dst]);
+        X[s] = b;
+        done[s] = 1;
+      }
+      __syncthreads();
+      int progress = 0;
+      for (int s = tid; s < S; s += kPoThreads)
+        if (done[s] == 1) {
+          done[s] = 2;
+          progress = 1;
+        }
+      if (!__syncthreads_or(progress)) break;
+    }
+    for (int i = tid; i < ne; i += kPoThreads) {
+      const pkb_lattice_arc_t &r = E[i];
+      A.arc_post[f0 + e_beg + i] = static_cast<float>(arc_posterior(total, alpha[e_beg + i], scaled_cost(A, r), X[r.dst]));
+    }
+    __syncthreads();
+    double *tx = X;
+    X = Y;
+    Y = tx;
+    end = e_beg;
+  }
+  if (tid == 0) {
+    A.total[u] = total;
+    A.n_post[u] = nout;
+  }
+}
+
+// Moves utterance u's frame entries from the end of its record range to out + off[u].
+__global__ void posterior_gather_kernel(const pkb_frame_post_t *__restrict__ tail, const long long *__restrict__ first,
+                                        const long long *__restrict__ n_arcs, const long long *__restrict__ n_post,
+                                        const long long *__restrict__ off, pkb_frame_post_t *__restrict__ out) {
+  const int u = blockIdx.x;
+  const long long k = n_post[u];
+  if (k <= 0) return;
+  const pkb_frame_post_t *src = tail + first[u] + n_arcs[u] - k;
+  for (long long i = threadIdx.x; i < k; i += blockDim.x) out[off[u] + i] = src[i];
+}
+
+}  // namespace
+
+int check_posterior_args(float acoustic_scale, float graph_scale, float min_post, const void *total_out,
+                         const void *n_post_out, const char *who) {
+  PKB_REQUIRE(acoustic_scale > 0.0f && acoustic_scale < INFINITY,
+              "%s: acoustic_scale must be finite and > 0 (got %g)", who, acoustic_scale);
+  PKB_REQUIRE(graph_scale >= 0.0f && graph_scale < INFINITY, "%s: graph_scale must be finite and >= 0 (got %g)",
+              who, graph_scale);
+  PKB_REQUIRE(min_post >= 0.0f && min_post <= 1.0f, "%s: min_post must be in [0, 1] (got %g)", who, min_post);
+  PKB_REQUIRE(total_out && n_post_out, "%s: NULL output argument", who);
+  return PKB_OK;
+}
+
+int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, const int32_t *d_tid2pdf, int num_pdfs,
+                      float acoustic_scale, float graph_scale, float min_post, PosteriorResults *res,
+                      double *total_out, int64_t *n_post_out) {
+  res->n_arcs = -1;
+  res->n_frames = 0;
+  const int U = lr.n_utts;
+  if (U == 0) {
+    res->n_arcs = 0;
+    return PKB_OK;
+  }
+  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
+  std::vector<long long> na(U), first(U + 1, 0);
+  PKB_CUDA(cudaMemcpyAsync(na.data(), lr.n_arcs, sizeof(long long) * U, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  for (int u = 0; u < U; ++u) first[u + 1] = first[u] + std::max(na[u], 0ll);
+  const long long R = first[U];
+  const int S = fst->num_states, P = num_pdfs, K = std::max(S, P), NA = std::max(fst->num_arcs, 1);
+  PKB_REQUIRE(K < (1 << 30), "pkb posteriors: %d states or pdfs are too many", K);
+  // results: arc posteriors; per call: frame entries at the end of each record range, totals,
+  // codes and the entries' output offsets
+  PKB_TRY(res->arc.ensure(sizeof(float) * std::max(R, 1ll)));
+  const size_t tail_bytes = (sizeof(pkb_frame_post_t) * std::max(R, 1ll) + 7) & ~size_t(7);
+  DevBuf scratch;
+  PKB_TRY(scratch.ensure(tail_bytes + sizeof(double) * U + sizeof(long long) * (2 * U + 1)));
+  pkb_frame_post_t *d_tail = scratch.as<pkb_frame_post_t>();
+  double *d_total = reinterpret_cast<double *>(scratch.as<char>() + tail_bytes);
+  long long *d_npost = reinterpret_cast<long long *>(d_total + U);
+  long long *d_off = d_npost + U;
+  // per block: sort order and group posteriors (NA each), and the per-state arrays when they do
+  // not fit in shared memory
+  const size_t state_bytes = sizeof(double) * (2 * static_cast<size_t>(S) + K) +
+                             sizeof(int) * (5 * static_cast<size_t>(S) + 2 * static_cast<size_t>(K) + 1);
+  const bool smem_state = state_bytes <= kPoSmemState;
+  const size_t stride = ((((sizeof(int) * NA + 7) & ~size_t(7)) + sizeof(double) * NA +
+                          (smem_state ? 0 : state_bytes)) + 255) & ~size_t(255);
+  // utterances in waves whose alpha and workspace fit the budget
+  size_t free_b = 0, total_b = 0;
+  PKB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  const size_t budget = std::min<size_t>(free_b / 2, size_t(8) << 30);
+  std::vector<int> wave_start{0};
+  size_t wave_max = 0;
+  for (int u0 = 0; u0 < U;) {
+    int m = 0;
+    size_t bytes = 0;
+    while (u0 + m < U) {
+      const size_t add = stride + sizeof(double) * std::max(na[u0 + m], 0ll);
+      if (m > 0 && bytes + add > budget) break;
+      bytes += add;
+      ++m;
+    }
+    wave_max = std::max(wave_max, bytes);
+    u0 += m;
+    wave_start.push_back(u0);
+  }
+  DevBuf wave_buf;
+  PKB_TRY(wave_buf.ensure(wave_max));
+  // the static shared memory and the per-state arrays together can pass the default 48 KiB
+  if (smem_state)
+    PKB_CUDA(cudaFuncSetAttribute(posterior_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  static_cast<int>(state_bytes)));
+  PostArgs A{};
+  A.arcs = lr.arcs;
+  A.first = lr.first;
+  A.n_arcs = lr.n_arcs;
+  A.best = lr.best;
+  A.final_w = fst->d_final;
+  A.tid2pdf = d_tid2pdf;
+  A.num_states = S;
+  A.num_pdfs = P;
+  A.num_arcs = NA;
+  A.start = fst->start;
+  A.as = acoustic_scale;
+  A.gs = graph_scale;
+  A.min_post = min_post;
+  A.work_stride = stride;
+  A.smem_state = smem_state;
+  A.arc_post = res->arc.as<float>();
+  A.tail = d_tail;
+  A.total = d_total;
+  A.n_post = d_npost;
+  for (size_t i = 0; i + 1 < wave_start.size(); ++i) {
+    const int u0 = wave_start[i], m = wave_start[i + 1] - u0;
+    A.u0 = u0;
+    A.work = wave_buf.as<char>();
+    A.alpha = reinterpret_cast<double *>(wave_buf.as<char>() + stride * m);
+    A.rec0 = first[u0];
+    LaunchScope scope(c, PKB_KERNEL_MISC);
+    posterior_kernel<<<m, kPoThreads, smem_state ? state_bytes : 0, c->stream>>>(A);
+    PKB_CUDA(cudaGetLastError());
+  }
+  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
+  PKB_CUDA(cudaMemcpyAsync(total_out, d_total, sizeof(double) * U, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaMemcpyAsync(n_post_out, d_npost, sizeof(long long) * U, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  std::vector<long long> off(U);
+  long long n_frames = 0;
+  for (int u = 0; u < U; ++u) {
+    off[u] = n_frames;
+    n_frames += std::max<long long>(n_post_out[u], 0);
+  }
+  PKB_TRY(res->frames.ensure(sizeof(pkb_frame_post_t) * std::max(n_frames, 1ll)));
+  PKB_CUDA(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * U, cudaMemcpyHostToDevice, c->stream));
+  {
+    LaunchScope scope(c, PKB_KERNEL_MISC);
+    posterior_gather_kernel<<<U, 256, 0, c->stream>>>(d_tail, lr.first, lr.n_arcs, d_npost, d_off,
+                                                       res->frames.as<pkb_frame_post_t>());
+    PKB_CUDA(cudaGetLastError());
+  }
+  // the host copy of off must outlive the copy
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  res->n_arcs = R;
+  res->n_frames = n_frames;
+  return PKB_OK;
+}
+
+int posteriors_get(Ctx *c, const PosteriorResults &res, float *arc_post_out, pkb_frame_post_t *frame_post_out) {
+  if (arc_post_out && res.n_arcs > 0)
+    PKB_CUDA(cudaMemcpyAsync(arc_post_out, res.arc.p, sizeof(float) * res.n_arcs, cudaMemcpyDeviceToHost, c->stream));
+  if (frame_post_out && res.n_frames > 0)
+    PKB_CUDA(cudaMemcpyAsync(frame_post_out, res.frames.p, sizeof(pkb_frame_post_t) * res.n_frames,
+                             cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  return PKB_OK;
+}
+
+}  // namespace pkb
