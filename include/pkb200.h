@@ -297,7 +297,8 @@ typedef struct {           /* 28 bytes, no padding */
  * lattice pruned to lattice_beam (> 0, may be +inf) on the device. max_arcs: unpruned arcs per
  * utterance, 8 bytes of device log each (<= 0: (frames of the longest utterance + 1) x arcs of the
  * graph, which no utterance can exceed; a word loop keeps nearly all its arcs inside the beam, so a
- * caller short of memory passes less). n_arcs_out[u]: kept arcs, or a
+ * caller short of memory passes less; at most INT32_MAX - arcs of the graph, the default capped
+ * there). n_arcs_out[u]: kept arcs, or a
  * negative code (-1 tokens, -2 word records, -3 epsilon closure, -4 more than max_arcs arcs);
  * best_cost_out[u]: min over final nodes of alpha + final (+inf: no final node or a failed search).
  * Synchronous. */

@@ -693,18 +693,12 @@ class Batch:
         """The search of decode() keeping its lattice pruned to lattice_beam (pkb_batch_lattice):
         returns ([LATTICE_ARC_DTYPE array per utterance, None where the search failed],
         best costs as float64)."""
-        n = len(self.num_samples)
-        na = np.zeros(max(n, 1), np.int64)
-        best = np.zeros(max(n, 1), np.float64)
-        _check(self.ctx.lib.pkb_batch_lattice(self.h, fst.h, beam, lattice_beam, max_tokens, max_arcs,
-                                              na.ctypes.data, best.ctypes.data))
-        kept = np.maximum(na[:n], 0)
-        arcs = np.empty(max(int(kept.sum()), 1), LATTICE_ARC_DTYPE)
-        _check(self.ctx.lib.pkb_batch_lattice_get(self.h, arcs.ctypes.data))
-        off = np.concatenate([[0], np.cumsum(kept)])
-        lats = [None if na[u] < 0 else arcs[off[u]:off[u + 1]].copy() for u in range(n)]
-        self._lat_n = na[:n].copy()
-        return lats, best[:n].copy()
+        lib = self.ctx.lib
+        lats, best, self._lat_n = _lattices(
+            len(self.num_samples),
+            lambda na, bc: lib.pkb_batch_lattice(self.h, fst.h, beam, lattice_beam, max_tokens, max_arcs, na, bc),
+            lambda arcs: lib.pkb_batch_lattice_get(self.h, arcs))
+        return lats, best
 
     def nbest(self, fst, n=10, max_words=256):
         """N-best lists of distinct word sequences over the latest lattice() (pkb_batch_nbest; fst
@@ -864,14 +858,10 @@ class Decoder:
     def lattice(self):
         """The lattices of the latest finish(): ([LATTICE_ARC_DTYPE array per stream, None where it
         failed], best costs as float64), as Batch.lattice returns them."""
-        na = np.zeros(self.n_streams, np.int64)
-        best = np.zeros(self.n_streams, np.float64)
-        _check(self.ctx.lib.pkb_decoder_lattice(self.h, na.ctypes.data, best.ctypes.data))
-        kept = np.maximum(na, 0)
-        arcs = np.empty(max(int(kept.sum()), 1), LATTICE_ARC_DTYPE)
-        _check(self.ctx.lib.pkb_decoder_lattice_get(self.h, arcs.ctypes.data))
-        off = np.concatenate([[0], np.cumsum(kept)])
-        return [None if na[s] < 0 else arcs[off[s]:off[s + 1]].copy() for s in range(self.n_streams)], best
+        lib = self.ctx.lib
+        lats, best, _ = _lattices(self.n_streams, lambda na, bc: lib.pkb_decoder_lattice(self.h, na, bc),
+                                  lambda arcs: lib.pkb_decoder_lattice_get(self.h, arcs))
+        return lats, best
 
     def nbest(self, n=10, max_words=256):
         """Batch.nbest over the lattices of the latest finish() (pkb_decoder_nbest)."""
@@ -888,6 +878,24 @@ class Decoder:
                            lambda tot, npost: lib.pkb_decoder_posteriors(self.h, acoustic_scale, graph_scale,
                                                                         min_post, tot, npost),
                            lambda arc, fr: lib.pkb_decoder_posteriors_get(self.h, arc, fr))
+
+
+def _split(flat, counts):
+    """Per utterance the next max(counts[u], 0) entries of flat, or None where counts[u] < 0."""
+    off = np.concatenate([[0], np.cumsum(np.maximum(counts, 0))])
+    return [None if counts[u] < 0 else flat[off[u]:off[u + 1]].copy() for u in range(len(counts))]
+
+
+def _lattices(n_utts, call, get):
+    """Runs call(n_arcs, best_costs) and get(records) for n_utts utterances and unpacks them as
+    Batch.lattice returns them, with the record counts."""
+    na = np.zeros(max(n_utts, 1), np.int64)
+    best = np.zeros(max(n_utts, 1), np.float64)
+    _check(call(na.ctypes.data, best.ctypes.data))
+    na = na[:n_utts].copy()
+    arcs = np.empty(max(int(np.maximum(na, 0).sum()), 1), LATTICE_ARC_DTYPE)
+    _check(get(arcs.ctypes.data))
+    return _split(arcs, na), best[:n_utts].copy(), na
 
 
 def _nbest(n_utts, n, max_words, call):
@@ -919,16 +927,11 @@ def _posteriors(n_arcs, n_utts, call, get):
     _check(call(tot.ctypes.data, npost.ctypes.data))
     if len(n_arcs) != n_utts:
         raise PkbError(1, "posteriors: the record counts of the latest lattice() are unknown")
-    kept = np.maximum(n_arcs, 0)
-    nf = np.maximum(npost[:n_utts], 0)
-    arc = np.empty(max(int(kept.sum()), 1), np.float32)
-    fr = np.empty(max(int(nf.sum()), 1), FRAME_POST_DTYPE)
+    npost = npost[:n_utts]
+    arc = np.empty(max(int(np.maximum(n_arcs, 0).sum()), 1), np.float32)
+    fr = np.empty(max(int(np.maximum(npost, 0).sum()), 1), FRAME_POST_DTYPE)
     _check(get(arc.ctypes.data, fr.ctypes.data))
-    ao = np.concatenate([[0], np.cumsum(kept)])
-    fo = np.concatenate([[0], np.cumsum(nf)])
-    arcs = [None if n_arcs[u] < 0 else arc[ao[u]:ao[u + 1]].copy() for u in range(n_utts)]
-    frames = [None if npost[u] < 0 else fr[fo[u]:fo[u + 1]].copy() for u in range(n_utts)]
-    return tot[:n_utts].copy(), arcs, frames
+    return tot[:n_utts].copy(), _split(arc, n_arcs), _split(fr, npost)
 
 
 class Stream:

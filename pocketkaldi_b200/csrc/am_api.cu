@@ -281,12 +281,8 @@ struct pkb_batch {
   bool compact = false;             // nnet stage writes loglik16 + loglik_off instead of loglik
   pkb::DevBuf loglik16, loglik_off;
   pkb::DevBuf vit_work, vit_out, vit_tid2pdf;  // GPU Viterbi: workspace, results, device tid2pdf
-  pkb::DevBuf lat_log, lat_aux, lat_arcs;      // lattices: arc logs, offsets and results, kept arcs
-  int64_t lat_total = -1;                      // kept arcs of the latest pkb_batch_lattice
-  const pkb_fst *lat_fst = nullptr;            // its graph, while its records are valid
-  pkb::LatticeRecords lat_rec;                 // its records on the device
-  pkb::DevBuf nbest_work;                      // outputs of pkb_batch_nbest
-  pkb::PosteriorResults post;                  // results of pkb_batch_posteriors
+  pkb::DevBuf lat_log, lat_aux;                // lattice search: arc logs, offsets and results
+  pkb::LatticeResults lat;                     // of the latest pkb_batch_lattice
   Workspace ws;
   pkb::Refine rf;
   pkb::PaddedPlanes planes;
@@ -906,17 +902,14 @@ int pkb_batch_lattice(pkb_batch_t *b, const pkb_fst_t *fst, float beam, float la
   PKB_REQUIRE(!b->compact, "pkb_batch_lattice: reads the FP32 log-likelihoods (switch the compact output off)");
   PKB_REQUIRE(lattice_beam > 0.0f, "pkb_batch_lattice: lattice_beam must be > 0 (got %g)", lattice_beam);
   PKB_TRY(pkb::check_decode_graph(b->c, b->am, fst, "pkb_batch_lattice"));
+  const int n = b->meta.n_utts;
+  int t_max = 0;
+  for (int u = 0; u < n; ++u) t_max = std::max(t_max, b->meta.num_frames[u]);
+  pkb::Lattice lat{};
+  PKB_TRY(pkb::lattice_max_arcs(fst, t_max, max_arcs, "pkb_batch_lattice", &lat.max_arcs));
   Ctx *c = b->c;
   PKB_CUDA(cudaSetDevice(c->device));
-  b->lat_total = 0;
-  b->lat_fst = nullptr;
-  b->post.n_arcs = -1;
-  const int n = b->meta.n_utts;
-  if (n == 0) {
-    b->lat_fst = fst;
-    b->lat_rec = pkb::LatticeRecords{};
-    return PKB_OK;
-  }
+  b->lat.invalidate("the latest pkb_batch_lattice failed");
   pkb::ViterbiConfig cfg;
   if (beam > 0.0f) cfg.beam = beam;
   if (max_tokens > 0) cfg.max_tokens = max_tokens;
@@ -926,77 +919,37 @@ int pkb_batch_lattice(pkb_batch_t *b, const pkb_fst_t *fst, float beam, float la
     PKB_TRY(b->vit_tid2pdf.ensure(tid_bytes));
     PKB_CUDA(cudaMemcpyAsync(b->vit_tid2pdf.p, am->tid2pdf.data(), tid_bytes, cudaMemcpyHostToDevice, c->stream));
   }
-  int t_max = 0;
-  for (int u = 0; u < n; ++u) t_max = std::max(t_max, b->meta.num_frames[u]);
-  pkb::Lattice lat{};
-  // default: the most the search can log, every arc of the graph at every time of the longest
-  // utterance (1.84 M entries, 14.7 MB, for 10 s on the 40-word loop; 33 M, 267 MB, on the 180-word loop)
-  const int64_t bound = static_cast<int64_t>(t_max + 1) * std::max(fst->num_arcs, 1);
-  lat.max_arcs = max_arcs > 0 ? max_arcs : static_cast<int>(std::min<int64_t>(bound, INT32_MAX));
   lat.grp_stride = 2 * (t_max + 1);
   lat.beam = lattice_beam;
-  // per utterance: the log; group offsets; kept count, best cost and first output record
+  // per utterance: the log; group offsets; kept count and best cost
   PKB_TRY(b->lat_log.ensure(static_cast<size_t>(n) * lat.max_arcs * sizeof(unsigned long long)));
   const size_t grp_bytes = (static_cast<size_t>(n) * lat.grp_stride * sizeof(int) + 7) & ~static_cast<size_t>(7);
-  PKB_TRY(b->lat_aux.ensure(grp_bytes + 3 * sizeof(int64_t) * static_cast<size_t>(n)));
+  PKB_TRY(b->lat_aux.ensure(grp_bytes + 2 * sizeof(int64_t) * static_cast<size_t>(n)));
   lat.log = b->lat_log.as<unsigned long long>();
   lat.grp = b->lat_aux.as<int>();
   lat.n_out = reinterpret_cast<long long *>(b->lat_aux.as<char>() + grp_bytes);
   lat.best_out = reinterpret_cast<double *>(lat.n_out + n);
-  long long *d_first = lat.n_out + 2 * n;
   PKB_TRY(pkb::launch_lattice(c, fst, cfg, b->loglik.as<float>(), am->num_pdfs, b->ws.pad_off.as<int64_t>(),
                               b->meta.d_num_frames, n, b->vit_tid2pdf.as<int32_t>(), &b->vit_work, lat));
-  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
-  PKB_CUDA(cudaMemcpyAsync(n_arcs_out, lat.n_out, sizeof(int64_t) * n, cudaMemcpyDeviceToHost, c->stream));
-  PKB_CUDA(cudaMemcpyAsync(best_cost_out, lat.best_out, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream));
-  PKB_CUDA(cudaStreamSynchronize(c->stream));
-  PKB_TRY(pkb::check_device_error(c, "pkb_batch_lattice"));
-  // the kept arcs as records, every utterance's back to back
-  std::vector<long long> first(n);
-  int64_t total = 0;
-  for (int u = 0; u < n; ++u) {
-    first[u] = total;
-    total += std::max<int64_t>(n_arcs_out[u], 0);
-  }
-  PKB_TRY(b->lat_arcs.ensure(std::max<int64_t>(total, 1) * sizeof(pkb_lattice_arc_t)));
-  PKB_CUDA(cudaMemcpyAsync(d_first, first.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, c->stream));
-  PKB_TRY(pkb::lattice_expand(c, fst, lat, b->loglik.as<float>(), am->num_pdfs, b->ws.pad_off.as<int64_t>(), n,
-                              b->vit_tid2pdf.as<int32_t>(), d_first, b->lat_arcs.as<pkb_lattice_arc_t>()));
-  PKB_CUDA(cudaStreamSynchronize(c->stream));
-  PKB_TRY(pkb::check_device_error(c, "pkb_batch_lattice"));
-  b->lat_total = total;
-  b->lat_fst = fst;
-  b->lat_rec.arcs = b->lat_arcs.as<pkb_lattice_arc_t>();
-  b->lat_rec.first = d_first;
-  b->lat_rec.n_arcs = lat.n_out;
-  b->lat_rec.best = lat.best_out;
-  b->lat_rec.n_utts = n;
+  PKB_TRY(b->lat.expand(c, fst, lat, n, b->loglik.as<float>(), am->num_pdfs, b->ws.pad_off.as<int64_t>(),
+                        b->vit_tid2pdf.as<int32_t>(), "pkb_batch_lattice"));
+  memcpy(n_arcs_out, b->lat.n_arcs.data(), sizeof(int64_t) * n);
+  memcpy(best_cost_out, b->lat.best.data(), sizeof(double) * n);
   return PKB_OK;
 }
 
 int pkb_batch_lattice_get(pkb_batch_t *b, pkb_lattice_arc_t *arcs_out) {
   PKB_REQUIRE(b, "pkb_batch_lattice_get: the batch is NULL");
-  PKB_REQUIRE(b->lat_total >= 0, "pkb_batch_lattice_get: no pkb_batch_lattice on this batch yet");
-  if (b->lat_total == 0) return PKB_OK;
-  PKB_REQUIRE(arcs_out, "pkb_batch_lattice_get: NULL argument");
-  PKB_CUDA(cudaSetDevice(b->c->device));
-  PKB_CUDA(cudaMemcpyAsync(arcs_out, b->lat_arcs.p, sizeof(pkb_lattice_arc_t) * b->lat_total,
-                           cudaMemcpyDeviceToHost, b->c->stream));
-  PKB_CUDA(cudaStreamSynchronize(b->c->stream));
-  return pkb::check_device_error(b->c, "pkb_batch_lattice_get");
+  return b->lat.get(arcs_out, "pkb_batch_lattice_get");
 }
 
 int pkb_batch_nbest(pkb_batch_t *b, const pkb_fst_t *fst, int n, int max_words, int32_t *words_out,
                     int32_t *n_words_out, double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out) {
   PKB_REQUIRE(b && fst, "pkb_batch_nbest: NULL argument");
-  PKB_REQUIRE(b->lat_fst, "pkb_batch_nbest: no valid pkb_batch_lattice on this batch");
-  PKB_REQUIRE(b->lat_fst == fst, "pkb_batch_nbest: the FST is not the one of the latest pkb_batch_lattice");
-  PKB_TRY(pkb::check_nbest_args(n, max_words, words_out, n_words_out, graph_cost_out, acoustic_cost_out,
-                                n_hyps_out, "pkb_batch_nbest"));
-  PKB_CUDA(cudaSetDevice(b->c->device));
-  PKB_TRY(pkb::launch_nbest(b->c, fst, b->lat_rec, n, max_words, &b->nbest_work, words_out, n_words_out,
-                            graph_cost_out, acoustic_cost_out, n_hyps_out));
-  return pkb::check_device_error(b->c, "pkb_batch_nbest");
+  PKB_REQUIRE(b->lat.total < 0 || b->lat.fst == fst,
+              "pkb_batch_nbest: the FST is not the one of the latest pkb_batch_lattice");
+  return b->lat.nbest(n, max_words, words_out, n_words_out, graph_cost_out, acoustic_cost_out, n_hyps_out,
+                      "pkb_batch_nbest");
 }
 
 static_assert(sizeof(pkb_frame_post_t) == 12 && offsetof(pkb_frame_post_t, post) == 8,
@@ -1005,22 +958,14 @@ static_assert(sizeof(pkb_frame_post_t) == 12 && offsetof(pkb_frame_post_t, post)
 int pkb_batch_posteriors(pkb_batch_t *b, const pkb_fst_t *fst, float acoustic_scale, float graph_scale,
                          float min_post, double *total_out, int64_t *n_post_out) {
   PKB_REQUIRE(b && fst, "pkb_batch_posteriors: NULL argument");
-  PKB_REQUIRE(b->lat_fst, "pkb_batch_posteriors: no valid pkb_batch_lattice on this batch");
-  PKB_REQUIRE(b->lat_fst == fst, "pkb_batch_posteriors: the FST is not the one of the latest pkb_batch_lattice");
-  PKB_TRY(pkb::check_posterior_args(acoustic_scale, graph_scale, min_post, total_out, n_post_out,
-                                    "pkb_batch_posteriors"));
-  PKB_CUDA(cudaSetDevice(b->c->device));
-  PKB_TRY(pkb::launch_posteriors(b->c, fst, b->lat_rec, b->vit_tid2pdf.as<int32_t>(), b->am->num_pdfs,
-                                 acoustic_scale, graph_scale, min_post, &b->post, total_out, n_post_out));
-  return pkb::check_device_error(b->c, "pkb_batch_posteriors");
+  PKB_REQUIRE(b->lat.total < 0 || b->lat.fst == fst,
+              "pkb_batch_posteriors: the FST is not the one of the latest pkb_batch_lattice");
+  return b->lat.posteriors(acoustic_scale, graph_scale, min_post, total_out, n_post_out, "pkb_batch_posteriors");
 }
 
 int pkb_batch_posteriors_get(pkb_batch_t *b, float *arc_post_out, pkb_frame_post_t *frame_post_out) {
   PKB_REQUIRE(b, "pkb_batch_posteriors_get: the batch is NULL");
-  PKB_REQUIRE(b->post.n_arcs >= 0, "pkb_batch_posteriors_get: no pkb_batch_posteriors since the latest pkb_batch_lattice");
-  PKB_CUDA(cudaSetDevice(b->c->device));
-  PKB_TRY(pkb::posteriors_get(b->c, b->post, arc_post_out, frame_post_out));
-  return pkb::check_device_error(b->c, "pkb_batch_posteriors_get");
+  return b->lat.posteriors_get(arc_post_out, frame_post_out, "pkb_batch_posteriors_get");
 }
 
 // ---------------------------------------------------------------- fused host path

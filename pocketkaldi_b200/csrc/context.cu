@@ -33,6 +33,8 @@ int DevBuf::ensure(size_t bytes) {
   size_t want = (bytes + (size_t(1) << 20) - 1) & ~((size_t(1) << 20) - 1);
   cudaError_t e = cudaMalloc(&p, want);
   if (e != cudaSuccess) {
+    // the failure is returned here: clear it, or the next launch's error check reports it again
+    cudaGetLastError();
     p = nullptr;
     set_error("cudaMalloc(%zu bytes): %s", want, cudaGetErrorString(e));
     return PKB_ERR_CUDA;

@@ -1555,15 +1555,64 @@ int launch_lattice(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const f
                                   work, nullptr, nullptr, nullptr, Carry{}, lat);
 }
 
-int lattice_expand(Ctx *c, const pkb_fst *fst, const Lattice &lat, const float *d_loglik, int num_pdfs,
-                   const int64_t *d_row_off, int n_utts, const int32_t *d_tid2pdf, const long long *d_first,
-                   pkb_lattice_arc_t *d_out) {
-  if (n_utts == 0) return PKB_OK;
-  LaunchScope scope(c, PKB_KERNEL_MISC);
-  lattice_expand_kernel<<<n_utts, kVitThreads, 0, c->stream>>>(fst_dev(fst), lat, d_loglik, num_pdfs, d_row_off,
-                                                               d_tid2pdf, d_first, d_out);
-  PKB_CUDA(cudaGetLastError());
+int lattice_max_arcs(const pkb_fst *fst, int frames, int max_arcs, const char *who, int *out) {
+  const int cap = INT32_MAX - std::max(fst->num_arcs, 1);
+  PKB_REQUIRE(max_arcs <= cap, "%s: max_arcs %d is more than %d", who, max_arcs, cap);
+  // default: 1.84 M entries, 14.7 MB, for 10 s on the 40-word loop; 33 M, 267 MB, on the 180-word loop
+  const int64_t bound = static_cast<int64_t>(frames + 1) * std::max(fst->num_arcs, 1);
+  *out = max_arcs > 0 ? max_arcs : static_cast<int>(std::min<int64_t>(bound, cap));
   return PKB_OK;
+}
+
+int LatticeResults::expand(Ctx *ctx, const pkb_fst *graph, const Lattice &lat, int n_utts, const float *d_loglik,
+                           int pdfs, const int64_t *d_row_off, const int32_t *tid2pdf, const char *who) {
+  c = ctx;
+  fst = graph;
+  d_tid2pdf = tid2pdf;
+  num_pdfs = pdfs;
+  const size_t U = n_utts;
+  n_arcs.resize(U);
+  first.resize(U);
+  best.resize(U);
+  if (U == 0) {
+    total = 0;
+    return PKB_OK;
+  }
+  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
+  PKB_CUDA(cudaMemcpyAsync(n_arcs.data(), lat.n_out, sizeof(int64_t) * U, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaMemcpyAsync(best.data(), lat.best_out, sizeof(double) * U, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  PKB_TRY(check_device_error(c, who));
+  int64_t sum = 0;
+  for (size_t u = 0; u < U; ++u) {
+    first[u] = sum;
+    sum += std::max<int64_t>(n_arcs[u], 0);
+  }
+  PKB_TRY(arcs.ensure(std::max<int64_t>(sum, 1) * sizeof(pkb_lattice_arc_t)));
+  PKB_TRY(meta.ensure(3 * sizeof(int64_t) * U));
+  PKB_CUDA(cudaMemcpyAsync(d_n_arcs(), n_arcs.data(), sizeof(int64_t) * U, cudaMemcpyHostToDevice, c->stream));
+  PKB_CUDA(cudaMemcpyAsync(d_first(), first.data(), sizeof(long long) * U, cudaMemcpyHostToDevice, c->stream));
+  PKB_CUDA(cudaMemcpyAsync(d_best(), best.data(), sizeof(double) * U, cudaMemcpyHostToDevice, c->stream));
+  {
+    LaunchScope scope(c, PKB_KERNEL_MISC);
+    lattice_expand_kernel<<<n_utts, kVitThreads, 0, c->stream>>>(fst_dev(fst), lat, d_loglik, num_pdfs, d_row_off,
+                                                                 d_tid2pdf, d_first(), arcs.as<pkb_lattice_arc_t>());
+    PKB_CUDA(cudaGetLastError());
+  }
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  PKB_TRY(check_device_error(c, who));
+  total = sum;
+  return PKB_OK;
+}
+
+int LatticeResults::get(pkb_lattice_arc_t *arcs_out, const char *who) const {
+  PKB_REQUIRE(total >= 0, "%s: no lattice: %s", who, why.c_str());
+  if (total == 0) return PKB_OK;
+  PKB_REQUIRE(arcs_out, "%s: NULL argument", who);
+  PKB_CUDA(cudaSetDevice(c->device));
+  PKB_CUDA(cudaMemcpyAsync(arcs_out, arcs.p, sizeof(pkb_lattice_arc_t) * total, cudaMemcpyDeviceToHost, c->stream));
+  PKB_CUDA(cudaStreamSynchronize(c->stream));
+  return check_device_error(c, who);
 }
 
 int ResumableSearch::setup(Ctx *ctx, const pkb_fst *graph, const ViterbiConfig &config, const int32_t *tid2pdf,
@@ -1611,27 +1660,22 @@ int ResumableSearch::setup(Ctx *ctx, const pkb_fst *graph, const ViterbiConfig &
 
 int ResumableSearch::set_lattice(float lattice_beam, int max_frames, int max_arcs) {
   lat = Lattice{};
-  lat_first = nullptr;
   lat_row_off = nullptr;
-  for (DevBuf *b : {&lat_log, &lat_aux, &lat_rows, &lat_arcs}) b->release();
+  for (DevBuf *b : {&lat_log, &lat_aux, &lat_rows}) b->release();
   if (lattice_beam == 0.0f) return PKB_OK;
   Lattice l{};
-  l.max_frames = max_frames > 0 ? max_frames : 6000;
-  // as pkb_batch_lattice: the most the search can log in an utterance of max_frames frames, capped
-  // so that the log count (an int that passes max_arcs by at most one group) cannot wrap
-  const int64_t bound = static_cast<int64_t>(l.max_frames + 1) * std::max(fst->num_arcs, 1);
-  l.max_arcs = max_arcs > 0 ? max_arcs
-                            : static_cast<int>(std::min<int64_t>(bound, INT32_MAX - std::max(fst->num_arcs, 1)));
+  l.max_frames = max_frames;
+  l.max_arcs = max_arcs;
   l.grp_stride = 2 * (l.max_frames + 1);
   l.beam = lattice_beam;
-  // per stream: the log; the row store; then group offsets, state, kept count, best cost, first
-  // record and row offset
+  // per stream: the log; the row store; then group offsets, state, kept count, best cost and row
+  // offset
   const size_t S = n;
   const size_t grp_bytes = (S * l.grp_stride * sizeof(int) + 7) & ~static_cast<size_t>(7);
   const size_t state_bytes = (S * 2 * sizeof(int) + 7) & ~static_cast<size_t>(7);
   int rc = lat_log.ensure(S * l.max_arcs * sizeof(unsigned long long));
   if (rc == PKB_OK) rc = lat_rows.ensure(S * l.max_frames * num_pdfs * sizeof(float));
-  if (rc == PKB_OK) rc = lat_aux.ensure(grp_bytes + state_bytes + 4 * S * sizeof(int64_t));
+  if (rc == PKB_OK) rc = lat_aux.ensure(grp_bytes + state_bytes + 3 * S * sizeof(int64_t));
   if (rc == PKB_OK) {
     char *p = lat_aux.as<char>();
     l.log = lat_log.as<unsigned long long>();
@@ -1640,19 +1684,15 @@ int ResumableSearch::set_lattice(float lattice_beam, int max_frames, int max_arc
     l.state = reinterpret_cast<int *>(p); p += state_bytes;
     l.n_out = reinterpret_cast<long long *>(p); p += S * sizeof(int64_t);
     l.best_out = reinterpret_cast<double *>(p); p += S * sizeof(int64_t);
-    lat_first = reinterpret_cast<long long *>(p); p += S * sizeof(int64_t);
     lat_row_off = reinterpret_cast<int64_t *>(p);
     std::vector<int64_t> off(S);
     for (size_t s = 0; s < S; ++s) off[s] = static_cast<int64_t>(s) * l.max_frames;
     rc = upload(c, lat_row_off, off.data(), S * sizeof(int64_t));
   }
   if (rc != PKB_OK) {
-    // the decoder stays usable without lattices (and the failed allocation is not reported again
-    // by the next launch's error check)
-    cudaGetLastError();
-    lat_first = nullptr;
+    // the decoder stays usable without lattices
     lat_row_off = nullptr;
-    for (DevBuf *b : {&lat_log, &lat_aux, &lat_rows, &lat_arcs}) b->release();
+    for (DevBuf *b : {&lat_log, &lat_aux, &lat_rows}) b->release();
     return rc;
   }
   lat = l;
@@ -1682,26 +1722,6 @@ int ResumableSearch::finish() {
   }
   return launch_plan<true, false>(c, fst, plan, cfg, nullptr, num_pdfs, nullptr, nullptr, n,
                                   d_tid2pdf.as<int32_t>(), &work, f_words, f_nw, f_weight, a, Lattice{});
-}
-
-int ResumableSearch::expand_lattice(int64_t *n_out, double *best_out, int64_t *total) {
-  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
-  PKB_CUDA(cudaMemcpyAsync(n_out, lat.n_out, sizeof(int64_t) * n, cudaMemcpyDeviceToHost, c->stream));
-  PKB_CUDA(cudaMemcpyAsync(best_out, lat.best_out, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream));
-  PKB_CUDA(cudaStreamSynchronize(c->stream));
-  std::vector<long long> first(n);
-  int64_t sum = 0;
-  for (int s = 0; s < n; ++s) {
-    first[s] = sum;
-    sum += std::max<int64_t>(n_out[s], 0);
-  }
-  PKB_TRY(lat_arcs.ensure(std::max<int64_t>(sum, 1) * sizeof(pkb_lattice_arc_t)));
-  PKB_CUDA(cudaMemcpyAsync(lat_first, first.data(), sizeof(long long) * n, cudaMemcpyHostToDevice, c->stream));
-  PKB_TRY(lattice_expand(c, fst, lat, lat.rows, num_pdfs, lat_row_off, n, d_tid2pdf.as<int32_t>(), lat_first,
-                         lat_arcs.as<pkb_lattice_arc_t>()));
-  PKB_CUDA(cudaStreamSynchronize(c->stream));
-  *total = sum;
-  return PKB_OK;
 }
 
 }  // namespace pkb

@@ -101,34 +101,20 @@ int launch_viterbi(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const f
                    int32_t *d_n_words, float *d_weight);
 
 // The search of launch_viterbi in lattice mode: per utterance lat.n_out / lat.best_out and the kept
-// arcs in lat.log (see Lattice). lattice_expand then writes utterance u's kept arcs as records from
-// out + first[u] on.
+// arcs in lat.log (see Lattice); LatticeResults::expand turns them into records.
 int launch_lattice(Ctx *c, const pkb_fst *fst, const ViterbiConfig &cfg, const float *d_loglik, int num_pdfs,
                    const int64_t *d_row_off, const int32_t *d_num_frames, int n_utts, const int32_t *d_tid2pdf,
                    DevBuf *work, const Lattice &lat);
-int lattice_expand(Ctx *c, const pkb_fst *fst, const Lattice &lat, const float *d_loglik, int num_pdfs,
-                   const int64_t *d_row_off, int n_utts, const int32_t *d_tid2pdf, const long long *d_first,
-                   pkb_lattice_arc_t *d_out);
+// Log entries per utterance of a lattice search over `frames` frames: max_arcs, or for max_arcs <= 0
+// the most the search can log, (frames + 1) x arcs of the graph. The log count is an int that passes
+// max_arcs by at most one group (at most the graph's arcs), so the default is capped at
+// INT32_MAX - arcs and a larger max_arcs is rejected.
+int lattice_max_arcs(const pkb_fst *fst, int frames, int max_arcs, const char *who, int *out);
 
-// The kept records of the latest lattice call, as the search left them on the device: utterance u's
-// n_arcs[u] records (or its negative code) from arcs + first[u] on, and its best cost.
-struct LatticeRecords {
-  const pkb_lattice_arc_t *arcs = nullptr;
-  const long long *first = nullptr, *n_arcs = nullptr;
-  const double *best = nullptr;
-  int n_utts = 0;
-};
-
-// N-best lists of distinct word sequences over the records of every utterance (nbest.cu), with the
-// arguments and host outputs of pkb_batch_nbest. work keeps the outputs and statistics; the
-// per-block lists (2 x states x n x 24 bytes) and word-history tables are allocated per call.
-int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, int max_words, DevBuf *work,
-                 int32_t *words_out, int32_t *n_words_out, double *graph_cost_out, double *acoustic_cost_out,
-                 int32_t *n_hyps_out);
-// The argument checks shared by pkb_batch_nbest and pkb_decoder_nbest.
-int check_nbest_args(int n, int max_words, const void *words_out, const void *n_words_out,
-                     const void *graph_cost_out, const void *acoustic_cost_out, const void *n_hyps_out,
-                     const char *who);
+// Utterances in waves whose bytes (bytes[u] per utterance) stay within 8 GiB or half the free device
+// memory, whichever is less, with at least one utterance each: wave i is [starts[i], starts[i + 1]).
+// *most (if not NULL): the bytes of the largest wave.
+int plan_waves(const std::vector<size_t> &bytes, std::vector<int> *starts, size_t *most);
 
 // Results of the latest posteriors call, kept on the device for the _get call: one float per
 // record, and every utterance's frame entries back to back.
@@ -137,17 +123,52 @@ struct PosteriorResults {
   int64_t n_arcs = -1;   // records covered (-1: no valid results)
   int64_t n_frames = 0;  // frame entries
 };
-// Arc and frame posteriors over the records of every utterance (posterior.cu), with the arguments
-// and host outputs of pkb_batch_posteriors; d_tid2pdf maps input labels to pdfs in [0, num_pdfs).
-// Alpha (8 bytes per record) and the per-block workspace are allocated per call, in waves.
-int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, const int32_t *d_tid2pdf, int num_pdfs,
-                      float acoustic_scale, float graph_scale, float min_post, PosteriorResults *res,
-                      double *total_out, int64_t *n_post_out);
-// The argument checks shared by pkb_batch_posteriors and pkb_decoder_posteriors.
-int check_posterior_args(float acoustic_scale, float graph_scale, float min_post, const void *total_out,
-                         const void *n_post_out, const char *who);
-// Copies the results out (either output may be NULL).
-int posteriors_get(Ctx *c, const PosteriorResults &res, float *arc_post_out, pkb_frame_post_t *frame_post_out);
+
+// The lattice of the latest search of a batch or decoder and what is computed from it: utterance u's
+// n_arcs[u] kept records (or its negative code) from arcs + first[u] on, and its best cost. Every
+// operation takes the name of its entry point for its messages and checks the results are valid.
+struct LatticeResults {
+  Ctx *c = nullptr;
+  const pkb_fst *fst = nullptr;          // the graph the records belong to
+  const int32_t *d_tid2pdf = nullptr;    // its input labels' pdfs, in [0, num_pdfs)
+  int num_pdfs = 0;
+  DevBuf arcs;                           // the records, every utterance's back to back
+  DevBuf meta;                           // device copy of n_arcs, first and best
+  std::vector<int64_t> n_arcs;
+  std::vector<long long> first;
+  std::vector<double> best;
+  int64_t total = -1;                    // records (-1: not valid, for the reason in why)
+  std::string why = "no lattice search yet";
+  DevBuf nbest_work;                     // outputs of nbest
+  PosteriorResults post;                 // results of posteriors, valid as the records are
+
+  long long *d_n_arcs() const { return meta.as<long long>(); }
+  long long *d_first() const { return d_n_arcs() + n_arcs.size(); }
+  double *d_best() const { return reinterpret_cast<double *>(d_first() + n_arcs.size()); }
+  void invalidate(std::string reason) {
+    total = -1;
+    why = std::move(reason);
+    post.n_arcs = -1;
+  }
+  // After launch_lattice (or the finish of a resumable search) over n_utts utterances whose rows
+  // start at d_loglik + d_row_off[u] * num_pdfs: copies lat.n_out / lat.best_out to the host and
+  // writes the kept arcs as records. Valid when it returns PKB_OK.
+  int expand(Ctx *ctx, const pkb_fst *graph, const Lattice &lat, int n_utts, const float *d_loglik, int pdfs,
+             const int64_t *d_row_off, const int32_t *tid2pdf, const char *who);
+  int get(pkb_lattice_arc_t *arcs_out, const char *who) const;
+  // N-best lists of distinct word sequences per utterance (nbest.cu), with the arguments and host
+  // outputs of pkb_batch_nbest. nbest_work keeps the outputs and statistics; the per-block lists
+  // (2 x states x n x 24 bytes) and word-history tables are allocated per call.
+  int nbest(int n, int max_words, int32_t *words_out, int32_t *n_words_out, double *graph_cost_out,
+            double *acoustic_cost_out, int32_t *n_hyps_out, const char *who);
+  // Arc and frame posteriors per utterance (posterior.cu), with the arguments and host outputs of
+  // pkb_batch_posteriors. Alpha (8 bytes per record) and the per-block workspace are allocated per
+  // call, in waves.
+  int posteriors(float acoustic_scale, float graph_scale, float min_post, double *total_out, int64_t *n_post_out,
+                 const char *who);
+  // Copies the results of the latest posteriors out (either output may be NULL).
+  int posteriors_get(float *arc_post_out, pkb_frame_post_t *frame_post_out, const char *who);
+};
 
 // The resumable search behind pkb_decoder: n streams, one thread block each, whose tokens and word
 // records stay in global memory between launches. advance() decodes the next rows of every stream
@@ -167,21 +188,17 @@ struct ResumableSearch {
   int32_t *f_words = nullptr, *f_nw = nullptr;
   float *f_weight = nullptr;
   // lattice mode (set_lattice): lat.log == nullptr when off. lat_aux holds the group offsets, the
-  // per-stream state, the finish results and the row offsets / first records of lattice_expand.
+  // per-stream state, the finish results and the row offsets of the row store.
   Lattice lat{};
-  DevBuf lat_log, lat_aux, lat_rows, lat_arcs;
-  long long *lat_first = nullptr;
+  DevBuf lat_log, lat_aux, lat_rows;
   int64_t *lat_row_off = nullptr;
   int setup(Ctx *ctx, const pkb_fst *graph, const ViterbiConfig &config, const int32_t *tid2pdf, int n_tids,
             int pdfs, int streams);
-  // lattice_beam > 0 switches lattice mode on (buffers for max_frames frames and max_arcs log
-  // entries per stream), 0 off. Only between utterances.
+  // lattice_beam > 0 switches lattice mode on (buffers for max_frames > 0 frames and max_arcs > 0
+  // log entries per stream), 0 off. Only between utterances.
   int set_lattice(float lattice_beam, int max_frames, int max_arcs);
   int advance(const float *d_loglik, int frame_stride, const int32_t *d_n_frames, int uniform_frames);
   int finish();
-  // after a finish in lattice mode: the kept arcs of every stream as records in lat_arcs, back to
-  // back; n_out / best_out on the host. Returns the total in *total.
-  int expand_lattice(int64_t *n_out, double *best_out, int64_t *total);
 };
 
 // Checks shared by pkb_batch_decode and pkb_decoder_create / _finish: the FST is from context c, the
@@ -204,13 +221,7 @@ struct pkb_decoder {
   pkb_stream *st = nullptr;     // attached stream (pkb_stream_set_decoder)
   bool flushed = false;         // the attached stream was flushed: finish before its next push
   bool in_utt = false;          // an advance, push or flush since create or the last finish
-  // results of the latest finish in lattice mode, valid until the next advance, push or flush
-  int64_t lat_total = -1;       // records in search.lat_arcs (-1: none valid, for the reason in lat_why)
-  std::string lat_why = "no pkb_decoder_finish yet";
-  std::vector<int64_t> lat_n;
-  std::vector<double> lat_best;
-  pkb::DevBuf nbest_work;       // outputs of pkb_decoder_nbest
-  pkb::PosteriorResults post;   // results of pkb_decoder_posteriors, valid as the lattice results are
+  pkb::LatticeResults lat;      // of the latest finish in lattice mode, valid until the next advance, push or flush
   pkb_decoder() = default;
   pkb_decoder(const pkb_decoder &) = delete;
   pkb_decoder &operator=(const pkb_decoder &) = delete;

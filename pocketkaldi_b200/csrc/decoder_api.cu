@@ -27,16 +27,6 @@ int check_decode_outputs(int max_words, const void *words_out, const void *n_wor
   return PKB_OK;
 }
 
-int check_nbest_args(int n, int max_words, const void *words_out, const void *n_words_out,
-                     const void *graph_cost_out, const void *acoustic_cost_out, const void *n_hyps_out,
-                     const char *who) {
-  PKB_REQUIRE(n >= 1 && n <= 1024, "%s: n must be in [1, 1024] (got %d)", who, n);
-  PKB_REQUIRE(max_words > 0, "%s: max_words must be > 0 (got %d)", who, max_words);
-  PKB_REQUIRE(words_out && n_words_out && graph_cost_out && acoustic_cost_out && n_hyps_out,
-              "%s: NULL output argument", who);
-  return PKB_OK;
-}
-
 int decoder_enqueue_advance(pkb_decoder *dec, const float *d_rows, int frame_stride, const int32_t *d_n_frames,
                             int uniform_frames) {
   PKB_TRY(dec->search.advance(d_rows, frame_stride, d_n_frames, uniform_frames));
@@ -47,8 +37,7 @@ int decoder_enqueue_advance(pkb_decoder *dec, const float *d_rows, int frame_str
 
 void decoder_begin_step(pkb_decoder *dec) {
   dec->in_utt = true;
-  dec->lat_total = -1;
-  dec->lat_why = "an advance, push or flush came after the latest pkb_decoder_finish";
+  dec->lat.invalidate("an advance, push or flush came after the latest pkb_decoder_finish");
 }
 
 }  // namespace pkb
@@ -152,23 +141,14 @@ int pkb_decoder_finish(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words_
   PKB_CUDA(cudaStreamSynchronize(c->stream));
   dec->flushed = false;
   dec->in_utt = false;
-  dec->lat_total = -1;
-  dec->lat_why = "the latest pkb_decoder_finish ran without lattices";
-  dec->post.n_arcs = -1;
+  dec->lat.invalidate("the latest pkb_decoder_finish ran without lattices");
   PKB_TRY(pkb::check_device_error(c, "pkb_decoder_finish"));
-  if (r.lat.log) {
-    // the words above are complete and the utterance is over: a lattice that cannot be expanded
-    // (the records of a large graph can take gigabytes) is reported by pkb_decoder_lattice instead
-    dec->lat_n.resize(S);
-    dec->lat_best.resize(S);
-    int64_t total = 0;
-    if (r.expand_lattice(dec->lat_n.data(), dec->lat_best.data(), &total) == PKB_OK) {
-      dec->lat_total = total;
-    } else {
-      dec->lat_why = std::string("expanding the lattices of the latest pkb_decoder_finish failed: ") + pkb_last_error();
-      cudaGetLastError();
-    }
-  }
+  // the words above are complete and the utterance is over: a lattice that cannot be expanded (the
+  // records of a large graph can take gigabytes) is reported by pkb_decoder_lattice instead
+  if (r.lat.log && dec->lat.expand(c, r.fst, r.lat, dec->n, r.lat.rows, r.num_pdfs, r.lat_row_off,
+                                   r.d_tid2pdf.as<int32_t>(), "pkb_decoder_finish") != PKB_OK)
+    dec->lat.invalidate(std::string("expanding the lattices of the latest pkb_decoder_finish failed: ") +
+                        pkb_last_error());
   return PKB_OK;
 }
 
@@ -176,9 +156,9 @@ int pkb_decoder_set_lattice(pkb_decoder_t *dec, float lattice_beam, int max_fram
   PKB_REQUIRE(dec, "pkb_decoder_set_lattice: decoder is NULL");
   PKB_REQUIRE(lattice_beam >= 0.0f, "pkb_decoder_set_lattice: lattice_beam must be >= 0 (got %g)", lattice_beam);
   PKB_REQUIRE(max_frames <= (1 << 24), "pkb_decoder_set_lattice: max_frames %d is more than %d", max_frames, 1 << 24);
-  // the log count is an int and passes max_arcs by at most one group (at most the graph's arcs)
-  const int arcs_cap = INT32_MAX - std::max(dec->search.fst->num_arcs, 1);
-  PKB_REQUIRE(max_arcs <= arcs_cap, "pkb_decoder_set_lattice: max_arcs %d is more than %d", max_arcs, arcs_cap);
+  const int frames = max_frames > 0 ? max_frames : 6000;
+  int arcs = 0;
+  PKB_TRY(pkb::lattice_max_arcs(dec->search.fst, frames, max_arcs, "pkb_decoder_set_lattice", &arcs));
   PKB_REQUIRE(!dec->in_utt,
               "pkb_decoder_set_lattice: only between utterances (after create or pkb_decoder_finish)");
   pkb::Ctx *c = dec->c;
@@ -187,80 +167,40 @@ int pkb_decoder_set_lattice(pkb_decoder_t *dec, float lattice_beam, int max_fram
   // the attached stream's captured pushes launch the advance with the old lattice arguments (or
   // none): they are captured again
   if (dec->st) pkb::stream_drop_graphs(dec->st);
-  dec->lat_total = -1;
-  dec->lat_why = "pkb_decoder_set_lattice came after the latest pkb_decoder_finish";
-  return dec->search.set_lattice(lattice_beam, max_frames, max_arcs);
+  dec->lat.invalidate("pkb_decoder_set_lattice came after the latest pkb_decoder_finish");
+  dec->lat.arcs.release();
+  return dec->search.set_lattice(lattice_beam, frames, arcs);
 }
 
 int pkb_decoder_lattice(pkb_decoder_t *dec, int64_t *n_arcs_out, double *best_cost_out) {
   PKB_REQUIRE(dec && n_arcs_out && best_cost_out, "pkb_decoder_lattice: NULL argument");
-  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_lattice: no lattice: %s", dec->lat_why.c_str());
-  memcpy(n_arcs_out, dec->lat_n.data(), sizeof(int64_t) * dec->n);
-  memcpy(best_cost_out, dec->lat_best.data(), sizeof(double) * dec->n);
+  PKB_REQUIRE(dec->lat.total >= 0, "pkb_decoder_lattice: no lattice: %s", dec->lat.why.c_str());
+  memcpy(n_arcs_out, dec->lat.n_arcs.data(), sizeof(int64_t) * dec->n);
+  memcpy(best_cost_out, dec->lat.best.data(), sizeof(double) * dec->n);
   return PKB_OK;
 }
 
 int pkb_decoder_lattice_get(pkb_decoder_t *dec, pkb_lattice_arc_t *arcs_out) {
   PKB_REQUIRE(dec, "pkb_decoder_lattice_get: decoder is NULL");
-  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_lattice_get: no lattice: %s", dec->lat_why.c_str());
-  if (dec->lat_total == 0) return PKB_OK;
-  PKB_REQUIRE(arcs_out, "pkb_decoder_lattice_get: NULL argument");
-  pkb::Ctx *c = dec->c;
-  PKB_CUDA(cudaSetDevice(c->device));
-  PKB_CUDA(cudaMemcpyAsync(arcs_out, dec->search.lat_arcs.p, sizeof(pkb_lattice_arc_t) * dec->lat_total,
-                           cudaMemcpyDeviceToHost, c->stream));
-  PKB_CUDA(cudaStreamSynchronize(c->stream));
-  return pkb::check_device_error(c, "pkb_decoder_lattice_get");
+  return dec->lat.get(arcs_out, "pkb_decoder_lattice_get");
 }
 
 int pkb_decoder_nbest(pkb_decoder_t *dec, int n, int max_words, int32_t *words_out, int32_t *n_words_out,
                       double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out) {
   PKB_REQUIRE(dec, "pkb_decoder_nbest: decoder is NULL");
-  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_nbest: no lattice: %s", dec->lat_why.c_str());
-  PKB_TRY(pkb::check_nbest_args(n, max_words, words_out, n_words_out, graph_cost_out, acoustic_cost_out,
-                                n_hyps_out, "pkb_decoder_nbest"));
-  pkb::Ctx *c = dec->c;
-  PKB_CUDA(cudaSetDevice(c->device));
-  const pkb::ResumableSearch &r = dec->search;
-  pkb::LatticeRecords lr;
-  lr.arcs = r.lat_arcs.as<pkb_lattice_arc_t>();
-  lr.first = r.lat_first;
-  lr.n_arcs = r.lat.n_out;
-  lr.best = r.lat.best_out;
-  lr.n_utts = dec->n;
-  PKB_TRY(pkb::launch_nbest(c, r.fst, lr, n, max_words, &dec->nbest_work, words_out, n_words_out, graph_cost_out,
-                            acoustic_cost_out, n_hyps_out));
-  return pkb::check_device_error(c, "pkb_decoder_nbest");
+  return dec->lat.nbest(n, max_words, words_out, n_words_out, graph_cost_out, acoustic_cost_out, n_hyps_out,
+                        "pkb_decoder_nbest");
 }
 
 int pkb_decoder_posteriors(pkb_decoder_t *dec, float acoustic_scale, float graph_scale, float min_post,
                            double *total_out, int64_t *n_post_out) {
   PKB_REQUIRE(dec, "pkb_decoder_posteriors: decoder is NULL");
-  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_posteriors: no lattice: %s", dec->lat_why.c_str());
-  PKB_TRY(pkb::check_posterior_args(acoustic_scale, graph_scale, min_post, total_out, n_post_out,
-                                    "pkb_decoder_posteriors"));
-  pkb::Ctx *c = dec->c;
-  PKB_CUDA(cudaSetDevice(c->device));
-  const pkb::ResumableSearch &r = dec->search;
-  pkb::LatticeRecords lr;
-  lr.arcs = r.lat_arcs.as<pkb_lattice_arc_t>();
-  lr.first = r.lat_first;
-  lr.n_arcs = r.lat.n_out;
-  lr.best = r.lat.best_out;
-  lr.n_utts = dec->n;
-  PKB_TRY(pkb::launch_posteriors(c, r.fst, lr, r.d_tid2pdf.as<int32_t>(), r.num_pdfs, acoustic_scale, graph_scale,
-                                 min_post, &dec->post, total_out, n_post_out));
-  return pkb::check_device_error(c, "pkb_decoder_posteriors");
+  return dec->lat.posteriors(acoustic_scale, graph_scale, min_post, total_out, n_post_out, "pkb_decoder_posteriors");
 }
 
 int pkb_decoder_posteriors_get(pkb_decoder_t *dec, float *arc_post_out, pkb_frame_post_t *frame_post_out) {
   PKB_REQUIRE(dec, "pkb_decoder_posteriors_get: decoder is NULL");
-  PKB_REQUIRE(dec->lat_total >= 0, "pkb_decoder_posteriors_get: no lattice: %s", dec->lat_why.c_str());
-  PKB_REQUIRE(dec->post.n_arcs >= 0, "pkb_decoder_posteriors_get: no pkb_decoder_posteriors since the latest finish");
-  pkb::Ctx *c = dec->c;
-  PKB_CUDA(cudaSetDevice(c->device));
-  PKB_TRY(pkb::posteriors_get(c, dec->post, arc_post_out, frame_post_out));
-  return pkb::check_device_error(c, "pkb_decoder_posteriors_get");
+  return dec->lat.posteriors_get(arc_post_out, frame_post_out, "pkb_decoder_posteriors_get");
 }
 
 }  // extern "C"

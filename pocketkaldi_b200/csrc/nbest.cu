@@ -461,11 +461,35 @@ __global__ void __launch_bounds__(kNbThreads) nbest_kernel(NbestArgs A) {
 
 }  // namespace
 
-int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, int max_words, DevBuf *work,
-                 int32_t *words_out, int32_t *n_words_out, double *graph_cost_out, double *acoustic_cost_out,
-                 int32_t *n_hyps_out) {
-  const int U = lr.n_utts;
+int plan_waves(const std::vector<size_t> &bytes, std::vector<int> *starts, size_t *most) {
+  size_t free_b = 0, total_b = 0;
+  PKB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+  const size_t budget = std::min<size_t>(free_b / 2, size_t(8) << 30);
+  const int U = static_cast<int>(bytes.size());
+  starts->assign(1, 0);
+  size_t top = 0;
+  for (int u0 = 0; u0 < U;) {
+    int m = 0;
+    size_t sum = 0;
+    while (u0 + m < U && (m == 0 || sum + bytes[u0 + m] <= budget)) sum += bytes[u0 + m++];
+    top = std::max(top, sum);
+    u0 += m;
+    starts->push_back(u0);
+  }
+  if (most) *most = top;
+  return PKB_OK;
+}
+
+int LatticeResults::nbest(int n, int max_words, int32_t *words_out, int32_t *n_words_out,
+                          double *graph_cost_out, double *acoustic_cost_out, int32_t *n_hyps_out, const char *who) {
+  PKB_REQUIRE(total >= 0, "%s: no lattice: %s", who, why.c_str());
+  PKB_REQUIRE(n >= 1 && n <= 1024, "%s: n must be in [1, 1024] (got %d)", who, n);
+  PKB_REQUIRE(max_words > 0, "%s: max_words must be > 0 (got %d)", who, max_words);
+  PKB_REQUIRE(words_out && n_words_out && graph_cost_out && acoustic_cost_out && n_hyps_out,
+              "%s: NULL output argument", who);
+  const int U = static_cast<int>(n_arcs.size());
   if (U == 0) return PKB_OK;
+  PKB_CUDA(cudaSetDevice(c->device));
   const int S = fst->num_states;
   const int scratch = std::max(fst->num_arcs, S) + S + 1;  // merge cursors at seg[d] + d
   // sizes: statistics and flags, then the outputs
@@ -479,8 +503,8 @@ int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, in
   const size_t stride = ((2 * sizeof(Entry) * S * static_cast<size_t>(n) + sizeof(int) * (4 * S + 1) +
                           2 * sizeof(int) * scratch) + 255) & ~static_cast<size_t>(255);
   // the first pass sizes the word-history stores
-  PKB_TRY(work->ensure(fixed));
-  char *p = work->as<char>();
+  PKB_TRY(nbest_work.ensure(fixed));
+  char *p = nbest_work.as<char>();
   long long *d_stats = reinterpret_cast<long long *>(p); p += stats_bytes;
   int *d_flags = reinterpret_cast<int *>(p); p += flag_bytes;
   int32_t *d_words = reinterpret_cast<int32_t *>(p); p += words_bytes;
@@ -492,9 +516,9 @@ int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, in
   PKB_CUDA(cudaMemsetAsync(d_words, 0, fixed - stats_bytes - flag_bytes, c->stream));
   {
     LaunchScope scope(c, PKB_KERNEL_MISC);
-    nbest_scan_kernel<<<U + 1, kNbThreads, 0, c->stream>>>(lr.arcs, lr.first, lr.n_arcs, U, fst->d_arc_dst,
-                                                          fst->d_arc_il, fst->d_arc_ol, fst->num_arcs, S, d_flags,
-                                                          d_stats);
+    nbest_scan_kernel<<<U + 1, kNbThreads, 0, c->stream>>>(arcs.as<pkb_lattice_arc_t>(), d_first(), d_n_arcs(), U,
+                                                          fst->d_arc_dst, fst->d_arc_il, fst->d_arc_ol,
+                                                          fst->num_arcs, S, d_flags, d_stats);
     PKB_CUDA(cudaGetLastError());
   }
   std::vector<long long> stats(3 * (U + 1));
@@ -514,26 +538,20 @@ int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, in
     slots[u] = sl;
   }
   // utterances in waves whose workspace fits the budget
-  size_t free_b = 0, total_b = 0;
-  PKB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-  const size_t budget = std::min<size_t>(free_b / 2, size_t(8) << 30);
+  std::vector<size_t> bytes(U);
+  for (int u = 0; u < U; ++u) bytes[u] = stride + slots[u] * sizeof(unsigned long long) + 4 * sizeof(long long);
+  std::vector<int> wave_start;
+  PKB_TRY(plan_waves(bytes, &wave_start, nullptr));
   DevBuf wave_buf;
-  for (int u0 = 0; u0 < U;) {
-    int m = 0;
-    size_t bytes = 0;
-    while (u0 + m < U) {
-      const size_t add = stride + slots[u0 + m] * sizeof(unsigned long long) + 4 * sizeof(long long);
-      if (m > 0 && bytes + add > budget) break;
-      bytes += add;
-      ++m;
-    }
+  for (size_t w = 0; w + 1 < wave_start.size(); ++w) {
+    const int u0 = wave_start[w], m = wave_start[w + 1] - u0;
     const size_t key_bytes = [&] {
       size_t s = 0;
       for (int i = 0; i < m; ++i) s += slots[u0 + i] * sizeof(unsigned long long);
       return s;
     }();
-    const size_t meta = (sizeof(long long) * (2 * m + 1) + sizeof(int) * m + 255) & ~static_cast<size_t>(255);
-    PKB_TRY(wave_buf.ensure(stride * m + key_bytes + meta));
+    const size_t meta_bytes = (sizeof(long long) * (2 * m + 1) + sizeof(int) * m + 255) & ~static_cast<size_t>(255);
+    PKB_TRY(wave_buf.ensure(stride * m + key_bytes + meta_bytes));
     char *q = wave_buf.as<char>();
     NbestArgs A{};
     A.work = q; q += stride * m;
@@ -550,10 +568,10 @@ int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, in
     A.hist_count = reinterpret_cast<int *>(d_meta + 2 * m + 1);
     PKB_CUDA(cudaMemsetAsync(A.hist_count, 0, sizeof(int) * m, c->stream));
     PKB_CUDA(cudaMemsetAsync(A.keys, 0xff, key_bytes, c->stream));
-    A.arcs = lr.arcs;
-    A.first = lr.first;
-    A.n_arcs = lr.n_arcs;
-    A.best = lr.best;
+    A.arcs = arcs.as<pkb_lattice_arc_t>();
+    A.first = d_first();
+    A.n_arcs = d_n_arcs();
+    A.best = d_best();
     A.stats = d_stats;
     A.final_w = fst->d_final;
     A.num_states = S;
@@ -575,7 +593,6 @@ int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, in
     }
     // the host copy of hm must outlive the copy
     PKB_CUDA(cudaStreamSynchronize(c->stream));
-    u0 += m;
   }
   PKB_CUDA(cudaMemcpyAsync(words_out, d_words, words_bytes, cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaMemcpyAsync(n_words_out, d_nw, sizeof(int32_t) * U * static_cast<size_t>(n), cudaMemcpyDeviceToHost,
@@ -584,7 +601,7 @@ int launch_nbest(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, int n, in
   PKB_CUDA(cudaMemcpyAsync(acoustic_cost_out, d_ac, cost_bytes, cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaMemcpyAsync(n_hyps_out, d_nh, sizeof(int32_t) * U, cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaStreamSynchronize(c->stream));
-  return PKB_OK;
+  return check_device_error(c, who);
 }
 
 }  // namespace pkb

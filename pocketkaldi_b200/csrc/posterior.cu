@@ -396,38 +396,29 @@ __global__ void posterior_gather_kernel(const pkb_frame_post_t *__restrict__ tai
 
 }  // namespace
 
-int check_posterior_args(float acoustic_scale, float graph_scale, float min_post, const void *total_out,
-                         const void *n_post_out, const char *who) {
+int LatticeResults::posteriors(float acoustic_scale, float graph_scale, float min_post, double *total_out,
+                               int64_t *n_post_out, const char *who) {
+  PKB_REQUIRE(total >= 0, "%s: no lattice: %s", who, why.c_str());
   PKB_REQUIRE(acoustic_scale > 0.0f && acoustic_scale < INFINITY,
               "%s: acoustic_scale must be finite and > 0 (got %g)", who, acoustic_scale);
   PKB_REQUIRE(graph_scale >= 0.0f && graph_scale < INFINITY, "%s: graph_scale must be finite and >= 0 (got %g)",
               who, graph_scale);
   PKB_REQUIRE(min_post >= 0.0f && min_post <= 1.0f, "%s: min_post must be in [0, 1] (got %g)", who, min_post);
   PKB_REQUIRE(total_out && n_post_out, "%s: NULL output argument", who);
-  return PKB_OK;
-}
-
-int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, const int32_t *d_tid2pdf, int num_pdfs,
-                      float acoustic_scale, float graph_scale, float min_post, PosteriorResults *res,
-                      double *total_out, int64_t *n_post_out) {
-  res->n_arcs = -1;
-  res->n_frames = 0;
-  const int U = lr.n_utts;
+  post.n_arcs = -1;
+  post.n_frames = 0;
+  const int U = static_cast<int>(n_arcs.size());
   if (U == 0) {
-    res->n_arcs = 0;
+    post.n_arcs = 0;
     return PKB_OK;
   }
-  static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
-  std::vector<long long> na(U), first(U + 1, 0);
-  PKB_CUDA(cudaMemcpyAsync(na.data(), lr.n_arcs, sizeof(long long) * U, cudaMemcpyDeviceToHost, c->stream));
-  PKB_CUDA(cudaStreamSynchronize(c->stream));
-  for (int u = 0; u < U; ++u) first[u + 1] = first[u] + std::max(na[u], 0ll);
-  const long long R = first[U];
+  PKB_CUDA(cudaSetDevice(c->device));
+  const long long R = total;
   const int S = fst->num_states, P = num_pdfs, K = std::max(S, P), NA = std::max(fst->num_arcs, 1);
   PKB_REQUIRE(K < (1 << 30), "pkb posteriors: %d states or pdfs are too many", K);
   // results: arc posteriors; per call: frame entries at the end of each record range, totals,
   // codes and the entries' output offsets
-  PKB_TRY(res->arc.ensure(sizeof(float) * std::max(R, 1ll)));
+  PKB_TRY(post.arc.ensure(sizeof(float) * std::max(R, 1ll)));
   const size_t tail_bytes = (sizeof(pkb_frame_post_t) * std::max(R, 1ll) + 7) & ~size_t(7);
   DevBuf scratch;
   PKB_TRY(scratch.ensure(tail_bytes + sizeof(double) * U + sizeof(long long) * (2 * U + 1)));
@@ -443,24 +434,11 @@ int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, cons
   const size_t stride = ((((sizeof(int) * NA + 7) & ~size_t(7)) + sizeof(double) * NA +
                           (smem_state ? 0 : state_bytes)) + 255) & ~size_t(255);
   // utterances in waves whose alpha and workspace fit the budget
-  size_t free_b = 0, total_b = 0;
-  PKB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-  const size_t budget = std::min<size_t>(free_b / 2, size_t(8) << 30);
-  std::vector<int> wave_start{0};
+  std::vector<size_t> bytes(U);
+  for (int u = 0; u < U; ++u) bytes[u] = stride + sizeof(double) * std::max<int64_t>(n_arcs[u], 0);
+  std::vector<int> wave_start;
   size_t wave_max = 0;
-  for (int u0 = 0; u0 < U;) {
-    int m = 0;
-    size_t bytes = 0;
-    while (u0 + m < U) {
-      const size_t add = stride + sizeof(double) * std::max(na[u0 + m], 0ll);
-      if (m > 0 && bytes + add > budget) break;
-      bytes += add;
-      ++m;
-    }
-    wave_max = std::max(wave_max, bytes);
-    u0 += m;
-    wave_start.push_back(u0);
-  }
+  PKB_TRY(plan_waves(bytes, &wave_start, &wave_max));
   DevBuf wave_buf;
   PKB_TRY(wave_buf.ensure(wave_max));
   // the static shared memory and the per-state arrays together can pass the default 48 KiB
@@ -468,10 +446,10 @@ int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, cons
     PKB_CUDA(cudaFuncSetAttribute(posterior_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(state_bytes)));
   PostArgs A{};
-  A.arcs = lr.arcs;
-  A.first = lr.first;
-  A.n_arcs = lr.n_arcs;
-  A.best = lr.best;
+  A.arcs = arcs.as<pkb_lattice_arc_t>();
+  A.first = d_first();
+  A.n_arcs = d_n_arcs();
+  A.best = d_best();
   A.final_w = fst->d_final;
   A.tid2pdf = d_tid2pdf;
   A.num_states = S;
@@ -483,7 +461,7 @@ int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, cons
   A.min_post = min_post;
   A.work_stride = stride;
   A.smem_state = smem_state;
-  A.arc_post = res->arc.as<float>();
+  A.arc_post = post.arc.as<float>();
   A.tail = d_tail;
   A.total = d_total;
   A.n_post = d_npost;
@@ -507,29 +485,33 @@ int launch_posteriors(Ctx *c, const pkb_fst *fst, const LatticeRecords &lr, cons
     off[u] = n_frames;
     n_frames += std::max<long long>(n_post_out[u], 0);
   }
-  PKB_TRY(res->frames.ensure(sizeof(pkb_frame_post_t) * std::max(n_frames, 1ll)));
+  PKB_TRY(post.frames.ensure(sizeof(pkb_frame_post_t) * std::max(n_frames, 1ll)));
   PKB_CUDA(cudaMemcpyAsync(d_off, off.data(), sizeof(long long) * U, cudaMemcpyHostToDevice, c->stream));
   {
     LaunchScope scope(c, PKB_KERNEL_MISC);
-    posterior_gather_kernel<<<U, 256, 0, c->stream>>>(d_tail, lr.first, lr.n_arcs, d_npost, d_off,
-                                                       res->frames.as<pkb_frame_post_t>());
+    posterior_gather_kernel<<<U, 256, 0, c->stream>>>(d_tail, d_first(), d_n_arcs(), d_npost, d_off,
+                                                       post.frames.as<pkb_frame_post_t>());
     PKB_CUDA(cudaGetLastError());
   }
   // the host copy of off must outlive the copy
   PKB_CUDA(cudaStreamSynchronize(c->stream));
-  res->n_arcs = R;
-  res->n_frames = n_frames;
-  return PKB_OK;
+  post.n_arcs = R;
+  post.n_frames = n_frames;
+  return check_device_error(c, who);
 }
 
-int posteriors_get(Ctx *c, const PosteriorResults &res, float *arc_post_out, pkb_frame_post_t *frame_post_out) {
-  if (arc_post_out && res.n_arcs > 0)
-    PKB_CUDA(cudaMemcpyAsync(arc_post_out, res.arc.p, sizeof(float) * res.n_arcs, cudaMemcpyDeviceToHost, c->stream));
-  if (frame_post_out && res.n_frames > 0)
-    PKB_CUDA(cudaMemcpyAsync(frame_post_out, res.frames.p, sizeof(pkb_frame_post_t) * res.n_frames,
+int LatticeResults::posteriors_get(float *arc_post_out, pkb_frame_post_t *frame_post_out, const char *who) {
+  PKB_REQUIRE(total >= 0, "%s: no lattice: %s", who, why.c_str());
+  PKB_REQUIRE(post.n_arcs >= 0, "%s: no posteriors since the latest lattice", who);
+  PKB_CUDA(cudaSetDevice(c->device));
+  if (arc_post_out && post.n_arcs > 0)
+    PKB_CUDA(cudaMemcpyAsync(arc_post_out, post.arc.p, sizeof(float) * post.n_arcs, cudaMemcpyDeviceToHost,
+                             c->stream));
+  if (frame_post_out && post.n_frames > 0)
+    PKB_CUDA(cudaMemcpyAsync(frame_post_out, post.frames.p, sizeof(pkb_frame_post_t) * post.n_frames,
                              cudaMemcpyDeviceToHost, c->stream));
   PKB_CUDA(cudaStreamSynchronize(c->stream));
-  return PKB_OK;
+  return check_device_error(c, who);
 }
 
 }  // namespace pkb

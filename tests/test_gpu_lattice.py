@@ -430,6 +430,8 @@ def test_invalid_uses_are_rejected(ctx):
     for lb in (0.0, -1.0, float("nan")):
         with pytest.raises(pk.PkbError):
             b.lattice(fst, lattice_beam=lb)
+    with pytest.raises(pk.PkbError):
+        b.lattice(fst, max_arcs=2 ** 31 - 1)   # the log count must not wrap
     b.set_compact(True)
     with pytest.raises(pk.PkbError):
         b.lattice(fst)
@@ -444,6 +446,37 @@ def test_invalid_uses_are_rejected(ctx):
         b2.lattice(fst)
     b2.close()
     bare.close()
+    fst.close()
+    am.close()
+
+
+@pytest.mark.gpu
+def test_a_failed_lattice_invalidates_its_results_and_leaves_the_batch_usable(ctx):
+    import torch
+    am, fst, _, _ = make_model(ctx, "loop")
+    # a log of utterances x max_arcs x 8 bytes above the card's memory: cudaMalloc refuses at once
+    max_arcs = 1 << 30
+    n = torch.cuda.mem_get_info(0)[1] // (8 * max_arcs) + 2
+    b, _ = batch_of(ctx, am, [4000] * n)
+    hyps, wts = b.decode(fst)
+    lats, best = b.lattice(fst, lattice_beam=4.0)
+    assert b.nbest(fst) and b.posteriors(fst)
+    na = np.zeros(n, np.int64)
+    bc = np.zeros(n, np.float64)
+    assert ctx.lib.pkb_batch_lattice(b.h, fst.h, 0.0, 4.0, 0, max_arcs, na.ctypes.data, bc.ctypes.data) != 0
+    arcs = np.empty(max(1, sum(len(x) for x in lats if x is not None)), pk.LATTICE_ARC_DTYPE)
+    assert ctx.lib.pkb_batch_lattice_get(b.h, arcs.ctypes.data) != 0
+    with pytest.raises(pk.PkbError):
+        b.nbest(fst)
+    with pytest.raises(pk.PkbError):
+        b.posteriors(fst)
+    assert ctx.lib.pkb_batch_posteriors_get(b.h, None, None) != 0
+    hyps2, wts2 = b.decode(fst)
+    assert hyps2 == hyps and wts2.tobytes() == wts.tobytes()
+    lats2, best2 = b.lattice(fst, lattice_beam=4.0)
+    assert all(x is y is None or same_records(x, y) for x, y in zip(lats2, lats))
+    assert best2.tobytes() == best.tobytes()
+    b.close()
     fst.close()
     am.close()
 
