@@ -261,8 +261,9 @@ int pkb_loglik16_expand(const uint16_t *h, const float *off, int64_t n_frames, i
  * utterance of a batch, one thread block per utterance, reading the log-likelihood rows where
  * pkb_batch_run left them in HBM: the [frames x pdfs] matrix never crosses PCIe and no host core
  * walks it. Costs, the beam (16 in the reference) and the best-path rule are the reference's;
- * differences (tightest instead of running cutoff, hard token capacity instead of the sampled
- * max-active estimate, tie-breaking) are listed in pocketkaldi_b200/csrc/decoder.cu. */
+ * differences (tightest instead of running cutoff, an exact optional max-active limit instead of
+ * the reference's sampled estimate, a hard token capacity, tie-breaking) are listed in
+ * pocketkaldi_b200/csrc/decoder.cu. */
 typedef struct pkb_fst pkb_fst_t;
 /* Fst::Read (src/fst.cc:29-92): "pk::fst_0" file. */
 int pkb_fst_load(pkb_ctx_t *ctx, const char *path, pkb_fst_t **fst);
@@ -280,6 +281,15 @@ void pkb_fst_destroy(pkb_fst_t *fst);
  * frame; 0 selects 4096); weight_out[u] = Hypothesis::weight(). Synchronous. */
 int pkb_batch_decode(pkb_batch_t *batch, const pkb_fst_t *fst, float beam, int max_tokens,
                      int max_words, int32_t *words_out, int32_t *n_words_out, float *weight_out);
+/* Max-active pruning (Kaldi's --max-active) for the later pkb_batch_decode and pkb_batch_lattice
+ * calls of this batch: on a frame with more than max_active tokens whose max_active-th smallest
+ * cost c_k is below best + beam, only the tokens of cost <= c_k are expanded (every tie at c_k) and
+ * the beam of the next frame's bound narrows to min(beam, (c_k - best) + 0.5). The best token is
+ * always expanded; the lattice holds what the pruned search relaxed. max_active = 0 (the default)
+ * switches it off; with it off, or on frames of at most max_active tokens, results are exactly those
+ * of the beam alone. It bounds the tokens expanded, not those created: max_tokens still applies.
+ * Negative values are rejected. */
+int pkb_batch_set_max_active(pkb_batch_t *batch, int max_active);
 
 /* ---- lattices of the batch search -------------------------------------------------------------
  * Every arc the search of pkb_batch_decode relaxed under its beam, kept when the best complete path
@@ -425,6 +435,12 @@ int pkb_decoder_finish(pkb_decoder_t *dec, int32_t *words_out, int32_t *n_words_
  * pkb_decoder_finish); an attached stream captures its CUDA graphs again. A failed allocation
  * leaves the decoder working without lattices. */
 int pkb_decoder_set_lattice(pkb_decoder_t *dec, float lattice_beam, int max_frames, int max_arcs);
+/* pkb_batch_set_max_active for the decoder's streams (0 after create): results stay bit-identical
+ * to pkb_batch_decode / pkb_batch_lattice with the same max_active, however the rows are split (each
+ * advance keeps every token of its last frame; the limit applies when the next frame expands them).
+ * Only between utterances (after create or pkb_decoder_finish); an attached stream captures its
+ * CUDA graphs again. Negative values are rejected. */
+int pkb_decoder_set_max_active(pkb_decoder_t *dec, int max_active);
 /* Per stream, for the latest finish: kept arcs or a negative code (those of pkb_batch_lattice, and
  * -5 more than max_frames frames; a lattice error fails only that stream's lattice) and the best
  * cost. Valid until the next advance, push or flush; rejected after one, or when the latest finish

@@ -109,6 +109,7 @@ _SIGNATURES = [
     ("pkb_fst_create", C.c_int, [_VP, C.c_int, C.c_int, _VP, _VP, C.c_int, _VP, C.POINTER(_VP)]),
     ("pkb_fst_destroy", None, [_VP]),
     ("pkb_batch_decode", C.c_int, [_VP, _VP, C.c_float, C.c_int, C.c_int, _VP, _VP, _VP]),
+    ("pkb_batch_set_max_active", C.c_int, [_VP, C.c_int]),
     ("pkb_batch_lattice", C.c_int, [_VP, _VP, C.c_float, C.c_float, C.c_int, C.c_int, _VP, _VP]),
     ("pkb_batch_lattice_get", C.c_int, [_VP, _VP]),
     ("pkb_batch_nbest", C.c_int, [_VP, _VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
@@ -121,6 +122,7 @@ _SIGNATURES = [
     ("pkb_decoder_partial", C.c_int, [_VP, _VP, _VP, _VP, _VP]),
     ("pkb_decoder_finish", C.c_int, [_VP, _VP, _VP, _VP]),
     ("pkb_decoder_set_lattice", C.c_int, [_VP, C.c_float, C.c_int, C.c_int]),
+    ("pkb_decoder_set_max_active", C.c_int, [_VP, C.c_int]),
     ("pkb_decoder_lattice", C.c_int, [_VP, _VP, _VP]),
     ("pkb_decoder_lattice_get", C.c_int, [_VP, _VP]),
     ("pkb_decoder_nbest", C.c_int, [_VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
@@ -689,6 +691,11 @@ class Batch:
         hyps = [None if nw[u] < 0 else [int(x) for x in words[u, :min(int(nw[u]), max_words)]] for u in range(n)]
         return hyps, wt[:n].copy()
 
+    def set_max_active(self, max_active):
+        """Expand at most max_active tokens per frame (ties at the cutoff included) in the later
+        decode() and lattice() calls (pkb_batch_set_max_active); 0 switches the limit off."""
+        _check(self.ctx.lib.pkb_batch_set_max_active(self.h, max_active))
+
     def lattice(self, fst, lattice_beam=8.0, beam=0.0, max_tokens=0, max_arcs=0):
         """The search of decode() keeping its lattice pruned to lattice_beam (pkb_batch_lattice):
         returns ([LATTICE_ARC_DTYPE array per utterance, None where the search failed],
@@ -854,6 +861,11 @@ class Decoder:
         Batch.lattice over the same rows (pkb_decoder_set_lattice); 0 switches lattices off. Only
         between utterances."""
         _check(self.ctx.lib.pkb_decoder_set_lattice(self.h, lattice_beam, max_frames, max_arcs))
+
+    def set_max_active(self, max_active):
+        """Batch.set_max_active for the decoder's streams (pkb_decoder_set_max_active). Only between
+        utterances."""
+        _check(self.ctx.lib.pkb_decoder_set_max_active(self.h, max_active))
 
     def lattice(self):
         """The lattices of the latest finish(): ([LATTICE_ARC_DTYPE array per stream, None where it

@@ -283,6 +283,7 @@ struct pkb_batch {
   pkb::DevBuf vit_work, vit_out, vit_tid2pdf;  // GPU Viterbi: workspace, results, device tid2pdf
   pkb::DevBuf lat_log, lat_aux;                // lattice search: arc logs, offsets and results
   pkb::LatticeResults lat;                     // of the latest pkb_batch_lattice
+  int max_active = 0;                          // pkb_batch_set_max_active
   Workspace ws;
   pkb::Refine rf;
   pkb::PaddedPlanes planes;
@@ -869,6 +870,7 @@ int pkb_batch_decode(pkb_batch_t *b, const pkb_fst_t *fst, float beam, int max_t
   if (beam > 0.0f) cfg.beam = beam;
   if (max_tokens > 0) cfg.max_tokens = max_tokens;
   cfg.max_words = max_words;
+  cfg.max_active = b->max_active;
   pkb_am *am = b->am;
   const size_t tid_bytes = am->tid2pdf.size() * sizeof(int32_t);
   if (b->vit_tid2pdf.cap < tid_bytes) {
@@ -892,6 +894,13 @@ int pkb_batch_decode(pkb_batch_t *b, const pkb_fst_t *fst, float beam, int max_t
   return pkb::check_device_error(c, "pkb_batch_decode");
 }
 
+int pkb_batch_set_max_active(pkb_batch_t *b, int max_active) {
+  PKB_REQUIRE(b, "pkb_batch_set_max_active: the batch is NULL");
+  PKB_REQUIRE(max_active >= 0, "pkb_batch_set_max_active: max_active must be >= 0 (got %d)", max_active);
+  b->max_active = max_active;
+  return PKB_OK;
+}
+
 static_assert(sizeof(pkb_lattice_arc_t) == 28 && offsetof(pkb_lattice_arc_t, acoustic_cost) == 24,
               "pkb_lattice_arc_t is 28 bytes without padding");
 
@@ -913,6 +922,7 @@ int pkb_batch_lattice(pkb_batch_t *b, const pkb_fst_t *fst, float beam, float la
   pkb::ViterbiConfig cfg;
   if (beam > 0.0f) cfg.beam = beam;
   if (max_tokens > 0) cfg.max_tokens = max_tokens;
+  cfg.max_active = b->max_active;
   pkb_am *am = b->am;
   const size_t tid_bytes = am->tid2pdf.size() * sizeof(int32_t);
   if (b->vit_tid2pdf.cap < tid_bytes) {

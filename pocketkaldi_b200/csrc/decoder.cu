@@ -16,8 +16,16 @@
 // early are tested against a looser bound and may create tokens that the final bound would not;
 // those tokens lie outside the next frame's beam and are dropped there. Here every arc is tested
 // against the final (tightest) bound. The max-active estimate by sampling (:141-200, more than
-// 30000 tokens) is replaced by a hard per-utterance capacity that fails the utterance. Ties between
-// equal float costs are broken by arc index instead of by list order.
+// 30000 tokens) is replaced by an exact, optional limit (ViterbiConfig::max_active, Kaldi's
+// --max-active): on a frame of more than max_active tokens whose max_active-th smallest cost c_k is
+// below float(best + beam), the tokens of cost <= c_k are expanded (all ties at c_k, so nothing
+// depends on scheduling) and the next bound is the least expanded total + float(min(beam,
+// (c_k - best) + 0.5)). The best token is always expanded, so partial hypotheses keep their
+// meaning; BestPath and the lattice's backward pass are unchanged, and a lattice holds what the
+// pruned search relaxed. With max_active = 0, or no more tokens than max_active, the arithmetic is
+// the beam's alone. max_tokens still bounds the tokens CREATED per frame: an overflow fails the
+// utterance whatever max_active says. Ties between equal float costs are broken by arc index
+// instead of by list order.
 
 #include <math.h>
 
@@ -311,6 +319,71 @@ __device__ void block_sort(unsigned long long *a, int n) {
   }
 }
 
+// The k-th smallest (1 <= k <= n) of the n keys key(0), ..., key(n - 1), equal keys counted
+// separately: radix select from the top byte down, one 256-bin shared histogram per byte of the
+// keys that match the bytes chosen so far. Exact, without sorting; everyone must call it.
+template <class Key>
+__device__ uint32_t block_select(int n, int k, Key key) {
+  __shared__ unsigned int hist[256];
+  __shared__ uint32_t s_prefix;
+  __shared__ int s_k;
+  const int tid = threadIdx.x;
+  uint32_t prefix = 0;
+  for (int shift = 24; shift >= 0; shift -= 8) {
+    const uint32_t above = shift == 24 ? 0u : ~0u << (shift + 8);  // the bytes already chosen
+    for (int i = tid; i < 256; i += kVitThreads) hist[i] = 0;
+    __syncthreads();
+    for (int i = tid; i < n; i += kVitThreads) {
+      const uint32_t v = key(i);
+      if ((v & above) == prefix) atomicAdd(&hist[(v >> shift) & 255u], 1u);
+    }
+    __syncthreads();
+    if (tid < 32) {
+      // lane l holds bins 8l .. 8l + 7; the lane whose count range holds the k-th key picks the bin
+      unsigned int c[8], sum = 0;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) { c[j] = hist[8 * tid + j]; sum += c[j]; }
+      unsigned int incl = sum;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const unsigned int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (tid >= o) incl += t;
+      }
+      unsigned int run = incl - sum;
+      if (run < static_cast<unsigned int>(k) && static_cast<unsigned int>(k) <= incl) {
+        for (int j = 0; j < 8; ++j) {
+          if (run + c[j] >= static_cast<unsigned int>(k)) {
+            s_prefix = prefix | (static_cast<uint32_t>(8 * tid + j) << shift);
+            s_k = k - static_cast<int>(run);
+            break;
+          }
+          run += c[j];
+        }
+      }
+    }
+    __syncthreads();
+    prefix = s_prefix;
+    k = s_k;
+  }
+  return prefix;
+}
+
+// Max-active pruning of one frame (Kaldi's --max-active; the reference estimates the same cutoff by
+// sampling above 30000 tokens, src/decoder.cc:141-200). With more than max_active live tokens whose
+// max_active-th smallest cost c_k is below the beam cutoff, the tokens expanded are those of cost
+// <= c_k (ties included) and the next bound uses the narrowed beam min(beam, (c_k - best) + 0.5)
+// (0.5: Kaldi's beam_delta). Called with ck_key = ord32(c_k) on frames of more than max_active
+// tokens; weight_cutoff and adaptive come in as float(best + beam) and beam.
+__device__ __forceinline__ void max_active_cutoff(uint32_t ck_key, float best, float beam, float *weight_cutoff,
+                                                  float *adaptive) {
+  const float ck = unord32(ck_key);
+  if (ck < *weight_cutoff) {
+    *weight_cutoff = ck;
+    *adaptive = static_cast<float>(fmin(static_cast<double>(beam),
+                                        (static_cast<double>(ck) - static_cast<double>(best)) + 0.5));
+  }
+}
+
 // Backward pass over utterance u's log once its search is complete, with `best` finite:
 //   beta(T, s) = final(s); beta(t, s) = min over logged arcs leaving (t, s) of
 //   (w + ac) + beta(head), epsilon arcs of a time relaxed to a fixpoint (also at T);
@@ -410,9 +483,11 @@ __device__ int lattice_prune(const FstDev &fst, const Lattice &lat, unsigned lon
   return kept;
 }
 
-template <int kVitGroup, bool kResume, bool kLattice>
+// kMaxActive: the max-active rule is compiled in (launches with max_active > 0 only), so that the
+// search without it keeps its registers and schedule.
+template <int kVitGroup, bool kResume, bool kLattice, bool kMaxActive>
 __global__ void __launch_bounds__(kVitThreads)
-viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, int max_words,
+viterbi_kernel(FstDev fst, float beam, int max_active, int max_tok, uint32_t mask, int max_log, int max_words,
                const float *__restrict__ loglik, int num_pdfs, const int64_t *__restrict__ row_off,
                const int32_t *__restrict__ num_frames, int n_utts, const int32_t *__restrict__ tid2pdf,
                char *work_base, size_t work_stride, int tables_in_smem, int32_t *__restrict__ words_out,
@@ -685,17 +760,21 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
       const Tab &tp = w.tab[prev], &tc = w.tab[cur];
       const int n_prev = s_ntok[prev];
       const float *ll = ll0 + static_cast<int64_t>(f) * num_pdfs;
-      // ---- GetCutoff (src/decoder.cc:141-200) below kBeamSize tokens: best cost + beam
+      // ---- GetCutoff (src/decoder.cc:141-200): best cost + beam, narrowed by max-active
       if (tid == 0) s_min = ~0ull;
       __syncthreads();
+      auto key = [&](int i) { return static_cast<uint32_t>(tp.vals[tp.list[i]] >> 32); };
       {
         uint32_t m = 0xffffffffu;
-        for (int i = tid; i < n_prev; i += kVitThreads) m = min(m, static_cast<uint32_t>(tp.vals[tp.list[i]] >> 32));
+        for (int i = tid; i < n_prev; i += kVitThreads) m = min(m, key(i));
         atomicMin(&s_min, static_cast<unsigned long long>(m));
       }
       __syncthreads();
       const float best = unord32(static_cast<uint32_t>(s_min));
-      const float weight_cutoff = static_cast<float>(static_cast<double>(best) + static_cast<double>(beam));
+      float weight_cutoff = static_cast<float>(static_cast<double>(best) + static_cast<double>(beam));
+      float adaptive = beam;
+      if (kMaxActive && n_prev > max_active)
+        max_active_cutoff(block_select(n_prev, max_active, key), best, beam, &weight_cutoff, &adaptive);
       __syncthreads();
       // ---- ProcessEmitting, pass 1: the bound on the next frame (min over kept arcs of total + beam)
       if (tid == 0) s_min = ~0ull;
@@ -725,7 +804,7 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
       }
       __syncthreads();
       if (s_min == ~0ull) { alive = false; break; }  // no arc left the beam: the reference has no tokens either
-      const double next_cutoff = unord64(s_min) + static_cast<double>(beam);
+      const double next_cutoff = unord64(s_min) + static_cast<double>(adaptive);
       const bool lat_on = kLattice && lat_live();
       if (lat_on) {
         if (tid == 0) go[2 * f + 1] = lat_shared().count;
@@ -874,9 +953,19 @@ viterbi_kernel(FstDev fst, float beam, int max_tok, uint32_t mask, int max_log, 
 //   bp[s]    newest word record of the token
 constexpr uint32_t kInactive = 0xffffffffu;
 
-template <int kArcsPerThread, bool kResume, bool kLattice>
+// The k-th smallest token cost (ord32) of a dense table of S states, or kInactive when it holds at
+// most k tokens. kInactive is above every cost, so with k <= tokens the empty states never reach
+// the k-th place.
+__device__ uint32_t dense_select(const uint32_t *cost, int S, int k) {
+  int n = 0;
+  for (int s0 = 0; s0 < S; s0 += kVitThreads)
+    n += __syncthreads_count(s0 + threadIdx.x < S && cost[s0 + threadIdx.x] != kInactive);
+  return n > k ? block_select(S, k, [&](int s) { return cost[s]; }) : kInactive;
+}
+
+template <int kArcsPerThread, bool kResume, bool kLattice, bool kMaxActive>
 __global__ void __launch_bounds__(kVitThreads, kArcsPerThread <= 8 ? 3 : 1)
-viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_words,
+viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_active, int max_log, int max_words,
                      const float *__restrict__ loglik, int num_pdfs, const int64_t *__restrict__ row_off,
                      const int32_t *__restrict__ num_frames, int n_utts, const int32_t *__restrict__ tid2pdf,
                      char *work_base, size_t work_stride, int32_t *__restrict__ words_out,
@@ -1186,9 +1275,16 @@ viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_
           ll_next[k] = (f + 1 < T && d < D) ? __ldg(&lln[s_pdf[d]]) : 0.0f;
         }
       }
-      // ---- GetCutoff below kBeamSize tokens: the best cost was reduced when the table was finished
+      // ---- GetCutoff: the best cost was reduced when the table was finished, + beam, narrowed by
+      // max-active (a graph of at most max_active states never has more tokens)
       if (s_best == kInactive) { alive = false; break; }
-      const float weight_cutoff = static_cast<float>(static_cast<double>(unord32(s_best)) + static_cast<double>(beam));
+      const float best = unord32(s_best);
+      float weight_cutoff = static_cast<float>(static_cast<double>(best) + static_cast<double>(beam));
+      float adaptive = beam;
+      if (kMaxActive) {
+        const uint32_t ck = dense_select(cost[prev], S, max_active);
+        if (ck != kInactive) max_active_cutoff(ck, best, beam, &weight_cutoff, &adaptive);
+      }
       // ---- ProcessEmitting, pass 1: totals of this thread's arcs, bound on the next frame
       double td[kArcsPerThread];
       bool live[kArcsPerThread];
@@ -1214,7 +1310,7 @@ viterbi_dense_kernel(FstDev fst, int num_arcs, float beam, int max_log, int max_
       }
       __syncthreads();
       if (s_min == ~0ull) { alive = false; break; }
-      const double next_cutoff = unord64(s_min) + static_cast<double>(beam);
+      const double next_cutoff = unord64(s_min) + static_cast<double>(adaptive);
       // ---- pass 2: token costs of this frame
 #pragma unroll
       for (int k = 0; k < kArcsPerThread; ++k) {
@@ -1482,8 +1578,8 @@ int init_workspace(Ctx *c, const VitPlan &p, DevBuf *work) {
   return PKB_OK;
 }
 
-template <bool kResume, bool kLattice>
-int launch_plan(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfig &cfg, const float *d_loglik,
+template <bool kResume, bool kLattice, bool kMaxActive>
+int launch_plan_ma(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfig &cfg, const float *d_loglik,
                 int num_pdfs, const int64_t *d_row_off, const int32_t *d_num_frames, int n_utts,
                 const int32_t *d_tid2pdf, DevBuf *work, int32_t *d_words, int32_t *d_n_words, float *d_weight,
                 const Carry &cr, const Lattice &lat) {
@@ -1492,10 +1588,11 @@ int launch_plan(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfi
 #define PKB_VIT_DENSE(APT)                                                                                   \
   do {                                                                                                       \
     if (p.smem > 48 * 1024)                                                                                  \
-      PKB_CUDA(cudaFuncSetAttribute(viterbi_dense_kernel<APT, kResume, kLattice>,                            \
+      PKB_CUDA(cudaFuncSetAttribute(viterbi_dense_kernel<APT, kResume, kLattice, kMaxActive>,                            \
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(p.smem))); \
-    viterbi_dense_kernel<APT, kResume, kLattice><<<p.grid, kVitThreads, p.smem, c->stream>>>(                \
-        fd, fst->num_arcs, cfg.beam, cfg.max_log, cfg.max_words, d_loglik, num_pdfs, d_row_off,              \
+    viterbi_dense_kernel<APT, kResume, kLattice, kMaxActive><<<p.grid, kVitThreads, p.smem, c->stream>>>(                \
+        fd, fst->num_arcs, cfg.beam, cfg.max_active, cfg.max_log, cfg.max_words, d_loglik, num_pdfs,          \
+        d_row_off,                                                                                           \
         d_num_frames, n_utts, d_tid2pdf, work->as<char>(), p.stride, d_words, d_n_words, d_weight, cr, lat); \
   } while (0)
   // (staging each frame's log-likelihood row in shared memory with cp.async was measured slower in
@@ -1504,10 +1601,11 @@ int launch_plan(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfi
 #define PKB_VIT_LAUNCH(G)                                                                                    \
   do {                                                                                                       \
     if (p.smem > 48 * 1024)                                                                                  \
-      PKB_CUDA(cudaFuncSetAttribute(viterbi_kernel<G, kResume, kLattice>,                                    \
+      PKB_CUDA(cudaFuncSetAttribute(viterbi_kernel<G, kResume, kLattice, kMaxActive>,                                    \
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(p.smem))); \
-    viterbi_kernel<G, kResume, kLattice><<<p.grid, kVitThreads, p.smem, c->stream>>>(                        \
-        fd, cfg.beam, p.max_tok, p.H - 1, cfg.max_log, cfg.max_words, d_loglik, num_pdfs, d_row_off,         \
+    viterbi_kernel<G, kResume, kLattice, kMaxActive><<<p.grid, kVitThreads, p.smem, c->stream>>>(                        \
+        fd, cfg.beam, cfg.max_active, p.max_tok, p.H - 1, cfg.max_log, cfg.max_words, d_loglik, num_pdfs,    \
+        d_row_off,                                                                                           \
         d_num_frames, n_utts, d_tid2pdf, work->as<char>(), p.stride, p.small ? 1 : 0, d_words, d_n_words,    \
         d_weight, cr, lat);                                                                                  \
   } while (0)
@@ -1523,6 +1621,19 @@ int launch_plan(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfi
 #undef PKB_VIT_LAUNCH
   PKB_CUDA(cudaGetLastError());
   return PKB_OK;
+}
+
+// The kernels with the max-active rule when it can prune: max_active > 0, and for the dense kernel
+// fewer than the graph's states (a frame never holds more tokens than states).
+template <bool kResume, bool kLattice>
+int launch_plan(Ctx *c, const pkb_fst *fst, const VitPlan &p, const ViterbiConfig &cfg, const float *d_loglik,
+                int num_pdfs, const int64_t *d_row_off, const int32_t *d_num_frames, int n_utts,
+                const int32_t *d_tid2pdf, DevBuf *work, int32_t *d_words, int32_t *d_n_words, float *d_weight,
+                const Carry &cr, const Lattice &lat) {
+  const bool prune = cfg.max_active > 0 && (!p.dense || cfg.max_active < fst->num_states);
+  return (prune ? launch_plan_ma<kResume, kLattice, true> : launch_plan_ma<kResume, kLattice, false>)(
+      c, fst, p, cfg, d_loglik, num_pdfs, d_row_off, d_num_frames, n_utts, d_tid2pdf, work, d_words, d_n_words,
+      d_weight, cr, lat);
 }
 
 }  // namespace

@@ -34,9 +34,10 @@ int fst_build(Ctx *c, int num_states, int start, const float *final_w, const int
 
 struct ViterbiConfig {
   float beam = 16.0f;        // Decoder::beam_ (src/decoder.cc:29)
-  int max_tokens = 4096;     // tokens per frame and utterance (the reference caps at 30000 by sampling)
+  int max_tokens = 4096;     // tokens created per frame and utterance; more fail the utterance
   int max_log = 1 << 18;     // word back-pointer records per utterance
   int max_words = 256;       // words returned per utterance
+  int max_active = 0;        // tokens expanded per frame, ties at the cutoff included (0: no limit)
 };
 
 // Kernel choice and workspace of one search (launch_viterbi picks the same for both entry points).

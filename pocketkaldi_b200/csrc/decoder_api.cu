@@ -172,6 +172,21 @@ int pkb_decoder_set_lattice(pkb_decoder_t *dec, float lattice_beam, int max_fram
   return dec->search.set_lattice(lattice_beam, frames, arcs);
 }
 
+int pkb_decoder_set_max_active(pkb_decoder_t *dec, int max_active) {
+  PKB_REQUIRE(dec, "pkb_decoder_set_max_active: decoder is NULL");
+  PKB_REQUIRE(max_active >= 0, "pkb_decoder_set_max_active: max_active must be >= 0 (got %d)", max_active);
+  PKB_REQUIRE(!dec->in_utt,
+              "pkb_decoder_set_max_active: only between utterances (after create or pkb_decoder_finish)");
+  // the attached stream's captured pushes launch the advance with the old value: they are captured again
+  if (dec->st) {
+    PKB_CUDA(cudaSetDevice(dec->c->device));
+    PKB_CUDA(cudaStreamSynchronize(dec->c->stream));
+    pkb::stream_drop_graphs(dec->st);
+  }
+  dec->search.cfg.max_active = max_active;
+  return PKB_OK;
+}
+
 int pkb_decoder_lattice(pkb_decoder_t *dec, int64_t *n_arcs_out, double *best_cost_out) {
   PKB_REQUIRE(dec && n_arcs_out && best_cost_out, "pkb_decoder_lattice: NULL argument");
   PKB_REQUIRE(dec->lat.total >= 0, "pkb_decoder_lattice: no lattice: %s", dec->lat.why.c_str());
