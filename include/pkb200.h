@@ -392,6 +392,43 @@ int pkb_batch_posteriors(pkb_batch_t *batch, const pkb_fst_t *fst, float acousti
  * frame_post_out: every utterance's entries back to back, each in (t, pdf) order. Either may be
  * NULL. */
 int pkb_batch_posteriors_get(pkb_batch_t *batch, float *arc_post_out, pkb_frame_post_t *frame_post_out);
+/* ---- best path and frame alignment over a lattice ----------------------------------------------
+ * Paths, T and final(s) as in the N-best comment above. The cost of a record is c(r) = graph_scale x
+ * graph_cost + acoustic_scale x acoustic_cost, plus word_penalty when olabel != 0, and of a final
+ * weight graph_scale x final(s), in double from the records' floats with the scaled costs of the
+ * posteriors (lattice-scale --inv-acoustic-scale, lattice-add-penalty, lattice-best-path):
+ *   alpha(0, start) = 0; a node takes its candidates alpha(t, src) + c(r) in the posteriors' fold
+ *   order (the emitting records into it from time t - 1 in record order, then the epsilon records
+ *   of time t into it in record order, in topological order) and a candidate replaces the held
+ *   value only when it is strictly smaller, so among equal values the first in fold order wins.
+ *   The best final node is the least alpha(T, s) + graph_scale x final(s), ties to the lowest state.
+ * Per utterance: cost, that minimum; graph_cost and acoustic_cost of its path, unscaled and without
+ * the penalty, summed in double in path order with the final weight once in the graph cost (as in
+ * N-best); its words (the nonzero olabels, in spoken order) and for each word_t, the t of the record
+ * that carries it (the frame an emitting record reads, the node time of an epsilon record); and its
+ * alignment, the ilabel (transition id) of the path's emitting record at each t < T. Word end times
+ * and boundaries need the word-boundary information of a transition model, which this library does
+ * not hold; the alignment is what a caller derives them from.
+ * n_words_out codes besides those of the lattice: -8 the kept epsilon records of one time form a
+ * cycle, as in the posteriors; only that utterance fails. A failed utterance has NaN costs; one
+ * without a complete path has +inf costs, no words and an empty alignment.
+ * Device memory per call: the results, 8 bytes per word and 4 per alignment entry, kept until the
+ * next call; 12 bytes per record of scratch; and per utterance in flight 12 bytes per record (alpha
+ * and the path) plus 4 bytes per graph arc and, for graphs whose per-state arrays pass 48 KiB, those
+ * arrays (28 bytes per state); utterances run in waves of at most 8 GiB (or half the free memory) of
+ * the latter. */
+/* The best path of the latest pkb_batch_lattice of this batch (fst: the graph of that call; another
+ * one is rejected). acoustic_scale > 0, graph_scale >= 0 and word_penalty (any sign), all finite.
+ * cost_out / graph_cost_out / acoustic_cost_out [n_utts]; n_words_out[u]: the words of utterance u,
+ * or its negative code; n_frames_out[u]: T, or 0 when it failed or has no complete path.
+ * Synchronous; the lattice, N-best, posterior and decode results are left unchanged. */
+int pkb_batch_best_path(pkb_batch_t *batch, const pkb_fst_t *fst, float acoustic_scale, float graph_scale,
+                        float word_penalty, double *cost_out, double *graph_cost_out, double *acoustic_cost_out,
+                        int32_t *n_words_out, int32_t *n_frames_out);
+/* The results of the latest pkb_batch_best_path, valid until the next lattice call on the batch:
+ * words_out and word_t_out hold every utterance's n_words_out entries back to back, ali_out every
+ * utterance's n_frames_out entries back to back. Any of them may be NULL. */
+int pkb_batch_best_path_get(pkb_batch_t *batch, int32_t *words_out, int32_t *word_t_out, int32_t *ali_out);
 
 /* ---- online decoding: the GPU Viterbi search, chunk by chunk ----------------------------------
  * n_streams searches whose tokens and word records stay on the device between calls, so that
@@ -459,6 +496,13 @@ int pkb_decoder_posteriors(pkb_decoder_t *dec, float acoustic_scale, float graph
                            double *total_out, int64_t *n_post_out);
 /* The results of the latest pkb_decoder_posteriors, valid until the next advance, push or flush. */
 int pkb_decoder_posteriors_get(pkb_decoder_t *dec, float *arc_post_out, pkb_frame_post_t *frame_post_out);
+/* pkb_batch_best_path for the lattices of the latest pkb_decoder_finish; valid when
+ * pkb_decoder_lattice is. */
+int pkb_decoder_best_path(pkb_decoder_t *dec, float acoustic_scale, float graph_scale, float word_penalty,
+                          double *cost_out, double *graph_cost_out, double *acoustic_cost_out,
+                          int32_t *n_words_out, int32_t *n_frames_out);
+/* The results of the latest pkb_decoder_best_path, valid until the next advance, push or flush. */
+int pkb_decoder_best_path_get(pkb_decoder_t *dec, int32_t *words_out, int32_t *word_t_out, int32_t *ali_out);
 
 /* Sum over all elements of a per-frame float buffer, computed on the device
  * in double (a cheap whole-output fingerprint for full-size runs). */

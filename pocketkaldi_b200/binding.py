@@ -115,6 +115,8 @@ _SIGNATURES = [
     ("pkb_batch_nbest", C.c_int, [_VP, _VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
     ("pkb_batch_posteriors", C.c_int, [_VP, _VP, C.c_float, C.c_float, C.c_float, _VP, _VP]),
     ("pkb_batch_posteriors_get", C.c_int, [_VP, _VP, _VP]),
+    ("pkb_batch_best_path", C.c_int, [_VP, _VP, C.c_float, C.c_float, C.c_float, _VP, _VP, _VP, _VP, _VP]),
+    ("pkb_batch_best_path_get", C.c_int, [_VP, _VP, _VP, _VP]),
     ("pkb_decoder_create", C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int,
                                      C.POINTER(_VP)]),
     ("pkb_decoder_destroy", None, [_VP]),
@@ -128,6 +130,8 @@ _SIGNATURES = [
     ("pkb_decoder_nbest", C.c_int, [_VP, C.c_int, C.c_int, _VP, _VP, _VP, _VP, _VP]),
     ("pkb_decoder_posteriors", C.c_int, [_VP, C.c_float, C.c_float, C.c_float, _VP, _VP]),
     ("pkb_decoder_posteriors_get", C.c_int, [_VP, _VP, _VP]),
+    ("pkb_decoder_best_path", C.c_int, [_VP, C.c_float, C.c_float, C.c_float, _VP, _VP, _VP, _VP, _VP]),
+    ("pkb_decoder_best_path_get", C.c_int, [_VP, _VP, _VP, _VP]),
     ("pkb_loglik16_expand", C.c_int, [_VP, _VP, C.c_int64, C.c_int, C.c_float, _VP]),
     ("pkb_stream_create", C.c_int, [_VP, _VP, C.c_int, C.c_int, _f32p, C.c_float, C.POINTER(_VP)]),
     ("pkb_stream_destroy", None, [_VP]),
@@ -725,6 +729,17 @@ class Batch:
                                                                       min_post, tot, npost),
                            lambda arc, fr: lib.pkb_batch_posteriors_get(self.h, arc, fr))
 
+    def best_path(self, fst, acoustic_scale=1.0, graph_scale=1.0, word_penalty=0.0):
+        """The best path of every utterance's latest lattice() at these scales and word insertion
+        penalty (pkb_batch_best_path; fst is the graph of that call): per utterance None where its
+        lattice or its best path failed, otherwise (cost, graph_cost, acoustic_cost, words as int32,
+        word_t as int32, alignment as int32 transition ids, one per frame)."""
+        lib = self.ctx.lib
+        return _best_path(len(self.num_samples),
+                          lambda *out: lib.pkb_batch_best_path(self.h, fst.h, acoustic_scale, graph_scale,
+                                                               word_penalty, *out),
+                          lambda *out: lib.pkb_batch_best_path_get(self.h, *out))
+
     def refine_stats(self):
         """(GEMM rows, frames recomputed) of the latest run under PREC_FP16R."""
         rows, sel = C.c_int64(0), C.c_int64(0)
@@ -891,6 +906,14 @@ class Decoder:
                                                                         min_post, tot, npost),
                            lambda arc, fr: lib.pkb_decoder_posteriors_get(self.h, arc, fr))
 
+    def best_path(self, acoustic_scale=1.0, graph_scale=1.0, word_penalty=0.0):
+        """Batch.best_path over the lattices of the latest finish() (pkb_decoder_best_path)."""
+        lib = self.ctx.lib
+        return _best_path(self.n_streams,
+                          lambda *out: lib.pkb_decoder_best_path(self.h, acoustic_scale, graph_scale, word_penalty,
+                                                                 *out),
+                          lambda *out: lib.pkb_decoder_best_path_get(self.h, *out))
+
 
 def _split(flat, counts):
     """Per utterance the next max(counts[u], 0) entries of flat, or None where counts[u] < 0."""
@@ -944,6 +967,24 @@ def _posteriors(n_arcs, n_utts, call, get):
     fr = np.empty(max(int(np.maximum(npost, 0).sum()), 1), FRAME_POST_DTYPE)
     _check(get(arc.ctypes.data, fr.ctypes.data))
     return tot[:n_utts].copy(), _split(arc, n_arcs), _split(fr, npost)
+
+
+def _best_path(n_utts, call, get):
+    """Runs call(costs, graph_costs, acoustic_costs, n_words, n_frames) and get(words, word_t, ali) for
+    n_utts utterances and unpacks them as Batch.best_path returns them."""
+    u = max(n_utts, 1)
+    cost, g, a = (np.zeros(u, np.float64) for _ in range(3))
+    nw = np.zeros(u, np.int32)
+    nf = np.zeros(u, np.int32)
+    _check(call(cost.ctypes.data, g.ctypes.data, a.ctypes.data, nw.ctypes.data, nf.ctypes.data))
+    nw, nf = nw[:n_utts], nf[:n_utts]
+    words = np.empty(max(int(np.maximum(nw, 0).sum()), 1), np.int32)
+    word_t = np.empty_like(words)
+    ali = np.empty(max(int(nf.sum()), 1), np.int32)
+    _check(get(words.ctypes.data, word_t.ctypes.data, ali.ctypes.data))
+    ws, ts, al = _split(words, nw), _split(word_t, nw), _split(ali, np.where(nw < 0, -1, nf))
+    return [None if nw[i] < 0 else (float(cost[i]), float(g[i]), float(a[i]), ws[i], ts[i], al[i])
+            for i in range(n_utts)]
 
 
 class Stream:

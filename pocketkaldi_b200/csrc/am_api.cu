@@ -978,6 +978,21 @@ int pkb_batch_posteriors_get(pkb_batch_t *b, float *arc_post_out, pkb_frame_post
   return b->lat.posteriors_get(arc_post_out, frame_post_out, "pkb_batch_posteriors_get");
 }
 
+int pkb_batch_best_path(pkb_batch_t *b, const pkb_fst_t *fst, float acoustic_scale, float graph_scale,
+                        float word_penalty, double *cost_out, double *graph_cost_out, double *acoustic_cost_out,
+                        int32_t *n_words_out, int32_t *n_frames_out) {
+  PKB_REQUIRE(b && fst, "pkb_batch_best_path: NULL argument");
+  PKB_REQUIRE(b->lat.total < 0 || b->lat.fst == fst,
+              "pkb_batch_best_path: the FST is not the one of the latest pkb_batch_lattice");
+  return b->lat.best_path(acoustic_scale, graph_scale, word_penalty, cost_out, graph_cost_out, acoustic_cost_out,
+                          n_words_out, n_frames_out, "pkb_batch_best_path");
+}
+
+int pkb_batch_best_path_get(pkb_batch_t *b, int32_t *words_out, int32_t *word_t_out, int32_t *ali_out) {
+  PKB_REQUIRE(b, "pkb_batch_best_path_get: the batch is NULL");
+  return b->lat.best_path_get(words_out, word_t_out, ali_out, "pkb_batch_best_path_get");
+}
+
 // ---------------------------------------------------------------- fused host path
 int pkb_pcm_to_loglik_i16(pkb_ctx_t *c, pkb_am_t *am, const int16_t *pcm,
                           const int32_t *num_samples, int n_utts, const float *global_stats,

@@ -125,6 +125,14 @@ struct PosteriorResults {
   int64_t n_frames = 0;  // frame entries
 };
 
+// Results of the latest best-path call, kept on the device for the _get call: every utterance's
+// words, then every utterance's word times, and every utterance's alignment, back to back.
+struct BestPathResults {
+  DevBuf words, ali;
+  int64_t n_words = -1;  // words (-1: no valid results)
+  int64_t n_frames = 0;  // alignment entries
+};
+
 // The lattice of the latest search of a batch or decoder and what is computed from it: utterance u's
 // n_arcs[u] kept records (or its negative code) from arcs + first[u] on, and its best cost. Every
 // operation takes the name of its entry point for its messages and checks the results are valid.
@@ -142,6 +150,7 @@ struct LatticeResults {
   std::string why = "no lattice search yet";
   DevBuf nbest_work;                     // outputs of nbest
   PosteriorResults post;                 // results of posteriors, valid as the records are
+  BestPathResults bp;                    // results of best_path, valid as the records are
 
   long long *d_n_arcs() const { return meta.as<long long>(); }
   long long *d_first() const { return d_n_arcs() + n_arcs.size(); }
@@ -150,6 +159,7 @@ struct LatticeResults {
     total = -1;
     why = std::move(reason);
     post.n_arcs = -1;
+    bp.n_words = -1;
   }
   // After launch_lattice (or the finish of a resumable search) over n_utts utterances whose rows
   // start at d_loglik + d_row_off[u] * num_pdfs: copies lat.n_out / lat.best_out to the host and
@@ -169,6 +179,14 @@ struct LatticeResults {
                  const char *who);
   // Copies the results of the latest posteriors out (either output may be NULL).
   int posteriors_get(float *arc_post_out, pkb_frame_post_t *frame_post_out, const char *who);
+  // The best path per utterance at the given scales and word insertion penalty (best_path.cu), with
+  // the arguments and host outputs of pkb_batch_best_path. Alpha and the path (12 bytes per record)
+  // and the per-block workspace are allocated per call, in waves.
+  int best_path(float acoustic_scale, float graph_scale, float word_penalty, double *cost_out,
+                double *graph_cost_out, double *acoustic_cost_out, int32_t *n_words_out, int32_t *n_frames_out,
+                const char *who);
+  // Copies the words, word times and alignments of the latest best_path out (any may be NULL).
+  int best_path_get(int32_t *words_out, int32_t *word_t_out, int32_t *ali_out, const char *who);
 };
 
 // The resumable search behind pkb_decoder: n streams, one thread block each, whose tokens and word

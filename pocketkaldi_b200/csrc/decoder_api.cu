@@ -218,4 +218,17 @@ int pkb_decoder_posteriors_get(pkb_decoder_t *dec, float *arc_post_out, pkb_fram
   return dec->lat.posteriors_get(arc_post_out, frame_post_out, "pkb_decoder_posteriors_get");
 }
 
+int pkb_decoder_best_path(pkb_decoder_t *dec, float acoustic_scale, float graph_scale, float word_penalty,
+                          double *cost_out, double *graph_cost_out, double *acoustic_cost_out, int32_t *n_words_out,
+                          int32_t *n_frames_out) {
+  PKB_REQUIRE(dec, "pkb_decoder_best_path: decoder is NULL");
+  return dec->lat.best_path(acoustic_scale, graph_scale, word_penalty, cost_out, graph_cost_out, acoustic_cost_out,
+                            n_words_out, n_frames_out, "pkb_decoder_best_path");
+}
+
+int pkb_decoder_best_path_get(pkb_decoder_t *dec, int32_t *words_out, int32_t *word_t_out, int32_t *ali_out) {
+  PKB_REQUIRE(dec, "pkb_decoder_best_path_get: decoder is NULL");
+  return dec->lat.best_path_get(words_out, word_t_out, ali_out, "pkb_decoder_best_path_get");
+}
+
 }  // extern "C"

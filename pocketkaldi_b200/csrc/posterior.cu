@@ -2,18 +2,13 @@
 // pkb_decoder_posteriors): a forward-backward pass in the log semiring, one thread block per
 // utterance, in the fold order of include/pkb200.h.
 //
-// The block walks the groups eps(0), emit(0), eps(1), ... forward and then backward, with the
-// costs of two times live as per-state double arrays (in shared memory when they fit):
-//   emit(t) forward   the group's records are grouped by destination with a stable counting sort
-//                     (below), then one thread per destination folds its incoming records in
-//                     record order into alpha(t + 1, dst).
-//   eps(t)            Kahn levels over the group: a node is folded once every source (forward) or
-//                     every head (backward) is complete, so the fold order is fixed and the result
-//                     does not depend on scheduling. Nodes left over when the levels stop lie on a
-//                     cycle of epsilon records: the utterance fails with -8.
+// The forward pass is the walk of lattice_walk.cuh with lse as its fold. The block then walks the
+// groups backward, with the costs of two times live as per-state double arrays (in shared memory
+// when they fit):
 //   backward          the records of a group are already grouped by source (the FST's arcs are
 //                     sorted by source state), so a node folds its outgoing epsilon records, then
-//                     its outgoing emitting records, from two contiguous ranges.
+//                     its outgoing emitting records, from two contiguous ranges; the epsilon records
+//                     of a time in Kahn levels, a node once every head is complete.
 // The forward pass saves alpha(t, src) per record (8 bytes), so the backward pass finishes each
 // record's posterior as soon as beta at its head is known. The frame posteriors of time t are the
 // emitting posteriors of the group grouped by pdf with the same stable sort, summed in record
@@ -24,42 +19,26 @@
 #include <math.h>
 
 #include <algorithm>
-#include <cub/block/block_radix_sort.cuh>
-#include <cub/block/block_scan.cuh>
 
-#include "decoder.cuh"
+#include "lattice_walk.cuh"
 
 namespace pkb {
 namespace {
 
-constexpr int kPoThreads = 512;
-constexpr int kPoItems = 4;                        // records per thread of a sort tile
-constexpr int kPoTile = kPoThreads * kPoItems;     // records per sort tile
-constexpr int kPoTileBits = 11;                    // log2(kPoTile)
-static_assert((1 << kPoTileBits) == kPoTile, "tile bits");
-constexpr size_t kPoSmemState = 48 << 10;          // per-state arrays go to shared memory up to this
+using lattice_walk::kThreads;
+using lattice_walk::kSmemState;
+using lattice_walk::scaled_cost;
 
-struct PostArgs {
-  const pkb_lattice_arc_t *arcs;
-  const long long *first, *n_arcs;
-  const double *best;
-  const float *final_w;
+// work: per block sort order and group posteriors [, per-state arrays]
+struct PostArgs : lattice_walk::WalkArgs {
   const int32_t *tid2pdf;
-  int num_states, num_pdfs, num_arcs, start, u0;
-  double as, gs;
+  int num_pdfs;
   float min_post;
-  char *work;               // per block: sort order and group posteriors [, per-state arrays]
-  size_t work_stride;
-  bool smem_state;          // per-state arrays in dynamic shared memory
-  double *alpha;            // alpha(t, src) of record first[u] + i at alpha[first[u] - rec0 + i]
-  long long rec0;
   float *arc_post;          // [records]
   pkb_frame_post_t *tail;   // [records]: utterance u's entries end at first[u] + n_arcs[u]
   double *total;            // [n_utts]
   long long *n_post;        // [n_utts]
 };
-
-__device__ __forceinline__ int group_of(const pkb_lattice_arc_t &r) { return 2 * r.t + (r.ilabel != 0); }
 
 // -log(exp(-a) + exp(-b)); +inf is the identity
 __device__ __forceinline__ double lse(double a, double b) {
@@ -67,25 +46,12 @@ __device__ __forceinline__ double lse(double a, double b) {
   return M == INFINITY ? m : m - log1p(exp(m - M));
 }
 
-__device__ __forceinline__ double scaled_cost(const PostArgs &A, const pkb_lattice_arc_t &r) {
-  return __dadd_rn(__dmul_rn(A.gs, static_cast<double>(r.graph_cost)),
-                   __dmul_rn(A.as, static_cast<double>(r.acoustic_cost)));
-}
-
 __device__ __forceinline__ double arc_posterior(double total, double alpha, double c, double beta) {
   return total < INFINITY ? exp(total - ((alpha + c) + beta)) : 0.0;
 }
 
-__device__ __forceinline__ int bit_width(unsigned x) { return 32 - __clz(x); }
-
-__global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
-  using Scan = cub::BlockScan<int, kPoThreads>;
-  using Sort = cub::BlockRadixSort<unsigned long long, kPoThreads, kPoItems>;
-  __shared__ union {
-    typename Scan::TempStorage scan;
-    typename Sort::TempStorage sort;
-  } tmp;
-  __shared__ int tkey[kPoTile];
+__global__ void __launch_bounds__(kThreads) posterior_kernel(PostArgs A) {
+  __shared__ lattice_walk::Shared sh;
   __shared__ double s_total;
   extern __shared__ double smem_state[];
   const int w = blockIdx.x, u = A.u0 + w, tid = threadIdx.x;
@@ -99,7 +65,7 @@ __global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
   }
   const long long f0 = A.first[u];
   if (!(A.best[u] < INFINITY)) {  // no complete path, so no records
-    for (long long i = tid; i < na; i += kPoThreads) A.arc_post[f0 + i] = 0.0f;
+    for (long long i = tid; i < na; i += kThreads) A.arc_post[f0 + i] = 0.0f;
     if (tid == 0) {
       A.total[u] = INFINITY;
       A.n_post[u] = 0;
@@ -121,156 +87,13 @@ __global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
   int *seg = fill + K;                         // [K + 1]
   int *eb = seg + K + 1, *ee = eb + S, *mb = ee + S, *me = mb + S;  // [S] each: runs by source
 
-  // the first index in [lo, min(na, lo + NA)] whose group is > grp (a group holds at most NA
-  // records); every thread probes once per round, so two rounds cover 2^18 records
-  auto group_end = [&](long long lo, int grp) {
-    long long a = lo, b = min(na, lo + NA);
-    while (b > a) {
-      const long long step = (b - a + kPoThreads - 1) / kPoThreads, p = a + tid * step;
-      const int k = __syncthreads_count(p < b && group_of(recs[p]) <= grp);
-      if (k == 0) break;
-      const long long nb = min(b, a + k * step);
-      a += (k - 1) * step + 1;
-      b = nb;
-    }
-    return a;
-  };
-  // Groups records [0, m) by key(i) in [0, K) stably: key k's records are perm[seg[k] .. seg[k + 1])
-  // in ascending order. Counts and a scan give the segments; then tiles of kPoTile records in
-  // order are radix-sorted by (key, index) and appended to their segments.
-  auto group_by_key = [&](int m, auto key) {
-    __syncthreads();
-    for (int k = tid; k < K; k += kPoThreads) fill[k] = 0;
-    __syncthreads();
-    for (int i = tid; i < m; i += kPoThreads) atomicAdd(&fill[key(i)], 1);
-    __syncthreads();
-    const int per = (K + kPoThreads - 1) / kPoThreads, k0 = min(K, tid * per), k1 = min(K, k0 + per);
-    int sum = 0;
-    for (int k = k0; k < k1; ++k) sum += fill[k];
-    int base = 0;
-    Scan(tmp.scan).ExclusiveSum(sum, base);
-    __syncthreads();
-    for (int k = k0; k < k1; ++k) {
-      const int c = fill[k];
-      seg[k] = base;
-      fill[k] = base;
-      base += c;
-    }
-    if (tid == 0) seg[K] = m;
-    const int end_bit = kPoTileBits + bit_width(static_cast<unsigned>(K));
-    for (int b0 = 0; b0 < m; b0 += kPoTile) {
-      unsigned long long keys[kPoItems];
-      for (int j = 0; j < kPoItems; ++j) {
-        const int li = tid * kPoItems + j;
-        keys[j] = b0 + li < m ? (static_cast<unsigned long long>(key(b0 + li)) << kPoTileBits) | li : ~0ull;
-      }
-      __syncthreads();
-      Sort(tmp.sort).Sort(keys, 0, end_bit);
-      for (int j = 0; j < kPoItems; ++j) {
-        const int r = tid * kPoItems + j;
-        tkey[r] = r < m - b0 ? static_cast<int>(keys[j] >> kPoTileBits) : -1;
-      }
-      __syncthreads();
-      // the first rank of each key's run in this tile moves its fill pointer back by that rank,
-      // every rank then lands at fill + rank, and the run's last rank moves it past the run
-      for (int j = 0; j < kPoItems; ++j) {
-        const int r = tid * kPoItems + j, k = tkey[r];
-        if (k >= 0 && (r == 0 || tkey[r - 1] != k)) fill[k] -= r;
-      }
-      __syncthreads();
-      for (int j = 0; j < kPoItems; ++j) {
-        const int r = tid * kPoItems + j, k = tkey[r];
-        if (k >= 0) perm[fill[k] + r] = b0 + static_cast<int>(keys[j] & (kPoTile - 1));
-      }
-      __syncthreads();
-      for (int j = 0; j < kPoItems; ++j) {
-        const int r = tid * kPoItems + j, k = tkey[r];
-        if (k >= 0 && (r == kPoTile - 1 || tkey[r + 1] != k)) fill[k] += r + 1;
-      }
-    }
-    __syncthreads();
-  };
-
-  // T: the last emitting record's t + 1 (records end with eps(T))
-  int T = 0;
-  if (na > 0) {
-    const pkb_lattice_arc_t last = recs[na - 1];
-    if (last.ilabel) {
-      T = last.t + 1;
-    } else {
-      const long long b = group_end(max(0ll, na - NA), 2 * last.t - 1);
-      T = b > 0 ? recs[b - 1].t + 1 : 0;
-    }
-  }
-
-  // ---- forward: alpha(t, .) in X
-  for (int s = tid; s < S; s += kPoThreads) X[s] = s == A.start ? 0.0 : INFINITY;
-  int err = 0;
-  long long pos = 0;
-  for (int t = 0;; ++t) {
-    const long long e_end = group_end(pos, 2 * t);
-    const int ne = static_cast<int>(e_end - pos);
-    if (ne > 0) {
-      const pkb_lattice_arc_t *E = recs + pos;
-      group_by_key(ne, [&](int i) { return E[i].dst; });
-      for (int s = tid; s < S; s += kPoThreads) done[s] = seg[s + 1] > seg[s] ? 0 : 2;
-      __syncthreads();
-      for (;;) {
-        for (int d = tid; d < S; d += kPoThreads) {
-          if (done[d]) continue;
-          bool ready = true;
-          for (int j = seg[d]; j < seg[d + 1] && ready; ++j) ready = done[E[perm[j]].src] == 2;
-          if (!ready) continue;
-          double a = X[d];
-          for (int j = seg[d]; j < seg[d + 1]; ++j) {
-            const pkb_lattice_arc_t &r = E[perm[j]];
-            a = lse(a, X[r.src] + scaled_cost(A, r));
-          }
-          X[d] = a;
-          done[d] = 1;
-        }
-        __syncthreads();
-        int progress = 0;
-        for (int d = tid; d < S; d += kPoThreads)
-          if (done[d] == 1) {
-            done[d] = 2;
-            progress = 1;
-          }
-        if (!__syncthreads_or(progress)) break;
-      }
-      int open = 0;
-      for (int d = tid; d < S && !open; d += kPoThreads) open = done[d] == 0;
-      if (__syncthreads_or(open)) {
-        err = 8;
-        break;
-      }
-    }
-    const long long m_end = t < T ? group_end(e_end, 2 * t + 1) : e_end;
-    for (long long i = pos + tid; i < m_end; i += kPoThreads) alpha[i] = X[recs[i].src];
-    if (t == T) break;
-    const int nm = static_cast<int>(m_end - e_end);
-    const pkb_lattice_arc_t *M = recs + e_end;
-    for (int s = tid; s < S; s += kPoThreads) Y[s] = INFINITY;
-    if (nm > 0) {
-      group_by_key(nm, [&](int i) { return M[i].dst; });
-      for (int d = tid; d < S; d += kPoThreads) {
-        if (seg[d + 1] == seg[d]) continue;
-        double a = INFINITY;
-        for (int j = seg[d]; j < seg[d + 1]; ++j) {
-          const pkb_lattice_arc_t &r = M[perm[j]];
-          a = lse(a, X[r.src] + scaled_cost(A, r));
-        }
-        Y[d] = a;
-      }
-    }
-    __syncthreads();
-    double *tx = X;
-    X = Y;
-    Y = tx;
-    pos = m_end;
-  }
+  const lattice_walk::Walk W{recs, na, NA, K, tid, perm, fill, seg, sh};
+  const int T = W.last_time();
+  const int err = W.forward(X, Y, done, S, A.start, T, alpha,
+                            [&](const pkb_lattice_arc_t &r) { return scaled_cost(A, r); },
+                            [](double held, double c) { return lse(held, c); });
   if (err) {
-    for (long long i = tid; i < na; i += kPoThreads) A.arc_post[f0 + i] = NAN;
+    for (long long i = tid; i < na; i += kThreads) A.arc_post[f0 + i] = NAN;
     if (tid == 0) {
       A.total[u] = NAN;
       A.n_post[u] = -err;
@@ -292,20 +115,20 @@ __global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
   long long end = na;
   int nout = 0;
   for (int t = T; t >= 0; --t) {
-    const long long m_beg = t < T ? group_end(max(0ll, end - NA), 2 * t) : end;
-    const long long e_beg = t > 0 ? group_end(max(0ll, m_beg - NA), 2 * t - 1) : 0;
+    const long long m_beg = t < T ? W.group_end(max(0ll, end - NA), 2 * t) : end;
+    const long long e_beg = t > 0 ? W.group_end(max(0ll, m_beg - NA), 2 * t - 1) : 0;
     const pkb_lattice_arc_t *E = recs + e_beg, *M = recs + m_beg;
     const int ne = static_cast<int>(m_beg - e_beg), nm = static_cast<int>(end - m_beg);
     if (nm > 0) {
       // posteriors of emit(t), then its frame posteriors
-      for (int i = tid; i < nm; i += kPoThreads) {
+      for (int i = tid; i < nm; i += kThreads) {
         const pkb_lattice_arc_t &r = M[i];
         const double p = arc_posterior(total, alpha[m_beg + i], scaled_cost(A, r), Y[r.dst]);
         pd[i] = p;
         A.arc_post[f0 + m_beg + i] = static_cast<float>(p);
       }
-      group_by_key(nm, [&](int i) { return A.tid2pdf[M[i].ilabel]; });
-      const int per = (P + kPoThreads - 1) / kPoThreads, k0 = min(P, tid * per), k1 = min(P, k0 + per);
+      W.group_by_key(nm, [&](int i) { return A.tid2pdf[M[i].ilabel]; });
+      const int per = (P + kThreads - 1) / kThreads, k0 = min(P, tid * per), k1 = min(P, k0 + per);
       int cnt = 0;
       for (int k = k0; k < k1; ++k) {
         if (seg[k + 1] == seg[k]) continue;
@@ -315,7 +138,7 @@ __global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
         cnt += static_cast<float>(sum) >= A.min_post;
       }
       int base = 0, kept = 0;
-      Scan(tmp.scan).ExclusiveSum(cnt, base, kept);
+      lattice_walk::Scan(sh.tmp.scan).ExclusiveSum(cnt, base, kept);
       pkb_frame_post_t *out = A.tail + f0 + na - nout - kept;
       for (int k = k0; k < k1; ++k) {
         if (seg[k + 1] == seg[k]) continue;
@@ -326,24 +149,24 @@ __global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
     }
     // beta(t, s): the final weight at T, then the outgoing epsilon and emitting records of s in
     // record order
-    for (int s = tid; s < S; s += kPoThreads) {
+    for (int s = tid; s < S; s += kThreads) {
       eb[s] = ee[s] = mb[s] = me[s] = 0;
       done[s] = 0;
     }
     __syncthreads();
-    for (int i = tid; i < ne; i += kPoThreads) {
+    for (int i = tid; i < ne; i += kThreads) {
       const int s = E[i].src;
       if (i == 0 || E[i - 1].src != s) eb[s] = i;
       if (i == ne - 1 || E[i + 1].src != s) ee[s] = i + 1;
     }
-    for (int i = tid; i < nm; i += kPoThreads) {
+    for (int i = tid; i < nm; i += kThreads) {
       const int s = M[i].src;
       if (i == 0 || M[i - 1].src != s) mb[s] = i;
       if (i == nm - 1 || M[i + 1].src != s) me[s] = i + 1;
     }
     __syncthreads();
     for (;;) {
-      for (int s = tid; s < S; s += kPoThreads) {
+      for (int s = tid; s < S; s += kThreads) {
         if (done[s]) continue;
         bool ready = true;
         for (int i = eb[s]; i < ee[s] && ready; ++i) ready = done[E[i].dst] == 2;
@@ -360,14 +183,14 @@ __global__ void __launch_bounds__(kPoThreads) posterior_kernel(PostArgs A) {
       }
       __syncthreads();
       int progress = 0;
-      for (int s = tid; s < S; s += kPoThreads)
+      for (int s = tid; s < S; s += kThreads)
         if (done[s] == 1) {
           done[s] = 2;
           progress = 1;
         }
       if (!__syncthreads_or(progress)) break;
     }
-    for (int i = tid; i < ne; i += kPoThreads) {
+    for (int i = tid; i < ne; i += kThreads) {
       const pkb_lattice_arc_t &r = E[i];
       A.arc_post[f0 + e_beg + i] = static_cast<float>(arc_posterior(total, alpha[e_beg + i], scaled_cost(A, r), X[r.dst]));
     }
@@ -430,7 +253,7 @@ int LatticeResults::posteriors(float acoustic_scale, float graph_scale, float mi
   // not fit in shared memory
   const size_t state_bytes = sizeof(double) * (2 * static_cast<size_t>(S) + K) +
                              sizeof(int) * (5 * static_cast<size_t>(S) + 2 * static_cast<size_t>(K) + 1);
-  const bool smem_state = state_bytes <= kPoSmemState;
+  const bool smem_state = state_bytes <= kSmemState;
   const size_t stride = ((((sizeof(int) * NA + 7) & ~size_t(7)) + sizeof(double) * NA +
                           (smem_state ? 0 : state_bytes)) + 255) & ~size_t(255);
   // utterances in waves whose alpha and workspace fit the budget
@@ -446,18 +269,9 @@ int LatticeResults::posteriors(float acoustic_scale, float graph_scale, float mi
     PKB_CUDA(cudaFuncSetAttribute(posterior_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(state_bytes)));
   PostArgs A{};
-  A.arcs = arcs.as<pkb_lattice_arc_t>();
-  A.first = d_first();
-  A.n_arcs = d_n_arcs();
-  A.best = d_best();
-  A.final_w = fst->d_final;
+  static_cast<lattice_walk::WalkArgs &>(A) = lattice_walk::walk_args(*this, acoustic_scale, graph_scale);
   A.tid2pdf = d_tid2pdf;
-  A.num_states = S;
   A.num_pdfs = P;
-  A.num_arcs = NA;
-  A.start = fst->start;
-  A.as = acoustic_scale;
-  A.gs = graph_scale;
   A.min_post = min_post;
   A.work_stride = stride;
   A.smem_state = smem_state;
@@ -472,7 +286,7 @@ int LatticeResults::posteriors(float acoustic_scale, float graph_scale, float mi
     A.alpha = reinterpret_cast<double *>(wave_buf.as<char>() + stride * m);
     A.rec0 = first[u0];
     LaunchScope scope(c, PKB_KERNEL_MISC);
-    posterior_kernel<<<m, kPoThreads, smem_state ? state_bytes : 0, c->stream>>>(A);
+    posterior_kernel<<<m, kThreads, smem_state ? state_bytes : 0, c->stream>>>(A);
     PKB_CUDA(cudaGetLastError());
   }
   static_assert(sizeof(long long) == sizeof(int64_t), "int64_t is long long");
